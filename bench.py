@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference ...                     # the reference's CPU algorithm (oracle)
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's results as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch: config[1] of BASELINE.json -- cvLDS on
 NPannual/NPpc (T=413, p=q=3), 100 make_Z hold-out folds x 100 restarts = 10 000 independent EM
@@ -32,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark writes nothing into it
 
 from ldsr_b200 import workloads as W  # noqa: E402
 
@@ -169,6 +171,28 @@ def oracle_check(w, res, args, seconds):
     return {"value": ns / dt, "unit": "fits/s", "cores": cores, "kind": "port",
             "sample": "first %d of %d groups (%d fits), %.1f s" % (g, len(w["group_series"]), ns, dt)}, \
         matches_oracle(ro, res, ns, g)
+
+
+DUMP_LIMIT = 64 << 20  # bytes of --dump-outputs, all arrays together
+
+
+def dump_outputs(dirname, res, fit_group):
+    """Writes the arrays of a fetched EM result as DIR/<name>.npy in float64.  A result above DUMP_LIMIT is cut
+    to a fixed sample of whole groups (their fits, selections and trajectory rows; traj_ptr renumbered), listed
+    in sample_groups.npy.  Groups differ in size, so the sample aims at half the limit."""
+    ng = res["best"].size
+    total = sum(np.asarray(a).size * 8 for a in res.values())
+    if total > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(ng, max(1, ng * DUMP_LIMIT // (2 * total)), replace=False))
+        ptr = res["traj_ptr"]
+        rows = np.concatenate([np.arange(ptr[g], ptr[g + 1]) for g in keep])
+        fits = np.isin(fit_group, keep)
+        res = dict({k: res[k][fits] for k in ("theta", "lik", "iters", "status")}, best=res["best"][keep],
+                   traj_ptr=np.concatenate([[0], np.cumsum(np.diff(ptr)[keep])]), sample_groups=keep,
+                   **{k: res[k][rows] for k in ("X", "Y", "V", "J")})
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in res.items():
+        np.save(os.path.join(dirname, k + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def device_steps(plan, args, steps, warmup, torch, flush, stream):
@@ -392,7 +416,11 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` block (configs 1, 4, 5)")
     ap.add_argument("--rep-replicates", type=int, default=100000, help="config 4: LDS_rep replicates")
     ap.add_argument("--scan-T", type=int, default=100000, help="config 5: series length")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (rank 0) as DIR/<name>.npy, float64, <= 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -452,7 +480,9 @@ def main():
         dist.all_reduce(tot_ms, op=dist.ReduceOp.MAX)
     tot_ms = float(tot_ms.item())
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
-    res = plan.fetch(want_traj=False)
+    res = plan.fetch(want_traj=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, w["fit_group"])
     iters = res["iters"].astype(np.float64)
     value = world * nf * K / (tot_ms * 1e-3)
 
