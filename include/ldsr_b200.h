@@ -229,6 +229,17 @@ int ldsr_shard_groups(const ldsr_batch *batch, int n_shards, int *group_shard, c
  *   out [n_folds][5]: R2, RE, CE, nRMSE, KGE (the column order of metrics.dist) */
 int ldsr_cv_metrics_batch(int device, int n, int n_folds, const double *sim, const double *obs, const int *z_ptr,
                           const int *z_idx, int exp_trans, double *out, char *errbuf, int errlen);
+/* The same for many stations in one launch (cvLDS over a set of gauges): station s has a target of n[s] >= 2
+ * values and the folds fold_ptr[s] .. fold_ptr[s+1]-1 (fold_ptr[0] = 0, non-decreasing, fold_ptr[n_stations]
+ * >= 1 folds in all).
+ *   sim: the folds' rows concatenated in fold order, each n[station] long
+ *   obs: the stations' targets concatenated in station order
+ *   z_ptr [n_folds+1], z_idx: CSR of each fold's hold-out indices, 1-BASED into its OWN station's target
+ *   out [n_folds][5] in fold order.
+ * ldsr_cv_metrics_batch is the one-station case (same kernel, same bits). */
+int ldsr_cv_metrics_stations(int device, int n_stations, const int *n, const int *fold_ptr, const double *sim,
+                             const double *obs, const int *z_ptr, const int *z_idx, int exp_trans, double *out,
+                             char *errbuf, int errlen);
 
 /* ---- objectives of the experimental learners, for a whole population of parameter vectors ------
  * One value per fit (= per theta0 row of the batch, on its group's y with its hold-outs removed):
@@ -253,6 +264,18 @@ int ldsr_objective_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int kind, doubl
 int ldsr_construct_rec_batch(int device, int n, int T, const double *X, const double *V, const double *Y,
                              const double *C, const double *R, double mu, int transform, double lambda, double *out,
                              double *mean, char *errbuf, int errlen);
+/* The same for many stations in one launch (LDS_reconstruction over a set of gauges): station s has T[s] >= 1
+ * years and the members member_ptr[s] .. member_ptr[s+1]-1 (member_ptr[0] = 0, at least one member each).
+ *   X, V, Y: the members' rows concatenated in member order, each T[station] long
+ *   C, R [n_members]: each member's theta$C and theta$R;  mu, lambda [n_stations]: per station (lambda is only
+ *   read with transform 2 and may be NULL otherwise); transform is shared
+ *   out: per member [6][T[station]], concatenated in member order
+ *   mean (may be NULL): per station [2][T[s]] (mean X, mean Q over its members), concatenated in station order
+ * ldsr_construct_rec_batch is the one-station case (same kernel, same bits). */
+int ldsr_construct_rec_stations(int device, int n_stations, const int *T, const int *member_ptr, const double *X,
+                                const double *V, const double *Y, const double *C, const double *R, const double *mu,
+                                const double *lambda, int transform, double *out, double *mean, char *errbuf,
+                                int errlen);
 
 /* ---- general state dimension, long series (beyond the reference) ----------------------------
  * The reference is scalar-state only (src/EM.cpp:20 "matrix inversion is treated as /").

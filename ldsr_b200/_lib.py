@@ -21,7 +21,8 @@ EXPORTS = ("ldsr_abi_version", "ldsr_device_count", "ldsr_ctx_create", "ldsr_ctx
            "ldsr_propagate_batch", "ldsr_rep_batch", "ldsr_shard_groups", "ldsr_measure_fp64_peak",
            "ldsr_smoother_d_batch", "ldsr_cv_metrics_batch", "ldsr_construct_rec_batch",
            "ldsr_objective_batch", "ldsr_rep_batch_r", "ldsr_r_rng_create", "ldsr_r_rng_unif", "ldsr_r_rng_norm",
-           "ldsr_r_rng_sample", "ldsr_r_rng_destroy", "ldsr_r_rnorm_device", "ldsr_last_device_ms")
+           "ldsr_r_rng_sample", "ldsr_r_rng_destroy", "ldsr_r_rnorm_device", "ldsr_last_device_ms",
+           "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations")
 
 
 class LdsrError(RuntimeError):
@@ -503,6 +504,37 @@ def cv_metrics(sim, obs, Z, exp_trans=False, device=0):
     return out
 
 
+def _ptr(lengths):
+    out = np.zeros(len(lengths) + 1, dtype=np.int32)
+    out[1:] = np.cumsum(lengths)
+    return out
+
+
+def cv_metrics_stations(sims, obss, Zs, exp_trans=False, device=0):
+    """ldsr_cv_metrics_stations: cv_metrics for several stations of different lengths in one launch.
+    sims[s] [n_folds_s, n_s]; obss[s] [n_s]; Zs[s]: station s's folds, 1-based into obss[s].
+    Returns one [n_folds_s, 5] array per station."""
+    sims = [np.atleast_2d(np.asarray(a, dtype=np.float64)) for a in sims]
+    obss = [np.asarray(a, dtype=np.float64).ravel() for a in obss]
+    if not (len(sims) == len(obss) == len(Zs)):
+        raise ValueError("one sim matrix, target and fold list per station")
+    n = np.asarray([o.size for o in obss], dtype=np.int32)
+    for s, (a, z) in enumerate(zip(sims, Zs)):
+        if a.shape != (len(z), n[s]):
+            raise ValueError("station %d: sim must be [%d folds, %d]" % (s, len(z), n[s]))
+    fp = _ptr([len(z) for z in Zs])
+    folds = [np.asarray(z, dtype=np.int32).ravel() for zs in Zs for z in zs]
+    zp = _ptr([z.size for z in folds])
+    zi = np.ascontiguousarray(np.concatenate(folds + [np.zeros(1, dtype=np.int32)]))
+    sim = np.ascontiguousarray(np.concatenate([a.ravel() for a in sims]))
+    obs = np.ascontiguousarray(np.concatenate(obss))
+    out = np.empty((int(fp[-1]), 5))
+    err = C.create_string_buffer(512)
+    _check(lib().ldsr_cv_metrics_stations(int(device), len(obss), _i(n), _i(fp), _d(sim), _d(obs), _i(zp), _i(zi),
+                                          int(bool(exp_trans)), _d(out), err, 512), err)
+    return [out[fp[s]:fp[s + 1]] for s in range(len(obss))]
+
+
 REC_COLUMNS = ("X", "Xl", "Xu", "Q", "Ql", "Qu")
 TRANSFORMS = {"none": 0, "log": 1, "boxcox": 2}
 
@@ -521,6 +553,38 @@ def construct_rec(X, V, Y, C_, R_, mu, transform="log", lam=0.0, device=0):
                                           C.c_double(mu), int(TRANSFORMS[transform]), C.c_double(lam), _d(out),
                                           _d(mean), err, 512), err)
     return out, mean
+
+
+def construct_rec_stations(Xs, Vs, Ys, Cs, Rs, mus, transform="log", lams=None, device=0):
+    """ldsr_construct_rec_stations: construct_rec for the members of several stations of different lengths in
+    one launch.  Xs[s], Vs[s], Ys[s]: [n_s, T_s]; Cs[s], Rs[s]: [n_s]; mus[s], lams[s]: station s's mean and
+    Box-Cox lambda.  Returns one (out [n_s, 6, T_s], mean [2, T_s]) pair per station."""
+    S = len(Xs)
+    Xs, Vs, Ys = ([np.atleast_2d(np.asarray(a, dtype=np.float64)) for a in arrs] for arrs in (Xs, Vs, Ys))
+    T = np.asarray([x.shape[1] for x in Xs], dtype=np.int32)
+    nm = [x.shape[0] for x in Xs]
+    for s in range(S):
+        if Vs[s].shape != Xs[s].shape or Ys[s].shape != Xs[s].shape:
+            raise ValueError("station %d: X, V and Y must have the same shape" % s)
+    mp = _ptr(nm)
+    X, V, Y = (np.ascontiguousarray(np.concatenate([a.ravel() for a in arrs])) for arrs in (Xs, Vs, Ys))
+    Cv, Rv = (np.ascontiguousarray(np.concatenate([np.broadcast_to(np.asarray(c, dtype=np.float64).ravel(), (k,))
+                                                   for c, k in zip(arrs, nm)])) for arrs in (Cs, Rs))
+    mu = np.ascontiguousarray(mus, dtype=np.float64)
+    lam = np.ascontiguousarray(np.zeros(S) if lams is None else [0.0 if l is None else l for l in lams],
+                               dtype=np.float64)
+    if mu.shape != (S,) or lam.shape != (S,):
+        raise ValueError("one mu and one lambda per station")
+    rows = np.concatenate([[0], np.cumsum(np.asarray(nm) * T)])
+    years = np.concatenate([[0], np.cumsum(T)])
+    out = np.empty(6 * int(rows[-1]))
+    mean = np.empty(2 * int(years[-1]))
+    err = C.create_string_buffer(512)
+    _check(lib().ldsr_construct_rec_stations(int(device), S, _i(T), _i(mp), _d(X), _d(V), _d(Y), _d(Cv), _d(Rv),
+                                             _d(mu), _d(lam), int(TRANSFORMS[transform]), _d(out), _d(mean), err, 512),
+           err)
+    return [(out[6 * rows[s]:6 * rows[s + 1]].reshape(nm[s], 6, T[s]), mean[2 * years[s]:2 * years[s + 1]].reshape(2, T[s]))
+            for s in range(S)]
 
 
 OBJECTIVES = {"penalized_likelihood": 0, "negLogLik": 1, "ssqTrain": 2}

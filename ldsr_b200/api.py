@@ -218,66 +218,140 @@ def _make_y(years_Qa, obs, start_year, N):
     return y, mu, years
 
 
-def _construct_rec(fit, theta, mu, transform, lam, years):
-    """R/LDS_reconstruction.R:190-212 through ldsr_construct_rec_batch (one member)."""
-    out, _ = _lib.construct_rec(fit["X"], fit["V"], fit["Y"], float(np.ravel(theta["C"])[0]),
-                                float(np.ravel(theta["R"])[0]), mu, transform, 0.0 if lam is None else float(lam))
-    rec = dict(year=years)
-    rec.update({k: out[0, j] for j, k in enumerate(_lib.REC_COLUMNS)})
-    return rec
+def _station(st, transform):
+    """Host-side set-up of one station, no random draws: the argument checks of LDS_reconstruction / cvLDS,
+    the transform, and y centred and NA-padded to the station's horizon (R/LDS_reconstruction.R:128-183)."""
+    single, us, vs, N = _prep_uv(st.get("u"), st.get("v"))
+    obs, lam = _transform(st["Qa"]["Qa"], transform)
+    qyears = np.asarray(st["Qa"]["year"])
+    y, mu, years = _make_y(qyears, obs, st["start_year"], N)
+    return dict(Qa=st["Qa"], single=single, N=N, obs=obs, lam=lam, qyears=qyears, mu=mu, years=years,
+                series=[_series(y, a, b) for a, b in zip(us, vs)])
+
+
+def _pack(P, groups):
+    """One em_batch over all stations.  groups: per station, its (member, held-out steps, initial thetas)
+    groups in batch order; series are numbered station-major, theta rows padded to the widest series.
+    Sets each station's first series / group / fit (s0, g0, f0) and its fit end f1; returns the em_batch
+    arguments."""
+    series, group_series, held, fit_group, th0 = [], [], [], [], []
+    for S, gs in zip(P, groups):
+        S.update(s0=len(series), g0=len(group_series), f0=len(fit_group))
+        for m, h, init in gs:
+            for t in init:
+                th0.append(theta_to_vec(t))
+                fit_group.append(len(group_series))
+            group_series.append(S["s0"] + m)
+            held.append(np.asarray(h, dtype=np.int64))
+        series += S["series"]
+        S["f1"] = len(fit_group)
+    stride = max(s["p"] + s["q"] + 6 for s in series)
+    return dict(series=series, group_series=group_series, held=held, fit_group=fit_group,
+                theta0=np.stack([np.pad(v, (0, stride - v.size)) for v in th0]))
+
+
+def _selected_thetas(r, best, series, group_series):
+    """The selected fits' theta rows for a propagate_batch: a narrower series' padding is zeroed."""
+    th = r["theta"][best].copy()
+    for i, g in enumerate(group_series):
+        s = series[g]
+        th[i, s["p"] + s["q"] + 6:] = 0.0
+    return th
+
+
+def reconstruction_batch(stations, transform="log", num_restarts=50, rng=None):
+    """Host half of LDS_reconstruction_stations, usable without a device: prepares every station, then, station
+    by station, draws what that station's own LDS_reconstruction call draws (make_init per member unless the
+    station gives `init`) and packs one em_batch (one group per member).  Returns (stations, em_batch args)."""
+    rng = rng or np.random.default_rng()
+    P = [_station(st, transform) for st in stations]
+    groups = []
+    for S, st in zip(P, stations):
+        init = st.get("init")
+        if init is None:
+            init = [make_init(s["p"], s["q"], num_restarts, rng) for s in S["series"]]
+        elif S["single"]:
+            init = [init]
+        S["init"] = init
+        groups.append([(m, [], ini) for m, ini in enumerate(init)])
+    return P, _pack(P, groups)
+
+
+def LDS_reconstruction_stations(stations, method="EM", transform="log", num_restarts=50, return_init=False,
+                                niter=1000, tol=1e-5, return_raw=False, rng=None, n_devices=1):
+    """LDS_reconstruction for many stations in one batched GPU call.  stations: list of
+    dict(Qa=dict(year=, Qa=), u=, v=, start_year=[, init=]); u / v as in LDS_reconstruction (matrix, None or an
+    ensemble list); stations may differ in T, p, q, instrumental period and start year.  The other arguments
+    are shared.  Random numbers are drawn station by station exactly as the single-station calls would draw
+    them in that order.  Returns one LDS_reconstruction result per station.
+    Device calls: one em_batch, one propagate_batch (return_raw), one construct_rec_stations."""
+    if method != "EM":
+        raise ValueError("only method = 'EM' is implemented (GA/BFGS are experimental in the reference)")
+    P, B = reconstruction_batch(stations, transform, num_restarts, rng)
+    r = _lib.em_batch(B["series"], B["group_series"], None, B["fit_group"], B["theta0"], niter, tol,
+                      n_devices=n_devices)
+    if np.any(r["status"] == _lib.FIT_SINGULAR):
+        raise _lib.LdsrError(_lib.ERR_ARG, "LDS_reconstruction: inv(): matrix is singular")
+    best = r["best"]
+    if np.any(best < 0):
+        raise _lib.LdsrError(_lib.ERR_ARG, "no restart produced a finite likelihood")
+    ns = len(B["series"])
+    # one group per series (member): group g == series g, and its winner's rows start at traj_ptr[g]
+    fits = [_fit_dict(r, int(r["traj_ptr"][g]), B["series"][g]["y"].size) for g in range(ns)]
+    thetas = [vec_to_theta(r["theta"][best[g]], B["series"][g]["p"], B["series"][g]["q"]) for g in range(ns)]
+    raws = None
+    if return_raw:
+        pr = _lib.propagate_batch(B["series"], np.arange(ns), None, np.arange(ns),
+                                  _selected_thetas(r, best, B["series"], range(ns)))
+        raws = [dict(X=pr["X"][g], Y=pr["Y"][g], V=pr["V"][g]) for g in range(ns)]
+    # construct_rec of every station's members in one launch; the raw trajectories are a second set of stations
+    blocks = [(fs, range(S["s0"], S["s0"] + len(S["series"])), S) for fs in ([fits, raws] if return_raw else [fits])
+              for S in P]
+    rec = _lib.construct_rec_stations([np.stack([fs[g]["X"] for g in gs]) for fs, gs, _ in blocks],
+                                      [np.stack([fs[g]["V"] for g in gs]) for fs, gs, _ in blocks],
+                                      [np.stack([fs[g]["Y"] for g in gs]) for fs, gs, _ in blocks],
+                                      [[thetas[g]["C"] for g in gs] for _, gs, _ in blocks],
+                                      [[thetas[g]["R"] for g in gs] for _, gs, _ in blocks],
+                                      [S["mu"] for _, _, S in blocks], transform, [S["lam"] for _, _, S in blocks])
+    out = []
+    for j, S in enumerate(P):
+        members = []
+        years = S["years"]
+
+        def cols(o, k):
+            d = dict(year=years)
+            d.update({c: o[k, i] for i, c in enumerate(_lib.REC_COLUMNS)})
+            return d
+        for k in range(len(S["series"])):
+            g = S["s0"] + k
+            b = int(best[g])
+            ans = dict(rec=cols(rec[j][0], k), theta=thetas[g], lik=float(r["lik"][b]))
+            if return_raw:
+                ans["rec2"] = cols(rec[len(P) + j][0], k)
+            if return_init:
+                ans["init"] = S["init"][k][b - S["f0"] - sum(len(i) for i in S["init"][:k])]
+            if transform == "boxcox":
+                ans["lambda"] = S["lam"]
+            members.append(ans)
+        if S["single"]:
+            out.append(members[0])
+            continue
+        mean = rec[j][1]
+        res = dict(rec=dict(year=years, X=mean[0], Q=mean[1]), ensemble=members)
+        if return_raw:
+            mean = rec[len(P) + j][1]
+            res["rec_raw"] = dict(year=years, X=mean[0], Q=mean[1])
+        out.append(res)
+    return out
 
 
 def LDS_reconstruction(Qa, u, v, start_year, method="EM", transform="log", init=None, num_restarts=50,
                        return_init=False, niter=1000, tol=1e-5, return_raw=False, rng=None, n_devices=1):
     """R/LDS_reconstruction.R:122-258.  Qa: dict(year=..., Qa=...).  Single model or ensemble
-    (u, v lists); all members x restarts go to the GPU as one batch."""
-    if method != "EM":
-        raise ValueError("only method = 'EM' is implemented (GA/BFGS are experimental in the reference)")
-    single, us, vs, N = _prep_uv(u, v)
-    rng = rng or np.random.default_rng()
-    if init is None:
-        init = [make_init(*_dims(a, b), num_restarts, rng) for a, b in zip(us, vs)]
-    elif single:
-        init = [init]
-    obs, lam = _transform(Qa["Qa"], transform)
-    y, mu, years = _make_y(np.asarray(Qa["year"]), obs, start_year, N)
-
-    series = [_series(y, a, b) for a, b in zip(us, vs)]
-    stride = max(s["p"] + s["q"] + 6 for s in series)
-    th0, fg = [], []
-    for m, ini in enumerate(init):
-        for t in ini:
-            vec = theta_to_vec(t)
-            th0.append(np.pad(vec, (0, stride - vec.size)))
-            fg.append(m)
-    r = _lib.em_batch(series, np.arange(len(series)), None, fg, np.stack(th0), niter, tol, n_devices=n_devices)
-    if np.any(r["status"] == _lib.FIT_SINGULAR):
-        raise _lib.LdsrError(_lib.ERR_ARG, "LDS_reconstruction: inv(): matrix is singular")
-    members = []
-    offs = np.cumsum([0] + [len(i) for i in init])
-    for m, s in enumerate(series):
-        b = int(r["best"][m])
-        if b < 0:
-            raise _lib.LdsrError(_lib.ERR_ARG, "no restart produced a finite likelihood")
-        theta = vec_to_theta(r["theta"][b], s["p"], s["q"])
-        fit = _fit_dict(r, int(r["traj_ptr"][m]), N)
-        ans = dict(rec=_construct_rec(fit, theta, mu, transform, lam, years), theta=theta, lik=float(r["lik"][b]))
-        if return_raw:
-            raw = propagate(theta, s["u"], s["v"], y)
-            ans["rec2"] = _construct_rec(raw, theta, mu, transform, lam, years)
-        if return_init:
-            ans["init"] = init[m][b - offs[m]]
-        if transform == "boxcox":
-            ans["lambda"] = lam
-        members.append(ans)
-    if single:
-        return members[0]
-    out = dict(rec=dict(year=years, X=np.mean([m["rec"]["X"] for m in members], axis=0),
-                        Q=np.mean([m["rec"]["Q"] for m in members], axis=0)), ensemble=members)
-    if return_raw:
-        out["rec_raw"] = dict(year=years, X=np.mean([m["rec2"]["X"] for m in members], axis=0),
-                              Q=np.mean([m["rec2"]["Q"] for m in members], axis=0))
-    return out
+    (u, v lists); all members x restarts go to the GPU as one batch.  The one-station case of
+    LDS_reconstruction_stations."""
+    return LDS_reconstruction_stations([dict(Qa=Qa, u=u, v=v, start_year=start_year, init=init)], method, transform,
+                                       num_restarts, return_init, niter, tol, return_raw, rng, n_devices)[0]
 
 
 def one_lds_cv(z, instPeriod, mu, y, u, v, method="EM", num_restarts=20, niter=1000, tol=1e-6, use_raw=False,
@@ -334,68 +408,95 @@ def tbrm(x, C=9.0):
     return float(np.sum(w * x) / np.sum(w))
 
 
+def cv_batch(stations, transform="log", num_restarts=50, rng=None):
+    """Host half of cvLDS_stations, usable without a device: prepares every station, then, station by station,
+    draws what that station's own cvLDS call draws -- make_Z if its Z is None, then make_init fold-major and
+    member-minor (the reference's nested foreach order, R/LDS_reconstruction.R:373-381) -- and packs one
+    em_batch (groups station-major, fold-major, member-minor).  Returns (stations, em_batch args)."""
+    rng = rng or np.random.default_rng()
+    P = [_station(st, transform) for st in stations]
+    groups = []
+    for S, st in zip(P, stations):
+        Z = st.get("Z")
+        if Z is None:
+            Z = make_Z(S["Qa"]["Qa"], rng=rng)
+        if not isinstance(Z, (list, tuple)):
+            raise ValueError("Please provide the cross-validation folds (Z) in a list.")
+        S["Z"] = Z
+        S["inst"] = np.nonzero(np.isin(S["years"], S["qyears"]))[0]  # 0-based instPeriod
+        groups.append([(m, S["inst"][np.asarray(z) - 1], make_init(s["p"], s["q"], num_restarts, rng))
+                       for z in Z for m, s in enumerate(S["series"])])
+    return P, _pack(P, groups)
+
+
+def cvLDS_stations(stations, method="EM", transform="log", num_restarts=50, metric_space="original", use_raw=False,
+                   niter=1000, tol=1e-5, rng=None, n_devices=1, use_robust_mean=True):
+    """cvLDS for many stations in one batched GPU call.  stations: list of
+    dict(Qa=dict(year=, Qa=), u=, v=, start_year=[, Z=]); u / v as in cvLDS (matrix, None or an ensemble list);
+    stations may differ in T, p, q, instrumental period and start year.  The other arguments are shared.
+    Random numbers are drawn station by station exactly as the single-station calls would draw them in that
+    order.  Returns one cvLDS result per station.
+    Device calls: one em_batch, one propagate_batch (use_raw), one cv_metrics_stations."""
+    if method != "EM":
+        raise ValueError("only method = 'EM' is implemented")
+    P, B = cv_batch(stations, transform, num_restarts, rng)
+    r = _lib.em_batch(B["series"], B["group_series"], B["held"], B["fit_group"], B["theta0"], niter, tol,
+                      n_devices=n_devices)
+    if np.any(r["status"] == _lib.FIT_SINGULAR):
+        raise _lib.LdsrError(_lib.ERR_ARG, "cvLDS: inv(): matrix is singular")
+    best = r["best"]
+    for S in P:
+        nm = len(S["series"])
+        bad = np.nonzero(best[S["g0"]:S["g0"] + len(S["Z"]) * nm] < 0)[0]
+        if bad.size:
+            raise _lib.LdsrError(_lib.ERR_ARG, "fold %d: no restart produced a finite likelihood" % (bad[0] // nm))
+    ng = len(B["group_series"])
+    if use_raw:  # propagate(theta_best, u, v, y_fold)$Y (:279-281): the selected fits, open loop, in one call
+        pr = _lib.propagate_batch(B["series"], B["group_series"], B["held"], np.arange(ng),
+                                  _selected_thetas(r, best, B["series"], B["group_series"]))
+        Yg = pr["Y"]
+    else:
+        Yg = [r["Y"][int(r["traj_ptr"][g]):int(r["traj_ptr"][g + 1])] for g in range(ng)]
+    sims, targets = [], []
+    for S in P:
+        nm, inst, mu = len(S["series"]), S["inst"], S["mu"]
+        Ycv = []
+        for k in range(len(S["Z"])):
+            g0 = S["g0"] + k * nm
+            Ycv.append(np.mean([Yg[g0 + m][inst] + mu for m in range(nm)], axis=0))  # fit$Y[instPeriod] + mu,
+        if metric_space == "original":                                              # .final = rowMeans (:379)
+            if transform == "log":
+                Ycv = [np.exp(a) for a in Ycv]
+            elif transform == "boxcox":
+                Ycv = [inv_boxcox(a, S["lam"]) for a in Ycv]
+            target = np.asarray(S["Qa"]["Qa"], dtype=float)
+        else:
+            target = S["obs"]
+        S["Ycv"], S["target"] = Ycv, target
+        sims.append(np.stack(Ycv))
+        targets.append(target)
+    # mapply(calculate_metrics, ...) (:395) for all folds of all stations in one device call
+    dists = _lib.cv_metrics_stations(sims, targets, [S["Z"] for S in P])
+    keys = _lib.METRIC_NAMES
+    mean_func = tbrm if use_robust_mean else np.mean  # R/LDS_reconstruction.R:397
+    out = []
+    for S, dist in zip(P, dists):
+        metrics_dist = {k: dist[:, j].copy() for j, k in enumerate(keys)}
+        g0, g1 = S["g0"], S["g0"] + len(S["Z"]) * len(S["series"])
+        out.append(dict(metrics_dist=metrics_dist, metrics={k: float(mean_func(metrics_dist[k])) for k in keys},
+                        target=dict(year=S["qyears"], y=S["target"]), Ycv=np.stack(S["Ycv"], axis=1), Z=S["Z"],
+                        best=best[g0:g1] - S["f0"], lik=r["lik"][S["f0"]:S["f1"]], iters=r["iters"][S["f0"]:S["f1"]]))
+    return out
+
+
 def cvLDS(Qa, u, v, start_year, method="EM", transform="log", num_restarts=50, Z=None, metric_space="original",
           use_raw=False, niter=1000, tol=1e-5, rng=None, n_devices=1, use_robust_mean=True):
     """R/LDS_reconstruction.R:308-409.  All folds x members x restarts run as ONE batch; initial
     values are drawn fold-major exactly as `foreach(z = Z) ... one_lds_cv` would under
-    registerDoSEQ (:373-381, :275)."""
-    if method != "EM":
-        raise ValueError("only method = 'EM' is implemented")
-    if use_raw:
-        raise ValueError("use_raw is experimental in the reference ('don't use'); not implemented")
-    single, us, vs, N = _prep_uv(u, v)
-    rng = rng or np.random.default_rng()
-    obs, lam = _transform(Qa["Qa"], transform)
-    qyears = np.asarray(Qa["year"])
-    if Z is None:
-        Z = make_Z(Qa["Qa"], rng=rng)
-    if not isinstance(Z, (list, tuple)):
-        raise ValueError("Please provide the cross-validation folds (Z) in a list.")
-    y, mu, years = _make_y(qyears, obs, start_year, N)
-    inst = np.nonzero(np.isin(years, qyears))[0]  # 0-based instPeriod
-
-    series = [_series(y, a, b) for a, b in zip(us, vs)]
-    stride = max(s["p"] + s["q"] + 6 for s in series)
-    group_series, held, fit_group, th0 = [], [], [], []
-    for z in Z:  # fold-major, member-minor: the reference's nested foreach order
-        for m, s in enumerate(series):
-            g = len(group_series)
-            group_series.append(m)
-            held.append(inst[np.asarray(z) - 1])
-            for t in make_init(s["p"], s["q"], num_restarts, rng):
-                vec = theta_to_vec(t)
-                th0.append(np.pad(vec, (0, stride - vec.size)))
-                fit_group.append(g)
-    r = _lib.em_batch(series, group_series, held, fit_group, np.stack(th0), niter, tol, n_devices=n_devices)
-    if np.any(r["status"] == _lib.FIT_SINGULAR):
-        raise _lib.LdsrError(_lib.ERR_ARG, "cvLDS: inv(): matrix is singular")
-    nm = len(series)
-    Ycv = []
-    for k in range(len(Z)):
-        cols = []
-        for m in range(nm):
-            g = k * nm + m
-            if r["best"][g] < 0:
-                raise _lib.LdsrError(_lib.ERR_ARG, "fold %d: no restart produced a finite likelihood" % k)
-            row = int(r["traj_ptr"][g])
-            cols.append(r["Y"][row + inst] + mu)  # fit$Y[instPeriod] + mu   (:283)
-        Ycv.append(np.mean(cols, axis=0))        # .final = rowMeans          (:379)
-    if metric_space == "original":
-        if transform == "log":
-            Ycv = [np.exp(a) for a in Ycv]
-        elif transform == "boxcox":
-            Ycv = [inv_boxcox(a, lam) for a in Ycv]
-        target = np.asarray(Qa["Qa"], dtype=float)
-    else:
-        target = obs
-    # mapply(calculate_metrics, ...) (:395) for all folds in one device call
-    keys = _lib.METRIC_NAMES
-    dist = _lib.cv_metrics(np.stack(Ycv), target, Z)
-    metrics_dist = {k: dist[:, j].copy() for j, k in enumerate(keys)}
-    mean_func = tbrm if use_robust_mean else np.mean  # R/LDS_reconstruction.R:397
-    return dict(metrics_dist=metrics_dist, metrics={k: float(mean_func(metrics_dist[k])) for k in keys},
-                target=dict(year=qyears, y=target), Ycv=np.stack(Ycv, axis=1), Z=Z,
-                best=r["best"], lik=r["lik"], iters=r["iters"])
+    registerDoSEQ (:373-381, :275).  use_raw: the fold output is the selected fit's open-loop
+    propagate(theta, u, v, y_fold)$Y[instPeriod] + mu (:279-281).  The one-station case of cvLDS_stations."""
+    return cvLDS_stations([dict(Qa=Qa, u=u, v=v, start_year=start_year, Z=Z)], method, transform, num_restarts,
+                          metric_space, use_raw, niter, tol, rng, n_devices, use_robust_mean)[0]
 
 
 # ---------------------------------------------------------------------------------------------

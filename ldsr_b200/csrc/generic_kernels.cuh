@@ -350,20 +350,26 @@ __global__ void pack_results_kernel(const PackParams P) {
 // ---- cross-validation skill metrics (the epilogue of cvLDS) --------------------------------------
 // calculate_metrics (R/utils.R:56-70) with the definitions of src/utils.cpp:13-97, one warp per
 // fold: R2 = NSE on the calibration part, RE, CE = NSE on the hold-out, nRMSE (normalised by
-// mean(obs)), KGE.  held [n_folds][n] marks the hold-out points; sim is exp()'d first when exp_trans
-// (cvLDS with transform = 'log', R/LDS_reconstruction.R:385-386).  Two passes (means, then moments
-// about the means) with shuffle reductions.
+// mean(obs)), KGE.  Folds of several stations share a launch: fold f has length f_n[f], its target
+// starts at obs + f_obs[f], its sim row and hold-out marks at sim / held + f_row[f].  held marks the
+// hold-out points; sim is exp()'d first when exp_trans (cvLDS with transform = 'log',
+// R/LDS_reconstruction.R:385-386).  Two passes (means, then moments about the means) with shuffle
+// reductions.
 __device__ __forceinline__ double warp_sum(double x) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(FULL, x, o);
     return x;
 }
-__global__ void cv_metrics_kernel(int n, int n_folds, const double *__restrict__ sim, const double *__restrict__ obs,
-                                  const unsigned char *__restrict__ held, int exp_trans, double *__restrict__ out) {
+__global__ void cv_metrics_kernel(int n_folds, const int *__restrict__ f_n, const long long *__restrict__ f_obs,
+                                  const long long *__restrict__ f_row, const double *__restrict__ sim,
+                                  const double *__restrict__ obs_all, const unsigned char *__restrict__ held,
+                                  int exp_trans, double *__restrict__ out) {
     const int f = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (f >= n_folds) return;
-    const double *__restrict__ s = sim + (size_t)f * n;
-    const unsigned char *__restrict__ h = held + (size_t)f * n;
+    const int n = f_n[f];
+    const double *__restrict__ s = sim + f_row[f];
+    const double *__restrict__ obs = obs_all + f_obs[f];
+    const unsigned char *__restrict__ h = held + f_row[f];
     double so = 0, sto = 0, nt = 0, svs = 0, svo = 0, nv = 0, no = 0;
     for (int i = lane; i < n; i += 32) {
         const double o = obs[i], x = exp_trans ? exp(s[i]) : s[i];
@@ -414,47 +420,63 @@ __global__ void cv_metrics_kernel(int n, int n_folds, const double *__restrict__
 
 
 // ---- construct_rec + ensemble mean (the step after restart selection in LDS_reconstruction) --------
-// R/LDS_reconstruction.R:190-212 with exp_ci / inv_boxcox of R/utils.R:112-125; one thread per year:
-// it walks the members in order, so the ensemble mean (:247-248) is a fixed-order sum.
-//   X,V,Y [n][T]; Cm,Rm [n]; out [n][6][T] = X, Xl, Xu, Q, Ql, Qu; mean [2][T] = mean X, mean Q.
-__global__ void construct_rec_kernel(int n, int T, const double *__restrict__ X, const double *__restrict__ V,
+// R/LDS_reconstruction.R:190-212 with exp_ci / inv_boxcox of R/utils.R:112-125; one thread per
+// (station, year): it walks the station's members in order, so the ensemble mean (:247-248) is a
+// fixed-order sum.  Station s has T_s = T[s] years and members m_ptr[s] .. m_ptr[s+1]-1; its member
+// rows X,V,Y [n_s][T_s] start at row_off[s], its out rows [n_s][6][T_s] (X, Xl, Xu, Q, Ql, Qu) at
+// 6 * row_off[s], its mean [2][T_s] (mean X, mean Q; not written when mean is NULL) at 2 * t_off[s].
+// Cm,Rm: per member; mu, lam: per station.  blockIdx.y strides over the stations.
+__global__ void construct_rec_kernel(int n_stations, const int *__restrict__ Ts, const int *__restrict__ m_ptr,
+                                     const long long *__restrict__ row_off, const long long *__restrict__ t_off,
+                                     const double *__restrict__ X, const double *__restrict__ V,
                                      const double *__restrict__ Y, const double *__restrict__ Cm,
-                                     const double *__restrict__ Rm, double mu, int transform, double lambda,
-                                     double *__restrict__ out, double *__restrict__ mean) {
+                                     const double *__restrict__ Rm, const double *__restrict__ mus,
+                                     const double *__restrict__ lams, int transform, double *__restrict__ out,
+                                     double *__restrict__ mean) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= T) return;
     const double QNORM_05 = -1.6448536269514722; // qnorm(0.05): qlnorm(p, m, s) = exp(m + s qnorm(p))
-    double sx = 0.0, sq = 0.0;
-    for (int m = 0; m < n; m++) {
-        const double x = X[(size_t)m * T + t], v = V[(size_t)m * T + t], y = Y[(size_t)m * T + t] + mu;
-        const double ciX = 1.96 * sqrt(v), sdY = sqrt(Cm[m] * v * Cm[m] + Rm[m]), ciY = 1.96 * sdY;
-        double q, ql, qu;
-        if (transform == 1 || (transform == 2 && lambda == 0.0)) {
-            q = exp(y);
-            ql = exp(y + sdY * QNORM_05);
-            qu = exp(y - sdY * QNORM_05);
-        } else if (transform == 0) {
-            q = y;
-            ql = y - ciY;
-            qu = y + ciY;
-        } else {
-            const double il = 1.0 / lambda;
-            q = pow(y * lambda + 1.0, il);
-            ql = pow((y - ciY) * lambda + 1.0, il);
-            qu = pow((y + ciY) * lambda + 1.0, il);
+    for (int st = blockIdx.y; st < n_stations; st += gridDim.y) {
+        const int T = Ts[st];
+        if (t >= T) continue;
+        const int m0 = m_ptr[st], n = m_ptr[st + 1] - m0;
+        const double mu = mus[st], lambda = lams[st];
+        const size_t r0 = (size_t)row_off[st];
+        double sx = 0.0, sq = 0.0;
+        for (int k = 0; k < n; k++) {
+            const size_t r = r0 + (size_t)k * T + t;
+            const double x = X[r], v = V[r], y = Y[r] + mu, c = Cm[m0 + k];
+            const double ciX = 1.96 * sqrt(v), sdY = sqrt(c * v * c + Rm[m0 + k]), ciY = 1.96 * sdY;
+            double q, ql, qu;
+            if (transform == 1 || (transform == 2 && lambda == 0.0)) {
+                q = exp(y);
+                ql = exp(y + sdY * QNORM_05);
+                qu = exp(y - sdY * QNORM_05);
+            } else if (transform == 0) {
+                q = y;
+                ql = y - ciY;
+                qu = y + ciY;
+            } else {
+                const double il = 1.0 / lambda;
+                q = pow(y * lambda + 1.0, il);
+                ql = pow((y - ciY) * lambda + 1.0, il);
+                qu = pow((y + ciY) * lambda + 1.0, il);
+            }
+            double *o = out + 6 * r0 + (size_t)k * 6 * T;
+            o[t] = x;
+            o[T + t] = x - ciX;
+            o[2 * T + t] = x + ciX;
+            o[3 * T + t] = q;
+            o[4 * T + t] = ql;
+            o[5 * T + t] = qu;
+            sx += x;
+            sq += q;
         }
-        double *o = out + (size_t)m * 6 * T;
-        o[t] = x;
-        o[T + t] = x - ciX;
-        o[2 * T + t] = x + ciX;
-        o[3 * T + t] = q;
-        o[4 * T + t] = ql;
-        o[5 * T + t] = qu;
-        sx += x;
-        sq += q;
+        if (mean) {
+            double *mo = mean + 2 * (size_t)t_off[st];
+            mo[t] = sx / n;
+            mo[T + t] = sq / n;
+        }
     }
-    mean[t] = sx / n;
-    mean[T + t] = sq / n;
 }
 
 // initial EM state: theta <- theta0, no E-step done, lik = NaN

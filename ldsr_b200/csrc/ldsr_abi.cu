@@ -2000,79 +2000,167 @@ int ldsr_objective_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int kind, doubl
     return report(run(), errbuf, errlen);
 }
 
+// construct_rec over stations of different lengths (one launch); ldsr_construct_rec_batch is its one-station case.
+static Err construct_rec_stations(int device, int n_stations, const int *T, const int *member_ptr, const double *X,
+                                  const double *V, const double *Y, const double *C, const double *R, const double *mu,
+                                  const double *lambda, int transform, double *out, double *mean) {
+    if (n_stations < 1) return fail(LDSR_ERR_ARG, "need n_stations >= 1");
+    if (!T || !member_ptr || !X || !V || !Y || !C || !R || !mu || !out) return fail(LDSR_ERR_ARG, "a required pointer is NULL");
+    if (transform < 0 || transform > 2) return fail(LDSR_ERR_ARG, "transform must be 0 (none), 1 (log) or 2 (boxcox)");
+    if (transform == 2 && !lambda) return fail(LDSR_ERR_ARG, "lambda is required with transform 2 (boxcox)");
+    if (member_ptr[0] != 0) return fail(LDSR_ERR_ARG, "member_ptr[0] must be 0");
+    std::vector<long long> row_off(n_stations), t_off(n_stations);
+    std::vector<double> lam(n_stations, 0.0);
+    long long rows = 0, years = 0;
+    int max_T = 0;
+    for (int s = 0; s < n_stations; s++) {
+        if (T[s] < 1) return fail(LDSR_ERR_ARG, "station %d: need T >= 1", s);
+        if (member_ptr[s + 1] <= member_ptr[s]) return fail(LDSR_ERR_ARG, "station %d: member_ptr not increasing (every station needs a member)", s);
+        row_off[s] = rows;
+        t_off[s] = years;
+        rows += (long long)(member_ptr[s + 1] - member_ptr[s]) * T[s];
+        years += T[s];
+        max_T = std::max(max_T, T[s]);
+        if (lambda) lam[s] = lambda[s];
+    }
+    const int n = member_ptr[n_stations];
+    if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
+    CU(cudaSetDevice(device));
+    const size_t nT = (size_t)rows, S = (size_t)n_stations;
+    double *d = nullptr;
+    struct Guard {
+        double *&p;
+        ~Guard() { cudaFree(p); }
+    } guard{d};
+    // one arena: X V Y | C R | mu lambda | out | mean | row_off t_off (8-byte integers) | T member_ptr (ints)
+    const size_t n_dbl = 3 * nT + 2 * (size_t)n + 2 * S + 6 * nT + 2 * (size_t)years + 2 * S;
+    CU(cudaMalloc(&d, sizeof(double) * n_dbl + sizeof(int) * (2 * S + 1)));
+    double *dX = d, *dV = dX + nT, *dY = dV + nT, *dC = dY + nT, *dR = dC + n, *dmu = dR + n, *dlam = dmu + S;
+    double *dO = dlam + S, *dM = dO + 6 * nT;
+    long long *d_roff = reinterpret_cast<long long *>(dM + 2 * years), *d_toff = d_roff + S;
+    int *d_T = reinterpret_cast<int *>(d_toff + S), *d_mp = d_T + S;
+    CU(cudaMemcpy(dX, X, sizeof(double) * nT, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dV, V, sizeof(double) * nT, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dY, Y, sizeof(double) * nT, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dC, C, sizeof(double) * n, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dR, R, sizeof(double) * n, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dmu, mu, sizeof(double) * S, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dlam, lam.data(), sizeof(double) * S, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_roff, row_off.data(), sizeof(long long) * S, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_toff, t_off.data(), sizeof(long long) * S, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_T, T, sizeof(int) * S, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_mp, member_ptr, sizeof(int) * (S + 1), cudaMemcpyHostToDevice));
+    const dim3 grid((max_T + 127) / 128, std::min(n_stations, 65535));
+    construct_rec_kernel<<<grid, 128>>>(n_stations, d_T, d_mp, d_roff, d_toff, dX, dV, dY, dC, dR, dmu, dlam, transform,
+                                        dO, mean ? dM : nullptr);
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(out, dO, sizeof(double) * 6 * nT, cudaMemcpyDeviceToHost));
+    if (mean) CU(cudaMemcpy(mean, dM, sizeof(double) * 2 * (size_t)years, cudaMemcpyDeviceToHost));
+    return Err();
+}
+
+int ldsr_construct_rec_stations(int device, int n_stations, const int *T, const int *member_ptr, const double *X,
+                                const double *V, const double *Y, const double *C, const double *R, const double *mu,
+                                const double *lambda, int transform, double *out, double *mean, char *errbuf,
+                                int errlen) {
+    return report(construct_rec_stations(device, n_stations, T, member_ptr, X, V, Y, C, R, mu, lambda, transform, out,
+                                         mean),
+                  errbuf, errlen);
+}
+
 int ldsr_construct_rec_batch(int device, int n, int T, const double *X, const double *V, const double *Y,
                              const double *C, const double *R, double mu, int transform, double lambda, double *out,
                              double *mean, char *errbuf, int errlen) {
-    auto run = [&]() -> Err {
-        if (n < 1 || T < 1) return fail(LDSR_ERR_ARG, "need n >= 1 and T >= 1");
-        if (!X || !V || !Y || !C || !R || !out) return fail(LDSR_ERR_ARG, "a required pointer is NULL");
-        if (transform < 0 || transform > 2) return fail(LDSR_ERR_ARG, "transform must be 0 (none), 1 (log) or 2 (boxcox)");
-        if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-        CU(cudaSetDevice(device));
-        const size_t nT = (size_t)n * T;
-        double *d = nullptr;
-        struct Guard {
-            double *&p;
-            ~Guard() { cudaFree(p); }
-        } guard{d};
-        // one arena: X V Y | C R | out | mean
-        CU(cudaMalloc(&d, sizeof(double) * (3 * nT + 2 * (size_t)n + 6 * nT + 2 * (size_t)T)));
-        double *dX = d, *dV = dX + nT, *dY = dV + nT, *dC = dY + nT, *dR = dC + n, *dO = dR + n, *dM = dO + 6 * nT;
-        CU(cudaMemcpy(dX, X, sizeof(double) * nT, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(dV, V, sizeof(double) * nT, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(dY, Y, sizeof(double) * nT, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(dC, C, sizeof(double) * n, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(dR, R, sizeof(double) * n, cudaMemcpyHostToDevice));
-        construct_rec_kernel<<<(T + 127) / 128, 128>>>(n, T, dX, dV, dY, dC, dR, mu, transform, lambda, dO, dM);
-        CU(cudaGetLastError());
-        CU(cudaMemcpy(out, dO, sizeof(double) * 6 * nT, cudaMemcpyDeviceToHost));
-        if (mean) CU(cudaMemcpy(mean, dM, sizeof(double) * 2 * T, cudaMemcpyDeviceToHost));
-        return Err();
-    };
-    return report(run(), errbuf, errlen);
+    const int member_ptr[2] = {0, n};
+    return report(construct_rec_stations(device, 1, &T, member_ptr, X, V, Y, C, R, &mu, &lambda, transform, out, mean),
+                  errbuf, errlen);
+}
+
+// cv metrics over stations of different lengths (one launch); ldsr_cv_metrics_batch is its one-station case.
+static Err cv_metrics_stations(int device, int n_stations, const int *n, const int *fold_ptr, const double *sim,
+                               const double *obs, const int *z_ptr, const int *z_idx, int exp_trans, double *out) {
+    if (n_stations < 1) return fail(LDSR_ERR_ARG, "need n_stations >= 1");
+    if (!n || !fold_ptr || !sim || !obs || !z_ptr || !z_idx || !out) return fail(LDSR_ERR_ARG, "a required pointer is NULL");
+    if (fold_ptr[0] != 0) return fail(LDSR_ERR_ARG, "fold_ptr[0] must be 0");
+    for (int s = 0; s < n_stations; s++) {
+        if (n[s] < 2) return fail(LDSR_ERR_ARG, "station %d: need a target of length n >= 2", s);
+        if (fold_ptr[s + 1] < fold_ptr[s]) return fail(LDSR_ERR_ARG, "fold_ptr not monotone at station %d", s);
+    }
+    const int n_folds = fold_ptr[n_stations];
+    if (n_folds < 1) return fail(LDSR_ERR_ARG, "need n_folds >= 1");
+    if (z_ptr[0] < 0) return fail(LDSR_ERR_ARG, "z_ptr[0] < 0");
+    // per fold: length, offset of its station's target, offset of its sim row (= of its hold-out marks)
+    std::vector<int> f_n(n_folds);
+    std::vector<long long> f_obs(n_folds), f_row(n_folds);
+    long long n_obs = 0, n_sim = 0;
+    for (int s = 0; s < n_stations; s++) {
+        for (int f = fold_ptr[s]; f < fold_ptr[s + 1]; f++) {
+            f_n[f] = n[s];
+            f_obs[f] = n_obs;
+            f_row[f] = n_sim;
+            n_sim += n[s];
+        }
+        n_obs += n[s];
+    }
+    std::vector<unsigned char> held((size_t)n_sim, 0);
+    for (int f = 0; f < n_folds; f++) {
+        if (z_ptr[f + 1] < z_ptr[f]) return fail(LDSR_ERR_ARG, "z_ptr not monotone at fold %d", f);
+        for (int k = z_ptr[f]; k < z_ptr[f + 1]; k++) {
+            const int i = z_idx[k] - 1; // R indices are 1-based
+            if (i < 0 || i >= f_n[f]) return fail(LDSR_ERR_ARG, "fold %d: hold-out index %d outside 1..%d", f, z_idx[k], f_n[f]);
+            held[(size_t)f_row[f] + i] = 1;
+        }
+    }
+    if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
+    CU(cudaSetDevice(device));
+    double *d_sim = nullptr, *d_obs = nullptr, *d_out = nullptr;
+    unsigned char *d_held = nullptr;
+    long long *d_off = nullptr;
+    int *d_n = nullptr;
+    struct Guard {
+        double *&a, *&b, *&c;
+        unsigned char *&h;
+        long long *&o;
+        int *&n;
+        ~Guard() {
+            cudaFree(a);
+            cudaFree(b);
+            cudaFree(c);
+            cudaFree(h);
+            cudaFree(o);
+            cudaFree(n);
+        }
+    } guard{d_sim, d_obs, d_out, d_held, d_off, d_n};
+    CU(cudaMalloc(&d_sim, sizeof(double) * (size_t)n_sim));
+    CU(cudaMalloc(&d_obs, sizeof(double) * (size_t)n_obs));
+    CU(cudaMalloc(&d_out, sizeof(double) * (size_t)n_folds * 5));
+    CU(cudaMalloc(&d_held, held.size()));
+    CU(cudaMalloc(&d_off, sizeof(long long) * 2 * (size_t)n_folds));
+    CU(cudaMalloc(&d_n, sizeof(int) * (size_t)n_folds));
+    CU(cudaMemcpy(d_sim, sim, sizeof(double) * (size_t)n_sim, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_obs, obs, sizeof(double) * (size_t)n_obs, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_held, held.data(), held.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_off, f_obs.data(), sizeof(long long) * n_folds, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_off + n_folds, f_row.data(), sizeof(long long) * n_folds, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_n, f_n.data(), sizeof(int) * n_folds, cudaMemcpyHostToDevice));
+    cv_metrics_kernel<<<(n_folds + 3) / 4, 128>>>(n_folds, d_n, d_off, d_off + n_folds, d_sim, d_obs, d_held, exp_trans,
+                                                  d_out);
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(out, d_out, sizeof(double) * (size_t)n_folds * 5, cudaMemcpyDeviceToHost));
+    return Err();
+}
+
+int ldsr_cv_metrics_stations(int device, int n_stations, const int *n, const int *fold_ptr, const double *sim,
+                             const double *obs, const int *z_ptr, const int *z_idx, int exp_trans, double *out,
+                             char *errbuf, int errlen) {
+    return report(cv_metrics_stations(device, n_stations, n, fold_ptr, sim, obs, z_ptr, z_idx, exp_trans, out), errbuf,
+                  errlen);
 }
 
 int ldsr_cv_metrics_batch(int device, int n, int n_folds, const double *sim, const double *obs, const int *z_ptr,
                           const int *z_idx, int exp_trans, double *out, char *errbuf, int errlen) {
-    auto run = [&]() -> Err {
-        if (n < 2 || n_folds < 1) return fail(LDSR_ERR_ARG, "need n >= 2 and n_folds >= 1");
-        if (!sim || !obs || !z_ptr || !z_idx || !out) return fail(LDSR_ERR_ARG, "a required pointer is NULL");
-        std::vector<unsigned char> held((size_t)n_folds * n, 0);
-        for (int f = 0; f < n_folds; f++) {
-            if (z_ptr[f + 1] < z_ptr[f]) return fail(LDSR_ERR_ARG, "z_ptr not monotone at fold %d", f);
-            for (int k = z_ptr[f]; k < z_ptr[f + 1]; k++) {
-                const int i = z_idx[k] - 1; // R indices are 1-based
-                if (i < 0 || i >= n) return fail(LDSR_ERR_ARG, "fold %d: hold-out index %d outside 1..%d", f, z_idx[k], n);
-                held[(size_t)f * n + i] = 1;
-            }
-        }
-        if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-        CU(cudaSetDevice(device));
-        double *d_sim = nullptr, *d_obs = nullptr, *d_out = nullptr;
-        unsigned char *d_held = nullptr;
-        struct Guard {
-            double *&a, *&b, *&c;
-            unsigned char *&h;
-            ~Guard() {
-                cudaFree(a);
-                cudaFree(b);
-                cudaFree(c);
-                cudaFree(h);
-            }
-        } guard{d_sim, d_obs, d_out, d_held};
-        CU(cudaMalloc(&d_sim, sizeof(double) * (size_t)n_folds * n));
-        CU(cudaMalloc(&d_obs, sizeof(double) * n));
-        CU(cudaMalloc(&d_out, sizeof(double) * (size_t)n_folds * 5));
-        CU(cudaMalloc(&d_held, held.size()));
-        CU(cudaMemcpy(d_sim, sim, sizeof(double) * (size_t)n_folds * n, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_obs, obs, sizeof(double) * n, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(d_held, held.data(), held.size(), cudaMemcpyHostToDevice));
-        cv_metrics_kernel<<<(n_folds + 3) / 4, 128>>>(n, n_folds, d_sim, d_obs, d_held, exp_trans, d_out);
-        CU(cudaGetLastError());
-        CU(cudaMemcpy(out, d_out, sizeof(double) * (size_t)n_folds * 5, cudaMemcpyDeviceToHost));
-        return Err();
-    };
-    return report(run(), errbuf, errlen);
+    const int fold_ptr[2] = {0, n_folds};
+    return report(cv_metrics_stations(device, 1, &n, fold_ptr, sim, obs, z_ptr, z_idx, exp_trans, out), errbuf, errlen);
 }
 
 int ldsr_smoother_d_batch(int device, int d, int T, int p, int q, const double *y, const double *u, const double *v,

@@ -65,8 +65,10 @@ one_lds_cv <- function(z, instPeriod, mu, y, u, v, method = 'EM', num.restarts =
 
 # The fold loop of cvLDS (R/LDS_reconstruction.R:372-382) as one batch.  Call it in place of the
 # `Ycv <- if (single) foreach(...) else foreach(...) %:% foreach(...)` block; everything before
-# (:308-370) and after (:384-409) stays as it is.
-cv_folds_batched <- function(Z, instPeriod, mu, y, u, v, num.restarts, niter, tol, n.devices = 0L) {
+# (:308-370) and after (:384-409) stays as it is.  use.raw = TRUE: the fold output is the selected
+# fit's open-loop propagate(theta, u, v, y_fold)$Y[instPeriod] + mu (:279-281).
+cv_folds_batched <- function(Z, instPeriod, mu, y, u, v, num.restarts, niter, tol, n.devices = 0L,
+                             use.raw = FALSE) {
   single <- is.matrix(u)
   if (single) { u <- list(u); v <- list(v) }
   series <- lapply(seq_along(u), function(i) list(y = y, u = u[[i]], v = v[[i]]))
@@ -76,14 +78,157 @@ cv_folds_batched <- function(Z, instPeriod, mu, y, u, v, num.restarts, niter, to
                                       init = make_init(nrow(u[[i]]), nrow(v[[i]]), num.restarts))
   res <- .em_batch(series, jobs, niter, tol, n.devices)
   if (any(res$status == 1L)) stop('inv(): matrix is singular')
-  nm <- length(u)
-  lapply(seq_along(Z), function(k) {
+  .fold_outputs(res, series, jobs, seq_along(jobs), length(u), instPeriod, mu, use.raw)
+}
+
+# Ycv of one station from a batch result: `gs` are its groups (fold-major, member-minor, nm members).
+.fold_outputs <- function(res, series, jobs, gs, nm, instPeriod, mu, use.raw) {
+  lapply(seq_len(length(gs) %/% nm), function(k) {
     cols <- sapply(seq_len(nm), function(i) {
-      g <- (k - 1L) * nm + i
+      g <- gs[(k - 1L) * nm + i]
       if (is.na(res$best[g])) stop('no restart produced a finite likelihood')
-      c(res$Y[[g]][instPeriod]) + mu           # fit$Y[instPeriod] + mu   (:283)
+      if (use.raw) {                           # propagate(theta, u, v, y)$Y[instPeriod] + mu   (:281)
+        s <- series[[jobs[[g]]$series]]
+        yz <- s$y
+        yz[jobs[[g]]$held] <- NA
+        th <- .theta_list(res$theta[, res$best[g]], nrow(s$u), nrow(s$v))
+        c(propagate(th, s$u, s$v, matrix(yz, nrow = 1))$Y[instPeriod]) + mu
+      } else c(res$Y[[g]][instPeriod]) + mu    # fit$Y[instPeriod] + mu   (:283)
     })
     rowMeans(matrix(cols, ncol = nm))           # .final = rowMeans         (:379)
+  })
+}
+
+# Host-side set-up of one station as LDS_reconstruction / cvLDS do it (R/LDS_reconstruction.R:128-183):
+# the NULL sentinel, the transform, y centred and NA-padded to the station's horizon.
+.station_setup <- function(st, transform) {
+  u <- st$u; v <- st$v
+  single <- !is.list(u) && !is.list(v)
+  if (single) {
+    if (is.null(u) && is.null(v)) stop('u and v cannot both be NULL')
+    u <- list(u); v <- list(v)
+  }
+  if (is.null(u)) u <- vector('list', length(v))
+  if (is.null(v)) v <- vector('list', length(u))
+  for (i in seq_along(u)) {
+    if (!is.null(u[[i]]) && !is.null(v[[i]]) && ncol(u[[i]]) != ncol(v[[i]]))
+      stop('u and v must have the same number of time steps.')
+  }
+  N <- ncol(if (is.null(u[[1]])) v[[1]] else u[[1]])
+  u <- lapply(u, function(m) if (is.null(m)) matrix(0) else m)
+  v <- lapply(v, function(m) if (is.null(m)) matrix(0) else m)
+  Qa <- st$Qa
+  lambda <- NULL
+  obs <- switch(transform,
+    log = log(Qa$Qa),
+    boxcox = {
+      bc <- MASS::boxcox(Qa$Qa ~ 1, plotit = FALSE)
+      lambda <- bc$x[which.max(bc$y)]
+      if (abs(lambda) < 0.01) lambda <- 0
+      if (lambda == 0) log(Qa$Qa) else (Qa$Qa^lambda - 1) / lambda
+    },
+    none = Qa$Qa,
+    stop('Accepted transformations are "log", "boxcox" and "none" only.'))
+  end.year <- st$start.year + N - 1
+  if (end.year < max(Qa$year)) stop('The last year of u is earlier than the last year of the instrumental period.')
+  mu <- mean(obs, na.rm = TRUE)
+  y <- c(rep(NA, min(Qa$year) - st$start.year), obs - mu, rep(NA, end.year - max(Qa$year)))
+  years <- st$start.year:end.year
+  list(Qa = Qa, single = single, u = u, v = v, obs = obs, lambda = lambda, mu = mu, years = years,
+       y = t(y), instPeriod = which(years %in% Qa$year))
+}
+
+.back_transform <- function(x, transform, lambda) {
+  switch(transform, log = exp(x), boxcox = if (lambda == 0) exp(x) else (x * lambda + 1)^(1 / lambda), none = x)
+}
+
+#' cvLDS for many stations in one batched call: one .em_batch over all stations' folds x members x restarts
+#' and one device call for all their metrics.  stations: list of list(Qa = data.frame(year, Qa), u, v,
+#' start.year[, Z]); u / v a matrix, NULL or a list (ensemble) as in cvLDS; stations may differ in T, p, q,
+#' instrumental period and start year.  Random numbers: station by station, make_Z (if Z is NULL) then make_init
+#' fold-major / member-minor -- what the single-station calls draw one after another, so set.seed() gives the
+#' same folds and restarts.  Returns one cvLDS-shaped list per station (mirrors api.cvLDS_stations).
+cvLDS_stations <- function(stations, transform = 'log', num.restarts = 50, metric.space = 'original',
+                           use.raw = FALSE, niter = 1000, tol = 1e-5, use.robust.mean = TRUE, n.devices = 0L) {
+  prep <- lapply(stations, .station_setup, transform = transform)
+  series <- list(); jobs <- list(); groups <- list()
+  for (j in seq_along(prep)) {
+    P <- prep[[j]]
+    Z <- if (is.null(stations[[j]]$Z)) make_Z(P$Qa$Qa) else stations[[j]]$Z
+    if (!is.list(Z)) stop('Please provide the cross-validation folds (Z) in a list.')
+    prep[[j]]$Z <- Z
+    s0 <- length(series)
+    for (i in seq_along(P$u)) series[[s0 + i]] <- list(y = P$y, u = P$u[[i]], v = P$v[[i]])
+    g0 <- length(jobs)
+    for (z in Z) for (i in seq_along(P$u))
+      jobs[[length(jobs) + 1L]] <- list(series = s0 + i, held = P$instPeriod[z],
+                                        init = make_init(nrow(P$u[[i]]), nrow(P$v[[i]]), num.restarts))
+    groups[[j]] <- (g0 + 1L):length(jobs)
+  }
+  res <- .em_batch(series, jobs, niter, tol, n.devices)
+  if (any(res$status == 1L)) stop('inv(): matrix is singular')
+  Ycv <- lapply(seq_along(prep), function(j) {
+    P <- prep[[j]]
+    y <- .fold_outputs(res, series, jobs, groups[[j]], length(P$u), P$instPeriod, P$mu, use.raw)
+    if (metric.space == 'original') lapply(y, .back_transform, transform = transform, lambda = P$lambda) else y
+  })
+  targets <- lapply(prep, function(P) if (metric.space == 'original') P$Qa$Qa else P$obs)
+  dist <- .Call('_ldsr_cv_metrics_stations', lapply(Ycv, function(y) do.call(cbind, y)), lapply(targets, as.numeric),
+                lapply(prep, function(P) lapply(P$Z, as.integer)), FALSE, PACKAGE = 'ldsr')
+  mean.func <- if (use.robust.mean) dplR::tbrm else mean
+  lapply(seq_along(prep), function(j) {
+    md <- data.table::as.data.table(t(dist[[j]]))
+    data.table::setnames(md, c('R2', 'RE', 'CE', 'nRMSE', 'KGE'))
+    list(metrics.dist = md, metrics = sapply(md, mean.func),
+         target = data.table::data.table(year = prep[[j]]$Qa$year, y = targets[[j]]),
+         Ycv = do.call(cbind, Ycv[[j]]), Z = prep[[j]]$Z)
+  })
+}
+
+#' LDS_reconstruction for many stations in one batched call: one .em_batch over all stations' members x
+#' restarts and one device call for all their reconstructions (construct_rec and the ensemble means).
+#' stations: list of list(Qa, u, v, start.year[, init]), as cvLDS_stations.  Random numbers: station by station,
+#' make_init per member unless `init` is given.  Returns one LDS_reconstruction-shaped list per station
+#' (mirrors api.LDS_reconstruction_stations).
+LDS_reconstruction_stations <- function(stations, transform = 'log', num.restarts = 50, return.init = FALSE,
+                                        niter = 1000, tol = 1e-5, n.devices = 0L) {
+  prep <- lapply(stations, .station_setup, transform = transform)
+  series <- list(); jobs <- list()
+  for (j in seq_along(prep)) {
+    P <- prep[[j]]
+    init <- stations[[j]]$init
+    if (is.null(init)) init <- lapply(seq_along(P$u), function(i) make_init(nrow(P$u[[i]]), nrow(P$v[[i]]), num.restarts))
+    else if (P$single) init <- list(init)
+    for (i in seq_along(P$u)) {
+      series[[length(series) + 1L]] <- list(y = P$y, u = P$u[[i]], v = P$v[[i]])
+      jobs[[length(jobs) + 1L]] <- list(series = length(series), held = integer(0), init = init[[i]])
+    }
+  }
+  res <- .em_batch(series, jobs, niter, tol, n.devices)
+  if (any(res$status == 1L)) stop('inv(): matrix is singular')
+  picks <- lapply(seq_along(jobs), function(g) .pick(res, g, series, jobs))
+  first <- cumsum(c(0L, sapply(prep, function(P) length(P$u))))
+  mine <- lapply(seq_along(prep), function(j) picks[(first[j] + 1L):first[j + 1L]])
+  col <- function(key) lapply(mine, function(m) sapply(m, function(a) c(a$fit[[key]])))
+  th <- function(key) lapply(mine, function(m) sapply(m, function(a) c(a$theta[[key]])))
+  tr <- match(transform, c('none', 'log', 'boxcox')) - 1L
+  rec <- .Call('_ldsr_construct_rec_stations', lapply(col('X'), as.matrix), lapply(col('V'), as.matrix),
+               lapply(col('Y'), as.matrix), th('C'), th('R'), sapply(prep, `[[`, 'mu'),
+               as.integer(tr), sapply(prep, function(P) if (is.null(P$lambda)) 0 else P$lambda), PACKAGE = 'ldsr')
+  lapply(seq_along(prep), function(j) {
+    P <- prep[[j]]; n <- length(P$u)
+    a <- array(rec[[j]]$rec, dim = c(length(P$years), 6L, n))
+    members <- lapply(seq_len(n), function(i) {
+      dt <- data.table::as.data.table(a[, , i]); data.table::setnames(dt, c('X', 'Xl', 'Xu', 'Q', 'Ql', 'Qu'))
+      out <- list(rec = cbind(data.table::data.table(year = P$years), dt), theta = mine[[j]][[i]]$theta,
+                  lik = mine[[j]][[i]]$lik)
+      if (return.init) out$init <- mine[[j]][[i]]$init
+      if (transform == 'boxcox') out$lambda <- P$lambda
+      out
+    })
+    if (P$single) members[[1]]
+    else list(rec = data.table::data.table(year = P$years, X = rec[[j]]$mean[, 1], Q = rec[[j]]$mean[, 2]),
+              ensemble = members)
   })
 }
 

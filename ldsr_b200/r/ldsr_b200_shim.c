@@ -16,6 +16,8 @@
  *     _ldsr_rep_batch(theta,u,v,n,num_reps,seed,mu,exp_trans,z,r_seed)               10
  *     _ldsr_cv_metrics(Ycv,target,Z,exp_trans)                                        4
  *     _ldsr_construct_rec(X,V,Y,C,R,mu,transform,lambda)                              8
+ *     _ldsr_cv_metrics_stations(Ycv,target,Z,exp_trans)   lists, one element per station    4
+ *     _ldsr_construct_rec_stations(X,V,Y,C,R,mu,transform,lambda)   lists / per-station vectors   8
  *     _ldsr_objective(y,u,v,thetas,kind,lambda)   thetas: (2d+6) x n matrix, one column per candidate   6
  *     _ldsr_smoother_d(y,u,v,theta,stdlik,method)                                     6
  *     _ldsr_trim()                                release the session's cached device memory  0
@@ -343,6 +345,117 @@ SEXP _ldsr_construct_rec(SEXP X, SEXP V, SEXP Y, SEXP C, SEXP R, SEXP muS, SEXP 
     return out;
 }
 
+/* _ldsr_cv_metrics for many stations in one device call (ldsr_cv_metrics_stations).  Ycv: list of n_s x n_folds_s
+ * matrices; target: list of numeric vectors (n_s); Z: list of lists of integer vectors (1-based into the station's
+ * target).  Returns a list of 5 x n_folds_s matrices. */
+SEXP _ldsr_cv_metrics_stations(SEXP Ycv, SEXP target, SEXP Z, SEXP expS) {
+    char err[512] = "";
+    const int S = (int)XLENGTH(Ycv);
+    if ((int)XLENGTH(target) != S || (int)XLENGTH(Z) != S) Rf_error("ldsr: one Ycv, target and Z per station");
+    int *n = (int *)R_alloc((size_t)S, sizeof(int)), *fp = (int *)R_alloc((size_t)S + 1, sizeof(int));
+    R_xlen_t n_sim = 0, n_obs = 0, n_idx = 0;
+    fp[0] = 0;
+    for (int s = 0; s < S; s++) {
+        SEXP Y = VECTOR_ELT(Ycv, s), zs = VECTOR_ELT(Z, s);
+        n[s] = (int)XLENGTH(VECTOR_ELT(target, s));
+        if (Rf_nrows(Y) != n[s] || Rf_ncols(Y) != (int)XLENGTH(zs))
+            Rf_error("ldsr: station %d: Ycv must be length(target) x length(Z)", s + 1);
+        fp[s + 1] = fp[s] + (int)XLENGTH(zs);
+        n_sim += XLENGTH(Y);
+        n_obs += n[s];
+        for (R_xlen_t f = 0; f < XLENGTH(zs); f++) n_idx += XLENGTH(VECTOR_ELT(zs, f));
+    }
+    const int nf = fp[S];
+    double *sim = (double *)R_alloc((size_t)(n_sim > 0 ? n_sim : 1), sizeof(double));
+    double *obs = (double *)R_alloc((size_t)(n_obs > 0 ? n_obs : 1), sizeof(double));
+    int *zp = (int *)R_alloc((size_t)nf + 1, sizeof(int)), *zi = (int *)R_alloc((size_t)(n_idx > 0 ? n_idx : 1), sizeof(int));
+    double *ps = sim, *po = obs;
+    int f = 0;
+    zp[0] = 0;
+    for (int s = 0; s < S; s++) {
+        SEXP zs = VECTOR_ELT(Z, s);
+        memcpy(ps, REAL(VECTOR_ELT(Ycv, s)), sizeof(double) * (size_t)XLENGTH(VECTOR_ELT(Ycv, s)));
+        ps += XLENGTH(VECTOR_ELT(Ycv, s));
+        memcpy(po, REAL(VECTOR_ELT(target, s)), sizeof(double) * (size_t)n[s]);
+        po += n[s];
+        for (R_xlen_t k = 0; k < XLENGTH(zs); k++, f++) {
+            const int len = (int)XLENGTH(VECTOR_ELT(zs, k));
+            memcpy(zi + zp[f], INTEGER(VECTOR_ELT(zs, k)), sizeof(int) * (size_t)len);
+            zp[f + 1] = zp[f] + len;
+        }
+    }
+    double *o = (double *)R_alloc((size_t)nf * 5, sizeof(double));
+    check(ldsr_cv_metrics_stations(0, S, n, fp, sim, obs, zp, zi, Rf_asLogical(expS), o, err, sizeof err), err);
+    SEXP out = PROTECT(Rf_allocVector(VECSXP, S));
+    for (int s = 0; s < S; s++) { /* 5 x n_folds_s, like mapply's result */
+        SEXP m = PROTECT(Rf_allocMatrix(REALSXP, 5, fp[s + 1] - fp[s]));
+        memcpy(REAL(m), o + (size_t)fp[s] * 5, sizeof(double) * 5 * (size_t)(fp[s + 1] - fp[s]));
+        SET_VECTOR_ELT(out, s, m);
+        UNPROTECT(1);
+    }
+    UNPROTECT(1);
+    return out;
+}
+
+/* _ldsr_construct_rec for many stations in one device call (ldsr_construct_rec_stations).  X, V, Y: lists of
+ * T_s x n_s matrices (one column per member); C, R: lists of numeric vectors (n_s); mu, lambda: numeric vectors
+ * (one value per station).  Returns a list of list(rec = T_s x 6 x n_s array, mean = T_s x 2). */
+SEXP _ldsr_construct_rec_stations(SEXP X, SEXP V, SEXP Y, SEXP C, SEXP R, SEXP muS, SEXP trS, SEXP lamS) {
+    char err[512] = "";
+    const int S = (int)XLENGTH(X);
+    if ((int)XLENGTH(V) != S || (int)XLENGTH(Y) != S || (int)XLENGTH(C) != S || (int)XLENGTH(R) != S ||
+        (int)XLENGTH(muS) != S || (int)XLENGTH(lamS) != S)
+        Rf_error("ldsr: one X, V, Y, C, R, mu and lambda per station");
+    int *T = (int *)R_alloc((size_t)S, sizeof(int)), *mp = (int *)R_alloc((size_t)S + 1, sizeof(int));
+    R_xlen_t rows = 0, years = 0;
+    mp[0] = 0;
+    for (int s = 0; s < S; s++) {
+        T[s] = Rf_nrows(VECTOR_ELT(X, s));
+        mp[s + 1] = mp[s] + Rf_ncols(VECTOR_ELT(X, s));
+        if (XLENGTH(VECTOR_ELT(V, s)) != XLENGTH(VECTOR_ELT(X, s)) || XLENGTH(VECTOR_ELT(Y, s)) != XLENGTH(VECTOR_ELT(X, s)) ||
+            (int)XLENGTH(VECTOR_ELT(C, s)) != mp[s + 1] - mp[s] || (int)XLENGTH(VECTOR_ELT(R, s)) != mp[s + 1] - mp[s])
+            Rf_error("ldsr: station %d: X, V, Y must be T x n and C, R of length n", s + 1);
+        rows += XLENGTH(VECTOR_ELT(X, s));
+        years += T[s];
+    }
+    const size_t nr = (size_t)(rows > 0 ? rows : 1);
+    double *x = (double *)R_alloc(nr, sizeof(double)), *v = (double *)R_alloc(nr, sizeof(double));
+    double *y = (double *)R_alloc(nr, sizeof(double));
+    double *c = (double *)R_alloc((size_t)mp[S] + 1, sizeof(double)), *r = (double *)R_alloc((size_t)mp[S] + 1, sizeof(double));
+    for (int s = 0, off = 0; s < S; s++) {
+        const size_t len = (size_t)XLENGTH(VECTOR_ELT(X, s));
+        memcpy(x + off, REAL(VECTOR_ELT(X, s)), sizeof(double) * len);
+        memcpy(v + off, REAL(VECTOR_ELT(V, s)), sizeof(double) * len);
+        memcpy(y + off, REAL(VECTOR_ELT(Y, s)), sizeof(double) * len);
+        memcpy(c + mp[s], REAL(VECTOR_ELT(C, s)), sizeof(double) * (size_t)(mp[s + 1] - mp[s]));
+        memcpy(r + mp[s], REAL(VECTOR_ELT(R, s)), sizeof(double) * (size_t)(mp[s + 1] - mp[s]));
+        off += (int)len;
+    }
+    double *rec = (double *)R_alloc(6 * nr, sizeof(double)), *mean = (double *)R_alloc(2 * (size_t)years + 1, sizeof(double));
+    check(ldsr_construct_rec_stations(0, S, T, mp, x, v, y, c, r, REAL(muS), REAL(lamS), Rf_asInteger(trS), rec, mean, err,
+                                      sizeof err),
+          err);
+    const char *nm[] = {"rec", "mean", ""};
+    SEXP out = PROTECT(Rf_allocVector(VECSXP, S));
+    double *pr = rec, *pm = mean;
+    for (int s = 0; s < S; s++) {
+        const size_t n6 = 6 * (size_t)XLENGTH(VECTOR_ELT(X, s));
+        SEXP one = PROTECT(Rf_mkNamed(VECSXP, nm));
+        SEXP a = PROTECT(Rf_allocVector(REALSXP, (R_xlen_t)n6)); /* [member][column][year], year fastest */
+        SEXP m = PROTECT(Rf_allocMatrix(REALSXP, T[s], 2));
+        memcpy(REAL(a), pr, sizeof(double) * n6);
+        memcpy(REAL(m), pm, sizeof(double) * 2 * (size_t)T[s]);
+        pr += n6;
+        pm += 2 * (size_t)T[s];
+        SET_VECTOR_ELT(one, 0, a);
+        SET_VECTOR_ELT(one, 1, m);
+        SET_VECTOR_ELT(out, s, one);
+        UNPROTECT(3);
+    }
+    UNPROTECT(1);
+    return out;
+}
+
 /* penalized_likelihood / negLogLik / ssqTrain (R/LDS_GA.R:28-44, 136-147) for a population of
  * parameter vectors (the columns of `thetas`, in vec_to_list order, R/LDS_GA.R:6-16) in one call. */
 SEXP _ldsr_objective(SEXP y, SEXP u, SEXP v, SEXP thetas, SEXP kindS, SEXP lamS) {
@@ -423,6 +536,8 @@ static const R_CallMethodDef CallEntries[] = {
     {"_ldsr_smoother_d", (DL_FUNC)&_ldsr_smoother_d, 6},
     {"_ldsr_cv_metrics", (DL_FUNC)&_ldsr_cv_metrics, 4},
     {"_ldsr_construct_rec", (DL_FUNC)&_ldsr_construct_rec, 8},
+    {"_ldsr_cv_metrics_stations", (DL_FUNC)&_ldsr_cv_metrics_stations, 4},
+    {"_ldsr_construct_rec_stations", (DL_FUNC)&_ldsr_construct_rec_stations, 8},
     {"_ldsr_objective", (DL_FUNC)&_ldsr_objective, 6},
     {"_ldsr_trim", (DL_FUNC)&_ldsr_trim, 0},
     {NULL, NULL, 0}};
