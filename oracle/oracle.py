@@ -268,18 +268,19 @@ def construct_rec(X, V, Y, C_, R_, mu, transform="log", lam=0.0):
     return out, mean
 
 
-def objective(y, u, v, theta_vec, kind, lam=1.0):
+def objective(y, u, v, theta_vec, kind, lam=1.0, p=None, q=None):
     """The experimental learners' objectives (R/LDS_GA.R:28-44, 136-147) from the oracle's
-    Kalman_smoother / propagate.  theta_vec is the reference's flat order (vec_to_list, R/LDS_GA.R:6-16)."""
+    Kalman_smoother / propagate.  theta_vec is the reference's flat order (vec_to_list, R/LDS_GA.R:6-16);
+    p / q give its widths when u / v is None but theta still has B / D entries."""
     y = np.asarray(y, dtype=np.float64).ravel()
     if kind == "penalized_likelihood":
-        s = kalman_smoother(y, u, v, theta_vec, stdlik=False)
-        p = 0 if u is None else np.asarray(u).shape[0]
+        s = kalman_smoother(y, u, v, theta_vec, p=p, q=q, stdlik=False)
+        p = (0 if u is None else np.asarray(u).shape[0]) if p is None else p
         A, B = theta_vec[0], np.asarray(theta_vec[1:1 + p])
         X = s["X"]
         Bu = B @ np.asarray(u)[:, :-1] if u is not None else 0.0
         return s["lik"] - lam * float(np.sum((X[1:] - A * X[:-1] - Bu) ** 2))
-    pr = propagate(theta_vec, u, v, y)
+    pr = propagate(theta_vec, u, v, y, p=p, q=q)
     if kind == "negLogLik":
         return -pr["lik"]
     return float(np.nansum((y - pr["Y"]) ** 2))

@@ -265,5 +265,9 @@ static inline int __popc(unsigned x) { return __builtin_popcount(x); }
 static inline int __clz(int x) { return x == 0 ? 32 : __builtin_clz((unsigned)x); }
 static inline int __ffs(int x) { return __builtin_ffs(x); }
 static inline long long clock64() { return 0; }
+static inline void sincospi(double x, double *s, double *c) { // the device generator of rep_kernel (unused in z mode)
+    *s = std::sin(M_PI * x);
+    *c = std::cos(M_PI * x);
+}
 using std::max;
 using std::min;

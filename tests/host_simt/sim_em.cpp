@@ -1,6 +1,6 @@
-// sim_em.cpp -- TEST INFRASTRUCTURE: the EM kernels' SOURCE (ldsr_b200/csrc/*.cuh) compiled for the CPU
-// and run by the coroutine emulator of host_simt.h on one series.  The host side here re-states what
-// plan_build / setup_kernel / compact_kernel prepare (blob, masks, Gram constants, task list) with
+// sim_em.cpp -- TEST INFRASTRUCTURE: the EM kernels' and the single-step kernels' SOURCE (ldsr_b200/csrc/*.cuh)
+// compiled for the CPU and run by the coroutine emulator of host_simt.h on one series.  The host side here
+// re-states what plan_build / setup_kernel / compact_kernel prepare (blob, masks, Gram constants, task list) with
 // plain loops, so the comparison with the oracle also covers those conventions.
 //
 //   g++ -O1 -g -std=c++17 -DLDSR_HOST_SIM -shared -fPIC sim_em.cpp -o libldsr_hostsim.so
@@ -15,6 +15,7 @@
 #ifdef LDSR_HAVE_SCAN
 #include "../../ldsr_b200/csrc/em_scan_kernel.cuh"
 #endif
+#include "../../ldsr_b200/csrc/aux_kernels.cuh"
 
 #include <vector>
 
@@ -108,79 +109,88 @@ template <int PQ> int launch_wide_hostsim(const EmParams &ep, const SeriesDev &S
 }
 #endif
 
-template <int PQ> int run(const Job &J) {
-    constexpr int NW = 4, MSEG = 4, UW = 32;
-    const int T = J.T, p = J.p, q = J.q, ng = J.n_groups, nf = J.n_fits;
-    constexpr int TL = 2 * PQ + 6;
-    // ---- blob (plan_build)
+// What plan_build and setup_kernel prepare for one series and its groups: the blob, the window Gram blocks of u,
+// the series constant (TuuInv over t < T - 1, then its singular flag), and per group the observed-step mask, the
+// Gram constants and the status.
+struct Prep {
     SeriesDev S;
+    std::vector<double> blob, uwin, sconst, gconst;
+    std::vector<unsigned> masks;
+    std::vector<long long> g_mask_off;
+    std::vector<int> g_status, g_series, g_nobs;
+    bool tuu_singular = false;
+};
+
+template <int PQ> void prepare(int T, int p, int q, const double *y, const double *u, const double *v, int ng,
+                               const int *held_ptr, const int *held_idx, Prep &P) {
+    constexpr int UW = 32;
+    // ---- blob (plan_build)
+    SeriesDev &S = P.S;
     std::memset(&S, 0, sizeof S);
     S.T = T;
     S.p = p;
     S.q = q;
-    S.has_u = J.u != nullptr;
-    S.has_v = J.v != nullptr;
-    S.same_uv = (J.u && J.v && p == q && std::memcmp(J.u, J.v, sizeof(double) * (size_t)p * T) == 0) || (!J.u && !J.v);
+    S.has_u = u != nullptr;
+    S.has_v = v != nullptr;
+    S.same_uv = (u && v && p == q && std::memcmp(u, v, sizeof(double) * (size_t)p * T) == 0) || (!u && !v);
     const int Ty = (T + 1) & ~1, nuv = T * PQ;
     S.y_off = 0;
     S.u_off = Ty;
     S.v_off = S.same_uv ? S.u_off : ((S.u_off + nuv + 1) & ~1);
     S.blob_doubles = ((S.v_off + nuv) + 1) & ~1;
-    S.blob_off = 0;
-    S.sconst_off = 0;
-    S.fit_begin = 0;
-    S.fit_end = nf;
-    S.uwin_off = 0;
-    std::vector<double> blob((size_t)S.blob_doubles, 0.0);
+    std::vector<double> &blob = P.blob;
+    blob.assign((size_t)S.blob_doubles, 0.0);
     for (int t = 0; t < T; t++) {
-        blob[t] = J.y[t];
-        if (J.u)
-            for (int j = 0; j < p; j++) blob[S.u_off + (size_t)t * PQ + j] = J.u[(size_t)t * p + j];
-        if (J.v && !S.same_uv)
-            for (int j = 0; j < q; j++) blob[S.v_off + (size_t)t * PQ + j] = J.v[(size_t)t * q + j];
+        blob[t] = y[t];
+        if (u)
+            for (int j = 0; j < p; j++) blob[S.u_off + (size_t)t * PQ + j] = u[(size_t)t * p + j];
+        if (v && !S.same_uv)
+            for (int j = 0; j < q; j++) blob[S.v_off + (size_t)t * PQ + j] = v[(size_t)t * q + j];
     }
     const int nwin = (T + UW - 1) / UW;
-    std::vector<double> uwin((size_t)nwin * PQ * PQ, 0.0);
-    if (J.u)
+    P.uwin.assign((size_t)nwin * PQ * PQ, 0.0);
+    if (u)
         for (int t = 0; t < T; t++)
             for (int a = 0; a < p; a++)
                 for (int c = 0; c < p; c++)
-                    uwin[(size_t)(t / UW) * PQ * PQ + a * PQ + c] += J.u[(size_t)t * p + a] * J.u[(size_t)t * p + c];
+                    P.uwin[(size_t)(t / UW) * PQ * PQ + a * PQ + c] += u[(size_t)t * p + a] * u[(size_t)t * p + c];
     // ---- series constant: TuuInv over t < T-1
-    std::vector<double> sconst;
     {
         std::vector<char> keep(T, 1);
-        if (!gram_inverse(blob.data() + S.u_off, T - 1, PQ, J.u ? p : 0, keep, sconst)) return 10;
-        sconst.push_back(0.0);
+        P.tuu_singular = !gram_inverse(blob.data() + S.u_off, T - 1, PQ, u ? p : 0, keep, P.sconst);
+        P.sconst.push_back(P.tuu_singular ? 1.0 : 0.0);
     }
-    // ---- groups: masks + constants (setup_kernel)
+    // ---- groups: masks + constants (setup_kernel, merge_status_kernel)
     const int nwords = (T + 31) / 32;
-    std::vector<unsigned> masks((size_t)ng * nwords, 0u);
-    std::vector<long long> g_mask_off(ng);
-    std::vector<double> gconst((size_t)ng * gconst_stride(PQ), 0.0);
-    std::vector<int> g_status(ng, 0), g_series(ng, 0);
+    P.masks.assign((size_t)ng * nwords, 0u);
+    P.g_mask_off.assign(ng, 0);
+    P.gconst.assign((size_t)ng * gconst_stride(PQ), 0.0);
+    P.g_status.assign(ng, 0);
+    P.g_series.assign(ng, 0);
+    P.g_nobs.assign(ng, 0);
     for (int g = 0; g < ng; g++) {
-        g_mask_off[g] = (long long)g * nwords;
+        P.g_mask_off[g] = (long long)g * nwords;
         std::vector<char> keep(T, 0);
-        for (int t = 0; t < T; t++) keep[t] = std::isfinite(J.y[t]) ? 1 : 0;
-        if (J.held_ptr)
-            for (int k = J.held_ptr[g]; k < J.held_ptr[g + 1]; k++) keep[J.held_idx[k]] = 0;
+        for (int t = 0; t < T; t++) keep[t] = std::isfinite(y[t]) ? 1 : 0;
+        if (held_ptr)
+            for (int k = held_ptr[g]; k < held_ptr[g + 1]; k++) keep[held_idx[k]] = 0;
         for (int t = 0; t < T; t++)
-            if (keep[t]) masks[(size_t)g * nwords + (t >> 5)] |= 1u << (t & 31);
-        double *gc = gconst.data() + (size_t)g * gconst_stride(PQ);
+            if (keep[t]) P.masks[(size_t)g * nwords + (t >> 5)] |= 1u << (t & 31);
+        double *gc = P.gconst.data() + (size_t)g * gconst_stride(PQ);
         const double *vr = blob.data() + S.v_off;
         std::vector<double> svv_inv;
-        if (!gram_inverse(vr, T, PQ, J.v ? q : 0, keep, svv_inv)) g_status[g] = 1;
+        if (!gram_inverse(vr, T, PQ, v ? q : 0, keep, svv_inv) || P.tuu_singular) P.g_status[g] = 1;
         double Syy = 0.0, n_obs = 0.0;
         std::vector<double> Syv(PQ, 0.0);
         for (int t = 0; t < T; t++) {
             if (!keep[t]) continue;
-            Syy += J.y[t] * J.y[t];
+            Syy += y[t] * y[t];
             n_obs += 1.0;
-            for (int a = 0; a < PQ; a++) Syv[a] += J.y[t] * vr[(size_t)t * PQ + a];
+            for (int a = 0; a < PQ; a++) Syv[a] += y[t] * vr[(size_t)t * PQ + a];
         }
         gc[0] = Syy;
         gc[1] = n_obs;
+        P.g_nobs[g] = (int)n_obs;
         for (int a = 0; a < PQ; a++) {
             gc[2 + a] = Syv[a];
             double acc = 0.0;
@@ -189,21 +199,48 @@ template <int PQ> int run(const Job &J) {
         }
         for (int e = 0; e < PQ * PQ; e++) gc[2 + 2 * PQ + e] = svv_inv[e];
     }
+}
+
+// a caller theta (p, q) in the device layout (PQ, PQ) and back (ldsr_abi.cu: pad_theta, unpad_theta)
+template <int PQ> void pad_theta(const double *src, int p, int q, bool has_u, bool has_v, double *dst) {
+    std::fill(dst, dst + 2 * PQ + 6, 0.0);
+    dst[0] = src[0];
+    if (has_u)
+        for (int j = 0; j < p; j++) dst[1 + j] = src[1 + j];
+    dst[1 + PQ] = src[1 + p];
+    if (has_v)
+        for (int j = 0; j < q; j++) dst[2 + PQ + j] = src[2 + p + j];
+    for (int k = 0; k < 4; k++) dst[2 + 2 * PQ + k] = src[2 + p + q + k];
+}
+template <int PQ> void unpad_theta(const double *src, int p, int q, bool has_u, bool has_v, double *dst) {
+    dst[0] = src[0];
+    for (int j = 0; j < p; j++) dst[1 + j] = has_u ? src[1 + j] : 0.0;
+    dst[1 + p] = src[1 + PQ];
+    for (int j = 0; j < q; j++) dst[2 + p + j] = has_v ? src[2 + PQ + j] : 0.0;
+    for (int k = 0; k < 4; k++) dst[2 + p + q + k] = src[2 + 2 * PQ + k];
+}
+
+template <int PQ> int run(const Job &J) {
+    constexpr int NW = 4, MSEG = 4, UW = 32;
+    const int T = J.T, p = J.p, q = J.q, ng = J.n_groups, nf = J.n_fits;
+    constexpr int TL = 2 * PQ + 6;
+    Prep Pr;
+    prepare<PQ>(T, p, q, J.y, J.u, J.v, ng, J.held_ptr, J.held_idx, Pr);
+    if (Pr.tuu_singular) return 10;
+    SeriesDev &S = Pr.S;
+    S.fit_begin = 0;
+    S.fit_end = nf;
+    std::vector<double> &blob = Pr.blob, &uwin = Pr.uwin, &sconst = Pr.sconst, &gconst = Pr.gconst;
+    std::vector<unsigned> &masks = Pr.masks;
+    std::vector<long long> &g_mask_off = Pr.g_mask_off;
+    std::vector<int> &g_status = Pr.g_status, &g_series = Pr.g_series;
     // ---- fits
     std::vector<double> theta((size_t)nf * TL, 0.0), l1(nf, 0.0), l2(nf, 0.0), lik(nf, std::nan(""));
     std::vector<int> ne(nf, 0), done(nf, 0), f_group(J.fit_group, J.fit_group + nf), f_user(nf);
     const int stride = p + q + 6;
     for (int f = 0; f < nf; f++) {
         f_user[f] = f;
-        const double *src = J.theta0 + (size_t)f * stride;
-        double *dst = &theta[(size_t)f * TL];
-        dst[0] = src[0];
-        if (J.u)
-            for (int j = 0; j < p; j++) dst[1 + j] = src[1 + j];
-        dst[1 + PQ] = src[1 + p];
-        if (J.v)
-            for (int j = 0; j < q; j++) dst[2 + PQ + j] = src[2 + p + j];
-        for (int k = 0; k < 4; k++) dst[2 + 2 * PQ + k] = src[2 + p + q + k];
+        pad_theta<PQ>(J.theta0 + (size_t)f * stride, p, q, J.u != nullptr, J.v != nullptr, &theta[(size_t)f * TL]);
     }
     std::vector<int> active(nf, 0);
     std::vector<int4> tasks(nf + 2);
@@ -361,16 +398,116 @@ template <int PQ> int run(const Job &J) {
     }
 #endif
     for (int f = 0; f < nf; f++) {
-        const double *src = &theta[(size_t)f * TL];
-        double *dst = J.theta_out + (size_t)f * stride;
-        dst[0] = src[0];
-        for (int j = 0; j < p; j++) dst[1 + j] = J.u ? src[1 + j] : 0.0;
-        dst[1 + p] = src[1 + PQ];
-        for (int j = 0; j < q; j++) dst[2 + p + j] = J.v ? src[2 + PQ + j] : 0.0;
-        for (int k = 0; k < 4; k++) dst[2 + p + q + k] = src[2 + 2 * PQ + k];
+        unpad_theta<PQ>(&theta[(size_t)f * TL], p, q, J.u != nullptr, J.v != nullptr, J.theta_out + (size_t)f * stride);
         J.lik_out[f] = lik[f];
         J.iters_out[f] = ne[f];
     }
+    return 0;
+}
+
+// The single-step kernels (aux_kernels.cuh) on one series: kind 0 = smoother_kernel, 1 = propagate_kernel, 2 =
+// mstep_kernel.  One job per row of X, Y, V, J ([n_jobs][T]); the M-step reads X, V, J and writes theta_out.
+struct StepJob {
+    int kind, T, p, q, n_groups, n_jobs, stdlik, order;
+    const double *y, *u, *v;
+    const int *held_ptr, *held_idx, *job_group, *job_theta;
+    const double *theta;
+    double *X, *Y, *V, *J, *lik, *aux, *theta_out;
+    int *status;
+};
+
+template <int PQ> int run_step(const StepJob &J) {
+    constexpr int TL = 2 * PQ + 6;
+    const int T = J.T, nj = J.n_jobs, stride = J.p + J.q + 6;
+    Prep Pr;
+    prepare<PQ>(T, J.p, J.q, J.y, J.u, J.v, J.n_groups, J.held_ptr, J.held_idx, Pr);
+    std::vector<long long> job_row(nj);
+    for (int j = 0; j < nj; j++) job_row[j] = (long long)j * T;
+    std::vector<double> th((size_t)nj * TL, 0.0);
+    const int block = 64, grid = (nj + block - 1) / block; // as kernels_inst.cu launches them
+    if (J.kind == 2) {
+        MstepParams mp;
+        std::memset(&mp, 0, sizeof mp);
+        mp.series = &Pr.S;
+        mp.blobs = Pr.blob.data();
+        mp.sconst = Pr.sconst.data();
+        mp.g_series = Pr.g_series.data();
+        mp.masks = Pr.masks.data();
+        mp.g_mask_off = Pr.g_mask_off.data();
+        mp.gconst = Pr.gconst.data();
+        mp.g_status = Pr.g_status.data();
+        mp.n_fits = nj;
+        mp.f_group = J.job_group;
+        mp.f_row = job_row.data();
+        mp.X = J.X;
+        mp.V = J.V;
+        mp.J = J.J;
+        mp.theta_out = th.data();
+        mp.status = J.status;
+        hostsim::launch(grid, block, 0, J.order, [&] { mstep_kernel<PQ>(mp); });
+        for (int j = 0; j < nj; j++)
+            unpad_theta<PQ>(&th[(size_t)j * TL], J.p, J.q, J.u != nullptr, J.v != nullptr, J.theta_out + (size_t)j * stride);
+        return 0;
+    }
+    for (int j = 0; j < nj; j++)
+        pad_theta<PQ>(J.theta + (size_t)j * stride, J.p, J.q, J.u != nullptr, J.v != nullptr, &th[(size_t)j * TL]);
+    SmootherParams sp;
+    std::memset(&sp, 0, sizeof sp);
+    sp.series = &Pr.S;
+    sp.blobs = Pr.blob.data();
+    sp.g_series = Pr.g_series.data();
+    sp.masks = Pr.masks.data();
+    sp.g_mask_off = Pr.g_mask_off.data();
+    sp.g_nobs = Pr.g_nobs.data();
+    sp.n_jobs = nj;
+    sp.job_group = J.job_group;
+    sp.job_theta = J.job_theta;
+    sp.job_row = job_row.data();
+    sp.theta = th.data();
+    sp.X = J.X;
+    sp.Y = J.Y;
+    sp.V = J.V;
+    sp.J = J.J;
+    sp.lik = J.lik;
+    sp.stdlik = J.stdlik;
+    sp.aux = J.aux;
+    if (J.kind == 0)
+        hostsim::launch(grid, block, 0, J.order, [&] { smoother_kernel<PQ>(sp); });
+    else if (J.kind == 1)
+        hostsim::launch(grid, block, 0, J.order, [&] { propagate_kernel<PQ>(sp); });
+    else
+        return 12;
+    return 0;
+}
+
+// rep_kernel with caller noise z ([n_reps][1 + 2n]); what ldsr_rep_batch prepares (padded theta, u, v)
+template <int PQ> int run_rep(int p, int q, const double *u, const double *v, int n, int n_reps, const double *z,
+                              const double *theta, double mu, int exp_trans, int order, double *simX, double *simY,
+                              double *simQ) {
+    std::vector<double> th(2 * PQ + 6), up((size_t)n * PQ, 0.0), vp((size_t)n * PQ, 0.0);
+    pad_theta<PQ>(theta, p, q, u != nullptr, v != nullptr, th.data());
+    for (int t = 0; t < n; t++) {
+        if (u)
+            for (int j = 0; j < p; j++) up[(size_t)t * PQ + j] = u[(size_t)t * p + j];
+        if (v)
+            for (int j = 0; j < q; j++) vp[(size_t)t * PQ + j] = v[(size_t)t * q + j];
+    }
+    RepParams rp;
+    std::memset(&rp, 0, sizeof rp);
+    rp.theta = th.data();
+    rp.u = up.data();
+    rp.v = vp.data();
+    rp.z = z;
+    rp.n = n;
+    rp.n_reps = n_reps;
+    rp.mu = mu;
+    rp.exp_trans = exp_trans;
+    rp.simX = simX;
+    rp.simY = simY;
+    rp.simQ = simQ;
+    const int per_cta = REP_WARPS * 32;
+    hostsim::launch((n_reps + per_cta - 1) / per_cta, per_cta, rep_smem_bytes(z != nullptr), order,
+                    [&] { rep_kernel<PQ>(rp); });
     return 0;
 }
 
@@ -403,5 +540,32 @@ extern "C" int hostsim_em_traj(int T, int p, int q, const double *y, const doubl
     const int need = std::max(u ? p : 1, v ? q : 1);
     if (need <= 3) return run<3>(J);
     if (need <= 10) return run<10>(J);
+    return 13;
+}
+
+// The single-step kernels, padded to width 3, 5 or 16 (steps per smoother block 8, 4, 1).  kind: 0 smoother, 1
+// propagate, 2 M-step (see StepJob); theta is [n_jobs][p + q + 6]; job_theta[j] < 0 marks a job without theta
+// (smoother only: NaN rows).
+extern "C" int hostsim_step(int kind, int T, int p, int q, const double *y, const double *u, const double *v,
+                            int n_groups, const int *held_ptr, const int *held_idx, int n_jobs, const int *job_group,
+                            const int *job_theta, const double *theta, int stdlik, int order, double *X, double *Y,
+                            double *V, double *J, double *lik, double *aux, double *theta_out, int *status) {
+    StepJob sj{kind, T, p, q, n_groups, n_jobs, stdlik, order, y, u, v, held_ptr, held_idx, job_group, job_theta, theta,
+               X, Y, V, J, lik, aux, theta_out, status};
+    const int need = std::max(1, std::max(u ? p : 0, v ? q : 0));
+    if (need <= 3) return run_step<3>(sj);
+    if (need <= 5) return run_step<5>(sj);
+    if (need <= 16) return run_step<16>(sj);
+    return 13;
+}
+
+// rep_kernel in caller-noise mode; any of simX, simY, simQ may be NULL
+extern "C" int hostsim_rep(int p, int q, const double *u, const double *v, int n, int n_reps, const double *z,
+                           const double *theta, double mu, int exp_trans, int order, double *simX, double *simY,
+                           double *simQ) {
+    const int need = std::max(1, std::max(u ? p : 0, v ? q : 0));
+    if (need <= 3) return run_rep<3>(p, q, u, v, n, n_reps, z, theta, mu, exp_trans, order, simX, simY, simQ);
+    if (need <= 5) return run_rep<5>(p, q, u, v, n, n_reps, z, theta, mu, exp_trans, order, simX, simY, simQ);
+    if (need <= 16) return run_rep<16>(p, q, u, v, n, n_reps, z, theta, mu, exp_trans, order, simX, simY, simQ);
     return 13;
 }

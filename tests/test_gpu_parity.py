@@ -594,62 +594,119 @@ def test_ranked_assignment_with_several_series_equals_separate_runs():
     assert_theta_close(a["theta"][f], o["theta"])
 
 
-@pytest.mark.parametrize("case", ["np413", "narrow_separate_v", "wide10", "wide10_separate_v", "long1500"])
-def test_winner_trajectories_equal_the_oracle_estep_with_the_same_theta(case):
-    """X, Y, V, J returned by ldsr_em_batch are the E-step (EM.cpp:43-110) of the selected restart's theta on the
-    group's y: compared with the oracle's smoother run with the GPU's OWN theta, so the tolerance is that of one
-    E-step (1e-10), not of a whole EM run.  Covers both trajectory paths: the scan kernel's trajectory mode
-    (narrow inputs, or wide with v == u, series up to 1024 / 512 steps) and the one-thread-per-winner kernel."""
+# (T, p, q, v == u) of the synthetic winner-trajectory cases.  The scan kernel's trajectory mode takes widths up to 10
+# (T <= 1024 up to width 4; T <= 512 and v == u from width 5); the others take smoother_kernel, one thread per winner.
+WINNER_CASES = dict(narrow_separate_v=(150, 3, 2, False), wide10=(300, 10, 10, True),
+                    wide10_separate_v=(120, 10, 4, False), long1500=(1500, 3, 3, True),
+                    wide12=(300, 12, 12, True), wide16=(300, 16, 16, True), wide24=(300, 24, 24, True),
+                    wide32=(300, 32, 32, True), wide6_separate_v=(200, 6, 3, False), pq4_long1100=(1100, 4, 4, True),
+                    pq6_long600=(600, 6, 6, True), singular_group=(300, 12, 12, True))
+
+
+def _winner_case(case):
+    """The em_batch job of a winner-trajectory case (also built by the child process of the sequential-path run)."""
     rng = np.random.default_rng(21)
     if case == "np413":
         from ldsr_b200 import workloads as W
-        w = W.np_cv(4, 10)
-    else:
-        T, p, q, same = dict(narrow_separate_v=(150, 3, 2, False), wide10=(300, 10, 10, True),
-                             wide10_separate_v=(120, 10, 4, False), long1500=(1500, 3, 3, True))[case]
-        u = rng.standard_normal((p, T))
-        v = u if same else rng.standard_normal((q, T))
-        x = np.zeros(T)
-        for t in range(1, T):
-            x[t] = 0.7 * x[t - 1] + 0.1 * u[0, t - 1] + 0.4 * rng.standard_normal()
-        y = 0.6 * x + 0.05 * v[0] + 0.2 * rng.standard_normal(T)
-        y[: T // 2] = np.nan
-        y[T // 2 + 7] = np.nan
-        inst = np.arange(T // 2, T)
-        inst = inst[np.isfinite(y[inst])]
-        held = [np.sort(rng.choice(inst, 9, replace=False)) for _ in range(3)] + [np.array([], dtype=int)]
-        th0 = rand_theta0(rng, p, q, 4 * 6)
-        th0[:, 1:1 + p] *= 0.2
-        th0[:, 2 + p:2 + p + q] *= 0.2
-        w = dict(series=[dict(y=y, u=u, v=v)], group_series=np.zeros(4, dtype=np.int32), held=held,
-                 fit_group=np.repeat(np.arange(4), 6), theta0=th0)
+        return W.np_cv(4, 10)
+    T, p, q, same = WINNER_CASES[case]
+    u = rng.standard_normal((p, T))
+    v = u if same else rng.standard_normal((q, T))
+    x = np.zeros(T)
+    for t in range(1, T):
+        x[t] = 0.7 * x[t - 1] + 0.1 * u[0, t - 1] + 0.4 * rng.standard_normal()
+    y = 0.6 * x + 0.05 * v[0] + 0.2 * rng.standard_normal(T)
+    y[: T // 2] = np.nan
+    y[T // 2 + 7] = np.nan
+    inst = np.arange(T // 2, T)
+    inst = inst[np.isfinite(y[inst])]
+    held = [np.sort(rng.choice(inst, 9, replace=False)) for _ in range(3)] + [np.array([], dtype=int)]
+    th0 = rand_theta0(rng, p, q, 4 * 6)
+    th0[:, 1:1 + p] *= 0.2
+    th0[:, 2 + p:2 + p + q] *= 0.2
+    series, group_series = [dict(y=y, u=u, v=v)], np.zeros(4, dtype=np.int32)
+    if case == "singular_group":
+        # group 1 on a second series whose Tuu is exactly singular (two equal +-1 rows over the 64 steps t < T - 1):
+        # all its fits are singular, it has no winner and its rows must be NaN; its neighbours are unaffected
+        us = rng.standard_normal((p, 65))
+        us[0] = us[1] = rng.choice([-1.0, 1.0], 65)
+        ys = 0.3 * rng.standard_normal(65)
+        series.append(dict(y=ys, u=us, v=us))
+        group_series[1] = 1
+        held[1] = np.array([], dtype=int)
+    return dict(series=series, group_series=group_series, held=held, fit_group=np.repeat(np.arange(4), 6), theta0=th0)
+
+
+@pytest.mark.parametrize("case", ["np413", "narrow_separate_v", "wide10", "wide10_separate_v", "long1500", "wide12",
+                                  "wide16", "wide24", "wide32", "wide6_separate_v", "pq4_long1100", "pq6_long600",
+                                  "singular_group"])
+def test_winner_trajectories_equal_the_oracle_estep_with_the_same_theta(case, tmp_path):
+    """X, Y, V, J returned by ldsr_em_batch are the E-step (EM.cpp:43-110) of the selected restart's theta on the
+    group's y: compared with the oracle's smoother run with the GPU's OWN theta, so the tolerance is that of one
+    E-step (1e-10), not of a whole EM run.  Covers both trajectory paths: the scan kernel's trajectory mode
+    (narrow inputs, or wide with v == u, series up to 1024 / 512 steps) and the one-thread-per-winner kernel
+    (wider inputs, v != u from width 5, longer series), whose rows are NaN for a group without a winner.
+    Where the scan kernel applies (np413, wide10), the one-thread-per-winner kernel is also run on the same job
+    (LDSR_SEQ_TRAJ=1, read once, so in a child process) and both paths must agree to 1e-10."""
+    w = _winner_case(case)
     g = _lib.em_batch(w["series"], w["group_series"], w["held"], w["fit_group"], w["theta0"], 40, 1e-5)
-    s0 = w["series"][0]
     for k in range(len(w["group_series"])):
+        row = slice(g["traj_ptr"][k], g["traj_ptr"][k + 1])
+        if case == "singular_group" and k == 1:
+            assert np.all(g["status"][w["fit_group"] == 1] == _lib.FIT_SINGULAR) and g["best"][k] == -1
+            for name in ("X", "Y", "V", "J"):
+                assert np.isnan(g[name][row]).all(), name
+            continue
+        s0 = w["series"][w["group_series"][k]]
         yy = np.array(s0["y"], dtype=float)
         yy[w["held"][k]] = np.nan
         s = O.kalman_smoother(yy, s0["u"], s0["v"], g["theta"][g["best"][k]])
-        row = slice(g["traj_ptr"][k], g["traj_ptr"][k + 1])
         for name in ("X", "Y", "V", "J"):
             assert np.allclose(g[name][row], s[name], rtol=1e-10, atol=1e-13), (k, name)
+    if case in ("np413", "wide10"):
+        import subprocess
+        import sys
+        f = str(tmp_path / "seq.npz")
+        code = ("import sys, numpy as np; sys.path.insert(0, %r)\n"
+                "from ldsr_b200 import _lib; from tests.test_gpu_parity import _winner_case\n"
+                "w = _winner_case(sys.argv[2])\n"
+                "r = _lib.em_batch(w['series'], w['group_series'], w['held'], w['fit_group'], w['theta0'], 40, 1e-5)\n"
+                "np.savez(sys.argv[1], **r)\n") % ROOT
+        subprocess.run([sys.executable, "-c", code, f, case], check=True, env=dict(os.environ, LDSR_SEQ_TRAJ="1"),
+                       timeout=300)
+        seq = np.load(f)
+        assert np.array_equal(seq["theta"], g["theta"]) and np.array_equal(seq["best"], g["best"])
+        for name in ("X", "Y", "V", "J"):
+            assert np.allclose(seq[name], g[name], rtol=1e-10, atol=1e-13), name
 
 
 def test_lds_rep_chunked_pipeline_equals_the_single_kernel_path(tmp_path):
     """ldsr_rep_batch simulates every replicate in one kernel when the output fits HBM and in pipelined chunks
     otherwise; the device generator is keyed by (seed, replicate, step), so both give the same bits.  The
-    chunked path is forced through LDSR_REP_CHUNKED in a child process (the switch is read once)."""
+    chunked path is forced through LDSR_REP_CHUNKED in a child process (the switch is read once).
+    seed: n = 813, 9000 replicates (two chunks).  z, r_seed, three_chunks: n = 4000, 4000 replicates are chunks of
+    1664, 1664 and 672 replicates, so the third chunk re-uses the first one's slot; the noise comes from the caller,
+    from R's stream after set.seed, or from the device generator."""
     import subprocess
     import sys
     code = ("import sys, numpy as np; sys.path.insert(0, %r); from ldsr_b200 import _lib; from tests import data\n"
             "d = data.load('np.json'); th = data.theta_of(d['theta']); y, u, mu, inst = data.np_case(1, 1200)\n"
-            "r = _lib.rep_batch(th, u, u, y.size, 9000, seed=7, mu=mu)\n"
-            "np.save(sys.argv[1], np.stack([r['simX'], r['simY'], r['simQ']]))\n") % ROOT
-    outs = []
-    for k, env in enumerate(({}, {"LDSR_REP_CHUNKED": "1"})):
-        f = str(tmp_path / ("rep%d.npy" % k))
-        subprocess.run([sys.executable, "-c", code, f], check=True, env=dict(os.environ, **env), timeout=300)
-        outs.append(np.load(f))
-    assert np.isfinite(outs[0]).all() and np.array_equal(outs[0], outs[1])
+            "case = sys.argv[2]\n"
+            "if case == 'seed':\n"
+            "    r = _lib.rep_batch(th, u, u, y.size, 9000, seed=7, mu=mu)\n"
+            "else:\n"
+            "    n = 4000; rng = np.random.default_rng(40); u = rng.standard_normal((3, n))\n"
+            "    kw = dict(z=rng.standard_normal((n, 1 + 2 * n))) if case == 'z' else (\n"
+            "        dict(r_seed=11) if case == 'r_seed' else dict(seed=5))\n"
+            "    r = _lib.rep_batch(th, u, u, n, n, mu=mu, want=('simQ',), **kw)\n"
+            "np.save(sys.argv[1], np.stack([r[k] for k in ('simX', 'simY', 'simQ') if k in r]))\n") % ROOT
+    for case in ("seed", "z", "r_seed", "three_chunks"):
+        outs = []
+        for k, env in enumerate(({}, {"LDSR_REP_CHUNKED": "1"})):
+            f = str(tmp_path / ("rep_%s%d.npy" % (case, k)))
+            subprocess.run([sys.executable, "-c", code, f, case], check=True, env=dict(os.environ, **env), timeout=300)
+            outs.append(np.load(f))
+        assert np.isfinite(outs[0]).all() and np.array_equal(outs[0], outs[1]), case
 
 
 def test_construct_rec_kernel_reproduces_the_stored_reconstruction():

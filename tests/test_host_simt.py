@@ -1,5 +1,5 @@
-"""The EM kernels' SOURCE run on the CPU by a coroutine-per-thread emulator (tests/host_simt/): checks,
-without a GPU and without compute-sanitizer (closed on the GPU pool), that
+"""The EM kernels' and the single-step kernels' SOURCE run on the CPU by a coroutine-per-thread emulator
+(tests/host_simt/): checks, without a GPU and without compute-sanitizer (closed on the GPU pool), that
   * the kernels' control flow, shared-memory carve-up and cross-warp exchanges reproduce the oracle,
   * results are BIT-IDENTICAL under different orders of resuming the CTA's threads between
     synchronisation points -- a shared-memory race (two accesses to one word that no barrier orders)
@@ -265,3 +265,154 @@ def test_emulated_scan_kernel_trajectory_mode(case):
     b = sim_em_traj(y, u, v, held, fg, th0, 6, chunk=6, order=3, grid_cap=2)
     for k in ("X", "Y", "V", "J"):
         assert np.array_equal(a[k], b[k], equal_nan=True), k
+
+
+# ---- the single-step kernels (aux_kernels.cuh) -------------------------------------------------------------------
+# Case generators of tests/test_gpu_step_kernels.py; here one series per case, padded to width 3, 5 or 16 (steps per
+# smoother block 8, 4 and 1), with one group per hold-out kind and two theta per group.
+from tests import test_gpu_step_kernels as SK  # noqa: E402
+
+STEP_WIDTHS = [(3, 3, "vu"), (3, 2, "sep"), (1, 3, "unone"), (5, 5, "vu"), (4, 2, "sep"), (13, 13, "vu"),
+               (16, 9, "sep")]
+
+
+def _held_arrays(held):
+    hp = np.zeros(len(held) + 1, dtype=np.int32)
+    hp[1:] = np.cumsum([len(h) for h in held])
+    hi = np.ascontiguousarray(np.concatenate([np.asarray(h, dtype=np.int32) for h in held] + [np.zeros(1, np.int32)]))
+    return hp, hi
+
+
+def sim_step(kind, s, held, job_group, theta=None, job_theta=None, stdlik=True, rows=None, order=0):
+    """hostsim_step: kind 0 smoother, 1 propagate, 2 M-step (from rows X, V, J).  s: dict(y, u, v, p, q)."""
+    L = _lib()
+    y = np.ascontiguousarray(s["y"], dtype=np.float64)
+    T, p, q = y.size, s["p"], s["q"]
+    uf = None if s["u"] is None else np.ascontiguousarray(np.asarray(s["u"], dtype=np.float64).T)
+    vf = None if s["v"] is None else np.ascontiguousarray(np.asarray(s["v"], dtype=np.float64).T)
+    hp, hi = _held_arrays(held)
+    jg = np.ascontiguousarray(job_group, dtype=np.int32)
+    nj = jg.size
+    jt = np.ascontiguousarray(np.arange(nj) if job_theta is None else job_theta, dtype=np.int32)
+    th = None if theta is None else np.ascontiguousarray(theta, dtype=np.float64)
+    # one guard row past the last job's: a write beyond a job's T steps lands there (or in the next job's row)
+    X, Y, V, J = (np.full((nj + 1, T), 12345.0) for _ in range(4))
+    if rows is not None:
+        for k, a in (("X", X), ("V", V), ("J", J)):
+            a[:nj] = [r[k] for r in rows]
+    lik, aux = np.full(nj, 12345.0), np.full(nj, 12345.0)
+    th_out, st = np.full((nj, p + q + 6), np.nan), np.full(nj, -1, dtype=np.int32)
+    d = lambda a: None if a is None else a.ctypes.data_as(_dp)
+    i = lambda a: a.ctypes.data_as(_ip)
+    rc = L.hostsim_step(kind, T, p, q, d(y), d(uf), d(vf), len(held), i(hp), i(hi), nj, i(jg), i(jt), d(th),
+                        int(stdlik), order, d(X), d(Y), d(V), d(J), d(lik), d(aux), d(th_out), i(st))
+    assert rc == 0, rc
+    for k, a in (("X", X), ("Y", Y), ("V", V), ("J", J)):
+        assert np.all(a[nj] == 12345.0), "%s written past the last job's row" % k
+    return dict(X=X[:nj], Y=Y[:nj], V=V[:nj], J=J[:nj], lik=lik, aux=aux, theta=th_out, status=st)
+
+
+def _step_case(p, q, form, seed, T=150):
+    rng = np.random.default_rng(seed)
+    s = SK.make_series(rng, p, q, form, T)
+    held = [SK.holdout(rng, s["y"], k) for k in SK.HOLD_KINDS]
+    job_group = np.repeat(np.arange(len(held)), 2)
+    return s, held, job_group, np.stack([SK.rand_theta(rng, p, q) for _ in job_group])
+
+
+def _y_of(s, held, g):
+    y = np.array(s["y"], dtype=float)
+    y[held[g]] = np.nan
+    return y
+
+
+@pytest.mark.parametrize("width", STEP_WIDTHS, ids=SK.case_id)
+def test_emulated_smoother_and_propagate_match_the_oracle(width):
+    """smoother_kernel (incl. a job without theta: NaN rows) and propagate_kernel from their source, against the
+    oracle: rows, lik, and the per-job sums of the experimental learners' objectives."""
+    p, q, _ = width
+    s, held, jg, th = _step_case(*width, seed=100 * p + q)
+    jt = np.arange(jg.size)
+    jt[3] = -1
+    sm = sim_step(0, s, held, jg, th, job_theta=jt, stdlik=True)
+    pr = sim_step(1, s, held, jg, th, stdlik=False)
+    for j in range(jg.size):
+        y = _y_of(s, held, jg[j])
+        if jt[j] < 0:
+            assert all(np.isnan(sm[k][j]).all() for k in "XYVJ") and np.isnan(sm["lik"][j])
+            continue
+        o = O.kalman_smoother(y, s["u"], s["v"], th[j], p=p, q=q, stdlik=True)
+        for k in "XYVJ":
+            assert SK.row_dev(sm[k][j], o[k]) < SK.ROW_RTOL, (j, k, SK.row_dev(sm[k][j], o[k]))
+        assert SK.rel_dev(sm["lik"][j], o["lik"]) < SK.LIK_RTOL, j
+        Bu = th[j][1:1 + p] @ s["u"][:, :-1] if s["u"] is not None else 0.0
+        ssq = np.sum((o["X"][1:] - th[j][0] * o["X"][:-1] - Bu) ** 2)
+        assert SK.rel_dev(sm["aux"][j], ssq) < SK.LIK_RTOL, j
+        o = O.propagate(th[j], s["u"], s["v"], y, p=p, q=q, stdlik=False)
+        for k in "XYV":
+            assert SK.row_dev(pr[k][j], o[k]) < SK.ROW_RTOL, (j, k)
+        assert SK.rel_dev(pr["lik"][j], o["lik"]) < SK.LIK_RTOL, j
+        assert SK.rel_dev(pr["aux"][j], np.nansum((y - o["Y"]) ** 2)) < SK.LIK_RTOL, j
+
+
+@pytest.mark.parametrize("width", STEP_WIDTHS, ids=SK.case_id)
+def test_emulated_mstep_matches_the_oracle(width):
+    """mstep_kernel from its source on the oracle smoother's rows, for the groups with at least 3 max(p, q) observed
+    steps (well-conditioned Gram blocks)."""
+    p, q, _ = width
+    s, held, jg, th = _step_case(*width, seed=100 * p + q)
+    rows = [O.kalman_smoother(_y_of(s, held, jg[j]), s["u"], s["v"], th[j], p=p, q=q) for j in range(jg.size)]
+    r = sim_step(2, s, held, jg, rows=rows)
+    checked = 0
+    for j in range(jg.size):
+        y = _y_of(s, held, jg[j])
+        if np.isfinite(y).sum() < 3 * max(p, q):
+            continue
+        assert r["status"][j] == 0, j
+        o = O.mstep(y, s["u"], s["v"], rows[j], p=p, q=q)
+        d = np.max(np.abs(r["theta"][j] - o) / np.maximum(np.abs(o), SK.THETA_FLOOR))
+        assert d < SK.THETA_RTOL, (j, d)
+        checked += 1
+    assert checked >= 6
+
+
+REP_HOST_WIDTHS = [(3, 3, "vu"), (1, 3, "unone"), (3, 2, "vnone"), (5, 5, "vu"), (4, 2, "sep"), (16, 16, "vu"),
+                   (13, 9, "sep")]
+
+
+def sim_rep(p, q, u, v, n, z, theta, mu, exp_trans, want, order=0):
+    L = _lib()
+    n_reps = z.shape[0]
+    uf = None if u is None else np.ascontiguousarray(np.asarray(u, dtype=np.float64).T)
+    vf = None if v is None else np.ascontiguousarray(np.asarray(v, dtype=np.float64).T)
+    outs = {k: np.full((n_reps, n), 12345.0) for k in want}
+    d = lambda a: None if a is None else a.ctypes.data_as(_dp)
+    rc = L.hostsim_rep(p, q, d(uf), d(vf), n, n_reps, d(np.ascontiguousarray(z)), d(np.ascontiguousarray(theta)),
+                       C.c_double(mu), int(exp_trans), order, *(d(outs.get(k)) for k in ("simX", "simY", "simQ")))
+    assert rc == 0, rc
+    return outs
+
+
+@pytest.mark.parametrize("width", REP_HOST_WIDTHS, ids=SK.case_id)
+def test_emulated_rep_kernel_matches_the_oracle_and_is_schedule_independent(width):
+    """rep_kernel with caller noise from its source: oracle parity replicate by replicate, and bit-identical outputs
+    under several thread schedules -- its tile transposes are the one cross-lane shared-memory exchange among the
+    single-step kernels, ordered by __syncwarp.  n is not a multiple of the 16-step tile, n_reps not one of 32."""
+    p, q, form = width
+    rng = np.random.default_rng(p * 100 + q)
+    for n, n_reps, exp_trans, want in ((17, 33, True, ("simX", "simY", "simQ")), (40, 70, False, ("simQ",)),
+                                       (1, 5, True, ("simX", "simQ"))):
+        u = None if form == "unone" else rng.standard_normal((p, n))
+        v = None if form == "vnone" else (u if form == "vu" else rng.standard_normal((q, n)))
+        th = SK.rand_theta(rng, p, q)
+        mu = 0.37 if exp_trans else -1.3
+        z = rng.standard_normal((n_reps, 1 + 2 * n))
+        base = sim_rep(p, q, u, v, n, z, th, mu, exp_trans, want)
+        for i in range(n_reps):
+            o = O.rep(th, u, v, n, z[i], mu=mu, exp_trans=exp_trans, p=p, q=q)
+            for k in want:
+                assert SK.row_dev(base[k][i], o[k]) < SK.ROW_RTOL, (n, i, k)
+        for order in (1, 2, 3):
+            r = sim_rep(p, q, u, v, n, z, th, mu, exp_trans, want, order=order)
+            for k in want:
+                assert np.array_equal(r[k], base[k]), (n, order, k)
