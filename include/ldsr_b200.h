@@ -191,8 +191,31 @@ int ldsr_rep_batch_r(ldsr_ctx *ctx, const double *theta, const double *u, const 
                      int p, int q, int n_reps, unsigned int r_seed, double mu, int exp_trans,
                      double *simX, double *simY, double *simQ, char *errbuf, int errlen);
 
-/* Device time in ms (CUDA events around the kernels, summed) of the last ldsr_rep_batch / ldsr_rep_batch_r call
- * made by the calling thread: the measurement hook of bench.py's config-4 record. */
+/* Replicates conditioned on the observed record (beyond the reference): draws of whole trajectories from the
+ * smoothing distribution p(x_0..T-1 | y, theta) by forward filtering, backward sampling.  Unlike LDS_rep's
+ * open-loop replicates they pass through the observed flows, and their year-wise spread is the reconstruction's
+ * band.  Every fit's theta0 row is one model, conditioned on its group's y with the group's held-out steps
+ * removed; the filter is Kalman_smoother's (mu1, V1 the prior of x_0, u with one step of lag, v without,
+ * u == NULL drops B u and v == NULL drops D v).  Per replicate, for t = T-1 down to 0:
+ *     x_t = m_t + J_t x_{t+1} + s_t zeta_t     (J_t = Vu_t A / Vp_{t+1}, m_t = Xu_t - J_t Xp_{t+1},
+ *                                               s_t = sqrt(Vu_t Q / Vp_{t+1}); at t = T-1: J = 0, m = Xu, s = sqrt(Vu))
+ *     simX_t = x_t
+ *     simY_t = y_t (bit for bit) at observed steps, else C x_t + D v_t + sqrt(R) eps_t
+ *     simQ_t = back-transform(simY_t + mu): transform 0 none, 1 exp, 2 inverse Box-Cox (lambda; 0 means exp)
+ * simY is on the centred, transformed scale.  With zeta = eps = 0, simX is the smoother's X and simY its Y at
+ * unobserved steps.  Outputs follow the caller's fit order: with fit_ptr the exclusive prefix sum of T over the
+ * fits (ldsr_smoother_batch's rows), fit f's replicate r starts at n_reps*fit_ptr[f] + r*T_f; any output may be
+ * NULL.  z (optional) holds fit f's replicate r at 2*(n_reps*fit_ptr[f] + r*T_f): T_f state draws zeta_t, then
+ * T_f observation draws eps_t (present but unused at observed steps).  Without z the draws come from a
+ * counter-based generator keyed by (seed, fit index, replicate, step): a replicate's draws do not depend on
+ * n_reps or on the other fits.  mu [n_fits] may be NULL (0); lambda [n_fits] is read with transform 2 only.
+ * One device (ctx device 0); arguments are checked before a device is touched. */
+int ldsr_posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                             unsigned long long seed, const double *mu, int transform, const double *lambda,
+                             double *simX, double *simY, double *simQ, char *errbuf, int errlen);
+
+/* Device time in ms (CUDA events around the kernels, summed) of the last ldsr_rep_batch / ldsr_rep_batch_r /
+ * ldsr_posterior_rep_batch call made by the calling thread: the measurement hook of bench.py's config-4 record. */
 double ldsr_last_device_ms(void);
 
 /* ---- the reference's random numbers (R's default generators after set.seed) ---------------

@@ -22,7 +22,7 @@ EXPORTS = ("ldsr_abi_version", "ldsr_device_count", "ldsr_ctx_create", "ldsr_ctx
            "ldsr_smoother_d_batch", "ldsr_cv_metrics_batch", "ldsr_construct_rec_batch",
            "ldsr_objective_batch", "ldsr_rep_batch_r", "ldsr_r_rng_create", "ldsr_r_rng_unif", "ldsr_r_rng_norm",
            "ldsr_r_rng_sample", "ldsr_r_rng_destroy", "ldsr_r_rnorm_device", "ldsr_last_device_ms",
-           "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations")
+           "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations", "ldsr_posterior_rep_batch")
 
 
 class LdsrError(RuntimeError):
@@ -373,6 +373,38 @@ def rep_batch(theta, u, v, n, n_reps, z=None, seed=0, mu=0.0, exp_trans=True, p=
     _check(rc, err)
     res = {k: v for k, v in outs.items() if v is not None}
     res["device_ms"] = float(lib().ldsr_last_device_ms())  # CUDA-event time of the replicate kernels
+    return res
+
+
+def posterior_rep_batch(series, group_series, held, fit_group, theta, n_reps, z=None, seed=0, mu=None, transform="log",
+                        lams=None, want=("simX", "simY", "simQ"), ctx=None):
+    """ldsr_posterior_rep_batch: n_reps replicates of every fit conditioned on its group's y (forward filtering,
+    backward sampling).  Batch arguments as smoother_batch; theta [n_fits, stride] holds one model per fit.
+    z (optional): 2 * n_reps * sum(T) standard normals in the ABI's layout; mu, lams: per fit (lams with
+    transform="boxcox" only).  Returns, per requested output, a list over fits of [n_reps, T_f] arrays (views of
+    one replicate-major buffer), and the kernels' device time."""
+    pb = PackedBatch(series, group_series, held, fit_group, theta)
+    nf = pb.n_fits
+    tot = int(pb.fit_ptr[-1]) * int(n_reps)
+    zz = None
+    if z is not None:
+        zz = np.ascontiguousarray(z, dtype=np.float64).ravel()
+        if zz.size != 2 * tot:
+            raise ValueError("z must hold 2 * n_reps * sum(T) = %d values" % (2 * tot))
+    code = TRANSFORMS[transform] if isinstance(transform, str) else int(transform)
+    mu_a = None if mu is None else np.ascontiguousarray(np.broadcast_to(np.asarray(mu, dtype=np.float64), (nf,)))
+    lam_a = None if lams is None else np.ascontiguousarray(np.broadcast_to(np.asarray(lams, dtype=np.float64), (nf,)))
+    outs = {k: (np.empty(tot) if k in want else None) for k in ("simX", "simY", "simQ")}
+    err = C.create_string_buffer(512)
+    rc = lib().ldsr_posterior_rep_batch(ctx.h if isinstance(ctx, Ctx) else ctx, C.byref(pb.c), int(n_reps), _d(zz),
+                                        C.c_ulonglong(int(seed)), _d(mu_a), code, _d(lam_a), _d(outs["simX"]),
+                                        _d(outs["simY"]), _d(outs["simQ"]), err, 512)
+    _check(rc, err)
+    ptr = pb.fit_ptr * int(n_reps)
+    T = np.diff(pb.fit_ptr)
+    res = {k: [o[ptr[f]:ptr[f + 1]].reshape(int(n_reps), int(T[f])) for f in range(nf)]
+           for k, o in outs.items() if o is not None}
+    res["device_ms"] = float(lib().ldsr_last_device_ms())
     return res
 
 

@@ -518,6 +518,38 @@ def LDS_rep(theta, u=None, v=None, years=None, num_reps=100, mu=0.0, exp_trans=T
                 simQ=r["simQ"].ravel(), rep=np.repeat(np.arange(1, num_reps + 1), n))
 
 
+def LDS_rep_posterior(theta, Qa, u, v, start_year, transform="log", num_reps=100, seed=0, z=None):
+    """Replicates conditioned on the observed record (beyond the reference): whole trajectories drawn from the
+    smoothing distribution p(x | y, theta) of the model LDS_reconstruction fitted (forward filtering, backward
+    sampling).  Each replicate passes through the observed flows, and its year-wise spread is the reconstruction's
+    band, so path statistics (runs below a threshold, worst n-year means) can be read off them.
+    theta: the fitted model (LDS_reconstruction(...)["theta"]), or a list of them for an ensemble with u / v lists.
+    y, mu and lambda are prepared exactly as LDS_reconstruction prepares them.  Inputs follow Kalman_smoother:
+    u = None drops B u and v = None drops D v (unlike LDS_rep, where u = None drops both).
+    Noise: the device's counter-based generator keyed by (seed, member, replicate), or z: 2 * num_reps * sum(T)
+    standard normals, member by member and replicate by replicate, T state draws then T observation draws each.
+    Returns LDS_rep's long format (year, simX, simY, simQ, rep) over the station's horizon, one dict per member for
+    an ensemble.  simY is on the centred, transformed scale; simQ = back-transform(simY + mu).  One device call."""
+    S = _station(dict(Qa=Qa, u=u, v=v, start_year=start_year), transform)
+    thetas = [theta] if S["single"] else list(theta)
+    if len(thetas) != len(S["series"]):
+        raise ValueError("theta must be one model per ensemble member (%d)" % len(S["series"]))
+    rows = [theta_to_vec(t) for t in thetas]
+    stride = max(s["p"] + s["q"] + 6 for s in S["series"])
+    for s, r in zip(S["series"], rows):
+        if r.size != s["p"] + s["q"] + 6:
+            raise ValueError("theta has %d entries, the member's inputs need %d" % (r.size, s["p"] + s["q"] + 6))
+    n = len(rows)
+    r = _lib.posterior_rep_batch(S["series"], np.arange(n), None, np.arange(n),
+                                 np.stack([np.pad(v, (0, stride - v.size)) for v in rows]), num_reps, z=z, seed=seed,
+                                 mu=np.full(n, S["mu"]), transform=transform,
+                                 lams=None if transform != "boxcox" else np.full(n, S["lam"]))
+    years = S["years"]
+    out = [dict(year=np.tile(years, num_reps), simX=r["simX"][k].ravel(), simY=r["simY"][k].ravel(),
+                simQ=r["simQ"][k].ravel(), rep=np.repeat(np.arange(1, num_reps + 1), years.size)) for k in range(n)]
+    return out[0] if S["single"] else out
+
+
 def one_LDS_rep(rep_num, theta, u=None, v=None, years=None, mu=0.0, exp_trans=True, seed=0, z=None):
     """R/stochastics.R:18-47."""
     out = LDS_rep(theta, u, v, years, 1, mu, exp_trans, seed=seed + rep_num, z=None if z is None else z[None, :])

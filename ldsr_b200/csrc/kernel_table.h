@@ -74,6 +74,7 @@ struct KernelTable {
     // the same kernel's E-step once, writing the smoothed trajectories of EmParams.n_jobs (group, fit) pairs
     cudaError_t (*em_scan_traj)(const EmParams &, int steps_per_thread, cudaStream_t);
     cudaError_t (*smoother)(const SmootherParams &, cudaStream_t);
+    cudaError_t (*smoother_coef)(const SmootherParams &, cudaStream_t); // its backward-sampling coefficient mode
     cudaError_t (*mstep)(const MstepParams &, cudaStream_t);
     cudaError_t (*propagate)(const SmootherParams &, cudaStream_t);
     cudaError_t (*rep)(const RepParams &, cudaStream_t);

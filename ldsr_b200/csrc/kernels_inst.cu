@@ -226,6 +226,10 @@ cudaError_t smoother(const SmootherParams &p, cudaStream_t st) {
     smoother_kernel<PQ><<<(p.n_jobs + 63) / 64, 64, 0, st>>>(p);
     return cudaGetLastError();
 }
+cudaError_t smoother_coef(const SmootherParams &p, cudaStream_t st) {
+    smoother_kernel<PQ, true><<<(p.n_jobs + 63) / 64, 64, 0, st>>>(p);
+    return cudaGetLastError();
+}
 cudaError_t mstep(const MstepParams &p, cudaStream_t st) {
     mstep_kernel<PQ><<<(p.n_fits + 63) / 64, 64, 0, st>>>(p);
     return cudaGetLastError();
@@ -264,6 +268,7 @@ const KernelTable table = {PQ,
                            em_scan,
                            em_scan_traj,
                            smoother,
+                           smoother_coef,
                            mstep,
                            propagate,
                            rep};

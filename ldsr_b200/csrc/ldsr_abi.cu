@@ -15,6 +15,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <memory>
 #include <mutex>
 #include <numeric>
@@ -1425,7 +1426,8 @@ static Err em_batch(ldsr_ctx *ctx, const ldsr_batch *b, int niter, double tol, c
     return Err();
 }
 
-// device time (CUDA events) of the kernels of the last ldsr_rep_batch* call of this thread (ldsr_last_device_ms)
+// device time (CUDA events) of the replicate kernels of the last ldsr_rep_batch* / ldsr_posterior_rep_batch call of
+// this thread (ldsr_last_device_ms)
 static thread_local double g_last_device_ms = 0.0;
 
 // ---- single-step batched entry points (one device: ctx device 0) ----------------------------
@@ -1575,6 +1577,181 @@ static Err mstep_batch(ldsr_ctx *ctx, const ldsr_batch *b, const double *X, cons
     return Err();
 }
 
+// device blocks taken from a pool for the length of one call
+struct DevBlocks {
+    DevicePool *pool;
+    std::vector<void *> held;
+    template <class T> cudaError_t alloc(size_t bytes, T **out) {
+        void *p = nullptr;
+        cudaError_t e = pool->alloc(bytes, &p);
+        if (e == cudaSuccess) held.push_back(p);
+        *out = static_cast<T *>(p);
+        return e;
+    }
+    ~DevBlocks() {
+        for (void *p : held) pool->release(p);
+    }
+};
+
+// The output pipeline of the replicate entry points.  Up to three outputs (simX, simY, simQ; null ones are
+// skipped) of lo.back() doubles each live in the caller's (pageable) memory.  Chunk c covers elements
+// lo[c] .. lo[c+1]-1 of every output and elements zlo[c] .. zlo[c+1]-1 of the noise (caller noise z on the host,
+// or z_dev already on the device).  One pass: the kernel of chunk c+1 runs while chunk c crosses PCIe into a
+// pinned slot and chunk c-1 is copied from its slot into the caller's arrays by host threads.
+// `launch(c, z, out)` enqueues chunk c's kernel on sk (c = -1: one launch for every chunk), reading noise from z
+// (the chunk's first element on the device, or null) and writing output k from out[k] (the chunk's first
+// element).  Every producer the kernels depend on is on sk too; their device time goes to g_last_device_ms.
+struct RepOutputs {
+    double *outs[3];
+    std::vector<size_t> lo, zlo;
+    const double *z = nullptr, *z_dev = nullptr;
+};
+using RepLaunch = std::function<Err(int c, const double *zdev, double *const *out)>;
+
+static Err rep_pipeline(DevicePool *pool, cudaStream_t sk, const RepOutputs &R, const RepLaunch &launch) {
+    double *const *outs = R.outs;
+    int n_out = 0;
+    for (int o = 0; o < 3; o++) n_out += outs[o] ? 1 : 0;
+    g_last_device_ms = 0.0;
+    if (n_out == 0) return Err();
+    const int n_chunks = (int)R.lo.size() - 1;
+    size_t chunk = 0, zchunk = 0;
+    for (int c = 0; c < n_chunks; c++) {
+        chunk = std::max(chunk, R.lo[c + 1] - R.lo[c]);
+        if (R.z) zchunk = std::max(zchunk, R.zlo[c + 1] - R.zlo[c]);
+    }
+    const size_t tot = R.lo[n_chunks], ztot = R.z ? R.zlo[n_chunks] : 0;
+    // When the whole output fits comfortably in HBM (up to 8 GB here) ONE kernel simulates every replicate --
+    // 782 CTAs for 100 000 replicates instead of 58 per chunk, each warp's 813-step chain hidden behind the
+    // others -- and only the copies are chunked.  Otherwise kernel and copies are chunked alike.
+    // (LDSR_REP_CHUNKED=1, development / tests: take the chunked path whatever the size)
+    static const bool force_chunked = std::getenv("LDSR_REP_CHUNKED") != nullptr;
+    const bool whole = !force_chunked && ((size_t)n_out * tot + ztot) * 8 <= ((size_t)8 << 30);
+    const size_t slot_doubles = (size_t)n_out * chunk;
+    DevBlocks dev{pool, {}};
+    double *d_whole = nullptr;
+    constexpr int SLOTS = 2;
+    double *d_out[SLOTS] = {nullptr, nullptr}, *h_out[SLOTS] = {nullptr, nullptr}, *d_z[SLOTS] = {nullptr, nullptr};
+    cudaEvent_t ev_k[SLOTS] = {nullptr, nullptr}, ev_c[SLOTS] = {nullptr, nullptr};
+    std::vector<cudaEvent_t> ev_t;
+    cudaStream_t sc = nullptr;
+    struct Cleanup {
+        DevicePool *pool;
+        double **h;
+        cudaEvent_t *a, *b;
+        std::vector<cudaEvent_t> *t;
+        cudaStream_t sk, *sc;
+        ~Cleanup() {
+            cudaStreamSynchronize(sk);
+            if (*sc) cudaStreamSynchronize(*sc);
+            for (int i = 0; i < SLOTS; i++) {
+                if (h[i]) pool->release_pinned(h[i]);
+                if (a[i]) cudaEventDestroy(a[i]);
+                if (b[i]) cudaEventDestroy(b[i]);
+            }
+            for (cudaEvent_t e : *t) cudaEventDestroy(e);
+            if (*sc) pool->put_stream(*sc);
+        }
+    } cleanup{pool, h_out, ev_k, ev_c, &ev_t, sk, &sc};
+    CU(pool->get_stream(&sc));
+    for (int i = 0; i < SLOTS && i < n_chunks; i++) {
+        if (!whole) CU(dev.alloc(slot_doubles * 8, &d_out[i]));
+        void *hp = nullptr;
+        CU(pool->alloc_pinned(slot_doubles * 8, &hp));
+        h_out[i] = static_cast<double *>(hp);
+        if (R.z && !whole) CU(dev.alloc(zchunk * 8, &d_z[i]));
+        CU(cudaEventCreateWithFlags(&ev_k[i], cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&ev_c[i], cudaEventDisableTiming));
+    }
+    auto copy_out = [&](int c) { // pinned slot -> the caller's arrays, a few host threads
+        const int slot = c % SLOTS;
+        const size_t bytes = (R.lo[c + 1] - R.lo[c]) * 8;
+        std::vector<std::thread> th;
+        int k = 0;
+        for (int o = 0; o < 3; o++) {
+            if (!outs[o]) continue;
+            const char *src = reinterpret_cast<const char *>(h_out[slot] + (size_t)k * chunk);
+            char *dst = reinterpret_cast<char *>(outs[o] + R.lo[c]);
+            const int parts = bytes > ((size_t)4 << 20) ? 2 : 1;
+            for (int pi = 0; pi < parts; pi++) {
+                const size_t lo = bytes * pi / parts, hi = bytes * (pi + 1) / parts;
+                th.emplace_back([=] { std::memcpy(dst + lo, src + lo, hi - lo); });
+            }
+            k++;
+        }
+        for (auto &t : th) t.join();
+    };
+    auto timed_launch = [&](int c, const double *zdev, double *base, size_t out_stride) -> Err {
+        double *o3[3] = {nullptr, nullptr, nullptr};
+        int k = 0;
+        for (int o = 0; o < 3; o++)
+            if (outs[o]) o3[o] = base + (size_t)(k++) * out_stride;
+        cudaEvent_t ta = nullptr, tb = nullptr;
+        CU(cudaEventCreate(&ta));
+        ev_t.push_back(ta);
+        CU(cudaEventCreate(&tb));
+        ev_t.push_back(tb);
+        CU(cudaEventRecord(ta, sk));
+        Err e = launch(c, zdev, o3);
+        if (!e.ok()) return e;
+        CU(cudaEventRecord(tb, sk));
+        return Err();
+    };
+    if (whole) {
+        CU(dev.alloc((size_t)n_out * tot * 8, &d_whole));
+        const double *zdev = R.z_dev;
+        if (R.z) {
+            double *dzw = nullptr;
+            CU(dev.alloc(ztot * 8, &dzw));
+            CU(cudaMemcpyAsync(dzw, R.z, ztot * 8, cudaMemcpyHostToDevice, sk));
+            zdev = dzw;
+        }
+        Err e = timed_launch(-1, zdev, d_whole, tot);
+        if (!e.ok()) return e;
+        CU(cudaEventRecord(ev_k[0], sk));
+        CU(cudaStreamWaitEvent(sc, ev_k[0], 0));
+    }
+    for (int c = 0; c < n_chunks; c++) {
+        const int slot = c % SLOTS;
+        if (c >= SLOTS) { // the slot's previous chunk must have left the device, then leave the pinned block
+            CU(cudaEventSynchronize(ev_c[slot]));
+            copy_out(c - SLOTS);
+        }
+        if (whole) { // the kernel is done (or running ahead of the copy stream's wait): only the copies are chunked
+            for (int k = 0; k < n_out; k++)
+                CU(cudaMemcpyAsync(h_out[slot] + (size_t)k * chunk, d_whole + (size_t)k * tot + R.lo[c],
+                                   (R.lo[c + 1] - R.lo[c]) * 8, cudaMemcpyDeviceToHost, sc));
+            CU(cudaEventRecord(ev_c[slot], sc));
+            continue;
+        }
+        const double *zdev = nullptr;
+        if (R.z) {
+            CU(cudaMemcpyAsync(d_z[slot], R.z + R.zlo[c], (R.zlo[c + 1] - R.zlo[c]) * 8, cudaMemcpyHostToDevice, sk));
+            zdev = d_z[slot];
+        } else if (R.z_dev) {
+            zdev = R.z_dev + R.zlo[c];
+        }
+        Err e = timed_launch(c, zdev, d_out[slot], chunk);
+        if (!e.ok()) return e;
+        CU(cudaEventRecord(ev_k[slot], sk));
+        CU(cudaStreamWaitEvent(sc, ev_k[slot], 0));
+        CU(cudaMemcpyAsync(h_out[slot], d_out[slot], slot_doubles * 8, cudaMemcpyDeviceToHost, sc));
+        CU(cudaEventRecord(ev_c[slot], sc));
+        // (the next kernel into this slot is enqueued only after the host has seen ev_c[slot], above)
+    }
+    for (int c = std::max(0, n_chunks - SLOTS); c < n_chunks; c++) {
+        CU(cudaEventSynchronize(ev_c[c % SLOTS]));
+        copy_out(c);
+    }
+    CU(cudaStreamSynchronize(sk));
+    for (size_t i = 0; i + 1 < ev_t.size(); i += 2) {
+        float ms = 0.f;
+        CU(cudaEventElapsedTime(&ms, ev_t[i], ev_t[i + 1]));
+        g_last_device_ms += ms;
+    }
+    return Err();
+}
+
 static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const double *v, int n, int p, int q,
                      int n_reps, const double *z, unsigned long long seed, double mu, int exp_trans, double *simX,
                      double *simY, double *simQ, const unsigned *r_seed = nullptr) {
@@ -1603,107 +1780,42 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
         if (v)
             for (int j = 0; j < q; j++) vp[(size_t)t * PQ + j] = v[(size_t)t * q + j];
     }
-    std::vector<void *> held;
-    auto dal = [&](size_t bytes, void **pp) -> cudaError_t {
-        cudaError_t e = pool->alloc(bytes, pp);
-        if (e == cudaSuccess) held.push_back(*pp);
-        return e;
-    };
-    struct Rel {
+    DevBlocks dev{pool, {}};
+    struct Stream { // declared after dev: synchronised before the blocks go back to the pool
         DevicePool *pool;
-        std::vector<void *> *h;
-        ~Rel() {
-            for (void *p : *h) pool->release(p);
+        cudaStream_t s = nullptr;
+        ~Stream() {
+            if (s) {
+                cudaStreamSynchronize(s);
+                pool->put_stream(s);
+            }
         }
-    } rel{pool, &held};
+    } sk{pool};
+    CU(pool->get_stream(&sk.s));
     double *dth, *du, *dv, *dz_all = nullptr;
-    CU(dal(th.size() * 8, (void **)&dth));
-    CU(dal(up.size() * 8, (void **)&du));
-    CU(dal(vp.size() * 8, (void **)&dv));
-    CU(cudaMemcpy(dth, th.data(), th.size() * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(du, up.data(), up.size() * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(dv, vp.data(), vp.size() * 8, cudaMemcpyHostToDevice));
+    CU(dev.alloc(th.size() * 8, &dth));
+    CU(dev.alloc(up.size() * 8, &du));
+    CU(dev.alloc(vp.size() * 8, &dv));
+    CU(cudaMemcpyAsync(dth, th.data(), th.size() * 8, cudaMemcpyHostToDevice, sk.s));
+    CU(cudaMemcpyAsync(du, up.data(), up.size() * 8, cudaMemcpyHostToDevice, sk.s));
+    CU(cudaMemcpyAsync(dv, vp.data(), vp.size() * 8, cudaMemcpyHostToDevice, sk.s));
     const size_t zrow = 1 + 2 * (size_t)n;
     if (r_seed) { // the reference's own stream: set.seed(*r_seed); rnorm(...) in replicate order, made on the device
         const long long nz = (long long)n_reps * (long long)zrow;
-        CU(dal((size_t)nz * 8, (void **)&dz_all));
-        CU(r_rnorm_device(*r_seed, nz, dz_all, 0));
+        CU(dev.alloc((size_t)nz * 8, &dz_all));
+        CU(r_rnorm_device(*r_seed, nz, dz_all, sk.s));
     }
-    // One pass over the replicates in chunks: the kernel of chunk c+1 runs while chunk c crosses PCIe into a
-    // pinned slot and chunk c-1 is copied from its slot into the caller's (pageable) arrays by host threads.
-    double *outs[3] = {simX, simY, simQ};
-    int n_out = 0;
-    for (double *o : outs) n_out += o ? 1 : 0;
-    g_last_device_ms = 0.0;
-    if (n_out == 0) return Err();
     // ~48 MB per output and chunk, a multiple of a CTA's 128 replicates (at T = 813: 58 CTAs per launch)
     int chunk = (int)std::max<size_t>(128, ((size_t)48 << 20) / ((size_t)n * 8));
     chunk = std::min(n_reps, (chunk + 127) / 128 * 128);
-    const int n_chunks = (n_reps + chunk - 1) / chunk;
-    const size_t slot_doubles = (size_t)n_out * chunk * n;
-    // When the whole output fits comfortably in HBM (up to 8 GB here) ONE kernel simulates every replicate --
-    // 782 CTAs for 100 000 replicates instead of 58 per chunk, each warp's 813-step chain hidden behind the
-    // others -- and only the copies are chunked.  Otherwise kernel and copies are chunked alike.
-    const size_t tot = (size_t)n * n_reps;
-    // (LDSR_REP_CHUNKED=1, development / tests: take the chunked path whatever the size)
-    static const bool force_chunked = std::getenv("LDSR_REP_CHUNKED") != nullptr;
-    const bool whole =
-        !force_chunked && (size_t)n_out * tot * 8 + (z ? (size_t)n_reps * zrow * 8 : 0) <= ((size_t)8 << 30);
-    double *d_whole = nullptr;
-    constexpr int SLOTS = 2;
-    double *d_out[SLOTS] = {nullptr, nullptr}, *h_out[SLOTS] = {nullptr, nullptr}, *d_z[SLOTS] = {nullptr, nullptr};
-    cudaEvent_t ev_k[SLOTS] = {nullptr, nullptr}, ev_c[SLOTS] = {nullptr, nullptr};
-    std::vector<cudaEvent_t> ev_t;
-    cudaStream_t sk = nullptr, sc = nullptr;
-    struct Cleanup {
-        DevicePool *pool;
-        double **h;
-        cudaEvent_t *a, *b;
-        std::vector<cudaEvent_t> *t;
-        cudaStream_t *sk, *sc;
-        ~Cleanup() {
-            if (*sk) cudaStreamSynchronize(*sk);
-            if (*sc) cudaStreamSynchronize(*sc);
-            for (int i = 0; i < SLOTS; i++) {
-                if (h[i]) pool->release_pinned(h[i]);
-                if (a[i]) cudaEventDestroy(a[i]);
-                if (b[i]) cudaEventDestroy(b[i]);
-            }
-            for (cudaEvent_t e : *t) cudaEventDestroy(e);
-            if (*sk) pool->put_stream(*sk);
-            if (*sc) pool->put_stream(*sc);
-        }
-    } cleanup{pool, h_out, ev_k, ev_c, &ev_t, &sk, &sc};
-    CU(pool->get_stream(&sk));
-    CU(pool->get_stream(&sc));
-    for (int i = 0; i < SLOTS && i < n_chunks; i++) {
-        if (!whole) CU(dal(slot_doubles * 8, (void **)&d_out[i]));
-        void *hp = nullptr;
-        CU(pool->alloc_pinned(slot_doubles * 8, &hp));
-        h_out[i] = static_cast<double *>(hp);
-        if (z && !whole) CU(dal((size_t)chunk * zrow * 8, (void **)&d_z[i]));
-        CU(cudaEventCreateWithFlags(&ev_k[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&ev_c[i], cudaEventDisableTiming));
+    RepOutputs R{{simX, simY, simQ}, {}, {}, z, dz_all};
+    for (int r0 = 0;; r0 = std::min(n_reps, r0 + chunk)) {
+        R.lo.push_back((size_t)r0 * n);
+        R.zlo.push_back((size_t)r0 * zrow);
+        if (r0 == n_reps) break;
     }
-    auto copy_out = [&](int c) { // pinned slot -> the caller's arrays, a few host threads
-        const int slot = c % SLOTS, r0 = c * chunk, nr = std::min(chunk, n_reps - r0);
-        const size_t bytes = (size_t)nr * n * 8;
-        std::vector<std::thread> th;
-        int k = 0;
-        for (int o = 0; o < 3; o++) {
-            if (!outs[o]) continue;
-            const char *src = reinterpret_cast<const char *>(h_out[slot] + (size_t)k * chunk * n);
-            char *dst = reinterpret_cast<char *>(outs[o] + (size_t)r0 * n);
-            const int parts = bytes > ((size_t)4 << 20) ? 2 : 1;
-            for (int pi = 0; pi < parts; pi++) {
-                const size_t lo = bytes * pi / parts, hi = bytes * (pi + 1) / parts;
-                th.emplace_back([=] { std::memcpy(dst + lo, src + lo, hi - lo); });
-            }
-            k++;
-        }
-        for (auto &t : th) t.join();
-    };
-    auto launch = [&](int r0, int nr, const double *zdev, double *base, size_t out_stride) -> Err {
+    return rep_pipeline(pool, sk.s, R, [&](int c, const double *zdev, double *const *o3) -> Err {
+        const int r0 = c < 0 ? 0 : c * chunk;
         RepParams rp;
         rp.theta = dth;
         rp.u = du;
@@ -1711,102 +1823,156 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
         rp.z = zdev;
         rp.seed = seed;
         rp.n = n;
-        rp.n_reps = nr;
+        rp.n_reps = c < 0 ? n_reps : std::min(chunk, n_reps - r0);
         rp.rep0 = r0;
         rp.mu = mu;
         rp.exp_trans = exp_trans;
-        int k = 0;
-        double *o3[3] = {nullptr, nullptr, nullptr};
-        for (int o = 0; o < 3; o++)
-            if (outs[o]) o3[o] = base + (size_t)(k++) * out_stride;
         rp.simX = o3[0];
         rp.simY = o3[1];
         rp.simQ = o3[2];
-        cudaEvent_t ta = nullptr, tb = nullptr;
-        CU(cudaEventCreate(&ta));
-        ev_t.push_back(ta);
-        CU(cudaEventCreate(&tb));
-        ev_t.push_back(tb);
-        CU(cudaEventRecord(ta, sk));
-        CU(kt->rep(rp, sk));
-        CU(cudaEventRecord(tb, sk));
+        CU(kt->rep(rp, sk.s));
         return Err();
+    });
+}
+
+// ---- replicates conditioned on the observed record (forward filtering, backward sampling) -----
+static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
+                               unsigned long long seed, const double *mu, int transform, const double *lambda,
+                               double *simX, double *simY, double *simQ) {
+    Err e = validate(b);
+    if (!e.ok()) return e;
+    if (n_reps < 1) return fail(LDSR_ERR_ARG, "n_reps=%d, need n_reps >= 1", n_reps);
+    if (transform < 0 || transform > 2) return fail(LDSR_ERR_ARG, "transform=%d, need 0 (none), 1 (log) or 2 (Box-Cox)", transform);
+    if (transform == 2 && !lambda) return fail(LDSR_ERR_ARG, "transform 2 (Box-Cox) needs lambda");
+    const int nf = b->n_fits;
+    std::vector<long long> fit_ptr(nf + 1, 0);
+    for (int f = 0; f < nf; f++) fit_ptr[f + 1] = fit_ptr[f] + b->T[b->group_series[b->fit_group[f]]];
+    std::vector<double> par((size_t)4 * nf);
+    for (int f = 0; f < nf; f++) {
+        const int s = b->group_series[b->fit_group[f]];
+        const double *th = b->theta0 + (size_t)f * b->theta_stride;
+        const double R = th[3 + b->p[s] + b->q[s]];
+        if (!(R >= 0.0)) return fail(LDSR_ERR_ARG, "fit %d: R=%g, need R >= 0", f, R);
+        par[4 * f] = th[1 + b->p[s]];
+        par[4 * f + 1] = std::sqrt(R);
+        par[4 * f + 2] = mu ? mu[f] : 0.0;
+        par[4 * f + 3] = transform == 2 ? lambda[f] : 0.0;
+    }
+    std::unique_ptr<ldsr_ctx> tmp_ctx;
+    if (!ctx) {
+        ldsr_ctx *c = nullptr;
+        char buf[256];
+        int rc = ldsr_ctx_create(1, nullptr, &c, buf, sizeof buf);
+        if (rc != LDSR_OK) return fail(rc, "%s", buf);
+        tmp_ctx.reset(c);
+        ctx = c;
+    }
+    ldsr_plan *P = nullptr;
+    if (!(e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P)).ok()) return e;
+    std::unique_ptr<ldsr_plan> guard(P);
+    // per fit: its coefficient rows (user order, as ldsr_smoother_batch) and its group's first mask word
+    std::vector<long long> jr(nf), f_mask_off(nf), g_mask_off(P->n_groups);
+    std::vector<int> jt(nf);
+    for (int gi = 0, w = 0; gi < P->n_groups; gi++) {
+        g_mask_off[gi] = w;
+        w += (P->s_T[P->h_g_series[gi]] + 31) / 32;
+    }
+    for (int fi = 0; fi < nf; fi++) {
+        jr[fi] = fit_ptr[P->f_user[fi]];
+        jt[fi] = fi;
+        f_mask_off[P->f_user[fi]] = g_mask_off[P->h_f_group[fi]];
+    }
+    const size_t tot = (size_t)fit_ptr[nf];
+    double *dm, *dO, *ds, *dJ, *d_par;
+    int *d_jt;
+    long long *d_jr, *d_fit_ptr, *d_fmo;
+    if (!(e = P->dalloc(&dm, tot)).ok()) return e;
+    if (!(e = P->dalloc(&dO, tot)).ok()) return e;
+    if (!(e = P->dalloc(&ds, tot)).ok()) return e;
+    if (!(e = P->dalloc(&dJ, tot)).ok()) return e;
+    if (!(e = P->upload(&d_jt, jt)).ok()) return e;
+    if (!(e = P->upload(&d_jr, jr)).ok()) return e;
+    if (!(e = P->upload(&d_fit_ptr, fit_ptr)).ok()) return e;
+    if (!(e = P->upload(&d_fmo, f_mask_off)).ok()) return e;
+    if (!(e = P->upload(&d_par, par)).ok()) return e;
+    SmootherParams sp = {};
+    sp.series = P->d_series;
+    sp.blobs = P->d_blobs;
+    sp.g_series = P->d_g_series;
+    sp.masks = P->d_masks;
+    sp.g_mask_off = P->d_g_mask_off;
+    sp.g_nobs = P->d_g_nobs;
+    sp.n_jobs = nf;
+    sp.job_group = P->d_f_group;
+    sp.job_theta = d_jt;
+    sp.job_row = d_jr;
+    sp.theta = P->d_theta0;
+    sp.X = dm;
+    sp.Y = dO;
+    sp.V = ds;
+    sp.J = dJ;
+    struct Events {
+        cudaEvent_t a = nullptr, b = nullptr;
+        ~Events() {
+            if (a) cudaEventDestroy(a);
+            if (b) cudaEventDestroy(b);
+        }
+    } ev;
+    CU(cudaEventCreate(&ev.a));
+    CU(cudaEventCreate(&ev.b));
+    CU(cudaEventRecord(ev.a, P->stream));
+    CU(P->kt->smoother_coef(sp, P->stream));
+    CU(cudaEventRecord(ev.b, P->stream));
+    // warps: (fit, 32 replicates) blocks in output order; a chunk is a range of whole blocks (~48 MB per output)
+    const int wpf = (n_reps + 31) / 32;
+    const long long n_blk = (long long)nf * wpf;
+    auto blk_end = [&](long long k) { // output offset just past block k
+        const int f = (int)(k / wpf), r1 = std::min(n_reps, (int)(k % wpf) * 32 + 32);
+        return (size_t)n_reps * fit_ptr[f] + (size_t)r1 * (fit_ptr[f + 1] - fit_ptr[f]);
     };
-    if (whole) {
-        CU(dal((size_t)n_out * tot * 8, (void **)&d_whole));
-        const double *zdev = dz_all;
-        if (z) {
-            double *dzw = nullptr;
-            CU(dal((size_t)n_reps * zrow * 8, (void **)&dzw));
-            CU(cudaMemcpyAsync(dzw, z, (size_t)n_reps * zrow * 8, cudaMemcpyHostToDevice, sk));
-            zdev = dzw;
+    const size_t chunk_target = ((size_t)48 << 20) / 8;
+    std::vector<long long> cb{0};
+    RepOutputs R{{simX, simY, simQ}, {0}, {0}, z, nullptr};
+    for (long long k = 0; k < n_blk; k++)
+        if (k == n_blk - 1 || blk_end(k) - R.lo.back() >= chunk_target) {
+            cb.push_back(k + 1);
+            R.lo.push_back(blk_end(k));
+            R.zlo.push_back(2 * blk_end(k));
         }
-        Err e = launch(0, n_reps, zdev, d_whole, tot);
-        if (!e.ok()) return e;
-        CU(cudaEventRecord(ev_k[0], sk));
-        CU(cudaStreamWaitEvent(sc, ev_k[0], 0));
-    }
-    for (int c = 0; c < n_chunks; c++) {
-        const int slot = c % SLOTS, r0 = c * chunk, nr = std::min(chunk, n_reps - r0);
-        if (c >= SLOTS) { // the slot's previous chunk must have left the device, then leave the pinned block
-            CU(cudaEventSynchronize(ev_c[slot]));
-            copy_out(c - SLOTS);
-        }
-        if (whole) { // the kernel is done (or running ahead of the copy stream's wait): only the copies are chunked
-            for (int k = 0; k < n_out; k++)
-                CU(cudaMemcpyAsync(h_out[slot] + (size_t)k * chunk * n, d_whole + (size_t)k * tot + (size_t)r0 * n,
-                                   (size_t)nr * n * 8, cudaMemcpyDeviceToHost, sc));
-            CU(cudaEventRecord(ev_c[slot], sc));
-            continue;
-        }
-        RepParams rp;
-        rp.theta = dth;
-        rp.u = du;
-        rp.v = dv;
-        rp.z = nullptr;
-        if (z) {
-            CU(cudaMemcpyAsync(d_z[slot], z + (size_t)r0 * zrow, (size_t)nr * zrow * 8, cudaMemcpyHostToDevice, sk));
-            rp.z = d_z[slot];
-        } else if (dz_all) {
-            rp.z = dz_all + (size_t)r0 * zrow;
-        }
-        rp.seed = seed;
-        rp.n = n;
-        rp.n_reps = nr;
-        rp.rep0 = r0;
-        rp.mu = mu;
-        rp.exp_trans = exp_trans;
-        int k = 0;
-        double *slot_out[3] = {nullptr, nullptr, nullptr};
-        for (int o = 0; o < 3; o++)
-            if (outs[o]) slot_out[o] = d_out[slot] + (size_t)(k++) * chunk * n;
-        rp.simX = slot_out[0];
-        rp.simY = slot_out[1];
-        rp.simQ = slot_out[2];
-        cudaEvent_t ta = nullptr, tb = nullptr;
-        CU(cudaEventCreate(&ta));
-        ev_t.push_back(ta);
-        CU(cudaEventCreate(&tb));
-        ev_t.push_back(tb);
-        CU(cudaEventRecord(ta, sk));
-        CU(kt->rep(rp, sk));
-        CU(cudaEventRecord(tb, sk));
-        CU(cudaEventRecord(ev_k[slot], sk));
-        CU(cudaStreamWaitEvent(sc, ev_k[slot], 0));
-        CU(cudaMemcpyAsync(h_out[slot], d_out[slot], slot_doubles * 8, cudaMemcpyDeviceToHost, sc));
-        CU(cudaEventRecord(ev_c[slot], sc));
-        // (the next kernel into this slot is enqueued only after the host has seen ev_c[slot], above)
-    }
-    for (int c = std::max(0, n_chunks - SLOTS); c < n_chunks; c++) {
-        CU(cudaEventSynchronize(ev_c[c % SLOTS]));
-        copy_out(c);
-    }
-    CU(cudaStreamSynchronize(sk));
-    for (size_t i = 0; i + 1 < ev_t.size(); i += 2) {
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, ev_t[i], ev_t[i + 1]));
-        g_last_device_ms += ms;
-    }
+    e = rep_pipeline(P->pool, P->stream, R, [&](int c, const double *zdev, double *const *o3) -> Err {
+        PostRepParams pp;
+        pp.m = dm;
+        pp.o = dO;
+        pp.s = ds;
+        pp.J = dJ;
+        pp.fit_ptr = d_fit_ptr;
+        pp.par = d_par;
+        pp.masks = P->d_masks;
+        pp.f_mask_off = d_fmo;
+        pp.z = zdev;
+        pp.seed = seed;
+        pp.n_reps = n_reps;
+        pp.wpf = wpf;
+        pp.blk0 = c < 0 ? 0 : cb[c];
+        pp.n_blk = c < 0 ? n_blk : cb[c + 1] - cb[c];
+        pp.out0 = c < 0 ? 0 : (long long)R.lo[c];
+        pp.transform = transform;
+        pp.simX = o3[0];
+        pp.simY = o3[1];
+        pp.simQ = o3[2];
+        const size_t smem = posterior_smem_bytes<REP_TT>(zdev != nullptr);
+        CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)posterior_smem_bytes<REP_TT>(true)));
+        const int per_cta = REP_WARPS;
+        posterior_rep_kernel<REP_TT><<<(unsigned)((pp.n_blk + per_cta - 1) / per_cta), REP_WARPS * 32, smem, P->stream>>>(pp);
+        CU(cudaGetLastError());
+        return Err();
+    });
+    if (!e.ok()) return e;
+    float ms = 0.f; // the coefficient pass counts as device time too
+    CU(cudaEventSynchronize(ev.b));
+    CU(cudaEventElapsedTime(&ms, ev.a, ev.b));
+    g_last_device_ms += ms;
     return Err();
 }
 
@@ -1924,6 +2090,13 @@ int ldsr_rep_batch_r(ldsr_ctx *ctx, const double *theta, const double *u, const 
                      double *simQ, char *errbuf, int errlen) {
     return report(rep_batch(ctx, theta, u, v, n, p, q, n_reps, nullptr, 0ull, mu, exp_trans, simX, simY, simQ, &r_seed),
                   errbuf, errlen);
+}
+
+int ldsr_posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                             unsigned long long seed, const double *mu, int transform, const double *lambda,
+                             double *simX, double *simY, double *simQ, char *errbuf, int errlen) {
+    return report(posterior_rep_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, simX, simY, simQ), errbuf,
+                  errlen);
 }
 
 struct ldsr_r_rng {

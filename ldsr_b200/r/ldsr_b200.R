@@ -270,6 +270,39 @@ LDS_rep <- function(theta, u = NULL, v = NULL, years, num.reps = 100, mu = 0, ex
 }
 
 
+# Replicates conditioned on the observed record (beyond ldsr): whole trajectories drawn from the smoothing
+# distribution p(x | y, theta) of the model LDS_reconstruction fitted, by forward filtering, backward sampling.
+# They pass through the observed flows and their year-wise spread is the reconstruction's band.  theta: the
+# fitted model, or a list of them for an ensemble (u / v lists).  y, mu and lambda are prepared as
+# LDS_reconstruction prepares them (.station_setup); u = NULL drops B u and v = NULL drops D v (Kalman_smoother's
+# convention, unlike LDS_rep).  exact.rng = TRUE: the noise is rnorm() in the documented order -- member by member,
+# replicate by replicate, N state draws then N observation draws -- so set.seed() reproduces the replicates;
+# exact.rng = FALSE uses the device's counter-based generator keyed by (seed, member, replicate).  Returns
+# LDS_rep's data.table (year, simX, simY, simQ, rep), a list of them for an ensemble; simY is centred and
+# transformed, simQ its back-transform.
+LDS_rep_posterior <- function(theta, Qa, u, v, start.year, transform = 'log', num.reps = 100, exact.rng = TRUE,
+                              seed = 0) {
+  P <- .station_setup(list(Qa = Qa, u = u, v = v, start.year = start.year), transform)
+  thetas <- if (P$single) list(theta) else theta
+  if (length(thetas) != length(P$u)) stop('theta must be one model per ensemble member')
+  series <- lapply(seq_along(P$u), function(k) list(y = P$y, u = P$u[[k]], v = P$v[[k]]))
+  cols <- lapply(thetas, function(th) c(th$A, th$B, th$C, th$D, th$Q, th$R, th$mu1, th$V1))
+  stride <- max(lengths(cols))
+  th <- sapply(cols, function(x) c(x, rep(0, stride - length(x))))
+  n <- length(P$years); nm <- length(series)
+  z <- if (exact.rng) stats::rnorm(2 * num.reps * n * nm) else NULL
+  code <- switch(transform, none = 0L, log = 1L, boxcox = 2L)
+  m <- .Call('_ldsr_posterior_rep_batch', series, matrix(th, nrow = stride), as.integer(num.reps), z,
+             as.numeric(seed), rep(P$mu, nm), code, if (transform == 'boxcox') rep(P$lambda, nm) else NULL,
+             PACKAGE = 'ldsr')
+  out <- lapply(seq_len(nm), function(k) {
+    r <- (k - 1) * num.reps * n + seq_len(num.reps * n)
+    data.table::data.table(year = rep(P$years, num.reps), simX = m[r, 1], simY = m[r, 2], simQ = m[r, 3],
+                           rep = rep(seq_len(num.reps), each = n))
+  })
+  if (P$single) out[[1]] else out
+}
+
 #' Kalman / RTS smoother for a state of dimension d > 1 (beyond ldsr, whose state is scalar).
 #' theta: list(A d x d, B d x p, C 1 x d, D 1 x q, Q d x d, R, mu1 d x 1, V1 d x d); y 1 x T with NA.
 #' method: 1 = associative scan over time (long series), 0 = sequential recursion.

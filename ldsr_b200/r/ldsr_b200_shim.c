@@ -14,6 +14,7 @@
  * and add the batched ones used by the drop-in R wrappers in ldsr_b200.R:
  *     _ldsr_em_batch(series,group_series,held,fit_group,theta0,niter,tol,n_devices)   8
  *     _ldsr_rep_batch(theta,u,v,n,num_reps,seed,mu,exp_trans,z,r_seed)               10
+ *     _ldsr_posterior_rep_batch(series,thetas,num_reps,z,seed,mu,transform,lambda)   8
  *     _ldsr_cv_metrics(Ycv,target,Z,exp_trans)                                        4
  *     _ldsr_construct_rec(X,V,Y,C,R,mu,transform,lambda)                              8
  *     _ldsr_cv_metrics_stations(Ycv,target,Z,exp_trans)   lists, one element per station    4
@@ -303,6 +304,48 @@ SEXP _ldsr_rep_batch(SEXP theta, SEXP u, SEXP v, SEXP nS, SEXP repsS, SEXP seedS
     return out;
 }
 
+/* Replicates conditioned on the observed record (LDS_rep_posterior in ldsr_b200.R): series is a list of
+ * list(y, u, v), one per ensemble member, each its own group and fit; thetas a stride x n matrix (one column per
+ * member, the flat order of R/LDS_GA.R:6-16); mu and lambda per member (lambda NULL unless transform = 2).
+ * Returns a 3-column matrix (simX, simY, simQ): member by member, replicate by replicate, T rows each. */
+SEXP _ldsr_posterior_rep_batch(SEXP series, SEXP thetas, SEXP repsS, SEXP zS, SEXP seedS, SEXP muS, SEXP transformS,
+                               SEXP lambdaS) {
+    const int ns = (int)XLENGTH(series), reps = Rf_asInteger(repsS);
+    int *T = (int *)R_alloc(ns, sizeof(int)), *p = (int *)R_alloc(ns, sizeof(int)), *q = (int *)R_alloc(ns, sizeof(int));
+    int *idx = (int *)R_alloc(ns, sizeof(int));
+    const double **y = (const double **)R_alloc(ns, sizeof(double *));
+    const double **u = (const double **)R_alloc(ns, sizeof(double *));
+    const double **v = (const double **)R_alloc(ns, sizeof(double *));
+    R_xlen_t tot = 0;
+    for (int s = 0; s < ns; s++) {
+        SEXP e = VECTOR_ELT(series, s);
+        T[s] = Rf_ncols(list_get(e, "y"));
+        y[s] = REAL(list_get(e, "y"));
+        u[s] = input_ptr(list_get(e, "u"), T[s], &p[s]);
+        v[s] = input_ptr(list_get(e, "v"), T[s], &q[s]);
+        idx[s] = s;
+        tot += (R_xlen_t)reps * T[s];
+    }
+    if (Rf_ncols(thetas) != ns) Rf_error("ldsr: thetas must have one column per series");
+    if (XLENGTH(muS) != ns) Rf_error("ldsr: mu must have one value per series");
+    const double *z = Rf_isNull(zS) ? NULL : REAL(zS);
+    if (z && XLENGTH(zS) != 2 * tot) Rf_error("ldsr: z must hold 2 * num.reps * sum(T) draws");
+    const double *lam = Rf_isNull(lambdaS) ? NULL : REAL(lambdaS);
+    if (lam && XLENGTH(lambdaS) != ns) Rf_error("ldsr: lambda must have one value per series");
+    ldsr_batch b; memset(&b, 0, sizeof b);
+    b.n_series = ns; b.T = T; b.p = p; b.q = q; b.y = y; b.u = u; b.v = v;
+    b.n_groups = ns; b.group_series = idx;
+    b.n_fits = ns; b.fit_group = idx; b.theta0 = REAL(thetas); b.theta_stride = Rf_nrows(thetas);
+    SEXP out = PROTECT(Rf_allocMatrix(REALSXP, tot, 3));
+    double *o = REAL(out);
+    char err[512] = "";
+    check(ldsr_posterior_rep_batch(ctx(), &b, reps, z, (unsigned long long)Rf_asReal(seedS), REAL(muS),
+                                   Rf_asInteger(transformS), lam, o, o + tot, o + 2 * tot, err, sizeof err),
+          err);
+    UNPROTECT(1);
+    return out;
+}
+
 /* same shape as src/RcppExports.cpp:132-148 */
 /* mapply(calculate_metrics, sim = Ycv, z = Z, MoreArgs = list(obs = target)) in one call
  * (R/LDS_reconstruction.R:395): Ycv is an n x n_folds matrix, Z a list of integer vectors. */
@@ -533,6 +576,7 @@ static const R_CallMethodDef CallEntries[] = {
     {"_ldsr_propagate", (DL_FUNC)&_ldsr_propagate, 5},
     {"_ldsr_em_batch", (DL_FUNC)&_ldsr_em_batch, 8},
     {"_ldsr_rep_batch", (DL_FUNC)&_ldsr_rep_batch, 10},
+    {"_ldsr_posterior_rep_batch", (DL_FUNC)&_ldsr_posterior_rep_batch, 8},
     {"_ldsr_smoother_d", (DL_FUNC)&_ldsr_smoother_d, 6},
     {"_ldsr_cv_metrics", (DL_FUNC)&_ldsr_cv_metrics, 4},
     {"_ldsr_construct_rec", (DL_FUNC)&_ldsr_construct_rec, 8},
