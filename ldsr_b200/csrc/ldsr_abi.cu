@@ -192,6 +192,132 @@ class DevicePool {
     std::vector<cudaStream_t> streams_;
 };
 
+// ---- the CUDA resources of one call (or of one plan), given back when it goes out of scope -----
+// With a pool, device and pinned blocks (and, after borrow_stream, the stream) come from it, and the owner waits for
+// its stream before they go back.  Without one (the entry points that take a device number) device blocks are
+// cudaMalloc'd and the work runs on the legacy stream, which cudaFree waits for.  Events die with the owner.
+class Resources {
+  public:
+    explicit Resources(DevicePool *pool = nullptr, cudaStream_t stream = nullptr) : stream(stream), pool_(pool) {}
+    Resources(const Resources &) = delete;
+    Resources &operator=(const Resources &) = delete;
+    ~Resources() {
+        if (pool_ && stream) cudaStreamSynchronize(stream);
+        for (cudaEvent_t e : events_) cudaEventDestroy(e);
+        for (void *p : pinned_) pool_->release_pinned(p);
+        for (void *p : blocks_) free_block(p);
+        if (own_stream_) pool_->put_stream(stream);
+    }
+    cudaStream_t stream; // where the work of the call is enqueued
+    DevicePool *pool() const { return pool_; }
+
+    cudaError_t borrow_stream() {
+        cudaError_t e = pool_->get_stream(&stream);
+        own_stream_ = e == cudaSuccess;
+        return e;
+    }
+    template <class T> cudaError_t alloc(T **out, size_t n) {
+        const size_t bytes = std::max<size_t>(n, 1) * sizeof(T);
+        void *p = nullptr;
+        cudaError_t e = pool_ ? pool_->alloc(bytes, &p) : cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) return e;
+        blocks_.push_back(p);
+        *out = static_cast<T *>(p);
+        return cudaSuccess;
+    }
+    // grow a block: the old one goes back at once (a plan re-used with a larger niter or with trace_liks must not
+    // accumulate dead blocks until it is destroyed)
+    template <class T> cudaError_t realloc(T **ptr, size_t n) {
+        if (*ptr) {
+            forget(blocks_, *ptr);
+            free_block(*ptr);
+            *ptr = nullptr;
+        }
+        return alloc(ptr, n);
+    }
+    template <class T> cudaError_t upload(T **out, const std::vector<T> &h) {
+        cudaError_t e = alloc(out, h.size());
+        if (e != cudaSuccess || h.empty()) return e;
+        return cudaMemcpyAsync(*out, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, stream);
+    }
+    template <class T> cudaError_t alloc_pinned(T **out, size_t n) {
+        void *p = nullptr;
+        cudaError_t e = pool_->alloc_pinned(n * sizeof(T), &p);
+        if (e != cudaSuccess) return e;
+        pinned_.push_back(p);
+        *out = static_cast<T *>(p);
+        return cudaSuccess;
+    }
+    template <class T> cudaError_t realloc_pinned(T **ptr, size_t n) {
+        if (*ptr) {
+            forget(pinned_, *ptr);
+            pool_->release_pinned(*ptr);
+            *ptr = nullptr;
+        }
+        return alloc_pinned(ptr, n);
+    }
+    cudaError_t event(cudaEvent_t *out, unsigned flags = cudaEventDefault) {
+        cudaError_t e = cudaEventCreateWithFlags(out, flags);
+        if (e == cudaSuccess) events_.push_back(*out);
+        return e;
+    }
+
+    // Device time of enqueued work: start() and stop() record a pair of events on the stream around it.
+    cudaError_t start() {
+        cudaEvent_t a = nullptr, b = nullptr;
+        cudaError_t e = event(&a);
+        if (e == cudaSuccess) e = event(&b);
+        if (e != cudaSuccess) return e;
+        laps_.push_back({a, b});
+        return cudaEventRecord(a, stream);
+    }
+    cudaError_t stop() { return cudaEventRecord(laps_.back().second, stream); }
+    size_t laps() const { return laps_.size(); }
+    // from the start of pair `first` to the stop of pair `last`, once the device has reached that stop
+    cudaError_t ms(size_t first, size_t last, float *out) const {
+        cudaError_t e = cudaEventSynchronize(laps_[last].second);
+        return e != cudaSuccess ? e : cudaEventElapsedTime(out, laps_[first].first, laps_[last].second);
+    }
+    cudaError_t total_ms(double *out) const {
+        *out = 0.0;
+        for (size_t i = 0; i < laps_.size(); i++) {
+            float m = 0.f;
+            cudaError_t e = ms(i, i, &m);
+            if (e != cudaSuccess) return e;
+            *out += m;
+        }
+        return cudaSuccess;
+    }
+
+  private:
+    static void forget(std::vector<void *> &v, void *p) { v.erase(std::remove(v.begin(), v.end(), p), v.end()); }
+    void free_block(void *p) {
+        if (pool_)
+            pool_->release(p);
+        else
+            cudaFree(p);
+    }
+    DevicePool *pool_;
+    bool own_stream_ = false;
+    std::vector<void *> blocks_, pinned_;
+    std::vector<cudaEvent_t> events_;
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> laps_;
+};
+
+// Every entry point finds its device here, after validating its arguments: the library has no CPU path.
+static Err check_device(int device) {
+    const int have = ldsr_device_count();
+    if (have < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
+    if (device < 0 || device >= have) return fail(LDSR_ERR_ARG, "device %d out of range (have %d)", device, have);
+    return Err();
+}
+static Err use_device(int device) {
+    Err e = check_device(device);
+    if (!e.ok()) return e;
+    CU(cudaSetDevice(device));
+    return Err();
+}
+
 } // namespace ldsr
 
 using namespace ldsr;
@@ -212,11 +338,13 @@ constexpr int SCAN_MAX_FITS = 1500;
 inline int scan_auto_fits(int pq) { return pq <= 4 ? 1200 : 900; }
 constexpr size_t COUNTS_CAP = 256; // (tasks, live fits) per chunk: room for 128 chunks without regrowing
 struct ldsr_plan {
+    ldsr_plan(int device, DevicePool *pool)
+        : device(device), own_pool(pool ? nullptr : new DevicePool(device)), cuda(pool ? pool : own_pool.get()) {}
+    ~ldsr_plan() { cudaSetDevice(device); } // then `cuda` waits for the plan's stream and gives everything back
     int device = 0;
     int n_sm = 148;
-    DevicePool *pool = nullptr;
     std::unique_ptr<DevicePool> own_pool;
-    cudaStream_t stream = nullptr;
+    Resources cuda; // the plan's stream, its device blocks and pinned blocks
     const KernelTable *kt = nullptr;
     int PQ = 0, TL = 0;
     int n_series = 0, n_groups = 0, n_fits = 0, theta_stride = 0;
@@ -233,7 +361,11 @@ struct ldsr_plan {
     std::vector<int> user_fit_series; // per USER fit: its series (filled only when the rows differ in width)
     std::vector<long long> h_traj_ptr_user; // per USER group: offset of its trajectory row
     long long traj_total = 0;
-    std::vector<void *> allocs;
+    std::vector<long long> h_g_mask_off; // per group: its first mask word
+    // one job per fit with its rows in the caller's fit order (ldsr_smoother_batch's layout): per USER fit the
+    // offset of its rows, and per fit the job's row offset and theta row
+    std::vector<long long> fit_row_user, fit_job_row;
+    std::vector<int> fit_job_theta;
     // device
     SeriesDev *d_series = nullptr;
     double *d_blobs = nullptr, *d_sconst = nullptr, *d_gconst = nullptr, *d_uwin = nullptr;
@@ -271,40 +403,6 @@ struct ldsr_plan {
     long long *d_job_row = nullptr;
     int *h_counts = nullptr; // pinned
     bool em_done = false;
-
-    template <class T> Err dalloc(T **out, size_t n) {
-        void *p = nullptr;
-        cudaError_t e = pool->alloc(std::max<size_t>(n, 1) * sizeof(T), &p);
-        if (e != cudaSuccess) return fail(LDSR_ERR_CUDA, "device allocation of %zu bytes failed: %s", n * sizeof(T),
-                                          cudaGetErrorString(e));
-        allocs.push_back(p);
-        *out = static_cast<T *>(p);
-        return Err();
-    }
-    // grow a block: the old one goes back to the pool at once (a plan re-used with a larger niter or
-    // with trace_liks must not accumulate dead blocks until it is destroyed)
-    template <class T> Err drealloc(T **ptr, size_t n) {
-        if (*ptr) {
-            allocs.erase(std::remove(allocs.begin(), allocs.end(), static_cast<void *>(*ptr)), allocs.end());
-            pool->release(*ptr);
-            *ptr = nullptr;
-        }
-        return dalloc(ptr, n);
-    }
-    template <class T> Err upload(T **out, const std::vector<T> &h) {
-        Err e = dalloc(out, h.size());
-        if (!e.ok()) return e;
-        if (!h.empty()) CU(cudaMemcpyAsync(*out, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, stream));
-        return Err();
-    }
-    ~ldsr_plan() {
-        cudaSetDevice(device);
-        if (stream) cudaStreamSynchronize(stream);
-        for (void *p : allocs) pool->release(p);
-        if (h_counts) pool->release_pinned(h_counts);
-        if (h_res) pool->release_pinned(h_res);
-        if (stream) pool->put_stream(stream);
-    }
 };
 
 namespace ldsr {
@@ -327,6 +425,42 @@ static void unpad_theta(const double *src, int p, int q, bool has_u, bool has_v,
     dst[1 + p] = src[1 + PQ];
     for (int j = 0; j < q; j++) dst[2 + p + j] = has_v ? src[2 + PQ + j] : 0.0;
     for (int k = 0; k < 4; k++) dst[2 + p + q + k] = src[2 + 2 * PQ + k];
+}
+// a caller's theta table (user fit order, theta_stride apart) in the plan's fit order and padded layout
+static std::vector<double> padded_thetas(const ldsr_plan *P, const double *theta) {
+    std::vector<double> th((size_t)P->n_fits * P->TL);
+    for (int fi = 0; fi < P->n_fits; fi++) {
+        const int s = P->h_g_series[P->h_f_group[fi]];
+        pad_theta(theta + (size_t)P->f_user[fi] * P->theta_stride, P->s_p[s], P->s_q[s], P->h_series[s].has_u != 0,
+                  P->h_series[s].has_v != 0, P->PQ, &th[(size_t)fi * P->TL]);
+    }
+    return th;
+}
+
+// the smoother / propagate / coefficient kernels over n_jobs jobs of a plan's series and masks
+static SmootherParams smoother_params(const ldsr_plan *P, int n_jobs, const int *job_group, const int *job_theta,
+                                      const long long *job_row, const double *theta, double *X, double *Y, double *V,
+                                      double *J, double *lik, int stdlik, double *aux) {
+    SmootherParams sp;
+    sp.series = P->d_series;
+    sp.blobs = P->d_blobs;
+    sp.g_series = P->d_g_series;
+    sp.masks = P->d_masks;
+    sp.g_mask_off = P->d_g_mask_off;
+    sp.g_nobs = P->d_g_nobs;
+    sp.n_jobs = n_jobs;
+    sp.job_group = job_group;
+    sp.job_theta = job_theta;
+    sp.job_row = job_row;
+    sp.theta = theta;
+    sp.X = X;
+    sp.Y = Y;
+    sp.V = V;
+    sp.J = J;
+    sp.lik = lik;
+    sp.stdlik = stdlik;
+    sp.aux = aux;
+    return sp;
 }
 
 static Err validate(const ldsr_batch *b) {
@@ -370,29 +504,46 @@ static Err validate(const ldsr_batch *b) {
     return Err();
 }
 
-static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_plan **out) {
-    Err e = validate(b);
-    if (!e.ok()) return e;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
-        return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-    if (device < 0 || device >= ndev) return fail(LDSR_ERR_ARG, "device %d out of range (have %d)", device, ndev);
-    CU(cudaSetDevice(device));
+// The widest input row of a batch (series s has input rows u[s] of width p[s], v[s] of width q[s], either may be
+// absent): the kernels are compiled per padded width.
+static int input_width(int n_series, const double *const *u, const double *const *v, const int *p, const int *q) {
+    int need = 1;
+    for (int s = 0; s < n_series; s++) {
+        if (u && u[s]) need = std::max(need, p[s]);
+        if (v && v[s]) need = std::max(need, q[s]);
+    }
+    return need;
+}
 
-    std::unique_ptr<ldsr_plan> P(new ldsr_plan());
-    P->device = device;
-    if (pool)
-        P->pool = pool;
-    else {
-        P->own_pool.reset(new DevicePool(device));
-        P->pool = P->own_pool.get();
+// per group: its fits are lo[g] .. hi[g] - 1 (fit_group is non-decreasing), or lo[g] = hi[g] = -1 without fits
+static void fit_ranges(const ldsr_batch *b, std::vector<int> &lo, std::vector<int> &hi) {
+    lo.assign(b->n_groups, -1);
+    hi.assign(b->n_groups, -1);
+    for (int f = 0; f < b->n_fits; f++) {
+        const int g = b->fit_group[f];
+        if (lo[g] < 0) lo[g] = f;
+        hi[g] = f + 1;
     }
-    CU(P->pool->get_stream(&P->stream));
-    {
-        void *hp = nullptr;
-        CU(P->pool->alloc_pinned(COUNTS_CAP * sizeof(int), &hp));
-        P->h_counts = static_cast<int *>(hp);
-    }
+}
+
+// A call given no context runs on a temporary one, which `tmp` owns: device 0, or the devices of ldsr_options.
+static Err default_ctx(ldsr_ctx *&ctx, std::unique_ptr<ldsr_ctx> &tmp, int n_devices = 1, const int *devices = nullptr) {
+    if (ctx) return Err();
+    char buf[256];
+    const int rc = ldsr_ctx_create(n_devices, devices, &ctx, buf, sizeof buf);
+    if (rc != LDSR_OK) return fail(rc, "%s", buf);
+    tmp.reset(ctx);
+    return Err();
+}
+
+// b has passed validate()
+static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_plan **out) {
+    Err e = use_device(device);
+    if (!e.ok()) return e;
+
+    std::unique_ptr<ldsr_plan> P(new ldsr_plan(device, pool));
+    CU(P->cuda.borrow_stream());
+    CU(P->cuda.alloc_pinned(&P->h_counts, COUNTS_CAP));
     CU(cudaDeviceGetAttribute(&P->n_sm, cudaDevAttrMultiProcessorCount, device));
 
     const int ns = b->n_series, ng = b->n_groups, nf = b->n_fits;
@@ -400,12 +551,7 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
     P->n_groups = ng;
     P->n_fits = nf;
     P->theta_stride = b->theta_stride;
-    int need = 1;
-    for (int s = 0; s < ns; s++) {
-        const bool hu = b->u && b->u[s], hv = b->v && b->v[s];
-        if (hu) need = std::max(need, b->p[s]);
-        if (hv) need = std::max(need, b->q[s]);
-    }
+    const int need = input_width(ns, b->u, b->v, b->p, b->q);
     P->kt = kernel_table_for(need);
     if (!P->kt) return fail(LDSR_ERR_UNSUPPORTED, "input width %d has no kernel instantiation", need);
     const int PQ = P->PQ = P->kt->pq;
@@ -415,12 +561,8 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
     P->s_T.assign(b->T, b->T + ns);
 
     // ---- internal order: groups sorted by series (stable), fits follow their groups
-    std::vector<int> fit_lo(ng, -1), fit_hi(ng, -1);
-    for (int f = 0; f < nf; f++) {
-        const int g = b->fit_group[f];
-        if (fit_lo[g] < 0) fit_lo[g] = f;
-        fit_hi[g] = f + 1;
-    }
+    std::vector<int> fit_lo, fit_hi;
+    fit_ranges(b, fit_lo, fit_hi);
     P->g_user.resize(ng);
     std::iota(P->g_user.begin(), P->g_user.end(), 0);
     std::stable_sort(P->g_user.begin(), P->g_user.end(),
@@ -440,6 +582,12 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
             }
     }
     P->h_g_fit_ptr[ng] = (int)P->f_user.size();
+    P->fit_row_user.assign(nf + 1, 0);
+    for (int f = 0; f < nf; f++) P->fit_row_user[f + 1] = P->fit_row_user[f] + b->T[b->group_series[b->fit_group[f]]];
+    P->fit_job_row.resize(nf);
+    for (int fi = 0; fi < nf; fi++) P->fit_job_row[fi] = P->fit_row_user[P->f_user[fi]];
+    P->fit_job_theta.resize(nf);
+    std::iota(P->fit_job_theta.begin(), P->fit_job_theta.end(), 0);
 
     // ---- series blobs
     P->h_series.resize(ns);
@@ -509,12 +657,12 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
     P->blob_in_smem = P->max_blob_bytes <= 200 * 1024;
 
     // ---- masks, hold-outs (internal group order)
-    std::vector<long long> mask_off(ng);
+    P->h_g_mask_off.resize(ng);
     long long nwords = 0;
     std::vector<int> held_ptr(ng + 1, 0), held_idx;
     for (int gi = 0; gi < ng; gi++) {
         const int gu = P->g_user[gi];
-        mask_off[gi] = nwords;
+        P->h_g_mask_off[gi] = nwords;
         nwords += (b->T[P->h_g_series[gi]] + 31) / 32;
         if (b->held_ptr)
             for (int k = b->held_ptr[gu]; k < b->held_ptr[gu + 1]; k++) held_idx.push_back(b->held_idx[k]);
@@ -526,28 +674,21 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
     for (int g = 0; g < ng; g++) P->h_traj_ptr_user[g + 1] = P->h_traj_ptr_user[g] + b->T[b->group_series[g]];
     P->traj_total = P->h_traj_ptr_user[ng];
 
-    // ---- thetas (internal order, padded)
-    std::vector<double> th0((size_t)nf * P->TL);
-    for (int fi = 0; fi < nf; fi++) {
-        const int s = P->h_g_series[P->h_f_group[fi]];
-        pad_theta(b->theta0 + (size_t)P->f_user[fi] * b->theta_stride, b->p[s], b->q[s], P->h_series[s].has_u != 0,
-                  P->h_series[s].has_v != 0, PQ, &th0[(size_t)fi * P->TL]);
-    }
-
     // ---- upload
-    if (!(e = P->upload(&P->d_series, P->h_series)).ok()) return e;
-    if (!(e = P->upload(&P->d_blobs, blobs)).ok()) return e;
+    Resources &cuda = P->cuda;
+    CU(cuda.upload(&P->d_series, P->h_series));
+    CU(cuda.upload(&P->d_blobs, blobs));
     if (uwin.empty()) uwin.push_back(0.0);
-    if (!(e = P->upload(&P->d_uwin, uwin)).ok()) return e;
-    if (!(e = P->upload(&P->d_g_series, P->h_g_series)).ok()) return e;
-    if (!(e = P->upload(&P->d_g_fit_ptr, P->h_g_fit_ptr)).ok()) return e;
-    if (!(e = P->upload(&P->d_g_mask_off, mask_off)).ok()) return e;
-    if (!(e = P->upload(&P->d_held_ptr, held_ptr)).ok()) return e;
+    CU(cuda.upload(&P->d_uwin, uwin));
+    CU(cuda.upload(&P->d_g_series, P->h_g_series));
+    CU(cuda.upload(&P->d_g_fit_ptr, P->h_g_fit_ptr));
+    CU(cuda.upload(&P->d_g_mask_off, P->h_g_mask_off));
+    CU(cuda.upload(&P->d_held_ptr, held_ptr));
     if (held_idx.empty()) held_idx.push_back(0);
-    if (!(e = P->upload(&P->d_held_idx, held_idx)).ok()) return e;
-    if (!(e = P->upload(&P->d_f_group, P->h_f_group)).ok()) return e;
-    if (!(e = P->upload(&P->d_f_user, P->f_user)).ok()) return e;
-    if (!(e = P->upload(&P->d_g_user, P->g_user)).ok()) return e;
+    CU(cuda.upload(&P->d_held_idx, held_idx));
+    CU(cuda.upload(&P->d_f_group, P->h_f_group));
+    CU(cuda.upload(&P->d_f_user, P->f_user));
+    CU(cuda.upload(&P->d_g_user, P->g_user));
     for (int s = 0; s < ns; s++) P->same_width = P->same_width && b->p[s] + b->q[s] + 6 == b->theta_stride;
     if (!P->same_width) {
         P->user_fit_series.resize(nf);
@@ -555,35 +696,35 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
     }
     P->res_head = (size_t)nf * b->theta_stride + nf + ((size_t)2 * nf + ng + 1) / 2;
     P->res_total = P->res_head + 4 * (size_t)P->traj_total; // allocated by the first ldsr_plan_em
-    if (!(e = P->upload(&P->d_theta0, th0)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_masks, (size_t)nwords)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_sconst, (size_t)sconst_off)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_gconst, (size_t)ng * gconst_stride(PQ))).ok()) return e;
-    if (!(e = P->dalloc(&P->d_g_status, ng)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_g_nobs, ng)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_theta, (size_t)nf * P->TL)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_l1, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_l2, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_lik, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_ne, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_done, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_status, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_active, nf)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_n_live, ns)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_task_off, ns + 1)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_counts, COUNTS_CAP)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_sum, 1)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_ticket, 1)).ok()) return e;
-    CU(cudaMemsetAsync(P->d_ticket, 0, sizeof(unsigned), P->stream));
+    CU(cuda.upload(&P->d_theta0, padded_thetas(P.get(), b->theta0)));
+    CU(cuda.alloc(&P->d_masks, (size_t)nwords));
+    CU(cuda.alloc(&P->d_sconst, (size_t)sconst_off));
+    CU(cuda.alloc(&P->d_gconst, (size_t)ng * gconst_stride(PQ)));
+    CU(cuda.alloc(&P->d_g_status, ng));
+    CU(cuda.alloc(&P->d_g_nobs, ng));
+    CU(cuda.alloc(&P->d_theta, (size_t)nf * P->TL));
+    CU(cuda.alloc(&P->d_l1, nf));
+    CU(cuda.alloc(&P->d_l2, nf));
+    CU(cuda.alloc(&P->d_lik, nf));
+    CU(cuda.alloc(&P->d_ne, nf));
+    CU(cuda.alloc(&P->d_done, nf));
+    CU(cuda.alloc(&P->d_status, nf));
+    CU(cuda.alloc(&P->d_active, nf));
+    CU(cuda.alloc(&P->d_n_live, ns));
+    CU(cuda.alloc(&P->d_task_off, ns + 1));
+    CU(cuda.alloc(&P->d_counts, COUNTS_CAP));
+    CU(cuda.alloc(&P->d_sum, 1));
+    CU(cuda.alloc(&P->d_ticket, 1));
+    CU(cudaMemsetAsync(P->d_ticket, 0, sizeof(unsigned), cuda.stream));
     // the time-split kernels take 32 fits per CTA; the small-batch scan kernel one fit per CTA
     P->max_tasks = std::max(nf / 32, std::min(nf, SCAN_MAX_FITS)) + ns + 1;
-    if (!(e = P->dalloc(&P->d_tasks, P->max_tasks)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_share_flags, P->max_tasks)).ok()) return e;
-    CU(cudaMemsetAsync(P->d_share_flags, 0, (size_t)P->max_tasks * sizeof(int), P->stream));
-    if (!(e = P->dalloc(&P->d_share_ctl, SHARE_CTL_LEN)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_share_order, P->max_tasks)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_share_key, P->max_tasks)).ok()) return e;
-    if (!(e = P->dalloc(&P->d_best, ng)).ok()) return e;
+    CU(cuda.alloc(&P->d_tasks, P->max_tasks));
+    CU(cuda.alloc(&P->d_share_flags, P->max_tasks));
+    CU(cudaMemsetAsync(P->d_share_flags, 0, (size_t)P->max_tasks * sizeof(int), cuda.stream));
+    CU(cuda.alloc(&P->d_share_ctl, SHARE_CTL_LEN));
+    CU(cuda.alloc(&P->d_share_order, P->max_tasks));
+    CU(cuda.alloc(&P->d_share_key, P->max_tasks));
+    CU(cuda.alloc(&P->d_best, ng));
 
     // ---- set-up kernel: masks + Gram constants
     SetupParams sp;
@@ -602,10 +743,10 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
     sp.g_nobs = P->d_g_nobs;
     sp.pq = PQ;
     const size_t sh = (size_t)(2 * PQ * PQ + 2 * PQ + 4) * sizeof(double);
-    setup_kernel<<<ng + ns, 128, sh, P->stream>>>(sp);
+    setup_kernel<<<ng + ns, 128, sh, cuda.stream>>>(sp);
     CU(cudaGetLastError());
-    merge_status_kernel<<<(ng + 127) / 128, 128, 0, P->stream>>>(P->d_series, P->d_sconst, P->d_g_series, ng, PQ,
-                                                                 P->d_g_status);
+    merge_status_kernel<<<(ng + 127) / 128, 128, 0, cuda.stream>>>(P->d_series, P->d_sconst, P->d_g_series, ng, PQ,
+                                                                P->d_g_status);
     CU(cudaGetLastError());
     // No synchronisation here: cudaMemcpyAsync from pageable memory returns once the source has
     // been staged, so the host vectors above may go out of scope; errors surface at the first sync.
@@ -616,21 +757,38 @@ static Err plan_build(const ldsr_batch *b, int device, DevicePool *pool, ldsr_pl
 // ---- the EM driver ---------------------------------------------------------------------------
 #ifdef LDSR_PHASE_CLOCKS
 static long long *sp_clk_last = nullptr; // development build only (DESIGN.md 4.5)
+// per-warp phase clocks of one launch of `grid` CTAs of nw warps: 21 counters per warp, the first `rows` printed
+static void dump_phase_clocks(const char *kernel, const char *const *names, int rows, int width, int grid, int nw,
+                              int chunk, cudaStream_t st) {
+    std::vector<long long> h((size_t)grid * nw * 21);
+    cudaStreamSynchronize(st);
+    cudaMemcpy(h.data(), sp_clk_last, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
+    std::fprintf(stderr, "[ldsr] %sphase clocks of launch 1 (cycles per iteration, mean over %d CTAs), per warp:\n",
+                 kernel, grid);
+    for (int i = 0; i < rows; i++) {
+        std::fprintf(stderr, "[ldsr]   %-14s", names[i]);
+        for (int w = 0; w < nw; w++) {
+            double sum = 0;
+            for (int b = 0; b < grid; b++) sum += (double)h[((size_t)b * nw + w) * 21 + i];
+            std::fprintf(stderr, " %*.0f", width, sum / grid / chunk);
+        }
+        std::fprintf(stderr, "\n");
+    }
+}
 #endif
 static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt, cudaStream_t st, bool want_liks,
                    std::atomic<int> *abort_flag, long long *stats) {
     if (niter < 2) return fail(LDSR_ERR_ARG, "niter=%d: the reference requires niter >= 2 (EM.cpp:247,256)", niter);
     if (!(tol == tol)) return fail(LDSR_ERR_ARG, "tol is NaN");
     CU(cudaSetDevice(P->device));
-    if (!st) st = P->stream;
-    if (st != P->stream) {
+    if (!st) st = P->cuda.stream;
+    Resources clk(nullptr, st); // events on the stream the EM runs on
+    if (st != P->cuda.stream) {
         // the plan's uploads and set-up kernels were enqueued on its own stream: order the caller's after them
         cudaEvent_t ready = nullptr;
-        CU(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-        cudaError_t e1 = cudaEventRecord(ready, P->stream);
-        if (e1 == cudaSuccess) e1 = cudaStreamWaitEvent(st, ready, 0);
-        cudaEventDestroy(ready);
-        CU(e1);
+        CU(clk.event(&ready, cudaEventDisableTiming));
+        CU(cudaEventRecord(ready, P->cuda.stream));
+        CU(cudaStreamWaitEvent(st, ready, 0));
     }
     const int nf = P->n_fits, ns = P->n_series, ng = P->n_groups;
     int chunk = (opt && opt->chunk_iters > 0) ? opt->chunk_iters : 100;
@@ -643,8 +801,7 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
         const size_t need = (size_t)nf * niter;
         if (P->liks_cap < need) {
             P->liks_cap = 0;
-            Err e = P->drealloc(&P->d_liks, need);
-            if (!e.ok()) return e;
+            CU(P->cuda.realloc(&P->d_liks, need));
             P->liks_cap = need;
         }
         fill_nan_kernel<<<(unsigned)((need + 255) / 256), 256, 0, st>>>(P->d_liks, need);
@@ -795,30 +952,17 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
         share_ranked = share_slots == 2 * P->n_sm && share_slots <= 1024 && !no_rank;
     }
     if ((int)P->counts_cap < 2 * max_chunks) {
-        Err e = P->drealloc(&P->d_counts, (size_t)2 * max_chunks);
-        if (!e.ok()) return e;
+        CU(P->cuda.realloc(&P->d_counts, (size_t)2 * max_chunks));
         P->counts_cap = 2 * max_chunks;
-        if (P->h_counts) P->pool->release_pinned(P->h_counts);
-        P->h_counts = nullptr;
-        void *hp = nullptr;
-        CU(P->pool->alloc_pinned((size_t)2 * max_chunks * sizeof(int), &hp));
-        P->h_counts = static_cast<int *>(hp);
+        CU(P->cuda.realloc_pinned(&P->h_counts, (size_t)2 * max_chunks));
     }
     const size_t ck_need = (mode == 2 || use_split || use_wide || use_scan) ? 0 : (size_t)grid0 * EM_WARPS * P->max_seg * 64;
     if (P->ckpt_cap < ck_need) {
         P->ckpt_cap = 0;
-        Err e = P->drealloc(&P->d_ckpt, ck_need);
-        if (!e.ok()) return e;
+        CU(P->cuda.realloc(&P->d_ckpt, ck_need));
         P->ckpt_cap = ck_need;
     }
     ep.ckpt = P->d_ckpt;
-    std::vector<cudaEvent_t> evs;
-    struct EvVecGuard {
-        std::vector<cudaEvent_t> &v;
-        ~EvVecGuard() {
-            for (cudaEvent_t e : v) cudaEventDestroy(e);
-        }
-    } evs_guard{evs};
     int enq = 0;
     for (int c = 0; c < max_chunks; ++c) {
         int *cnt = P->d_counts + 2 * c;
@@ -853,14 +997,7 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
             }
         }
         ep.n_tasks = cnt;
-        if (stats) {
-            cudaEvent_t a = nullptr, b = nullptr;
-            CU(cudaEventCreate(&a));
-            evs.push_back(a);
-            CU(cudaEventCreate(&b));
-            evs.push_back(b);
-            CU(cudaEventRecord(a, st));
-        }
+        if (stats) CU(clk.start());
         if (use_scan) {
             ep.max_seg = P->max_T; // the scan kernel sizes its block from the longest series
             ep.mode = nf > 2 * P->n_sm ? 1 : 0; // more than two fits per SM: the three-CTAs-per-SM build (em_scan_kernel.cuh)
@@ -884,23 +1021,10 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
             CU(P->kt->em_wide(wp, grid, smem, st));
 #ifdef LDSR_PHASE_CLOCKS
             if (c == 1 && grid <= 2048) {
-                const int nw = P->kt->wide_nw;
-                std::vector<long long> h((size_t)grid * nw * 21);
-                cudaStreamSynchronize(st);
-                cudaMemcpy(h.data(), sp_clk_last, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
                 static const char *names[21] = {"P1", "B1 wait", "prefix+P2", "B2 wait", "P4", "B3 wait", "-",
                                                 "B4 wait", "store sums", "B5 wait", "totals", "B5b wait", "matvec rows",
                                                 "B5c wait", "M-step scalars", "B6 wait", "phase A", "chain+stop", "phase C", "-", "-"};
-                std::fprintf(stderr, "[ldsr] wide kernel, phase clocks of launch 1 (cycles per iteration, mean over %d CTAs), per warp:\n", grid);
-                for (int i = 0; i < 19; i++) {
-                    std::fprintf(stderr, "[ldsr]   %-14s", names[i]);
-                    for (int w = 0; w < nw; w++) {
-                        double sum = 0;
-                        for (int b = 0; b < grid; b++) sum += (double)h[((size_t)b * nw + w) * 21 + i];
-                        std::fprintf(stderr, " %8.0f", sum / grid / chunk);
-                    }
-                    std::fprintf(stderr, "\n");
-                }
+                dump_phase_clocks("wide kernel, ", names, 19, 8, grid, P->kt->wide_nw, chunk, st);
             }
 #endif
         } else if (use_split) {
@@ -940,27 +1064,14 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
         } else {
             CU(P->kt->em_chunk(ep, grid, smem, st));
         }
-        if (stats) CU(cudaEventRecord(evs.back(), st));
+        if (stats) CU(clk.stop());
 #ifdef LDSR_PHASE_CLOCKS
         if (use_split && c == 1 && grid <= 4096) {
-            const int nw = P->kt->split_nw;
-            std::vector<long long> h((size_t)grid * nw * 21);
-            cudaStreamSynchronize(st);
-            cudaMemcpy(h.data(), sp_clk_last, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
             static const char *names[21] = {"P1 loops", "B1 wait", "P2", "B2 wait", "chain+stop", "B2' wait",
                                             "P4", "B3 wait", "M-step", "constants", "prefix", "reduce",
                                             "-", "P2 U words", "P2 M units", "P2 M1 units",
                                             "P2 US units", "P4 U words", "P4 M units", "P4 M1 units", "P4 US units"};
-            std::fprintf(stderr, "[ldsr] phase clocks of launch 1 (cycles per iteration, mean over %d CTAs), per warp:\n", grid);
-            for (int i = 0; i < 21; i++) {
-                std::fprintf(stderr, "[ldsr]   %-14s", names[i]);
-                for (int w = 0; w < nw; w++) {
-                    double sum = 0;
-                    for (int b = 0; b < grid; b++) sum += (double)h[((size_t)b * nw + w) * 21 + i];
-                    std::fprintf(stderr, " %9.0f", sum / grid / chunk);
-                }
-                std::fprintf(stderr, "\n");
-            }
+            dump_phase_clocks("", names, 21, 9, grid, P->kt->split_nw, chunk, st);
         }
 #endif
         launches++;
@@ -978,7 +1089,7 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
         if (P->h_counts[2 * c + 1] > 0) chunks++; // launches that had live fits
         if (stats) {
             float ms = 0.f;
-            CU(cudaEventElapsedTime(&ms, evs[2 * c], evs[2 * c + 1]));
+            CU(clk.ms(c, c, &ms));
             if (P->h_counts[2 * c + 1] > 0) em_ms += ms;
             if (trace_chunks)
                 std::fprintf(stderr, "[ldsr] chunk %d: %d tasks, %d live fits, %.3f ms\n", c, P->h_counts[2 * c],
@@ -986,19 +1097,14 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
         }
     }
     // ---- selection + the winners' smoothed trajectories
-    cudaEvent_t tail_a = nullptr, tail_b = nullptr;
-    if (trace_chunks && stats) {
-        cudaEventCreate(&tail_a);
-        cudaEventCreate(&tail_b);
-        cudaEventRecord(tail_a, st);
-    }
+    const bool trace_tail = trace_chunks && stats;
+    if (trace_tail) CU(clk.start());
     select_kernel<<<(ng + 3) / 4, 128, 0, st>>>(ng, P->d_g_fit_ptr, P->d_theta, P->TL, 1 + P->PQ, P->d_lik,
                                                     P->d_g_status, P->d_best, P->d_status);
     CU(cudaGetLastError());
     launches++;
     if (!P->d_X) {
-        Err e;
-        if (!(e = P->dalloc(&P->d_res, P->res_total)).ok()) return e;
+        CU(P->cuda.alloc(&P->d_res, P->res_total));
         P->d_X = P->d_res + P->res_head;
         P->d_Y = P->d_X + P->traj_total;
         P->d_V = P->d_Y + P->traj_total;
@@ -1009,31 +1115,14 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
             jg[gi] = gi;
             jr[gi] = P->h_traj_ptr_user[P->g_user[gi]];
         }
-        cudaStream_t keep = P->stream;
-        P->stream = st;
-        if (!(e = P->upload(&P->d_job_group, jg)).ok()) return e;
-        if (!(e = P->upload(&P->d_job_row, jr)).ok()) return e;
-        P->stream = keep;
+        CU(P->cuda.alloc(&P->d_job_group, ng));
+        CU(cudaMemcpyAsync(P->d_job_group, jg.data(), ng * sizeof(int), cudaMemcpyHostToDevice, st));
+        CU(P->cuda.alloc(&P->d_job_row, ng));
+        CU(cudaMemcpyAsync(P->d_job_row, jr.data(), ng * sizeof(long long), cudaMemcpyHostToDevice, st));
     }
-    SmootherParams sp;
-    sp.series = P->d_series;
-    sp.blobs = P->d_blobs;
-    sp.g_series = P->d_g_series;
-    sp.masks = P->d_masks;
-    sp.g_mask_off = P->d_g_mask_off;
-    sp.g_nobs = P->d_g_nobs;
-    sp.n_jobs = ng;
-    sp.job_group = P->d_job_group;
-    sp.job_theta = P->d_best; // best fit (internal index) or -1
-    sp.job_row = P->d_job_row;
-    sp.theta = P->d_theta;
-    sp.X = P->d_X;
-    sp.Y = P->d_Y;
-    sp.V = P->d_V;
-    sp.J = P->d_J;
-    sp.lik = nullptr;
-    sp.stdlik = 1;
-    sp.aux = nullptr;
+    // job_theta: the best fit (internal index) or -1
+    const SmootherParams sp = smoother_params(P, ng, P->d_job_group, P->d_best, P->d_job_row, P->d_theta, P->d_X,
+                                              P->d_Y, P->d_V, P->d_J, nullptr, 1, nullptr);
     // One thread per winner walks 2 T dependent steps (0.12 ms at T = 413, however few the groups); where the scan
     // kernel applies (its width / length / v == u conditions, whatever the batch size) its E-step does it in a few us
     static const bool seq_traj = std::getenv("LDSR_SEQ_TRAJ") != nullptr; // development: A/B measurement
@@ -1053,7 +1142,7 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
         CU(P->kt->smoother(sp, st));
     }
     launches++;
-    if (tail_a) cudaEventRecord(tail_b, st);
+    if (trace_tail) CU(clk.stop());
     CU(cudaMemsetAsync(P->d_sum, 0, sizeof(unsigned long long), st));
     sum_int_kernel<<<64, 256, 0, st>>>(P->d_ne, nf, P->d_sum);
     launches++;
@@ -1062,13 +1151,11 @@ static Err plan_em(ldsr_plan *P, int niter, double tol, const ldsr_options *opt,
     CU(cudaStreamSynchronize(st));
     CU(cudaGetLastError());
     P->em_done = true;
-    if (tail_a) {
+    if (trace_tail) { // the last pair; pairs 0 .. enq - 1 are the chunks
         float ms = 0.f, all = 0.f;
-        cudaEventElapsedTime(&ms, tail_a, tail_b);
-        if (!evs.empty()) cudaEventElapsedTime(&all, evs.front(), tail_b);
+        clk.ms(enq, enq, &ms);
+        if (enq > 0) clk.ms(0, enq, &all);
         std::fprintf(stderr, "[ldsr] selection + winners' smoother %.3f ms; first chunk start -> end %.3f ms\n", ms, all);
-        cudaEventDestroy(tail_a);
-        cudaEventDestroy(tail_b);
     }
     if (stats) {
         stats[0] = launches;
@@ -1096,7 +1183,7 @@ static Err plan_fetch(ldsr_plan *P, ldsr_em_result *out, const FetchMap *map = n
     if (!out) return fail(LDSR_ERR_ARG, "result struct is NULL");
     CU(cudaSetDevice(P->device));
     const int nf = P->n_fits, ng = P->n_groups, stride = P->theta_stride;
-    cudaStream_t st = P->stream;
+    cudaStream_t st = P->cuda.stream;
     // pack on the device (caller's order and layout), one copy into pinned memory, then plain memcpys
     double *d_theta_u = P->d_res, *d_lik_u = d_theta_u + (size_t)nf * stride;
     int *d_int = reinterpret_cast<int *>(d_lik_u + nf);
@@ -1123,11 +1210,7 @@ static Err plan_fetch(ldsr_plan *P, ldsr_em_result *out, const FetchMap *map = n
     pk.best_u = d_int + 2 * (size_t)nf;
     pack_results_kernel<<<(std::max(nf, ng) + 255) / 256, 256, 0, st>>>(pk);
     CU(cudaGetLastError());
-    if (!P->h_res) {
-        void *hp = nullptr;
-        CU(P->pool->alloc_pinned(P->res_total * sizeof(double), &hp));
-        P->h_res = static_cast<double *>(hp);
-    }
+    if (!P->h_res) CU(P->cuda.alloc_pinned(&P->h_res, P->res_total));
     const bool traj = out->X || out->Y || out->V || out->J;
     CU(cudaMemcpyAsync(P->h_res, P->d_res, (traj ? P->res_total : P->res_head) * sizeof(double),
                        cudaMemcpyDeviceToHost, st));
@@ -1268,14 +1351,7 @@ static Err em_batch(ldsr_ctx *ctx, const ldsr_batch *b, int niter, double tol, c
     if (!e.ok()) return e;
     if (!out) return fail(LDSR_ERR_ARG, "result struct is NULL");
     std::unique_ptr<ldsr_ctx> tmp_ctx;
-    if (!ctx) {
-        ldsr_ctx *c = nullptr;
-        char buf[256];
-        int rc = ldsr_ctx_create(opt ? opt->n_devices : 0, opt ? opt->devices : nullptr, &c, buf, sizeof buf);
-        if (rc != LDSR_OK) return fail(rc, "%s", buf);
-        tmp_ctx.reset(c);
-        ctx = c;
-    }
+    if (!(e = default_ctx(ctx, tmp_ctx, opt ? opt->n_devices : 0, opt ? opt->devices : nullptr)).ok()) return e;
     int nd = (int)ctx->devices.size();
     if (opt && opt->n_devices > 0) nd = std::min(nd, opt->n_devices);
     nd = std::max(1, std::min(nd, b->n_groups));
@@ -1311,12 +1387,8 @@ static Err em_batch(ldsr_ctx *ctx, const ldsr_batch *b, int niter, double tol, c
 
     // ---- shard groups over devices (no data-path collective: a group's restarts stay together)
     const int ng = b->n_groups;
-    std::vector<int> fit_lo(ng, -1), fit_hi(ng, -1);
-    for (int f = 0; f < b->n_fits; f++) {
-        const int g = b->fit_group[f];
-        if (fit_lo[g] < 0) fit_lo[g] = f;
-        fit_hi[g] = f + 1;
-    }
+    std::vector<int> fit_lo, fit_hi;
+    fit_ranges(b, fit_lo, fit_hi);
     {   // a group without fits costs nothing: never more shards than groups that have work, so that no
         // device is handed an empty sub-batch
         int nonempty = 0;
@@ -1339,12 +1411,7 @@ static Err em_batch(ldsr_ctx *ctx, const ldsr_batch *b, int niter, double tol, c
     wopt.poll = nullptr;
     wopt.poll_arg = nullptr;
     if (wopt.variant == 0) { // the kernel follows the whole batch, not the shard (see plan_em, variant 6)
-        int width = 1;
-        for (int s = 0; s < b->n_series; s++) {
-            if (b->u && b->u[s]) width = std::max(width, b->p[s]);
-            if (b->v && b->v[s]) width = std::max(width, b->q[s]);
-        }
-        const KernelTable *kt_all = kernel_table_for(width);
+        const KernelTable *kt_all = kernel_table_for(input_width(b->n_series, b->u, b->v, b->p, b->q));
         if (kt_all && b->n_fits > scan_auto_fits(kt_all->pq)) wopt.variant = 6;
     }
     const bool caller_polls = opt && opt->poll;
@@ -1435,63 +1502,32 @@ enum class StepKind { Smoother, Propagate };
 
 static Err step_batch(ldsr_ctx *ctx, const ldsr_batch *b, StepKind kind, int stdlik, double *X, double *Y, double *V,
                       double *J, double *lik, double *aux = nullptr, bool rows_to_host = true) {
-    std::unique_ptr<ldsr_ctx> tmp_ctx;
-    if (!ctx) {
-        ldsr_ctx *c = nullptr;
-        char buf[256];
-        int rc = ldsr_ctx_create(1, nullptr, &c, buf, sizeof buf);
-        if (rc != LDSR_OK) return fail(rc, "%s", buf);
-        tmp_ctx.reset(c);
-        ctx = c;
-    }
     if (rows_to_host && (!X || !Y || !V)) return fail(LDSR_ERR_ARG, "X, Y and V outputs are required");
-    ldsr_plan *P = nullptr;
-    Err e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P);
+    Err e = validate(b);
     if (!e.ok()) return e;
+    std::unique_ptr<ldsr_ctx> tmp_ctx;
+    if (!(e = default_ctx(ctx, tmp_ctx)).ok()) return e;
+    ldsr_plan *P = nullptr;
+    if (!(e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P)).ok()) return e;
     std::unique_ptr<ldsr_plan> guard(P);
+    Resources &cuda = P->cuda;
     const int nf = P->n_fits;
-    // job rows follow the USER fit order
-    std::vector<long long> row_user(nf + 1, 0);
-    for (int f = 0; f < nf; f++) row_user[f + 1] = row_user[f] + b->T[b->group_series[b->fit_group[f]]];
-    std::vector<long long> jr(nf);
-    std::vector<int> jt(nf);
-    for (int fi = 0; fi < nf; fi++) {
-        jr[fi] = row_user[P->f_user[fi]];
-        jt[fi] = fi;
-    }
-    const size_t tot = (size_t)row_user[nf];
+    const size_t tot = (size_t)P->fit_row_user[nf];
     double *dX, *dY, *dV, *dJ = nullptr, *dlik, *daux = nullptr;
     int *d_jt;
     long long *d_jr;
-    if (!(e = P->dalloc(&dX, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dY, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dV, tot)).ok()) return e;
-    if (J && !(e = P->dalloc(&dJ, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dlik, nf)).ok()) return e;
-    if (aux && !(e = P->dalloc(&daux, nf)).ok()) return e;
-    if (!(e = P->upload(&d_jt, jt)).ok()) return e;
-    if (!(e = P->upload(&d_jr, jr)).ok()) return e;
-    SmootherParams sp;
-    sp.series = P->d_series;
-    sp.blobs = P->d_blobs;
-    sp.g_series = P->d_g_series;
-    sp.masks = P->d_masks;
-    sp.g_mask_off = P->d_g_mask_off;
-    sp.g_nobs = P->d_g_nobs;
-    sp.n_jobs = nf;
-    sp.job_group = P->d_f_group;
-    sp.job_theta = d_jt;
-    sp.job_row = d_jr;
-    sp.theta = P->d_theta0;
-    sp.X = dX;
-    sp.Y = dY;
-    sp.V = dV;
-    sp.J = dJ;
-    sp.lik = dlik;
-    sp.stdlik = stdlik;
-    sp.aux = daux;
-    CU(kind == StepKind::Smoother ? P->kt->smoother(sp, P->stream) : P->kt->propagate(sp, P->stream));
-    CU(cudaStreamSynchronize(P->stream));
+    CU(cuda.alloc(&dX, tot));
+    CU(cuda.alloc(&dY, tot));
+    CU(cuda.alloc(&dV, tot));
+    if (J) CU(cuda.alloc(&dJ, tot));
+    CU(cuda.alloc(&dlik, nf));
+    if (aux) CU(cuda.alloc(&daux, nf));
+    CU(cuda.upload(&d_jt, P->fit_job_theta));
+    CU(cuda.upload(&d_jr, P->fit_job_row));
+    const SmootherParams sp =
+        smoother_params(P, nf, P->d_f_group, d_jt, d_jr, P->d_theta0, dX, dY, dV, dJ, dlik, stdlik, daux);
+    CU(kind == StepKind::Smoother ? P->kt->smoother(sp, cuda.stream) : P->kt->propagate(sp, cuda.stream));
+    CU(cudaStreamSynchronize(cuda.stream));
     if (rows_to_host) {
         CU(cudaMemcpy(X, dX, tot * sizeof(double), cudaMemcpyDeviceToHost));
         CU(cudaMemcpy(Y, dY, tot * sizeof(double), cudaMemcpyDeviceToHost));
@@ -1513,38 +1549,29 @@ static Err step_batch(ldsr_ctx *ctx, const ldsr_batch *b, StepKind kind, int std
 
 static Err mstep_batch(ldsr_ctx *ctx, const ldsr_batch *b, const double *X, const double *V, const double *J,
                        double *theta_out, int *status) {
-    std::unique_ptr<ldsr_ctx> tmp_ctx;
-    if (!ctx) {
-        ldsr_ctx *c = nullptr;
-        char buf[256];
-        int rc = ldsr_ctx_create(1, nullptr, &c, buf, sizeof buf);
-        if (rc != LDSR_OK) return fail(rc, "%s", buf);
-        tmp_ctx.reset(c);
-        ctx = c;
-    }
     if (!X || !V || !J || !theta_out) return fail(LDSR_ERR_ARG, "X, V, J and theta_out are required");
-    ldsr_plan *P = nullptr;
-    Err e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P);
+    Err e = validate(b);
     if (!e.ok()) return e;
+    std::unique_ptr<ldsr_ctx> tmp_ctx;
+    if (!(e = default_ctx(ctx, tmp_ctx)).ok()) return e;
+    ldsr_plan *P = nullptr;
+    if (!(e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P)).ok()) return e;
     std::unique_ptr<ldsr_plan> guard(P);
+    Resources &cuda = P->cuda;
     const int nf = P->n_fits;
-    std::vector<long long> row_user(nf + 1, 0);
-    for (int f = 0; f < nf; f++) row_user[f + 1] = row_user[f] + b->T[b->group_series[b->fit_group[f]]];
-    std::vector<long long> fr(nf);
-    for (int fi = 0; fi < nf; fi++) fr[fi] = row_user[P->f_user[fi]];
-    const size_t tot = (size_t)row_user[nf];
+    const size_t tot = (size_t)P->fit_row_user[nf];
     double *dX, *dV, *dJ, *dth;
     int *dst;
     long long *d_fr;
-    if (!(e = P->dalloc(&dX, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dV, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dJ, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dth, (size_t)nf * P->TL)).ok()) return e;
-    if (!(e = P->dalloc(&dst, nf)).ok()) return e;
-    if (!(e = P->upload(&d_fr, fr)).ok()) return e;
-    CU(cudaMemcpyAsync(dX, X, tot * sizeof(double), cudaMemcpyHostToDevice, P->stream));
-    CU(cudaMemcpyAsync(dV, V, tot * sizeof(double), cudaMemcpyHostToDevice, P->stream));
-    CU(cudaMemcpyAsync(dJ, J, tot * sizeof(double), cudaMemcpyHostToDevice, P->stream));
+    CU(cuda.alloc(&dX, tot));
+    CU(cuda.alloc(&dV, tot));
+    CU(cuda.alloc(&dJ, tot));
+    CU(cuda.alloc(&dth, (size_t)nf * P->TL));
+    CU(cuda.alloc(&dst, nf));
+    CU(cuda.upload(&d_fr, P->fit_job_row));
+    CU(cudaMemcpyAsync(dX, X, tot * sizeof(double), cudaMemcpyHostToDevice, cuda.stream));
+    CU(cudaMemcpyAsync(dV, V, tot * sizeof(double), cudaMemcpyHostToDevice, cuda.stream));
+    CU(cudaMemcpyAsync(dJ, J, tot * sizeof(double), cudaMemcpyHostToDevice, cuda.stream));
     MstepParams mp;
     mp.series = P->d_series;
     mp.blobs = P->d_blobs;
@@ -1562,8 +1589,8 @@ static Err mstep_batch(ldsr_ctx *ctx, const ldsr_batch *b, const double *X, cons
     mp.J = dJ;
     mp.theta_out = dth;
     mp.status = dst;
-    CU(P->kt->mstep(mp, P->stream));
-    CU(cudaStreamSynchronize(P->stream));
+    CU(P->kt->mstep(mp, cuda.stream));
+    CU(cudaStreamSynchronize(cuda.stream));
     std::vector<double> th((size_t)nf * P->TL);
     std::vector<int> stt(nf);
     CU(cudaMemcpy(th.data(), dth, th.size() * sizeof(double), cudaMemcpyDeviceToHost));
@@ -1577,30 +1604,15 @@ static Err mstep_batch(ldsr_ctx *ctx, const ldsr_batch *b, const double *X, cons
     return Err();
 }
 
-// device blocks taken from a pool for the length of one call
-struct DevBlocks {
-    DevicePool *pool;
-    std::vector<void *> held;
-    template <class T> cudaError_t alloc(size_t bytes, T **out) {
-        void *p = nullptr;
-        cudaError_t e = pool->alloc(bytes, &p);
-        if (e == cudaSuccess) held.push_back(p);
-        *out = static_cast<T *>(p);
-        return e;
-    }
-    ~DevBlocks() {
-        for (void *p : held) pool->release(p);
-    }
-};
-
 // The output pipeline of the replicate entry points.  Up to three outputs (simX, simY, simQ; null ones are
 // skipped) of lo.back() doubles each live in the caller's (pageable) memory.  Chunk c covers elements
 // lo[c] .. lo[c+1]-1 of every output and elements zlo[c] .. zlo[c+1]-1 of the noise (caller noise z on the host,
 // or z_dev already on the device).  One pass: the kernel of chunk c+1 runs while chunk c crosses PCIe into a
 // pinned slot and chunk c-1 is copied from its slot into the caller's arrays by host threads.
-// `launch(c, z, out)` enqueues chunk c's kernel on sk (c = -1: one launch for every chunk), reading noise from z
-// (the chunk's first element on the device, or null) and writing output k from out[k] (the chunk's first
-// element).  Every producer the kernels depend on is on sk too; their device time goes to g_last_device_ms.
+// `launch(c, z, out)` enqueues chunk c's kernel on run.stream (c = -1: one launch for every chunk), reading noise
+// from z (the chunk's first element on the device, or null) and writing output k from out[k] (the chunk's first
+// element).  Every producer the kernels depend on is on run.stream too, and the device blocks come from `run`.
+// g_last_device_ms is the time of every piece of work timed on `run`: the caller's and the kernels.
 struct RepOutputs {
     double *outs[3];
     std::vector<size_t> lo, zlo;
@@ -1608,12 +1620,16 @@ struct RepOutputs {
 };
 using RepLaunch = std::function<Err(int c, const double *zdev, double *const *out)>;
 
-static Err rep_pipeline(DevicePool *pool, cudaStream_t sk, const RepOutputs &R, const RepLaunch &launch) {
+static Err rep_pipeline(Resources &run, const RepOutputs &R, const RepLaunch &launch) {
     double *const *outs = R.outs;
+    const cudaStream_t sk = run.stream;
     int n_out = 0;
     for (int o = 0; o < 3; o++) n_out += outs[o] ? 1 : 0;
     g_last_device_ms = 0.0;
-    if (n_out == 0) return Err();
+    if (n_out == 0) {
+        CU(run.total_ms(&g_last_device_ms));
+        return Err();
+    }
     const int n_chunks = (int)R.lo.size() - 1;
     size_t chunk = 0, zchunk = 0;
     for (int c = 0; c < n_chunks; c++) {
@@ -1628,40 +1644,21 @@ static Err rep_pipeline(DevicePool *pool, cudaStream_t sk, const RepOutputs &R, 
     static const bool force_chunked = std::getenv("LDSR_REP_CHUNKED") != nullptr;
     const bool whole = !force_chunked && ((size_t)n_out * tot + ztot) * 8 <= ((size_t)8 << 30);
     const size_t slot_doubles = (size_t)n_out * chunk;
-    DevBlocks dev{pool, {}};
     double *d_whole = nullptr;
     constexpr int SLOTS = 2;
     double *d_out[SLOTS] = {nullptr, nullptr}, *h_out[SLOTS] = {nullptr, nullptr}, *d_z[SLOTS] = {nullptr, nullptr};
     cudaEvent_t ev_k[SLOTS] = {nullptr, nullptr}, ev_c[SLOTS] = {nullptr, nullptr};
-    std::vector<cudaEvent_t> ev_t;
-    cudaStream_t sc = nullptr;
-    struct Cleanup {
-        DevicePool *pool;
-        double **h;
-        cudaEvent_t *a, *b;
-        std::vector<cudaEvent_t> *t;
-        cudaStream_t sk, *sc;
-        ~Cleanup() {
-            cudaStreamSynchronize(sk);
-            if (*sc) cudaStreamSynchronize(*sc);
-            for (int i = 0; i < SLOTS; i++) {
-                if (h[i]) pool->release_pinned(h[i]);
-                if (a[i]) cudaEventDestroy(a[i]);
-                if (b[i]) cudaEventDestroy(b[i]);
-            }
-            for (cudaEvent_t e : *t) cudaEventDestroy(e);
-            if (*sc) pool->put_stream(*sc);
-        }
-    } cleanup{pool, h_out, ev_k, ev_c, &ev_t, sk, &sc};
-    CU(pool->get_stream(&sc));
+    // the copy stream with its pinned slots and events (given back once the copy stream is idle; the device
+    // blocks stay with `run` until run.stream is)
+    Resources copy(run.pool());
+    CU(copy.borrow_stream());
+    const cudaStream_t sc = copy.stream;
     for (int i = 0; i < SLOTS && i < n_chunks; i++) {
-        if (!whole) CU(dev.alloc(slot_doubles * 8, &d_out[i]));
-        void *hp = nullptr;
-        CU(pool->alloc_pinned(slot_doubles * 8, &hp));
-        h_out[i] = static_cast<double *>(hp);
-        if (R.z && !whole) CU(dev.alloc(zchunk * 8, &d_z[i]));
-        CU(cudaEventCreateWithFlags(&ev_k[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&ev_c[i], cudaEventDisableTiming));
+        if (!whole) CU(run.alloc(&d_out[i], slot_doubles));
+        CU(copy.alloc_pinned(&h_out[i], slot_doubles));
+        if (R.z && !whole) CU(run.alloc(&d_z[i], zchunk));
+        CU(copy.event(&ev_k[i], cudaEventDisableTiming));
+        CU(copy.event(&ev_c[i], cudaEventDisableTiming));
     }
     auto copy_out = [&](int c) { // pinned slot -> the caller's arrays, a few host threads
         const int slot = c % SLOTS;
@@ -1686,23 +1683,18 @@ static Err rep_pipeline(DevicePool *pool, cudaStream_t sk, const RepOutputs &R, 
         int k = 0;
         for (int o = 0; o < 3; o++)
             if (outs[o]) o3[o] = base + (size_t)(k++) * out_stride;
-        cudaEvent_t ta = nullptr, tb = nullptr;
-        CU(cudaEventCreate(&ta));
-        ev_t.push_back(ta);
-        CU(cudaEventCreate(&tb));
-        ev_t.push_back(tb);
-        CU(cudaEventRecord(ta, sk));
+        CU(run.start());
         Err e = launch(c, zdev, o3);
         if (!e.ok()) return e;
-        CU(cudaEventRecord(tb, sk));
+        CU(run.stop());
         return Err();
     };
     if (whole) {
-        CU(dev.alloc((size_t)n_out * tot * 8, &d_whole));
+        CU(run.alloc(&d_whole, (size_t)n_out * tot));
         const double *zdev = R.z_dev;
         if (R.z) {
             double *dzw = nullptr;
-            CU(dev.alloc(ztot * 8, &dzw));
+            CU(run.alloc(&dzw, ztot));
             CU(cudaMemcpyAsync(dzw, R.z, ztot * 8, cudaMemcpyHostToDevice, sk));
             zdev = dzw;
         }
@@ -1744,11 +1736,7 @@ static Err rep_pipeline(DevicePool *pool, cudaStream_t sk, const RepOutputs &R, 
         copy_out(c);
     }
     CU(cudaStreamSynchronize(sk));
-    for (size_t i = 0; i + 1 < ev_t.size(); i += 2) {
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, ev_t[i], ev_t[i + 1]));
-        g_last_device_ms += ms;
-    }
+    CU(run.total_ms(&g_last_device_ms));
     return Err();
 }
 
@@ -1758,19 +1746,12 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
     if (!theta || n < 1 || n_reps < 1 || p < 0 || q < 0) return fail(LDSR_ERR_ARG, "bad theta/n/n_reps/p/q");
     if (p > LDSR_MAX_PQ || q > LDSR_MAX_PQ) return fail(LDSR_ERR_UNSUPPORTED, "p or q exceeds LDSR_MAX_PQ");
     std::unique_ptr<ldsr_ctx> tmp_ctx;
-    if (!ctx) {
-        ldsr_ctx *c = nullptr;
-        char buf[256];
-        int rc = ldsr_ctx_create(1, nullptr, &c, buf, sizeof buf);
-        if (rc != LDSR_OK) return fail(rc, "%s", buf);
-        tmp_ctx.reset(c);
-        ctx = c;
-    }
+    Err e = default_ctx(ctx, tmp_ctx);
+    if (!e.ok()) return e;
     CU(cudaSetDevice(ctx->devices[0]));
-    DevicePool *pool = ctx->pools[0].get();
-    const int need = std::max(1, std::max(u ? p : 0, v ? q : 0));
+    const int need = input_width(1, &u, &v, &p, &q);
     const KernelTable *kt = kernel_table_for(need);
-    if (!kt) return fail(LDSR_ERR_UNSUPPORTED, "no kernel for width %d", need);
+    if (!kt) return fail(LDSR_ERR_UNSUPPORTED, "input width %d has no kernel instantiation", need);
     const int PQ = kt->pq;
     std::vector<double> th(2 * PQ + 6), up((size_t)n * PQ, 0.0), vp((size_t)n * PQ, 0.0);
     pad_theta(theta, p, q, u != nullptr, v != nullptr, PQ, th.data());
@@ -1780,30 +1761,17 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
         if (v)
             for (int j = 0; j < q; j++) vp[(size_t)t * PQ + j] = v[(size_t)t * q + j];
     }
-    DevBlocks dev{pool, {}};
-    struct Stream { // declared after dev: synchronised before the blocks go back to the pool
-        DevicePool *pool;
-        cudaStream_t s = nullptr;
-        ~Stream() {
-            if (s) {
-                cudaStreamSynchronize(s);
-                pool->put_stream(s);
-            }
-        }
-    } sk{pool};
-    CU(pool->get_stream(&sk.s));
+    Resources run(ctx->pools[0].get());
+    CU(run.borrow_stream());
     double *dth, *du, *dv, *dz_all = nullptr;
-    CU(dev.alloc(th.size() * 8, &dth));
-    CU(dev.alloc(up.size() * 8, &du));
-    CU(dev.alloc(vp.size() * 8, &dv));
-    CU(cudaMemcpyAsync(dth, th.data(), th.size() * 8, cudaMemcpyHostToDevice, sk.s));
-    CU(cudaMemcpyAsync(du, up.data(), up.size() * 8, cudaMemcpyHostToDevice, sk.s));
-    CU(cudaMemcpyAsync(dv, vp.data(), vp.size() * 8, cudaMemcpyHostToDevice, sk.s));
+    CU(run.upload(&dth, th));
+    CU(run.upload(&du, up));
+    CU(run.upload(&dv, vp));
     const size_t zrow = 1 + 2 * (size_t)n;
     if (r_seed) { // the reference's own stream: set.seed(*r_seed); rnorm(...) in replicate order, made on the device
         const long long nz = (long long)n_reps * (long long)zrow;
-        CU(dev.alloc((size_t)nz * 8, &dz_all));
-        CU(r_rnorm_device(*r_seed, nz, dz_all, sk.s));
+        CU(run.alloc(&dz_all, (size_t)nz));
+        CU(r_rnorm_device(*r_seed, nz, dz_all, run.stream));
     }
     // ~48 MB per output and chunk, a multiple of a CTA's 128 replicates (at T = 813: 58 CTAs per launch)
     int chunk = (int)std::max<size_t>(128, ((size_t)48 << 20) / ((size_t)n * 8));
@@ -1814,7 +1782,7 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
         R.zlo.push_back((size_t)r0 * zrow);
         if (r0 == n_reps) break;
     }
-    return rep_pipeline(pool, sk.s, R, [&](int c, const double *zdev, double *const *o3) -> Err {
+    return rep_pipeline(run, R, [&](int c, const double *zdev, double *const *o3) -> Err {
         const int r0 = c < 0 ? 0 : c * chunk;
         RepParams rp;
         rp.theta = dth;
@@ -1830,7 +1798,7 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
         rp.simX = o3[0];
         rp.simY = o3[1];
         rp.simQ = o3[2];
-        CU(kt->rep(rp, sk.s));
+        CU(kt->rep(rp, run.stream));
         return Err();
     });
 }
@@ -1845,8 +1813,6 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
     if (transform < 0 || transform > 2) return fail(LDSR_ERR_ARG, "transform=%d, need 0 (none), 1 (log) or 2 (Box-Cox)", transform);
     if (transform == 2 && !lambda) return fail(LDSR_ERR_ARG, "transform 2 (Box-Cox) needs lambda");
     const int nf = b->n_fits;
-    std::vector<long long> fit_ptr(nf + 1, 0);
-    for (int f = 0; f < nf; f++) fit_ptr[f + 1] = fit_ptr[f] + b->T[b->group_series[b->fit_group[f]]];
     std::vector<double> par((size_t)4 * nf);
     for (int f = 0; f < nf; f++) {
         const int s = b->group_series[b->fit_group[f]];
@@ -1859,70 +1825,34 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
         par[4 * f + 3] = transform == 2 ? lambda[f] : 0.0;
     }
     std::unique_ptr<ldsr_ctx> tmp_ctx;
-    if (!ctx) {
-        ldsr_ctx *c = nullptr;
-        char buf[256];
-        int rc = ldsr_ctx_create(1, nullptr, &c, buf, sizeof buf);
-        if (rc != LDSR_OK) return fail(rc, "%s", buf);
-        tmp_ctx.reset(c);
-        ctx = c;
-    }
+    if (!(e = default_ctx(ctx, tmp_ctx)).ok()) return e;
     ldsr_plan *P = nullptr;
     if (!(e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P)).ok()) return e;
     std::unique_ptr<ldsr_plan> guard(P);
-    // per fit: its coefficient rows (user order, as ldsr_smoother_batch) and its group's first mask word
-    std::vector<long long> jr(nf), f_mask_off(nf), g_mask_off(P->n_groups);
-    std::vector<int> jt(nf);
-    for (int gi = 0, w = 0; gi < P->n_groups; gi++) {
-        g_mask_off[gi] = w;
-        w += (P->s_T[P->h_g_series[gi]] + 31) / 32;
-    }
-    for (int fi = 0; fi < nf; fi++) {
-        jr[fi] = fit_ptr[P->f_user[fi]];
-        jt[fi] = fi;
-        f_mask_off[P->f_user[fi]] = g_mask_off[P->h_f_group[fi]];
-    }
+    Resources &cuda = P->cuda;
+    // per USER fit: its group's first mask word
+    std::vector<long long> f_mask_off(nf);
+    for (int fi = 0; fi < nf; fi++) f_mask_off[P->f_user[fi]] = P->h_g_mask_off[P->h_f_group[fi]];
+    const std::vector<long long> &fit_ptr = P->fit_row_user;
     const size_t tot = (size_t)fit_ptr[nf];
     double *dm, *dO, *ds, *dJ, *d_par;
     int *d_jt;
     long long *d_jr, *d_fit_ptr, *d_fmo;
-    if (!(e = P->dalloc(&dm, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dO, tot)).ok()) return e;
-    if (!(e = P->dalloc(&ds, tot)).ok()) return e;
-    if (!(e = P->dalloc(&dJ, tot)).ok()) return e;
-    if (!(e = P->upload(&d_jt, jt)).ok()) return e;
-    if (!(e = P->upload(&d_jr, jr)).ok()) return e;
-    if (!(e = P->upload(&d_fit_ptr, fit_ptr)).ok()) return e;
-    if (!(e = P->upload(&d_fmo, f_mask_off)).ok()) return e;
-    if (!(e = P->upload(&d_par, par)).ok()) return e;
-    SmootherParams sp = {};
-    sp.series = P->d_series;
-    sp.blobs = P->d_blobs;
-    sp.g_series = P->d_g_series;
-    sp.masks = P->d_masks;
-    sp.g_mask_off = P->d_g_mask_off;
-    sp.g_nobs = P->d_g_nobs;
-    sp.n_jobs = nf;
-    sp.job_group = P->d_f_group;
-    sp.job_theta = d_jt;
-    sp.job_row = d_jr;
-    sp.theta = P->d_theta0;
-    sp.X = dm;
-    sp.Y = dO;
-    sp.V = ds;
-    sp.J = dJ;
-    struct Events {
-        cudaEvent_t a = nullptr, b = nullptr;
-        ~Events() {
-            if (a) cudaEventDestroy(a);
-            if (b) cudaEventDestroy(b);
-        }
-    } ev;
-    CU(cudaEventCreate(&ev.a));
-    CU(cudaEventCreate(&ev.b));
-    CU(cudaEventRecord(ev.a, P->stream));
-    CU(P->kt->smoother_coef(sp, P->stream));
-    CU(cudaEventRecord(ev.b, P->stream));
+    CU(cuda.alloc(&dm, tot));
+    CU(cuda.alloc(&dO, tot));
+    CU(cuda.alloc(&ds, tot));
+    CU(cuda.alloc(&dJ, tot));
+    CU(cuda.upload(&d_jt, P->fit_job_theta));
+    CU(cuda.upload(&d_jr, P->fit_job_row));
+    CU(cuda.upload(&d_fit_ptr, fit_ptr));
+    CU(cuda.upload(&d_fmo, f_mask_off));
+    CU(cuda.upload(&d_par, par));
+    // the coefficient rows (user order, as ldsr_smoother_batch): m, o, s, J
+    const SmootherParams sp =
+        smoother_params(P, nf, P->d_f_group, d_jt, d_jr, P->d_theta0, dm, dO, ds, dJ, nullptr, 0, nullptr);
+    CU(cuda.start()); // the coefficient pass counts as device time too
+    CU(P->kt->smoother_coef(sp, cuda.stream));
+    CU(cuda.stop());
     // warps: (fit, 32 replicates) blocks in output order; a chunk is a range of whole blocks (~48 MB per output)
     const int wpf = (n_reps + 31) / 32;
     const long long n_blk = (long long)nf * wpf;
@@ -1939,7 +1869,7 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
             R.lo.push_back(blk_end(k));
             R.zlo.push_back(2 * blk_end(k));
         }
-    e = rep_pipeline(P->pool, P->stream, R, [&](int c, const double *zdev, double *const *o3) -> Err {
+    return rep_pipeline(P->cuda, R, [&](int c, const double *zdev, double *const *o3) -> Err {
         PostRepParams pp;
         pp.m = dm;
         pp.o = dO;
@@ -1964,16 +1894,10 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
         CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)posterior_smem_bytes<REP_TT>(true)));
         const int per_cta = REP_WARPS;
-        posterior_rep_kernel<REP_TT><<<(unsigned)((pp.n_blk + per_cta - 1) / per_cta), REP_WARPS * 32, smem, P->stream>>>(pp);
+        posterior_rep_kernel<REP_TT><<<(unsigned)((pp.n_blk + per_cta - 1) / per_cta), REP_WARPS * 32, smem, P->cuda.stream>>>(pp);
         CU(cudaGetLastError());
         return Err();
     });
-    if (!e.ok()) return e;
-    float ms = 0.f; // the coefficient pass counts as device time too
-    CU(cudaEventSynchronize(ev.b));
-    CU(cudaEventElapsedTime(&ms, ev.a, ev.b));
-    g_last_device_ms += ms;
-    return Err();
 }
 
 } // namespace ldsr
@@ -1996,15 +1920,12 @@ int ldsr_device_count(void) {
 
 int ldsr_ctx_create(int n_devices, const int *devices, ldsr_ctx **out, char *errbuf, int errlen) {
     if (!out) return report(fail(LDSR_ERR_ARG, "out is NULL"), errbuf, errlen);
-    const int have = ldsr_device_count();
-    if (have < 1)
-        return report(fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)"), errbuf, errlen);
-    if (n_devices <= 0) n_devices = have;
+    if (n_devices <= 0) n_devices = std::max(1, ldsr_device_count());
     std::unique_ptr<ldsr_ctx> c(new ldsr_ctx());
     for (int i = 0; i < n_devices; i++) {
         const int d = devices ? devices[i] : i;
-        if (d < 0 || d >= have)
-            return report(fail(LDSR_ERR_ARG, "device %d out of range (have %d)", d, have), errbuf, errlen);
+        Err e = check_device(d);
+        if (!e.ok()) return report(e, errbuf, errlen);
         c->devices.push_back(d);
         c->pools.emplace_back(new DevicePool(d));
     }
@@ -2032,7 +1953,9 @@ int ldsr_em_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int niter, double tol,
 
 int ldsr_plan_create(const ldsr_batch *batch, int device, ldsr_plan **out, char *errbuf, int errlen) {
     if (!out) return report(fail(LDSR_ERR_ARG, "out is NULL"), errbuf, errlen);
-    return report(plan_build(batch, device, nullptr, out), errbuf, errlen);
+    Err e = validate(batch);
+    if (e.ok()) e = plan_build(batch, device, nullptr, out);
+    return report(e, errbuf, errlen);
 }
 
 int ldsr_plan_em(ldsr_plan *plan, int niter, double tol, const ldsr_options *opt, void *stream, long long *stats,
@@ -2043,17 +1966,17 @@ int ldsr_plan_em(ldsr_plan *plan, int niter, double tol, const ldsr_options *opt
 }
 
 int ldsr_plan_set_theta0(ldsr_plan *plan, const double *theta0_host, char *errbuf, int errlen) {
-    if (!plan || !theta0_host) return report(fail(LDSR_ERR_ARG, "plan or theta0 is NULL"), errbuf, errlen);
-    cudaSetDevice(plan->device);
-    std::vector<double> th0((size_t)plan->n_fits * plan->TL);
-    for (int fi = 0; fi < plan->n_fits; fi++) {
-        const int s = plan->h_g_series[plan->h_f_group[fi]];
-        pad_theta(theta0_host + (size_t)plan->f_user[fi] * plan->theta_stride, plan->s_p[s], plan->s_q[s],
-                  plan->h_series[s].has_u != 0, plan->h_series[s].has_v != 0, plan->PQ, &th0[(size_t)fi * plan->TL]);
-    }
-    cudaError_t e = cudaMemcpy(plan->d_theta0, th0.data(), th0.size() * sizeof(double), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) return report(fail(LDSR_ERR_CUDA, "theta0 upload: %s", cudaGetErrorString(e)), errbuf, errlen);
-    return LDSR_OK;
+    auto run = [&]() -> Err {
+        if (!plan || !theta0_host) return fail(LDSR_ERR_ARG, "plan or theta0 is NULL");
+        CU(cudaSetDevice(plan->device));
+        // on the plan's stream: after the plan's own upload of theta0, and before its next ldsr_plan_em
+        const std::vector<double> th0 = padded_thetas(plan, theta0_host);
+        const cudaStream_t st = plan->cuda.stream;
+        CU(cudaMemcpyAsync(plan->d_theta0, th0.data(), th0.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));
+        return Err();
+    };
+    return report(run(), errbuf, errlen);
 }
 
 int ldsr_plan_fetch(ldsr_plan *plan, ldsr_em_result *out, char *errbuf, int errlen) {
@@ -2133,14 +2056,11 @@ void ldsr_r_rng_destroy(ldsr_r_rng *rng) { delete rng; }
 int ldsr_r_rnorm_device(int device, unsigned int seed, long long n, double *out, char *errbuf, int errlen) {
     auto run = [&]() -> Err {
         if (n < 1 || !out) return fail(LDSR_ERR_ARG, "need n >= 1 and out");
-        if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-        CU(cudaSetDevice(device));
+        Err e = use_device(device);
+        if (!e.ok()) return e;
+        Resources cuda;
         double *d = nullptr;
-        struct Guard {
-            double *&p;
-            ~Guard() { cudaFree(p); }
-        } guard{d};
-        CU(cudaMalloc(&d, sizeof(double) * (size_t)n));
+        CU(cuda.alloc(&d, (size_t)n));
         CU(r_rnorm_device(seed, n, d, 0));
         CU(cudaMemcpy(out, d, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost));
         return Err();
@@ -2197,17 +2117,15 @@ static Err construct_rec_stations(int device, int n_stations, const int *T, cons
         if (lambda) lam[s] = lambda[s];
     }
     const int n = member_ptr[n_stations];
-    if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-    CU(cudaSetDevice(device));
+    Err e = use_device(device);
+    if (!e.ok()) return e;
     const size_t nT = (size_t)rows, S = (size_t)n_stations;
-    double *d = nullptr;
-    struct Guard {
-        double *&p;
-        ~Guard() { cudaFree(p); }
-    } guard{d};
     // one arena: X V Y | C R | mu lambda | out | mean | row_off t_off (8-byte integers) | T member_ptr (ints)
     const size_t n_dbl = 3 * nT + 2 * (size_t)n + 2 * S + 6 * nT + 2 * (size_t)years + 2 * S;
-    CU(cudaMalloc(&d, sizeof(double) * n_dbl + sizeof(int) * (2 * S + 1)));
+    Resources cuda;
+    char *arena = nullptr;
+    CU(cuda.alloc(&arena, sizeof(double) * n_dbl + sizeof(int) * (2 * S + 1)));
+    double *d = reinterpret_cast<double *>(arena);
     double *dX = d, *dV = dX + nT, *dY = dV + nT, *dC = dY + nT, *dR = dC + n, *dmu = dR + n, *dlam = dmu + S;
     double *dO = dlam + S, *dM = dO + 6 * nT;
     long long *d_roff = reinterpret_cast<long long *>(dM + 2 * years), *d_toff = d_roff + S;
@@ -2284,32 +2202,19 @@ static Err cv_metrics_stations(int device, int n_stations, const int *n, const i
             held[(size_t)f_row[f] + i] = 1;
         }
     }
-    if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-    CU(cudaSetDevice(device));
+    Err e = use_device(device);
+    if (!e.ok()) return e;
+    Resources cuda;
     double *d_sim = nullptr, *d_obs = nullptr, *d_out = nullptr;
     unsigned char *d_held = nullptr;
     long long *d_off = nullptr;
     int *d_n = nullptr;
-    struct Guard {
-        double *&a, *&b, *&c;
-        unsigned char *&h;
-        long long *&o;
-        int *&n;
-        ~Guard() {
-            cudaFree(a);
-            cudaFree(b);
-            cudaFree(c);
-            cudaFree(h);
-            cudaFree(o);
-            cudaFree(n);
-        }
-    } guard{d_sim, d_obs, d_out, d_held, d_off, d_n};
-    CU(cudaMalloc(&d_sim, sizeof(double) * (size_t)n_sim));
-    CU(cudaMalloc(&d_obs, sizeof(double) * (size_t)n_obs));
-    CU(cudaMalloc(&d_out, sizeof(double) * (size_t)n_folds * 5));
-    CU(cudaMalloc(&d_held, held.size()));
-    CU(cudaMalloc(&d_off, sizeof(long long) * 2 * (size_t)n_folds));
-    CU(cudaMalloc(&d_n, sizeof(int) * (size_t)n_folds));
+    CU(cuda.alloc(&d_sim, (size_t)n_sim));
+    CU(cuda.alloc(&d_obs, (size_t)n_obs));
+    CU(cuda.alloc(&d_out, (size_t)n_folds * 5));
+    CU(cuda.alloc(&d_held, held.size()));
+    CU(cuda.alloc(&d_off, 2 * (size_t)n_folds));
+    CU(cuda.alloc(&d_n, (size_t)n_folds));
     CU(cudaMemcpy(d_sim, sim, sizeof(double) * (size_t)n_sim, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(d_obs, obs, sizeof(double) * (size_t)n_obs, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(d_held, held.data(), held.size(), cudaMemcpyHostToDevice));
@@ -2351,8 +2256,8 @@ int ldsr_smoother_d_batch(int device, int d, int T, int p, int q, const double *
         if (method != 0 && method != 1) return fail(LDSR_ERR_ARG, "method must be 0 (sequential) or 1 (scan)");
         for (int t = 0; t < T; t++)
             if (std::isinf(y[t])) return fail(LDSR_ERR_ARG, "y[%d] is +-Inf", t);
-        if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available (this library has no CPU path)");
-        CU(cudaSetDevice(device));
+        Err e = use_device(device);
+        if (!e.ok()) return e;
         ScanParams P;
         std::memset(&P, 0, sizeof P);
         P.n_fits = n_fits;
@@ -2381,78 +2286,55 @@ int ldsr_smoother_d_batch(int device, int d, int T, int p, int q, const double *
             P.L = L;
         }
         P.n_chunks = (T + P.L - 1) / P.L;
-        std::vector<void *> bufs;
-        struct Guard {
-            std::vector<void *> &b;
-            ~Guard() {
-                for (void *p : b) cudaFree(p);
-            }
-        } guard{bufs};
-        auto dalloc = [&](double **out, size_t n) -> cudaError_t {
-            void *ptr = nullptr;
-            cudaError_t e = cudaMalloc(&ptr, std::max<size_t>(n, 1) * sizeof(double));
-            if (e == cudaSuccess) {
-                bufs.push_back(ptr);
-                *out = static_cast<double *>(ptr);
-            }
-            return e;
-        };
+        Resources cuda;
         const size_t nT = (size_t)n_fits * T, D = d, nC = (size_t)n_fits * P.n_chunks;
         double *dy = nullptr, *du = nullptr, *dv_in = nullptr, *dth = nullptr;
-        CU(dalloc(&dy, T));
+        CU(cuda.alloc(&dy, T));
         CU(cudaMemcpy(dy, y, sizeof(double) * T, cudaMemcpyHostToDevice));
         if (u) {
-            CU(dalloc(&du, (size_t)T * p));
+            CU(cuda.alloc(&du, (size_t)T * p));
             CU(cudaMemcpy(du, u, sizeof(double) * (size_t)T * p, cudaMemcpyHostToDevice));
         }
         if (v) {
-            CU(dalloc(&dv_in, (size_t)T * q));
+            CU(cuda.alloc(&dv_in, (size_t)T * q));
             CU(cudaMemcpy(dv_in, v, sizeof(double) * (size_t)T * q, cudaMemcpyHostToDevice));
         }
         std::vector<double> th((size_t)n_fits * tl);
         for (int f = 0; f < n_fits; f++) std::memcpy(&th[(size_t)f * tl], theta + (size_t)f * theta_stride, sizeof(double) * tl);
-        CU(dalloc(&dth, th.size()));
+        CU(cuda.alloc(&dth, th.size()));
         CU(cudaMemcpy(dth, th.data(), sizeof(double) * th.size(), cudaMemcpyHostToDevice));
         P.y = dy;
         P.u = du;
         P.v = dv_in;
         P.theta = dth;
-        CU(dalloc(&P.c, nT * D));
-        CU(dalloc(&P.dv, nT));
-        CU(dalloc(&P.Xu, nT * D));
-        CU(dalloc(&P.Vu, nT * D * D));
-        CU(dalloc(&P.fagg, nC * (3 * D * D + 2 * D)));
-        CU(dalloc(&P.sagg, nC * (2 * D * D + D)));
-        CU(dalloc(&P.pre, nC * (D + D * D)));
-        CU(dalloc(&P.suf, nC * (D + D * D)));
-        CU(dalloc(&P.likp, nC * 2));
+        CU(cuda.alloc(&P.c, nT * D));
+        CU(cuda.alloc(&P.dv, nT));
+        CU(cuda.alloc(&P.Xu, nT * D));
+        CU(cuda.alloc(&P.Vu, nT * D * D));
+        CU(cuda.alloc(&P.fagg, nC * (3 * D * D + 2 * D)));
+        CU(cuda.alloc(&P.sagg, nC * (2 * D * D + D)));
+        CU(cuda.alloc(&P.pre, nC * (D + D * D)));
+        CU(cuda.alloc(&P.suf, nC * (D + D * D)));
+        CU(cuda.alloc(&P.likp, nC * 2));
         P.n_groups = scan_groups_for(P.n_chunks);
         if (const char *ev = std::getenv("LDSR_SCAN_GROUPS")) // development: 1 = one CTA per fit scans all chunks
             if (std::atoi(ev) == 1) P.n_groups = 1;
         if (P.n_groups > 1) {
             const size_t nG = (size_t)n_fits * P.n_groups;
-            CU(dalloc(&P.fgagg, nG * (3 * D * D + 2 * D)));
-            CU(dalloc(&P.fgpre, nG * (3 * D * D + 2 * D)));
-            CU(dalloc(&P.sgagg, nG * (2 * D * D + D)));
-            CU(dalloc(&P.sgsuf, nG * (2 * D * D + D)));
+            CU(cuda.alloc(&P.fgagg, nG * (3 * D * D + 2 * D)));
+            CU(cuda.alloc(&P.fgpre, nG * (3 * D * D + 2 * D)));
+            CU(cuda.alloc(&P.sgagg, nG * (2 * D * D + D)));
+            CU(cuda.alloc(&P.sgsuf, nG * (2 * D * D + D)));
         }
-        CU(dalloc(&P.X, nT * D));
-        CU(dalloc(&P.V, nT * D * D));
-        CU(dalloc(&P.Y, nT));
-        CU(dalloc(&P.lik, n_fits));
-        cudaEvent_t a, b;
-        CU(cudaEventCreate(&a));
-        CU(cudaEventCreate(&b));
-        CU(cudaEventRecord(a, nullptr));
-        cudaError_t le = scan_smoother_launch(d, P, nullptr);
-        cudaEventRecord(b, nullptr);
-        cudaError_t se = cudaEventSynchronize(b);
+        CU(cuda.alloc(&P.X, nT * D));
+        CU(cuda.alloc(&P.V, nT * D * D));
+        CU(cuda.alloc(&P.Y, nT));
+        CU(cuda.alloc(&P.lik, n_fits));
+        CU(cuda.start());
+        CU(scan_smoother_launch(d, P, nullptr));
+        CU(cuda.stop());
         float ms = 0.f;
-        cudaEventElapsedTime(&ms, a, b);
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-        CU(le);
-        CU(se);
+        CU(cuda.ms(0, 0, &ms));
         CU(cudaGetLastError());
         if (kernel_ms) *kernel_ms = ms;
         CU(cudaMemcpy(lik, P.lik, sizeof(double) * n_fits, cudaMemcpyDeviceToHost));
@@ -2467,30 +2349,24 @@ int ldsr_smoother_d_batch(int device, int d, int T, int p, int q, const double *
 int ldsr_measure_fp64_peak(int device, double *tflops, char *errbuf, int errlen) {
     auto run = [&]() -> Err {
         if (!tflops) return fail(LDSR_ERR_ARG, "tflops is NULL");
-        if (ldsr_device_count() < 1) return fail(LDSR_ERR_CUDA, "no CUDA device available");
-        CU(cudaSetDevice(device));
+        Err e = use_device(device);
+        if (!e.ok()) return e;
         cudaDeviceProp prop;
         CU(cudaGetDeviceProperties(&prop, device));
+        Resources cuda;
         double *d = nullptr;
-        CU(cudaMalloc(&d, 64));
-        cudaEvent_t a, b;
-        CU(cudaEventCreate(&a));
-        CU(cudaEventCreate(&b));
+        CU(cuda.alloc(&d, 8));
         const int blocks = prop.multiProcessorCount * 2, threads = 1024, iters = 4096;
         double best = 0.0;
         for (int rep = 0; rep < 6; rep++) {
-            CU(cudaEventRecord(a));
+            CU(cuda.start());
             dfma_peak_kernel<<<blocks, threads>>>(d, iters, 1.0000001, 1e-9);
-            CU(cudaEventRecord(b));
-            CU(cudaEventSynchronize(b));
+            CU(cuda.stop());
             float ms = 0.f;
-            CU(cudaEventElapsedTime(&ms, a, b));
+            CU(cuda.ms(rep, rep, &ms));
             const double fl = 2.0 * 64.0 * iters * (double)blocks * threads;
             if (rep > 0) best = std::max(best, fl / (ms * 1e-3) / 1e12);
         }
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-        cudaFree(d);
         *tflops = best;
         return Err();
     };
