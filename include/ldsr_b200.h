@@ -214,8 +214,50 @@ int ldsr_posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps,
                              unsigned long long seed, const double *mu, int transform, const double *lambda,
                              double *simX, double *simY, double *simQ, char *errbuf, int errlen);
 
+/* Drought statistics of conditioned replicates (beyond the reference), reduced on the device: the replicates of
+ * ldsr_posterior_rep_batch with the same arguments (the same draws bit for bit, from seed or from z), of which only
+ * a few numbers per replicate leave the device.  Let Q_t be a replicate's simQ and [lo, hi) its fit's range of steps
+ * (range[2f], range[2f+1] with 0 <= lo < hi <= T_f; range NULL: the whole series).
+ *   Moving-mean extremes, per window length w = windows[k] (1 <= w <= LDSR_STATS_MAX_WINDOW, at most
+ *   LDSR_STATS_MAX_WINDOWS of them): over every start t with lo <= t <= hi - w, the minimum and maximum of
+ *   (1/w) sum_{j<w} Q_{t+j} and their starts t; on a tie the smallest t.  w > hi - lo: NaN and start -1.
+ *   Runs below threshold[f] (finite, on the Q scale): a run is a maximal set of consecutive steps of the range
+ *   with Q_t < thr, clipped to the range.  run_len / run_at: the longest run's length and first step; deficit /
+ *   deficit_at: the largest sum over a run of (thr - Q_t) and that run's first step; n_runs: the number of runs.
+ *   On a tie the earliest run.  No run: length 0, deficit 0, steps -1, count 0.  threshold NULL: no run statistics
+ *   (their outputs must be NULL).
+ *   A replicate with a non-finite Q in its range (inverse Box-Cox of (y + mu) lambda + 1 < 0) has every double
+ *   output NaN and every int output (steps, length, count) -1.
+ * Outputs are structure-of-arrays in the caller's fit order, row n_reps*f + r; window outputs are
+ * [n_windows][n_fits*n_reps].  Any output may be NULL.  Steps are 0-based within the fit's series.  Arguments are
+ * checked before a device is touched (as ldsr_posterior_rep_batch's, plus the spec); one device (ctx device 0), no
+ * CPU fallback.  ldsr_last_device_ms covers the coefficient pass and the sampler. */
+#define LDSR_STATS_MAX_WINDOWS 4
+#define LDSR_STATS_MAX_WINDOW 64
+typedef struct {
+    int n_windows;           /* 0 .. LDSR_STATS_MAX_WINDOWS */
+    const int *windows;      /* [n_windows] */
+    const double *threshold; /* [n_fits] or NULL */
+    const int *range;        /* [2*n_fits] or NULL */
+} ldsr_stats_spec;
+typedef struct {
+    double *wmin;
+    int *wmin_at;
+    double *wmax;
+    int *wmax_at;
+    int *run_len;
+    int *run_at;
+    double *deficit;
+    int *deficit_at;
+    int *n_runs;
+} ldsr_stats_out;
+int ldsr_posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                               unsigned long long seed, const double *mu, int transform, const double *lambda,
+                               const ldsr_stats_spec *spec, const ldsr_stats_out *out, char *errbuf, int errlen);
+
 /* Device time in ms (CUDA events around the kernels, summed) of the last ldsr_rep_batch / ldsr_rep_batch_r /
- * ldsr_posterior_rep_batch call made by the calling thread: the measurement hook of bench.py's config-4 record. */
+ * ldsr_posterior_rep_batch / ldsr_posterior_stats_batch call made by the calling thread: the measurement hook of
+ * bench.py's config-4 record. */
 double ldsr_last_device_ms(void);
 
 /* ---- the reference's random numbers (R's default generators after set.seed) ---------------

@@ -22,7 +22,8 @@ EXPORTS = ("ldsr_abi_version", "ldsr_device_count", "ldsr_ctx_create", "ldsr_ctx
            "ldsr_smoother_d_batch", "ldsr_cv_metrics_batch", "ldsr_construct_rec_batch",
            "ldsr_objective_batch", "ldsr_rep_batch_r", "ldsr_r_rng_create", "ldsr_r_rng_unif", "ldsr_r_rng_norm",
            "ldsr_r_rng_sample", "ldsr_r_rng_destroy", "ldsr_r_rnorm_device", "ldsr_last_device_ms",
-           "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations", "ldsr_posterior_rep_batch")
+           "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations", "ldsr_posterior_rep_batch",
+           "ldsr_posterior_stats_batch")
 
 
 class LdsrError(RuntimeError):
@@ -41,6 +42,15 @@ class Batch(C.Structure):
 class EmResult(C.Structure):
     _fields_ = [("theta", _dp), ("lik", _dp), ("iters", _ip), ("status", _ip), ("liks", _dp),
                 ("best", _ip), ("X", _dp), ("Y", _dp), ("V", _dp), ("J", _dp)]
+
+
+class StatsSpec(C.Structure):
+    _fields_ = [("n_windows", C.c_int), ("windows", _ip), ("threshold", _dp), ("range", _ip)]
+
+
+class StatsOut(C.Structure):
+    _fields_ = [("wmin", _dp), ("wmin_at", _ip), ("wmax", _dp), ("wmax_at", _ip), ("run_len", _ip), ("run_at", _ip),
+                ("deficit", _dp), ("deficit_at", _ip), ("n_runs", _ip)]
 
 
 POLL_FN = C.CFUNCTYPE(C.c_int, C.c_void_p)
@@ -406,6 +416,54 @@ def posterior_rep_batch(series, group_series, held, fit_group, theta, n_reps, z=
            for k, o in outs.items() if o is not None}
     res["device_ms"] = float(lib().ldsr_last_device_ms())
     return res
+
+
+WINDOW_STATS = ("wmin", "wmin_at", "wmax", "wmax_at")
+RUN_STATS = ("run_len", "run_at", "deficit", "deficit_at", "n_runs")
+
+
+def posterior_stats_batch(series, group_series, held, fit_group, theta, n_reps, z=None, seed=0, mu=None,
+                          transform="log", lams=None, windows=(10,), threshold=None, ranges=None, want=None, ctx=None):
+    """ldsr_posterior_stats_batch: the drought statistics of posterior_rep_batch's replicates (same arguments, the
+    same draws), reduced on the device.  windows: up to 4 moving-mean lengths in 1..64; threshold: per fit, on the Q
+    scale (None: no run statistics); ranges: [n_fits, 2] step ranges [lo, hi) (None: whole series).  want: the
+    outputs to return (default: all that the spec defines).  Returns window outputs shaped [n_windows, n_fits,
+    n_reps], run outputs [n_fits, n_reps] (steps as int32, -1 where undefined), and the device time."""
+    pb = PackedBatch(series, group_series, held, fit_group, theta)
+    nf, n_reps = pb.n_fits, int(n_reps)
+    zz = None
+    if z is not None:
+        zz = np.ascontiguousarray(z, dtype=np.float64).ravel()
+        if zz.size != 2 * int(pb.fit_ptr[-1]) * n_reps:
+            raise ValueError("z must hold 2 * n_reps * sum(T) = %d values" % (2 * int(pb.fit_ptr[-1]) * n_reps))
+    code = TRANSFORMS[transform] if isinstance(transform, str) else int(transform)
+    mu_a = None if mu is None else np.ascontiguousarray(np.broadcast_to(np.asarray(mu, dtype=np.float64), (nf,)))
+    lam_a = None if lams is None else np.ascontiguousarray(np.broadcast_to(np.asarray(lams, dtype=np.float64), (nf,)))
+    win = np.ascontiguousarray(np.atleast_1d(np.asarray(windows if windows is not None else (), dtype=np.int32)))
+    thr = None if threshold is None else np.ascontiguousarray(
+        np.broadcast_to(np.asarray(threshold, dtype=np.float64), (nf,)))
+    rng = None if ranges is None else np.ascontiguousarray(np.broadcast_to(np.asarray(ranges, dtype=np.int32),
+                                                                           (nf, 2)))
+    if want is None:
+        want = WINDOW_STATS + (RUN_STATS if thr is not None else ())
+    nw = win.size
+    outs = {}
+    for k in WINDOW_STATS:
+        if k in want:
+            outs[k] = np.empty((nw, nf, n_reps), dtype=np.int32 if k.endswith("_at") else np.float64)
+    for k in RUN_STATS:
+        if k in want:
+            outs[k] = np.empty((nf, n_reps), dtype=np.float64 if k == "deficit" else np.int32)
+    spec = StatsSpec(nw, _i(win) if nw else None, _d(thr), _i(rng))
+    out = StatsOut(*(_d(outs.get(k)) if k in ("wmin", "wmax", "deficit") else _i(outs.get(k))
+                     for k, _ in StatsOut._fields_))
+    err = C.create_string_buffer(512)
+    rc = lib().ldsr_posterior_stats_batch(ctx.h if isinstance(ctx, Ctx) else ctx, C.byref(pb.c), n_reps, _d(zz),
+                                          C.c_ulonglong(int(seed)), _d(mu_a), code, _d(lam_a), C.byref(spec),
+                                          C.byref(out), err, 512)
+    _check(rc, err)
+    outs["device_ms"] = float(lib().ldsr_last_device_ms())
+    return outs
 
 
 class RRandom:

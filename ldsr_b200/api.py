@@ -550,6 +550,54 @@ def LDS_rep_posterior(theta, Qa, u, v, start_year, transform="log", num_reps=100
     return out[0] if S["single"] else out
 
 
+def LDS_rep_posterior_stats(theta, Qa, u, v, start_year, transform="log", num_reps=100, seed=0, z=None, windows=(10,),
+                            threshold=None, period=None):
+    """Drought statistics of LDS_rep_posterior's replicates (the same arguments give the same draws), computed on the
+    device in the sampler's walk, so that no trajectory is written or copied: a few numbers per replicate instead of
+    whole series, which makes 10^6 replicates and more practical for tail probabilities.
+    windows: up to 4 moving-mean lengths of 1..64 years: per replicate the lowest and highest w-year mean flow and
+    the first year of that window (the earliest on a tie).  threshold: flow (Q scale) below which a year is in
+    drought; None means the mean of the observed Qa.  A run is a maximal stretch of years below it: per replicate
+    the longest run (years, first year), the largest run deficit sum(threshold - Q) (value, first year) and the
+    number of runs, the earliest run on a tie.  period = (first_year, last_year) restricts every statistic to those
+    years (runs are clipped to it); None: the whole horizon.  Undefined values (a window longer than the period, no
+    run) are NaN / year -1 / 0; a replicate with a non-finite flow in the period (Box-Cox) has NaN and -1 throughout.
+    Returns a dict with windows, threshold, period and arrays over replicates: wmin, wmin_year, wmax, wmax_year
+    ([n_windows, num_reps]), run_len, run_year, deficit, deficit_year, n_runs ([num_reps]); one dict per member for
+    an ensemble.  One device call."""
+    S = _station(dict(Qa=Qa, u=u, v=v, start_year=start_year), transform)
+    thetas = [theta] if S["single"] else list(theta)
+    if len(thetas) != len(S["series"]):
+        raise ValueError("theta must be one model per ensemble member (%d)" % len(S["series"]))
+    rows = [theta_to_vec(t) for t in thetas]
+    stride = max(s["p"] + s["q"] + 6 for s in S["series"])
+    for s, r in zip(S["series"], rows):
+        if r.size != s["p"] + s["q"] + 6:
+            raise ValueError("theta has %d entries, the member's inputs need %d" % (r.size, s["p"] + s["q"] + 6))
+    years = np.asarray(S["years"])
+    y0 = int(years[0])
+    if period is None:
+        lo, hi = 0, years.size
+    else:
+        lo, hi = int(period[0]) - y0, int(period[1]) - y0 + 1
+        if not (0 <= lo < hi <= years.size):
+            raise ValueError("period %r is not inside %d..%d" % (tuple(period), y0, int(years[-1])))
+    thr = float(np.mean(np.asarray(Qa["Qa"], dtype=float))) if threshold is None else float(threshold)
+    n = len(rows)
+    r = _lib.posterior_stats_batch(S["series"], np.arange(n), None, np.arange(n),
+                                   np.stack([np.pad(v, (0, stride - v.size)) for v in rows]), num_reps, z=z, seed=seed,
+                                   mu=np.full(n, S["mu"]), transform=transform,
+                                   lams=None if transform != "boxcox" else np.full(n, S["lam"]), windows=windows,
+                                   threshold=np.full(n, thr), ranges=np.tile([lo, hi], (n, 1)))
+    year = lambda a: np.where(a >= 0, a + y0, -1)
+    out = [dict(windows=tuple(int(w) for w in windows), threshold=thr, period=(y0 + lo, y0 + hi - 1),
+                wmin=r["wmin"][:, k], wmin_year=year(r["wmin_at"][:, k]), wmax=r["wmax"][:, k],
+                wmax_year=year(r["wmax_at"][:, k]), run_len=r["run_len"][k], run_year=year(r["run_at"][k]),
+                deficit=r["deficit"][k], deficit_year=year(r["deficit_at"][k]), n_runs=r["n_runs"][k])
+           for k in range(n)]
+    return out[0] if S["single"] else out
+
+
 def one_LDS_rep(rep_num, theta, u=None, v=None, years=None, mu=0.0, exp_trans=True, seed=0, z=None):
     """R/stochastics.R:18-47."""
     out = LDS_rep(theta, u, v, years, 1, mu, exp_trans, seed=seed + rep_num, z=None if z is None else z[None, :])

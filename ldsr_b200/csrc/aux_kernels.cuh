@@ -431,6 +431,8 @@ template <int PQ> __global__ void __launch_bounds__(REP_WARPS * 32) rep_kernel(c
 // The width of the inputs does not enter (D v is in o): one instantiation, compiled where it is
 // launched (a template, so that the per-width units do not carry it).
 // ------------------------------------------------------------------------------------------
+constexpr int POST_MAX_WIN = 4;   // windows per statistics call (LDSR_STATS_MAX_WINDOWS)
+constexpr int POST_MAX_RING = 64; // longest window (LDSR_STATS_MAX_WINDOW): the Q ring covers the last 64 steps
 struct PostRepParams {
     const double *m, *o, *s, *J;  // coefficient rows, fit f's T_f steps at fit_ptr[f]
     const long long *fit_ptr;     // [n_fits + 1]
@@ -444,6 +446,15 @@ struct PostRepParams {
     long long out0;               // output offset of the launch's first element (outputs are written at - out0)
     int transform;                // 0 none, 1 log, 2 Box-Cox
     double *simX, *simY, *simQ;   // any may be null
+    // statistics mode (posterior_rep_kernel<TT, true>, one launch, blk0 = out0 = 0): per (fit, replicate) row
+    // n_reps f + r, window k's outputs at k n_rows + row; any output may be null
+    int n_win, win[POST_MAX_WIN]; // moving-mean window lengths, 1 .. POST_MAX_RING
+    int ring;                     // Q ring slots per lane: a power of two >= every window (0 without windows)
+    long long n_rows;             // n_fits n_reps
+    const int *range;             // [n_fits][2]: the statistics range [lo, hi) of steps
+    const double *thr;            // [n_fits] run threshold on the Q scale, or null (no run statistics)
+    double *wmin, *wmax, *deficit;
+    int *wmin_at, *wmax_at, *run_len, *run_at, *deficit_at, *n_runs;
 };
 
 __device__ __forceinline__ unsigned long long posterior_key(unsigned long long seed, int fit, long long rep) {
@@ -454,8 +465,18 @@ __device__ __forceinline__ unsigned long long posterior_key(unsigned long long s
 template <int TT> __host__ __device__ inline size_t posterior_smem_bytes(bool with_z) {
     return (size_t)REP_WARPS * ((3 + (with_z ? 2 : 0)) * TT * 33 + 4 * TT) * sizeof(double);
 }
+// statistics mode: no output tiles; the noise tiles (with z), the coefficient tile and the lanes' Q rings
+template <int TT> __host__ __device__ inline size_t posterior_stats_smem_bytes(bool with_z, int ring) {
+    return (size_t)REP_WARPS * ((with_z ? 2 : 0) * TT * 33 + 4 * TT + 32 * ring) * sizeof(double);
+}
 
-template <int TT> __global__ void __launch_bounds__(REP_WARPS * 32) posterior_rep_kernel(const PostRepParams P) {
+// STATS = false: the trajectories (simX, simY, simQ).  STATS = true: the same draws, reduced in the walk to each
+// replicate's drought statistics over its fit's range [lo, hi) (ldsr_posterior_stats_batch); no trajectory leaves
+// the SM.  Both modes run the one step body below, so a replicate's Q_t is the same value in either.
+// The statistics mode's accumulators take it to 168 registers: three CTAs an SM, stated so that ptxas does not cap
+// it at 128 and spill (0 leaves the trajectory mode to ptxas's default, 96).
+template <int TT, bool STATS = false>
+__global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_kernel(const PostRepParams P) {
     static_assert(32 % TT == 0 && TT <= 16, "a tile's mask bits sit in one word; a half-warp loads a tile row");
     LDSR_DYN_SMEM(smem_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -466,10 +487,12 @@ template <int TT> __global__ void __launch_bounds__(REP_WARPS * 32) posterior_re
     const int n_rows = P.n_reps - r0 < 32 ? P.n_reps - r0 : 32;
     const bool have_z = P.z != nullptr;
     constexpr int TILE = TT * 33;
-    double *const tiles = reinterpret_cast<double *>(smem_raw) + (size_t)warp * ((3 + (have_z ? 2 : 0)) * TILE + 4 * TT);
+    constexpr int N_OUT = STATS ? 0 : 3; // output tiles
+    double *const tiles = reinterpret_cast<double *>(smem_raw) +
+                          (size_t)warp * ((N_OUT + (have_z ? 2 : 0)) * TILE + 4 * TT + (STATS ? 32 * P.ring : 0));
     double *const tX = tiles, *const tY = tiles + TILE, *const tQ = tiles + 2 * TILE;
-    double *const tZq = tiles + 3 * TILE, *const tZe = tiles + 4 * TILE;
-    double *const tC = tiles + (3 + (have_z ? 2 : 0)) * TILE; // [m | s | o | J] of the tile's steps
+    double *const tZq = tiles + N_OUT * TILE, *const tZe = tiles + (N_OUT + 1) * TILE;
+    double *const tC = tiles + (N_OUT + (have_z ? 2 : 0)) * TILE; // [m | s | o | J] of the tile's steps
     const long long fp = P.fit_ptr[f];
     const int T = (int)(P.fit_ptr[f + 1] - fp);
     const unsigned *__restrict__ mw = P.masks + P.f_mask_off[f];
@@ -479,13 +502,40 @@ template <int TT> __global__ void __launch_bounds__(REP_WARPS * 32) posterior_re
     const long long base = (long long)P.n_reps * fp + (long long)r0 * T - P.out0; // row rr at base + rr T
     const unsigned long long key = posterior_key(P.seed, f, r0 + lane); // lanes >= n_rows: never stored
     const int half = lane >> 4, hl = lane & 15;
+    // statistics state, one replicate per lane.  The walk runs downwards, so at step t the window starting at t is
+    // complete: its sum gains Q_t and loses Q_{t+w}, read from the lane's ring (slot (t mod ring) of column `lane`)
+    // before Q_t takes that slot.  Updating on <= / >= lets the smaller start, and the earlier run, win ties.
+    double *const ring = tC + 4 * TT + lane;
+    const int rmask = P.ring - 1;
+    const int rlo = STATS ? P.range[2 * f] : 0, rhi = STATS ? P.range[2 * f + 1] : 0;
+    const bool runs = STATS && P.thr != nullptr;
+    const double thr = runs ? P.thr[f] : 0.0;
+    double wsum[POST_MAX_WIN], wmn[POST_MAX_WIN], wmx[POST_MAX_WIN];
+    int wmn_at[POST_MAX_WIN], wmx_at[POST_MAX_WIN];
+#pragma unroll
+    for (int k = 0; k < POST_MAX_WIN; k++) {
+        wsum[k] = 0.0;
+        wmn[k] = INFINITY;
+        wmx[k] = -INFINITY;
+        wmn_at[k] = wmx_at[k] = -1;
+    }
+    int cur_len = 0, best_len = 0, best_len_at = -1, best_def_at = -1, n_runs = 0;
+    double cur_def = 0.0, best_def = 0.0;
+    bool finite = true;
+    auto close_run = [&](int first) {
+        n_runs++;
+        if (cur_len >= best_len) best_len = cur_len, best_len_at = first;
+        if (cur_def >= best_def) best_def = cur_def, best_def_at = first;
+        cur_len = 0;
+        cur_def = 0.0;
+    };
     // the coefficients of a tile: half-warp 0 loads m and o, half-warp 1 s and J (128 contiguous bytes each); the
     // next tile's are in flight while this one's chain runs, then read back from shared memory as broadcasts
     const double *__restrict__ ca = (half ? P.s : P.m) + fp, *__restrict__ cb = (half ? P.J : P.o) + fp;
     int lo = ((T - 1) / TT) * TT;
     double na = hl < T - lo ? ca[lo + hl] : 0.0, nb = hl < T - lo ? cb[lo + hl] : 0.0;
     double x1 = 0.0; // x_{t+1}
-    for (; lo >= 0; lo -= TT) {
+    for (; lo >= 0 && (!STATS || lo + TT > rlo); lo -= TT) { // statistics: no tile below the range
         const int cnt = T - lo < TT ? T - lo : TT;
         tC[half * TT + hl] = na;
         tC[(2 + half) * TT + hl] = nb;
@@ -515,23 +565,75 @@ template <int TT> __global__ void __launch_bounds__(REP_WARPS * 32) posterior_re
             const double x = fma(tC[TT + j], zq, fma(tC[3 * TT + j], x1, tC[j]));
             const double y = (bits >> j) & 1u ? tC[2 * TT + j] : fma(sR, ze, fma(C, x, tC[2 * TT + j]));
             const double yq = y + mu;
-            tX[j * 33 + lane] = x;
-            tY[j * 33 + lane] = y;
-            tQ[j * 33 + lane] = tr == 1 ? exp(yq) : (tr == 0 ? yq : pow(fma(yq, lam, 1.0), il));
+            const double q = tr == 1 ? exp(yq) : (tr == 0 ? yq : pow(fma(yq, lam, 1.0), il));
+            if (!STATS) {
+                tX[j * 33 + lane] = x;
+                tY[j * 33 + lane] = y;
+                tQ[j * 33 + lane] = q;
+            }
             x1 = x;
+            if (!STATS) continue;
+            const int t = lo + j;
+            if (t < rlo || t >= rhi) continue;
+            finite = finite && fabs(q) < INFINITY; // false for NaN and +-Inf
+            const int seen = rhi - t; // steps of the range walked so far, t included
+#pragma unroll
+            for (int k = 0; k < POST_MAX_WIN; k++) {
+                if (k >= P.n_win) break;
+                const int w = P.win[k];
+                double sum = wsum[k] + q;
+                if (seen > w) sum -= ring[((t + w) & rmask) * 32]; // Q_{t+w} leaves the window
+                wsum[k] = sum;
+                if (seen >= w) {
+                    if (sum <= wmn[k]) wmn[k] = sum, wmn_at[k] = t;
+                    if (sum >= wmx[k]) wmx[k] = sum, wmx_at[k] = t;
+                }
+            }
+            if (P.n_win > 0) ring[(t & rmask) * 32] = q;
+            if (runs) {
+                if (q < thr) {
+                    cur_len++;
+                    cur_def += thr - q;
+                } else if (cur_len > 0) {
+                    close_run(t + 1);
+                }
+            }
         }
-        __syncwarp();
-        // each half-warp writes one replicate row of the tile (up to 128 contiguous bytes) per instruction
-        for (int rr = half; rr < n_rows; rr += 2) {
-            if (hl < cnt) {
-                const long long off = base + (long long)rr * T + lo + hl;
-                if (P.simX) P.simX[off] = tX[hl * 33 + rr];
-                if (P.simY) P.simY[off] = tY[hl * 33 + rr];
-                if (P.simQ) P.simQ[off] = tQ[hl * 33 + rr];
+        if (!STATS) {
+            __syncwarp();
+            // each half-warp writes one replicate row of the tile (up to 128 contiguous bytes) per instruction
+            for (int rr = half; rr < n_rows; rr += 2) {
+                if (hl < cnt) {
+                    const long long off = base + (long long)rr * T + lo + hl;
+                    if (P.simX) P.simX[off] = tX[hl * 33 + rr];
+                    if (P.simY) P.simY[off] = tY[hl * 33 + rr];
+                    if (P.simQ) P.simQ[off] = tQ[hl * 33 + rr];
+                }
             }
         }
         __syncwarp();
     }
+    if (!STATS || lane >= n_rows) return;
+    if (cur_len > 0) close_run(rlo); // a run reaching the range's lower end
+    // one row per lane: consecutive rows across the warp
+    const long long row = (long long)P.n_reps * f + r0 + lane;
+#pragma unroll
+    for (int k = 0; k < POST_MAX_WIN; k++) {
+        if (k >= P.n_win) break;
+        const double w = P.win[k];
+        const bool ok = finite && wmn_at[k] >= 0;
+        const long long o = k * P.n_rows + row;
+        if (P.wmin) P.wmin[o] = ok ? wmn[k] / w : NAN;
+        if (P.wmin_at) P.wmin_at[o] = ok ? wmn_at[k] : -1;
+        if (P.wmax) P.wmax[o] = ok ? wmx[k] / w : NAN;
+        if (P.wmax_at) P.wmax_at[o] = ok ? wmx_at[k] : -1;
+    }
+    if (!runs) return;
+    if (P.run_len) P.run_len[row] = finite ? best_len : -1;
+    if (P.run_at) P.run_at[row] = finite ? best_len_at : -1;
+    if (P.deficit) P.deficit[row] = finite ? best_def : NAN;
+    if (P.deficit_at) P.deficit_at[row] = finite ? best_def_at : -1;
+    if (P.n_runs) P.n_runs[row] = finite ? n_runs : -1;
 }
 
 } // namespace ldsr

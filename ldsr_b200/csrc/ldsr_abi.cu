@@ -1493,8 +1493,8 @@ static Err em_batch(ldsr_ctx *ctx, const ldsr_batch *b, int niter, double tol, c
     return Err();
 }
 
-// device time (CUDA events) of the replicate kernels of the last ldsr_rep_batch* / ldsr_posterior_rep_batch call of
-// this thread (ldsr_last_device_ms)
+// device time (CUDA events) of the replicate kernels of the last ldsr_rep_batch* / ldsr_posterior_rep_batch /
+// ldsr_posterior_stats_batch call of this thread (ldsr_last_device_ms)
 static thread_local double g_last_device_ms = 0.0;
 
 // ---- single-step batched entry points (one device: ctx device 0) ----------------------------
@@ -1804,16 +1804,16 @@ static Err rep_batch(ldsr_ctx *ctx, const double *theta, const double *u, const 
 }
 
 // ---- replicates conditioned on the observed record (forward filtering, backward sampling) -----
-static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
-                               unsigned long long seed, const double *mu, int transform, const double *lambda,
-                               double *simX, double *simY, double *simQ) {
+// The argument checks of the conditioned replicates (no device touched) and the per-fit table C, sqrt(R), mu, lambda.
+static Err posterior_args(const ldsr_batch *b, int n_reps, const double *mu, int transform, const double *lambda,
+                          std::vector<double> &par) {
     Err e = validate(b);
     if (!e.ok()) return e;
     if (n_reps < 1) return fail(LDSR_ERR_ARG, "n_reps=%d, need n_reps >= 1", n_reps);
     if (transform < 0 || transform > 2) return fail(LDSR_ERR_ARG, "transform=%d, need 0 (none), 1 (log) or 2 (Box-Cox)", transform);
     if (transform == 2 && !lambda) return fail(LDSR_ERR_ARG, "transform 2 (Box-Cox) needs lambda");
     const int nf = b->n_fits;
-    std::vector<double> par((size_t)4 * nf);
+    par.assign((size_t)4 * nf, 0.0);
     for (int f = 0; f < nf; f++) {
         const int s = b->group_series[b->fit_group[f]];
         const double *th = b->theta0 + (size_t)f * b->theta_stride;
@@ -1824,17 +1824,33 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
         par[4 * f + 2] = mu ? mu[f] : 0.0;
         par[4 * f + 3] = transform == 2 ? lambda[f] : 0.0;
     }
+    return Err();
+}
+
+// The device half of the set-up both conditioned-replicate entry points share: the plan, the backward-sampling
+// coefficient rows (smoother_kernel's coefficient mode, timed on the plan's Resources), and every PostRepParams
+// field but the launch range, the noise and the outputs.
+struct PosteriorSetup {
     std::unique_ptr<ldsr_ctx> tmp_ctx;
-    if (!(e = default_ctx(ctx, tmp_ctx)).ok()) return e;
+    std::unique_ptr<ldsr_plan> plan;
+    PostRepParams pp{};
+    std::vector<long long> fit_ptr; // user order, as ldsr_smoother_batch's rows
+};
+
+static Err posterior_setup(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, unsigned long long seed, int transform,
+                           const std::vector<double> &par, PosteriorSetup &S) {
+    Err e = default_ctx(ctx, S.tmp_ctx);
+    if (!e.ok()) return e;
     ldsr_plan *P = nullptr;
     if (!(e = plan_build(b, ctx->devices[0], ctx->pools[0].get(), &P)).ok()) return e;
-    std::unique_ptr<ldsr_plan> guard(P);
+    S.plan.reset(P);
     Resources &cuda = P->cuda;
+    const int nf = b->n_fits;
     // per USER fit: its group's first mask word
     std::vector<long long> f_mask_off(nf);
     for (int fi = 0; fi < nf; fi++) f_mask_off[P->f_user[fi]] = P->h_g_mask_off[P->h_f_group[fi]];
-    const std::vector<long long> &fit_ptr = P->fit_row_user;
-    const size_t tot = (size_t)fit_ptr[nf];
+    S.fit_ptr = P->fit_row_user;
+    const size_t tot = (size_t)S.fit_ptr[nf];
     double *dm, *dO, *ds, *dJ, *d_par;
     int *d_jt;
     long long *d_jr, *d_fit_ptr, *d_fmo;
@@ -1844,7 +1860,7 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
     CU(cuda.alloc(&dJ, tot));
     CU(cuda.upload(&d_jt, P->fit_job_theta));
     CU(cuda.upload(&d_jr, P->fit_job_row));
-    CU(cuda.upload(&d_fit_ptr, fit_ptr));
+    CU(cuda.upload(&d_fit_ptr, S.fit_ptr));
     CU(cuda.upload(&d_fmo, f_mask_off));
     CU(cuda.upload(&d_par, par));
     // the coefficient rows (user order, as ldsr_smoother_batch): m, o, s, J
@@ -1853,8 +1869,34 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
     CU(cuda.start()); // the coefficient pass counts as device time too
     CU(P->kt->smoother_coef(sp, cuda.stream));
     CU(cuda.stop());
-    // warps: (fit, 32 replicates) blocks in output order; a chunk is a range of whole blocks (~48 MB per output)
-    const int wpf = (n_reps + 31) / 32;
+    PostRepParams &pp = S.pp;
+    pp.m = dm;
+    pp.o = dO;
+    pp.s = ds;
+    pp.J = dJ;
+    pp.fit_ptr = d_fit_ptr;
+    pp.par = d_par;
+    pp.masks = P->d_masks;
+    pp.f_mask_off = d_fmo;
+    pp.seed = seed;
+    pp.n_reps = n_reps;
+    pp.wpf = (n_reps + 31) / 32; // warps: (fit, 32 replicates) blocks in output order
+    pp.transform = transform;
+    return Err();
+}
+
+static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
+                               unsigned long long seed, const double *mu, int transform, const double *lambda,
+                               double *simX, double *simY, double *simQ) {
+    std::vector<double> par;
+    Err e = posterior_args(b, n_reps, mu, transform, lambda, par);
+    if (!e.ok()) return e;
+    PosteriorSetup S;
+    if (!(e = posterior_setup(ctx, b, n_reps, seed, transform, par, S)).ok()) return e;
+    const int nf = b->n_fits;
+    const std::vector<long long> &fit_ptr = S.fit_ptr;
+    // a chunk is a range of whole (fit, 32 replicates) blocks (~48 MB per output)
+    const int wpf = S.pp.wpf;
     const long long n_blk = (long long)nf * wpf;
     auto blk_end = [&](long long k) { // output offset just past block k
         const int f = (int)(k / wpf), r1 = std::min(n_reps, (int)(k % wpf) * 32 + 32);
@@ -1869,24 +1911,13 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
             R.lo.push_back(blk_end(k));
             R.zlo.push_back(2 * blk_end(k));
         }
-    return rep_pipeline(P->cuda, R, [&](int c, const double *zdev, double *const *o3) -> Err {
-        PostRepParams pp;
-        pp.m = dm;
-        pp.o = dO;
-        pp.s = ds;
-        pp.J = dJ;
-        pp.fit_ptr = d_fit_ptr;
-        pp.par = d_par;
-        pp.masks = P->d_masks;
-        pp.f_mask_off = d_fmo;
+    Resources &cuda = S.plan->cuda;
+    return rep_pipeline(cuda, R, [&](int c, const double *zdev, double *const *o3) -> Err {
+        PostRepParams pp = S.pp;
         pp.z = zdev;
-        pp.seed = seed;
-        pp.n_reps = n_reps;
-        pp.wpf = wpf;
         pp.blk0 = c < 0 ? 0 : cb[c];
         pp.n_blk = c < 0 ? n_blk : cb[c + 1] - cb[c];
         pp.out0 = c < 0 ? 0 : (long long)R.lo[c];
-        pp.transform = transform;
         pp.simX = o3[0];
         pp.simY = o3[1];
         pp.simQ = o3[2];
@@ -1894,10 +1925,110 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
         CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)posterior_smem_bytes<REP_TT>(true)));
         const int per_cta = REP_WARPS;
-        posterior_rep_kernel<REP_TT><<<(unsigned)((pp.n_blk + per_cta - 1) / per_cta), REP_WARPS * 32, smem, P->cuda.stream>>>(pp);
+        posterior_rep_kernel<REP_TT><<<(unsigned)((pp.n_blk + per_cta - 1) / per_cta), REP_WARPS * 32, smem, cuda.stream>>>(pp);
         CU(cudaGetLastError());
         return Err();
     });
+}
+
+// ---- drought statistics of the conditioned replicates, reduced in the sampler's walk -------------------------
+static Err posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
+                                 unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                 const ldsr_stats_spec *spec, const ldsr_stats_out *out) {
+    std::vector<double> par;
+    Err e = posterior_args(b, n_reps, mu, transform, lambda, par);
+    if (!e.ok()) return e;
+    if (!spec || !out) return fail(LDSR_ERR_ARG, "spec and out are required");
+    const int nw = spec->n_windows, nf = b->n_fits;
+    if (nw < 0 || nw > LDSR_STATS_MAX_WINDOWS)
+        return fail(LDSR_ERR_ARG, "n_windows=%d, need 0 .. %d", nw, LDSR_STATS_MAX_WINDOWS);
+    if (nw > 0 && !spec->windows) return fail(LDSR_ERR_ARG, "windows is NULL");
+    int wmax = 0;
+    for (int k = 0; k < nw; k++) {
+        const int w = spec->windows[k];
+        if (w < 1 || w > LDSR_STATS_MAX_WINDOW)
+            return fail(LDSR_ERR_ARG, "windows[%d]=%d, need 1 .. %d", k, w, LDSR_STATS_MAX_WINDOW);
+        wmax = std::max(wmax, w);
+    }
+    if (nw == 0 && !spec->threshold) return fail(LDSR_ERR_ARG, "no statistics asked for: no window and no threshold");
+    if (!spec->threshold && (out->run_len || out->run_at || out->deficit || out->deficit_at || out->n_runs))
+        return fail(LDSR_ERR_ARG, "run outputs need a threshold");
+    std::vector<int> range((size_t)2 * nf);
+    for (int f = 0; f < nf; f++) {
+        const int T = b->T[b->group_series[b->fit_group[f]]];
+        const int lo = spec->range ? spec->range[2 * f] : 0, hi = spec->range ? spec->range[2 * f + 1] : T;
+        if (!(0 <= lo && lo < hi && hi <= T))
+            return fail(LDSR_ERR_ARG, "fit %d: range [%d, %d), need 0 <= lo < hi <= T = %d", f, lo, hi, T);
+        if (spec->threshold && !std::isfinite(spec->threshold[f]))
+            return fail(LDSR_ERR_ARG, "fit %d: threshold %g is not finite", f, spec->threshold[f]);
+        range[2 * f] = lo;
+        range[2 * f + 1] = hi;
+    }
+    PosteriorSetup S;
+    if (!(e = posterior_setup(ctx, b, n_reps, seed, transform, par, S)).ok()) return e;
+    Resources &cuda = S.plan->cuda;
+    const long long rows = (long long)nf * n_reps, wrows = rows * nw;
+    PostRepParams pp = S.pp;
+    pp.blk0 = 0;
+    pp.n_blk = (long long)nf * pp.wpf;
+    pp.out0 = 0;
+    if (z) { // the test and parity path: the whole noise array at once
+        double *dz;
+        const size_t nz = 2 * (size_t)n_reps * (size_t)S.fit_ptr[nf];
+        CU(cuda.alloc(&dz, nz));
+        CU(cudaMemcpyAsync(dz, z, nz * sizeof(double), cudaMemcpyHostToDevice, cuda.stream));
+        pp.z = dz;
+    }
+    pp.n_win = nw;
+    for (int k = 0; k < nw; k++) pp.win[k] = spec->windows[k];
+    pp.ring = 1;
+    while (pp.ring < wmax) pp.ring *= 2;
+    if (nw == 0) pp.ring = 0;
+    pp.n_rows = rows;
+    int *d_range;
+    CU(cuda.upload(&d_range, range));
+    pp.range = d_range;
+    if (spec->threshold) {
+        double *d_thr;
+        CU(cuda.upload(&d_thr, std::vector<double>(spec->threshold, spec->threshold + nf)));
+        pp.thr = d_thr;
+    }
+    // device outputs of the requested statistics, copied into the caller's arrays once the kernel is done
+    std::vector<std::function<cudaError_t()>> copies;
+    auto out_block = [&](auto **dev, auto *host, long long n) -> cudaError_t {
+        *dev = nullptr;
+        if (!host) return cudaSuccess;
+        cudaError_t ce = cuda.alloc(dev, (size_t)n);
+        if (ce == cudaSuccess) {
+            auto *d = *dev;
+            copies.push_back([=, &cuda] {
+                return cudaMemcpyAsync(host, d, (size_t)n * sizeof(*host), cudaMemcpyDeviceToHost, cuda.stream);
+            });
+        }
+        return ce;
+    };
+    CU(out_block(&pp.wmin, out->wmin, wrows));
+    CU(out_block(&pp.wmin_at, out->wmin_at, wrows));
+    CU(out_block(&pp.wmax, out->wmax, wrows));
+    CU(out_block(&pp.wmax_at, out->wmax_at, wrows));
+    CU(out_block(&pp.run_len, out->run_len, rows));
+    CU(out_block(&pp.run_at, out->run_at, rows));
+    CU(out_block(&pp.deficit, out->deficit, rows));
+    CU(out_block(&pp.deficit_at, out->deficit_at, rows));
+    CU(out_block(&pp.n_runs, out->n_runs, rows));
+    const size_t smem = posterior_stats_smem_bytes<REP_TT>(z != nullptr, pp.ring);
+    CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)posterior_stats_smem_bytes<REP_TT>(true, POST_MAX_RING)));
+    CU(cuda.start());
+    posterior_rep_kernel<REP_TT, true>
+        <<<(unsigned)((pp.n_blk + REP_WARPS - 1) / REP_WARPS), REP_WARPS * 32, smem, cuda.stream>>>(pp);
+    CU(cudaGetLastError());
+    CU(cuda.stop());
+    for (auto &c : copies) CU(c());
+    CU(cudaStreamSynchronize(cuda.stream));
+    g_last_device_ms = 0.0;
+    CU(cuda.total_ms(&g_last_device_ms));
+    return Err();
 }
 
 } // namespace ldsr
@@ -2019,6 +2150,13 @@ int ldsr_posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps,
                              unsigned long long seed, const double *mu, int transform, const double *lambda,
                              double *simX, double *simY, double *simQ, char *errbuf, int errlen) {
     return report(posterior_rep_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, simX, simY, simQ), errbuf,
+                  errlen);
+}
+
+int ldsr_posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                               unsigned long long seed, const double *mu, int transform, const double *lambda,
+                               const ldsr_stats_spec *spec, const ldsr_stats_out *out, char *errbuf, int errlen) {
+    return report(posterior_stats_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, spec, out), errbuf,
                   errlen);
 }
 

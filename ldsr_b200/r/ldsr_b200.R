@@ -303,6 +303,48 @@ LDS_rep_posterior <- function(theta, Qa, u, v, start.year, transform = 'log', nu
   if (P$single) out[[1]] else out
 }
 
+# Drought statistics of LDS_rep_posterior's replicates (the same arguments and exact.rng / seed give the same draws),
+# computed on the device in the sampler's walk: no trajectory is written, so 10^6 replicates and more fit.  windows:
+# up to 4 moving-mean lengths of 1..64 years (lowest and highest mean and its first year, the earliest on a tie);
+# threshold: flow below which a year is in drought (NULL: mean of the observed Qa); runs are maximal stretches below
+# it (longest run and its first year, largest deficit sum(threshold - Q) and its first year, number of runs, the
+# earliest on a tie); period = c(first.year, last.year) restricts every statistic (runs clipped), NULL the whole
+# horizon.  Undefined values are NA / year NA; a replicate with a non-finite flow in the period has NA throughout.
+# Returns a list with windows, threshold, period, data.tables `window` (rep, window, min, min.year, max, max.year)
+# and `run` (rep, run.len, run.year, deficit, deficit.year, n.runs); a list of them for an ensemble.
+LDS_rep_posterior_stats <- function(theta, Qa, u, v, start.year, transform = 'log', num.reps = 100, exact.rng = TRUE,
+                                    seed = 0, windows = 10L, threshold = NULL, period = NULL) {
+  P <- .station_setup(list(Qa = Qa, u = u, v = v, start.year = start.year), transform)
+  thetas <- if (P$single) list(theta) else theta
+  if (length(thetas) != length(P$u)) stop('theta must be one model per ensemble member')
+  series <- lapply(seq_along(P$u), function(k) list(y = P$y, u = P$u[[k]], v = P$v[[k]]))
+  cols <- lapply(thetas, function(th) c(th$A, th$B, th$C, th$D, th$Q, th$R, th$mu1, th$V1))
+  stride <- max(lengths(cols))
+  th <- sapply(cols, function(x) c(x, rep(0, stride - length(x))))
+  n <- length(P$years); nm <- length(series); y0 <- P$years[1]
+  if (is.null(period)) period <- range(P$years)
+  rg <- c(period[1] - y0, period[2] - y0 + 1)
+  if (rg[1] < 0 || rg[2] > n || rg[1] >= rg[2]) stop('period must lie inside the reconstruction horizon')
+  if (is.null(threshold)) threshold <- mean(Qa$Qa)
+  z <- if (exact.rng) stats::rnorm(2 * num.reps * n * nm) else NULL
+  code <- switch(transform, none = 0L, log = 1L, boxcox = 2L)
+  m <- .Call('_ldsr_posterior_stats_batch', series, matrix(th, nrow = stride), as.integer(num.reps), z,
+             as.numeric(seed), rep(P$mu, nm), code, if (transform == 'boxcox') rep(P$lambda, nm) else NULL,
+             as.integer(windows), rep(as.numeric(threshold), nm), as.integer(rep(rg, nm)), PACKAGE = 'ldsr')
+  yr <- function(a) ifelse(a < 0, NA_integer_, a + y0)
+  na <- function(a) ifelse(a < 0, NA_integer_, a)
+  out <- lapply(seq_len(nm), function(k) {
+    r <- (k - 1) * num.reps + seq_len(num.reps)
+    win <- data.table::rbindlist(lapply(seq_along(windows), function(j) data.table::data.table(
+      rep = seq_len(num.reps), window = windows[j], min = m[[1]][r, j], min.year = yr(m[[2]][r, j]),
+      max = m[[3]][r, j], max.year = yr(m[[4]][r, j]))))
+    run <- data.table::data.table(rep = seq_len(num.reps), run.len = na(m[[5]][r]), run.year = yr(m[[6]][r]),
+                                  deficit = m[[7]][r], deficit.year = yr(m[[8]][r]), n.runs = na(m[[9]][r]))
+    list(windows = windows, threshold = threshold, period = period, window = win, run = run)
+  })
+  if (P$single) out[[1]] else out
+}
+
 #' Kalman / RTS smoother for a state of dimension d > 1 (beyond ldsr, whose state is scalar).
 #' theta: list(A d x d, B d x p, C 1 x d, D 1 x q, Q d x d, R, mu1 d x 1, V1 d x d); y 1 x T with NA.
 #' method: 1 = associative scan over time (long series), 0 = sequential recursion.

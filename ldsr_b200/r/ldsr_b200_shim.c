@@ -15,6 +15,7 @@
  *     _ldsr_em_batch(series,group_series,held,fit_group,theta0,niter,tol,n_devices)   8
  *     _ldsr_rep_batch(theta,u,v,n,num_reps,seed,mu,exp_trans,z,r_seed)               10
  *     _ldsr_posterior_rep_batch(series,thetas,num_reps,z,seed,mu,transform,lambda)   8
+ *     _ldsr_posterior_stats_batch(series,thetas,num_reps,z,seed,mu,transform,lambda,windows,threshold,range)   11
  *     _ldsr_cv_metrics(Ycv,target,Z,exp_trans)                                        4
  *     _ldsr_construct_rec(X,V,Y,C,R,mu,transform,lambda)                              8
  *     _ldsr_cv_metrics_stations(Ycv,target,Z,exp_trans)   lists, one element per station    4
@@ -346,6 +347,70 @@ SEXP _ldsr_posterior_rep_batch(SEXP series, SEXP thetas, SEXP repsS, SEXP zS, SE
     return out;
 }
 
+/* Drought statistics of the same replicates, reduced on the device (LDS_rep_posterior_stats in ldsr_b200.R):
+ * arguments as _ldsr_posterior_rep_batch, then windows (integer, up to 4 lengths of 1..64), threshold (one per
+ * series, Q scale, or NULL) and range (a 2 x n integer matrix of 0-based [lo, hi) per series, or NULL).  Returns
+ * list(wmin, wmin_at, wmax, wmax_at) as (num_reps * n) x n_windows matrices and, with a threshold, run_len, run_at,
+ * deficit, deficit_at, n_runs as vectors of num_reps * n: member by member, replicate by replicate; steps 0-based,
+ * -1 where undefined. */
+SEXP _ldsr_posterior_stats_batch(SEXP series, SEXP thetas, SEXP repsS, SEXP zS, SEXP seedS, SEXP muS,
+                                 SEXP transformS, SEXP lambdaS, SEXP windowsS, SEXP thresholdS, SEXP rangeS) {
+    const int ns = (int)XLENGTH(series), reps = Rf_asInteger(repsS), nw = (int)XLENGTH(windowsS);
+    int *T = (int *)R_alloc(ns, sizeof(int)), *p = (int *)R_alloc(ns, sizeof(int)), *q = (int *)R_alloc(ns, sizeof(int));
+    int *idx = (int *)R_alloc(ns, sizeof(int));
+    const double **y = (const double **)R_alloc(ns, sizeof(double *));
+    const double **u = (const double **)R_alloc(ns, sizeof(double *));
+    const double **v = (const double **)R_alloc(ns, sizeof(double *));
+    R_xlen_t tot = 0;
+    for (int s = 0; s < ns; s++) {
+        SEXP e = VECTOR_ELT(series, s);
+        T[s] = Rf_ncols(list_get(e, "y"));
+        y[s] = REAL(list_get(e, "y"));
+        u[s] = input_ptr(list_get(e, "u"), T[s], &p[s]);
+        v[s] = input_ptr(list_get(e, "v"), T[s], &q[s]);
+        idx[s] = s;
+        tot += (R_xlen_t)reps * T[s];
+    }
+    if (Rf_ncols(thetas) != ns) Rf_error("ldsr: thetas must have one column per series");
+    if (XLENGTH(muS) != ns) Rf_error("ldsr: mu must have one value per series");
+    const double *z = Rf_isNull(zS) ? NULL : REAL(zS);
+    if (z && XLENGTH(zS) != 2 * tot) Rf_error("ldsr: z must hold 2 * num.reps * sum(T) draws");
+    const double *lam = Rf_isNull(lambdaS) ? NULL : REAL(lambdaS);
+    if (lam && XLENGTH(lambdaS) != ns) Rf_error("ldsr: lambda must have one value per series");
+    const double *thr = Rf_isNull(thresholdS) ? NULL : REAL(thresholdS);
+    if (thr && XLENGTH(thresholdS) != ns) Rf_error("ldsr: threshold must have one value per series");
+    const int *range = Rf_isNull(rangeS) ? NULL : INTEGER(rangeS);
+    if (range && XLENGTH(rangeS) != 2 * (R_xlen_t)ns) Rf_error("ldsr: range must hold 2 values per series");
+    ldsr_batch b; memset(&b, 0, sizeof b);
+    b.n_series = ns; b.T = T; b.p = p; b.q = q; b.y = y; b.u = u; b.v = v;
+    b.n_groups = ns; b.group_series = idx;
+    b.n_fits = ns; b.fit_group = idx; b.theta0 = REAL(thetas); b.theta_stride = Rf_nrows(thetas);
+    const R_xlen_t rows = (R_xlen_t)reps * ns;
+    ldsr_stats_spec spec = {nw, INTEGER(windowsS), thr, range};
+    ldsr_stats_out so; memset(&so, 0, sizeof so);
+    const int n_out = thr ? 9 : 4;
+    SEXP out = PROTECT(Rf_allocVector(VECSXP, n_out));
+    for (int k = 0; k < n_out; k++) {
+        const int is_real = k == 0 || k == 2 || k == 6;
+        SEXP a = k < 4 ? Rf_allocMatrix(is_real ? REALSXP : INTSXP, rows, nw)
+                       : Rf_allocVector(is_real ? REALSXP : INTSXP, rows);
+        SET_VECTOR_ELT(out, k, a);
+    }
+    so.wmin = REAL(VECTOR_ELT(out, 0)); so.wmin_at = INTEGER(VECTOR_ELT(out, 1));
+    so.wmax = REAL(VECTOR_ELT(out, 2)); so.wmax_at = INTEGER(VECTOR_ELT(out, 3));
+    if (thr) {
+        so.run_len = INTEGER(VECTOR_ELT(out, 4)); so.run_at = INTEGER(VECTOR_ELT(out, 5));
+        so.deficit = REAL(VECTOR_ELT(out, 6)); so.deficit_at = INTEGER(VECTOR_ELT(out, 7));
+        so.n_runs = INTEGER(VECTOR_ELT(out, 8));
+    }
+    char err[512] = "";
+    check(ldsr_posterior_stats_batch(ctx(), &b, reps, z, (unsigned long long)Rf_asReal(seedS), REAL(muS),
+                                     Rf_asInteger(transformS), lam, &spec, &so, err, sizeof err),
+          err);
+    UNPROTECT(1);
+    return out;
+}
+
 /* same shape as src/RcppExports.cpp:132-148 */
 /* mapply(calculate_metrics, sim = Ycv, z = Z, MoreArgs = list(obs = target)) in one call
  * (R/LDS_reconstruction.R:395): Ycv is an n x n_folds matrix, Z a list of integer vectors. */
@@ -577,6 +642,7 @@ static const R_CallMethodDef CallEntries[] = {
     {"_ldsr_em_batch", (DL_FUNC)&_ldsr_em_batch, 8},
     {"_ldsr_rep_batch", (DL_FUNC)&_ldsr_rep_batch, 10},
     {"_ldsr_posterior_rep_batch", (DL_FUNC)&_ldsr_posterior_rep_batch, 8},
+    {"_ldsr_posterior_stats_batch", (DL_FUNC)&_ldsr_posterior_stats_batch, 11},
     {"_ldsr_smoother_d", (DL_FUNC)&_ldsr_smoother_d, 6},
     {"_ldsr_cv_metrics", (DL_FUNC)&_ldsr_cv_metrics, 4},
     {"_ldsr_construct_rec", (DL_FUNC)&_ldsr_construct_rec, 8},
