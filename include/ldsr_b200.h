@@ -255,9 +255,47 @@ int ldsr_posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_rep
                                unsigned long long seed, const double *mu, int transform, const double *lambda,
                                const ldsr_stats_spec *spec, const ldsr_stats_out *out, char *errbuf, int errlen);
 
+/* Year-by-year drought counts of conditioned replicates (beyond the reference), reduced across replicates on the
+ * device: the replicates of ldsr_posterior_rep_batch with the same arguments (the same draws bit for bit, from seed
+ * or from z), of which no trajectory and no per-replicate value leaves the device.  For fit f let Q_t be a
+ * replicate's simQ, [lo, hi) the fit's range of steps (range[2f], range[2f+1] with 0 <= lo < hi <= T_f; range NULL:
+ * the whole series) and thr = threshold[f] (required, finite, on the Q scale).  Step t is below when Q_t < thr (a
+ * non-finite Q_t is not).  A run is a maximal stretch of consecutive below steps inside [lo, hi): runs are clipped
+ * to the range, as in ldsr_posterior_stats_batch.  Each output counts replicates, per step t of the range:
+ *   below                     Q_t is below;
+ *   in_run[k]                 t lies in a run of length >= lengths[k];
+ *   wbelow[k]                 Q_t .. Q_{t+w-1} (w = windows[k]) are finite and sum to less than w thr; defined
+ *                             for lo <= t <= hi - w (the start convention of ldsr_posterior_stats_batch's wmin_at);
+ *   nonfinite                 Q_t is not finite (inverse Box-Cox of (y + mu) lambda + 1 < 0).
+ * Rows are ldsr_smoother_batch's: fit f's step t at fit_ptr[f] + t (fit_ptr the exclusive prefix sum of T over the
+ * fits, caller order); in_run and wbelow are [n_lengths] / [n_windows] blocks of fit_ptr[n_fits] rows.  Rows
+ * outside [lo, hi), and window starts t > hi - w, are -1.  Any output may be NULL.  Counts are integers, so the
+ * result does not depend on the order in which the device adds them: it is the same bit for bit from run to run,
+ * and a fit's counts do not depend on the other fits.  Identities: in_run with length 1 and wbelow with window 1
+ * equal below, and in_run does not increase with the length.  Arguments are checked before a device is touched (as
+ * ldsr_posterior_rep_batch's, plus the spec); one device (ctx device 0), one launch after the coefficient pass, no
+ * CPU fallback.  ldsr_last_device_ms covers the coefficient pass and the sampler. */
+typedef struct {
+    int n_windows;           /* 0 .. LDSR_STATS_MAX_WINDOWS, each 1 .. LDSR_STATS_MAX_WINDOW */
+    const int *windows;      /* [n_windows] */
+    int n_lengths;           /* 0 .. LDSR_STATS_MAX_WINDOWS, each 1 .. LDSR_STATS_MAX_WINDOW */
+    const int *lengths;      /* [n_lengths] */
+    const double *threshold; /* [n_fits], required, finite */
+    const int *range;        /* [2*n_fits] or NULL */
+} ldsr_yearly_spec;
+typedef struct {
+    int *below;     /* [fit_ptr[n_fits]] */
+    int *in_run;    /* [n_lengths][fit_ptr[n_fits]] */
+    int *wbelow;    /* [n_windows][fit_ptr[n_fits]] */
+    int *nonfinite; /* [fit_ptr[n_fits]] */
+} ldsr_yearly_out;
+int ldsr_posterior_yearly_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                                unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                const ldsr_yearly_spec *spec, const ldsr_yearly_out *out, char *errbuf, int errlen);
+
 /* Device time in ms (CUDA events around the kernels, summed) of the last ldsr_rep_batch / ldsr_rep_batch_r /
- * ldsr_posterior_rep_batch / ldsr_posterior_stats_batch call made by the calling thread: the measurement hook of
- * bench.py's config-4 record. */
+ * ldsr_posterior_rep_batch / ldsr_posterior_stats_batch / ldsr_posterior_yearly_batch call made by the calling
+ * thread: the measurement hook of bench.py's config-4 record. */
 double ldsr_last_device_ms(void);
 
 /* ---- the reference's random numbers (R's default generators after set.seed) ---------------

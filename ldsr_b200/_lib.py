@@ -23,7 +23,7 @@ EXPORTS = ("ldsr_abi_version", "ldsr_device_count", "ldsr_ctx_create", "ldsr_ctx
            "ldsr_objective_batch", "ldsr_rep_batch_r", "ldsr_r_rng_create", "ldsr_r_rng_unif", "ldsr_r_rng_norm",
            "ldsr_r_rng_sample", "ldsr_r_rng_destroy", "ldsr_r_rnorm_device", "ldsr_last_device_ms",
            "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations", "ldsr_posterior_rep_batch",
-           "ldsr_posterior_stats_batch")
+           "ldsr_posterior_stats_batch", "ldsr_posterior_yearly_batch")
 
 
 class LdsrError(RuntimeError):
@@ -51,6 +51,15 @@ class StatsSpec(C.Structure):
 class StatsOut(C.Structure):
     _fields_ = [("wmin", _dp), ("wmin_at", _ip), ("wmax", _dp), ("wmax_at", _ip), ("run_len", _ip), ("run_at", _ip),
                 ("deficit", _dp), ("deficit_at", _ip), ("n_runs", _ip)]
+
+
+class YearlySpec(C.Structure):
+    _fields_ = [("n_windows", C.c_int), ("windows", _ip), ("n_lengths", C.c_int), ("lengths", _ip),
+                ("threshold", _dp), ("range", _ip)]
+
+
+class YearlyOut(C.Structure):
+    _fields_ = [("below", _ip), ("in_run", _ip), ("wbelow", _ip), ("nonfinite", _ip)]
 
 
 POLL_FN = C.CFUNCTYPE(C.c_int, C.c_void_p)
@@ -464,6 +473,53 @@ def posterior_stats_batch(series, group_series, held, fit_group, theta, n_reps, 
     _check(rc, err)
     outs["device_ms"] = float(lib().ldsr_last_device_ms())
     return outs
+
+
+YEARLY_COUNTS = ("below", "in_run", "wbelow", "nonfinite")
+
+
+def posterior_yearly_batch(series, group_series, held, fit_group, theta, n_reps, z=None, seed=0, mu=None,
+                           transform="log", lams=None, windows=(10,), lengths=(5,), threshold=None, ranges=None,
+                           want=YEARLY_COUNTS, ctx=None):
+    """ldsr_posterior_yearly_batch: per step, the number of posterior_rep_batch's replicates (same arguments, the
+    same draws) below the threshold, inside a run below it of at least lengths[k] steps, starting a windows[k]-step
+    window whose sum is below windows[k] * threshold, and not finite; reduced on the device.  windows, lengths: up
+    to 4 each, in 1..64; threshold: per fit, on the Q scale (required); ranges: [n_fits, 2] step ranges [lo, hi)
+    (None: whole series).  want: the counts to return.  Returns, per requested count, a list over fits of int32
+    arrays: below and nonfinite [T_f], in_run [n_lengths, T_f], wbelow [n_windows, T_f] (-1 outside the range and at
+    window starts past hi - w), and the device time."""
+    pb = PackedBatch(series, group_series, held, fit_group, theta)
+    nf, n_reps = pb.n_fits, int(n_reps)
+    zz = None
+    if z is not None:
+        zz = np.ascontiguousarray(z, dtype=np.float64).ravel()
+        if zz.size != 2 * int(pb.fit_ptr[-1]) * n_reps:
+            raise ValueError("z must hold 2 * n_reps * sum(T) = %d values" % (2 * int(pb.fit_ptr[-1]) * n_reps))
+    code = TRANSFORMS[transform] if isinstance(transform, str) else int(transform)
+    mu_a = None if mu is None else np.ascontiguousarray(np.broadcast_to(np.asarray(mu, dtype=np.float64), (nf,)))
+    lam_a = None if lams is None else np.ascontiguousarray(np.broadcast_to(np.asarray(lams, dtype=np.float64), (nf,)))
+    win = np.ascontiguousarray(np.atleast_1d(np.asarray(windows if windows is not None else (), dtype=np.int32)))
+    lens = np.ascontiguousarray(np.atleast_1d(np.asarray(lengths if lengths is not None else (), dtype=np.int32)))
+    thr = None if threshold is None else np.ascontiguousarray(
+        np.broadcast_to(np.asarray(threshold, dtype=np.float64), (nf,)))
+    rng = None if ranges is None else np.ascontiguousarray(np.broadcast_to(np.asarray(ranges, dtype=np.int32),
+                                                                           (nf, 2)))
+    ns = int(pb.fit_ptr[-1])
+    rows = {"below": 1, "in_run": lens.size, "wbelow": win.size, "nonfinite": 1}
+    outs = {k: np.empty((rows[k], ns), dtype=np.int32) for k in YEARLY_COUNTS if k in want}
+    spec = YearlySpec(win.size, _i(win) if win.size else None, lens.size, _i(lens) if lens.size else None, _d(thr),
+                      _i(rng))
+    out = YearlyOut(*(_i(outs.get(k)) for k in YEARLY_COUNTS))
+    err = C.create_string_buffer(512)
+    rc = lib().ldsr_posterior_yearly_batch(ctx.h if isinstance(ctx, Ctx) else ctx, C.byref(pb.c), n_reps, _d(zz),
+                                           C.c_ulonglong(int(seed)), _d(mu_a), code, _d(lam_a), C.byref(spec),
+                                           C.byref(out), err, 512)
+    _check(rc, err)
+    ptr = pb.fit_ptr
+    res = {k: [o[:, ptr[f]:ptr[f + 1]] if k in ("in_run", "wbelow") else o[0, ptr[f]:ptr[f + 1]] for f in range(nf)]
+           for k, o in outs.items()}
+    res["device_ms"] = float(lib().ldsr_last_device_ms())
+    return res
 
 
 class RRandom:

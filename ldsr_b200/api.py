@@ -550,21 +550,9 @@ def LDS_rep_posterior(theta, Qa, u, v, start_year, transform="log", num_reps=100
     return out[0] if S["single"] else out
 
 
-def LDS_rep_posterior_stats(theta, Qa, u, v, start_year, transform="log", num_reps=100, seed=0, z=None, windows=(10,),
-                            threshold=None, period=None):
-    """Drought statistics of LDS_rep_posterior's replicates (the same arguments give the same draws), computed on the
-    device in the sampler's walk, so that no trajectory is written or copied: a few numbers per replicate instead of
-    whole series, which makes 10^6 replicates and more practical for tail probabilities.
-    windows: up to 4 moving-mean lengths of 1..64 years: per replicate the lowest and highest w-year mean flow and
-    the first year of that window (the earliest on a tie).  threshold: flow (Q scale) below which a year is in
-    drought; None means the mean of the observed Qa.  A run is a maximal stretch of years below it: per replicate
-    the longest run (years, first year), the largest run deficit sum(threshold - Q) (value, first year) and the
-    number of runs, the earliest run on a tie.  period = (first_year, last_year) restricts every statistic to those
-    years (runs are clipped to it); None: the whole horizon.  Undefined values (a window longer than the period, no
-    run) are NaN / year -1 / 0; a replicate with a non-finite flow in the period (Box-Cox) has NaN and -1 throughout.
-    Returns a dict with windows, threshold, period and arrays over replicates: wmin, wmin_year, wmax, wmax_year
-    ([n_windows, num_reps]), run_len, run_year, deficit, deficit_year, n_runs ([num_reps]); one dict per member for
-    an ensemble.  One device call."""
+def _posterior_reduce_setup(theta, Qa, u, v, start_year, transform, threshold, period):
+    """The station set-up of the reducing posterior calls: the station (as LDS_reconstruction sets it up), one padded
+    theta row per member, the first year, the period's step range [lo, hi) and the threshold (None: mean(Qa))."""
     S = _station(dict(Qa=Qa, u=u, v=v, start_year=start_year), transform)
     thetas = [theta] if S["single"] else list(theta)
     if len(thetas) != len(S["series"]):
@@ -583,9 +571,27 @@ def LDS_rep_posterior_stats(theta, Qa, u, v, start_year, transform="log", num_re
         if not (0 <= lo < hi <= years.size):
             raise ValueError("period %r is not inside %d..%d" % (tuple(period), y0, int(years[-1])))
     thr = float(np.mean(np.asarray(Qa["Qa"], dtype=float))) if threshold is None else float(threshold)
-    n = len(rows)
-    r = _lib.posterior_stats_batch(S["series"], np.arange(n), None, np.arange(n),
-                                   np.stack([np.pad(v, (0, stride - v.size)) for v in rows]), num_reps, z=z, seed=seed,
+    return S, np.stack([np.pad(r, (0, stride - r.size)) for r in rows]), y0, lo, hi, thr
+
+
+def LDS_rep_posterior_stats(theta, Qa, u, v, start_year, transform="log", num_reps=100, seed=0, z=None, windows=(10,),
+                            threshold=None, period=None):
+    """Drought statistics of LDS_rep_posterior's replicates (the same arguments give the same draws), computed on the
+    device in the sampler's walk, so that no trajectory is written or copied: a few numbers per replicate instead of
+    whole series, which makes 10^6 replicates and more practical for tail probabilities.
+    windows: up to 4 moving-mean lengths of 1..64 years: per replicate the lowest and highest w-year mean flow and
+    the first year of that window (the earliest on a tie).  threshold: flow (Q scale) below which a year is in
+    drought; None means the mean of the observed Qa.  A run is a maximal stretch of years below it: per replicate
+    the longest run (years, first year), the largest run deficit sum(threshold - Q) (value, first year) and the
+    number of runs, the earliest run on a tie.  period = (first_year, last_year) restricts every statistic to those
+    years (runs are clipped to it); None: the whole horizon.  Undefined values (a window longer than the period, no
+    run) are NaN / year -1 / 0; a replicate with a non-finite flow in the period (Box-Cox) has NaN and -1 throughout.
+    Returns a dict with windows, threshold, period and arrays over replicates: wmin, wmin_year, wmax, wmax_year
+    ([n_windows, num_reps]), run_len, run_year, deficit, deficit_year, n_runs ([num_reps]); one dict per member for
+    an ensemble.  One device call."""
+    S, thetas, y0, lo, hi, thr = _posterior_reduce_setup(theta, Qa, u, v, start_year, transform, threshold, period)
+    n = thetas.shape[0]
+    r = _lib.posterior_stats_batch(S["series"], np.arange(n), None, np.arange(n), thetas, num_reps, z=z, seed=seed,
                                    mu=np.full(n, S["mu"]), transform=transform,
                                    lams=None if transform != "boxcox" else np.full(n, S["lam"]), windows=windows,
                                    threshold=np.full(n, thr), ranges=np.tile([lo, hi], (n, 1)))
@@ -595,6 +601,38 @@ def LDS_rep_posterior_stats(theta, Qa, u, v, start_year, transform="log", num_re
                 wmax_year=year(r["wmax_at"][:, k]), run_len=r["run_len"][k], run_year=year(r["run_at"][k]),
                 deficit=r["deficit"][k], deficit_year=year(r["deficit_at"][k]), n_runs=r["n_runs"][k])
            for k in range(n)]
+    return out[0] if S["single"] else out
+
+
+def LDS_rep_posterior_yearly(theta, Qa, u, v, start_year, transform="log", num_reps=100, seed=0, z=None,
+                             windows=(10,), lengths=(5,), threshold=None, period=None):
+    """Year-by-year drought probabilities over LDS_rep_posterior's replicates (the same arguments give the same
+    draws), counted on the device in the sampler's walk: no trajectory and no per-replicate value is written, so
+    10^6 replicates and more are practical.  A year is below when its flow is below threshold (Q scale; None: the
+    mean of the observed Qa; a non-finite flow is not below); a run is a maximal stretch of years below it inside
+    period (runs are clipped to it).  Per year of period = (first_year, last_year) (None: the whole horizon):
+      p_below               the share of replicates with the year below;
+      p_run [n_lengths]     the share with the year inside a run of at least lengths[k] years (up to 4, 1..64);
+      p_window [n_windows]  the share whose windows[k]-year mean flow starting that year (all flows finite) is below
+                            the threshold (up to 4, 1..64); NaN where the window passes the period's end;
+      n_nonfinite           the number of replicates with a non-finite flow that year (Box-Cox).
+    Returns a dict with windows, lengths, threshold, period, year (the period's years), those arrays and the raw
+    counts below, in_run, wbelow (-1 where undefined); one dict per member for an ensemble.  One device call."""
+    S, thetas, y0, lo, hi, thr = _posterior_reduce_setup(theta, Qa, u, v, start_year, transform, threshold, period)
+    n = thetas.shape[0]
+    r = _lib.posterior_yearly_batch(S["series"], np.arange(n), None, np.arange(n), thetas, num_reps, z=z, seed=seed,
+                                    mu=np.full(n, S["mu"]), transform=transform,
+                                    lams=None if transform != "boxcox" else np.full(n, S["lam"]), windows=windows,
+                                    lengths=lengths, threshold=np.full(n, thr), ranges=np.tile([lo, hi], (n, 1)))
+    share = lambda c: np.where(c >= 0, c / float(num_reps), np.nan)
+    out = []
+    for k in range(n):
+        c = {name: r[name][k][..., lo:hi] for name in _lib.YEARLY_COUNTS}
+        out.append(dict(windows=tuple(int(w) for w in np.atleast_1d(windows)),
+                        lengths=tuple(int(x) for x in np.atleast_1d(lengths)), threshold=thr,
+                        period=(y0 + lo, y0 + hi - 1), year=np.arange(y0 + lo, y0 + hi), below=c["below"],
+                        in_run=c["in_run"], wbelow=c["wbelow"], p_below=share(c["below"]), p_run=share(c["in_run"]),
+                        p_window=share(c["wbelow"]), n_nonfinite=c["nonfinite"]))
     return out[0] if S["single"] else out
 
 

@@ -455,6 +455,13 @@ struct PostRepParams {
     const double *thr;            // [n_fits] run threshold on the Q scale, or null (no run statistics)
     double *wmin, *wmax, *deficit;
     int *wmin_at, *wmax_at, *run_len, *run_at, *deficit_at, *n_runs;
+    // yearly mode (posterior_rep_kernel<TT, POST_YEARLY>, one launch, blk0 = out0 = 0; win, n_win, ring, range and
+    // thr as above, thr required): counts of replicates added at row fit_ptr[f] + t, length / window k's at
+    // k n_steps + fit_ptr[f] + t; any output may be null
+    int n_len, len[POST_MAX_WIN]; // run lengths L_k, 1 .. POST_MAX_RING
+    int delay;                    // D = max L_k: step s is decided when the walk reaches s - D + 1 (0 without lengths)
+    long long n_steps;            // fit_ptr[n_fits]
+    int *y_below, *y_in_run, *y_wbelow, *y_nonfinite;
 };
 
 __device__ __forceinline__ unsigned long long posterior_key(unsigned long long seed, int fit, long long rep) {
@@ -465,19 +472,24 @@ __device__ __forceinline__ unsigned long long posterior_key(unsigned long long s
 template <int TT> __host__ __device__ inline size_t posterior_smem_bytes(bool with_z) {
     return (size_t)REP_WARPS * ((3 + (with_z ? 2 : 0)) * TT * 33 + 4 * TT) * sizeof(double);
 }
-// statistics mode: no output tiles; the noise tiles (with z), the coefficient tile and the lanes' Q rings
+// statistics and yearly modes: no output tiles; the noise tiles (with z), the coefficient tile and the lanes' Q rings
 template <int TT> __host__ __device__ inline size_t posterior_stats_smem_bytes(bool with_z, int ring) {
     return (size_t)REP_WARPS * ((with_z ? 2 : 0) * TT * 33 + 4 * TT + 32 * ring) * sizeof(double);
 }
 
-// STATS = false: the trajectories (simX, simY, simQ).  STATS = true: the same draws, reduced in the walk to each
-// replicate's drought statistics over its fit's range [lo, hi) (ldsr_posterior_stats_batch); no trajectory leaves
-// the SM.  Both modes run the one step body below, so a replicate's Q_t is the same value in either.
+// The modes of posterior_rep_kernel.  POST_STATS is 1, so the statistics mode may also be named <TT, true>.
+constexpr int POST_TRAJ = 0, POST_STATS = 1, POST_YEARLY = 2;
+
+// POST_TRAJ: the trajectories (simX, simY, simQ).  POST_STATS: the same draws, reduced in the walk to each
+// replicate's drought statistics over its fit's range [lo, hi) (ldsr_posterior_stats_batch).  POST_YEARLY: the
+// same draws, reduced across replicates to per-step counts (ldsr_posterior_yearly_batch).  In the two reducing modes
+// no trajectory leaves the SM.  All modes run the one step body below, so a replicate's Q_t is the same value in each.
 // The statistics mode's accumulators take it to 168 registers: three CTAs an SM, stated so that ptxas does not cap
-// it at 128 and spill (0 leaves the trajectory mode to ptxas's default, 96).
-template <int TT, bool STATS = false>
-__global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_kernel(const PostRepParams P) {
+// it at 128 and spill (0 leaves the other modes to ptxas's default: 96 registers for the trajectories).
+template <int TT, int MODE = POST_TRAJ>
+__global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS ? 3 : 0) posterior_rep_kernel(const PostRepParams P) {
     static_assert(32 % TT == 0 && TT <= 16, "a tile's mask bits sit in one word; a half-warp loads a tile row");
+    constexpr bool STATS = MODE == POST_STATS, YEARLY = MODE == POST_YEARLY, REDUCE = STATS || YEARLY;
     LDSR_DYN_SMEM(smem_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long blk = (long long)blockIdx.x * REP_WARPS + warp;
@@ -487,9 +499,9 @@ __global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_k
     const int n_rows = P.n_reps - r0 < 32 ? P.n_reps - r0 : 32;
     const bool have_z = P.z != nullptr;
     constexpr int TILE = TT * 33;
-    constexpr int N_OUT = STATS ? 0 : 3; // output tiles
+    constexpr int N_OUT = REDUCE ? 0 : 3; // output tiles
     double *const tiles = reinterpret_cast<double *>(smem_raw) +
-                          (size_t)warp * ((N_OUT + (have_z ? 2 : 0)) * TILE + 4 * TT + (STATS ? 32 * P.ring : 0));
+                          (size_t)warp * ((N_OUT + (have_z ? 2 : 0)) * TILE + 4 * TT + (REDUCE ? 32 * P.ring : 0));
     double *const tX = tiles, *const tY = tiles + TILE, *const tQ = tiles + 2 * TILE;
     double *const tZq = tiles + N_OUT * TILE, *const tZe = tiles + (N_OUT + 1) * TILE;
     double *const tC = tiles + (N_OUT + (have_z ? 2 : 0)) * TILE; // [m | s | o | J] of the tile's steps
@@ -507,9 +519,9 @@ __global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_k
     // before Q_t takes that slot.  Updating on <= / >= lets the smaller start, and the earlier run, win ties.
     double *const ring = tC + 4 * TT + lane;
     const int rmask = P.ring - 1;
-    const int rlo = STATS ? P.range[2 * f] : 0, rhi = STATS ? P.range[2 * f + 1] : 0;
+    const int rlo = REDUCE ? P.range[2 * f] : 0, rhi = REDUCE ? P.range[2 * f + 1] : 0;
     const bool runs = STATS && P.thr != nullptr;
-    const double thr = runs ? P.thr[f] : 0.0;
+    const double thr = runs || YEARLY ? P.thr[f] : 0.0;
     double wsum[POST_MAX_WIN], wmn[POST_MAX_WIN], wmx[POST_MAX_WIN];
     int wmn_at[POST_MAX_WIN], wmx_at[POST_MAX_WIN];
 #pragma unroll
@@ -529,13 +541,44 @@ __global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_k
         cur_len = 0;
         cur_def = 0.0;
     };
+    // yearly state.  Bit i of `below` / `bad` is whether Q_{t+i} < thr / Q_{t+i} is not finite, for the last 64
+    // steps walked (steps at or above hi: neither).  A count of the replicates is kept per step, by lane j for
+    // step j of the tile (ballot and popc), and added to the output once a tile by the lanes that hold one.
+    // A run's length is known only when it closes, so in_run decides step s with a delay: when the walk reaches
+    // t = s - D + 1, down(s) = the consecutive below steps from s downwards, capped at D, is in bits D-1 .. 0 of
+    // `below`, and `up` = the consecutive below steps from s upwards.  s lies in a run of length >= L
+    // iff below(s) and up + down - 1 >= L; the caps are exact because every L <= D.
+    const bool live = lane < n_rows;
+    const int D = YEARLY ? P.delay : 1; // (1: the other modes never decide a step)
+    unsigned long long below = 0ull, bad = 0ull;
+    int up = 0, c_below = 0, c_bad = 0, c_win[POST_MAX_WIN] = {}, c_run[POST_MAX_WIN] = {};
+    auto count = [&](int &c, bool pred, int j) { // c of lane j <- the live replicates with pred
+        const int n = __popc(__ballot_sync(0xffffffffu, live && pred));
+        if (lane == j) c = n;
+    };
+    auto add = [&](int *out, long long row, int &c) { // the lane's count into out[row]
+        if (out && c) atomicAdd(out + row, c);
+        c = 0;
+    };
+    auto decide = [&](int s, int j) { // step s, now that the walk is at s - D + 1 (or below lo)
+        const bool b = (below >> (D - 1)) & 1ull;
+        up = b ? up + 1 : 0;
+        const unsigned long long top = below << (64 - D); // step s in bit 63
+        const unsigned nh = ~(unsigned)(top >> 32), nl = ~(unsigned)top;
+        const int len = up + (nh ? __clz((int)nh) : 32 + __clz((int)nl)) - 1; // up + down(s) - 1
+#pragma unroll
+        for (int k = 0; k < POST_MAX_WIN; k++) {
+            if (k >= P.n_len) break;
+            count(c_run[k], s < rhi && b && len >= P.len[k], j);
+        }
+    };
     // the coefficients of a tile: half-warp 0 loads m and o, half-warp 1 s and J (128 contiguous bytes each); the
     // next tile's are in flight while this one's chain runs, then read back from shared memory as broadcasts
     const double *__restrict__ ca = (half ? P.s : P.m) + fp, *__restrict__ cb = (half ? P.J : P.o) + fp;
     int lo = ((T - 1) / TT) * TT;
     double na = hl < T - lo ? ca[lo + hl] : 0.0, nb = hl < T - lo ? cb[lo + hl] : 0.0;
     double x1 = 0.0; // x_{t+1}
-    for (; lo >= 0 && (!STATS || lo + TT > rlo); lo -= TT) { // statistics: no tile below the range
+    for (; lo >= 0 && (!REDUCE || lo + TT > rlo); lo -= TT) { // statistics, yearly: no tile below the range
         const int cnt = T - lo < TT ? T - lo : TT;
         tC[half * TT + hl] = na;
         tC[(2 + half) * TT + hl] = nb;
@@ -566,40 +609,71 @@ __global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_k
             const double y = (bits >> j) & 1u ? tC[2 * TT + j] : fma(sR, ze, fma(C, x, tC[2 * TT + j]));
             const double yq = y + mu;
             const double q = tr == 1 ? exp(yq) : (tr == 0 ? yq : pow(fma(yq, lam, 1.0), il));
-            if (!STATS) {
+            if (!REDUCE) {
                 tX[j * 33 + lane] = x;
                 tY[j * 33 + lane] = y;
                 tQ[j * 33 + lane] = q;
             }
             x1 = x;
-            if (!STATS) continue;
+            if (!REDUCE) continue;
             const int t = lo + j;
             if (t < rlo || t >= rhi) continue;
             finite = finite && fabs(q) < INFINITY; // false for NaN and +-Inf
             const int seen = rhi - t; // steps of the range walked so far, t included
+            if constexpr (YEARLY) {
+                const bool fin = fabs(q) < INFINITY;
+                below = below << 1 | (unsigned long long)(q < thr); // NaN: not below
+                bad = bad << 1 | (unsigned long long)!fin;
+                count(c_below, q < thr, j);
+                count(c_bad, !fin, j);
+                // window sums of finite flows only; a window with a non-finite flow (a bit of `bad`) counts nowhere
+                const double qf = fin ? q : 0.0;
 #pragma unroll
-            for (int k = 0; k < POST_MAX_WIN; k++) {
-                if (k >= P.n_win) break;
-                const int w = P.win[k];
-                double sum = wsum[k] + q;
-                if (seen > w) sum -= ring[((t + w) & rmask) * 32]; // Q_{t+w} leaves the window
-                wsum[k] = sum;
-                if (seen >= w) {
-                    if (sum <= wmn[k]) wmn[k] = sum, wmn_at[k] = t;
-                    if (sum >= wmx[k]) wmx[k] = sum, wmx_at[k] = t;
+                for (int k = 0; k < POST_MAX_WIN; k++) {
+                    if (k >= P.n_win) break;
+                    const int w = P.win[k];
+                    double sum = wsum[k] + qf;
+                    if (seen > w) sum -= ring[((t + w) & rmask) * 32];
+                    wsum[k] = sum;
+                    count(c_win[k], seen >= w && !(bad & (~0ull >> (64 - w))) && sum < w * thr, j);
                 }
-            }
-            if (P.n_win > 0) ring[(t & rmask) * 32] = q;
-            if (runs) {
-                if (q < thr) {
-                    cur_len++;
-                    cur_def += thr - q;
-                } else if (cur_len > 0) {
-                    close_run(t + 1);
+                if (P.n_win > 0) ring[(t & rmask) * 32] = qf;
+                if (D > 0) decide(t + D - 1, j);
+            } else {
+#pragma unroll
+                for (int k = 0; k < POST_MAX_WIN; k++) {
+                    if (k >= P.n_win) break;
+                    const int w = P.win[k];
+                    double sum = wsum[k] + q;
+                    if (seen > w) sum -= ring[((t + w) & rmask) * 32]; // Q_{t+w} leaves the window
+                    wsum[k] = sum;
+                    if (seen >= w) {
+                        if (sum <= wmn[k]) wmn[k] = sum, wmn_at[k] = t;
+                        if (sum >= wmx[k]) wmx[k] = sum, wmx_at[k] = t;
+                    }
+                }
+                if (P.n_win > 0) ring[(t & rmask) * 32] = q;
+                if (runs) {
+                    if (q < thr) {
+                        cur_len++;
+                        cur_def += thr - q;
+                    } else if (cur_len > 0) {
+                        close_run(t + 1);
+                    }
                 }
             }
         }
-        if (!STATS) {
+        if constexpr (YEARLY) { // lane j < TT holds step lo + j's counts, and in_run's of step lo + j + D - 1
+            const long long row = fp + lo + lane;
+            add(P.y_below, row, c_below);
+            add(P.y_nonfinite, row, c_bad);
+#pragma unroll
+            for (int k = 0; k < POST_MAX_WIN; k++) {
+                if (k < P.n_win) add(P.y_wbelow, k * P.n_steps + row, c_win[k]);
+                if (k < P.n_len) add(P.y_in_run, k * P.n_steps + row + D - 1, c_run[k]);
+            }
+        }
+        if (!REDUCE) {
             __syncwarp();
             // each half-warp writes one replicate row of the tile (up to 128 contiguous bytes) per instruction
             for (int rr = half; rr < n_rows; rr += 2) {
@@ -612,6 +686,18 @@ __global__ void __launch_bounds__(REP_WARPS * 32, STATS ? 3 : 0) posterior_rep_k
             }
         }
         __syncwarp();
+    }
+    if constexpr (YEARLY) {
+        // the steps lo - 1 .. lo - D + 1 are not below: this decides lo + D - 2 .. lo, one step at a time (lane 0
+        // holds and adds the counts), and clips runs at lo
+        for (int s = rlo + D - 2; s >= rlo; s--) {
+            below <<= 1;
+            decide(s, 0);
+#pragma unroll
+            for (int k = 0; k < POST_MAX_WIN; k++)
+                if (k < P.n_len) add(P.y_in_run, k * P.n_steps + fp + s, c_run[k]);
+        }
+        return;
     }
     if (!STATS || lane >= n_rows) return;
     if (cur_len > 0) close_run(rlo); // a run reaching the range's lower end

@@ -1494,7 +1494,7 @@ static Err em_batch(ldsr_ctx *ctx, const ldsr_batch *b, int niter, double tol, c
 }
 
 // device time (CUDA events) of the replicate kernels of the last ldsr_rep_batch* / ldsr_posterior_rep_batch /
-// ldsr_posterior_stats_batch call of this thread (ldsr_last_device_ms)
+// ldsr_posterior_stats_batch / ldsr_posterior_yearly_batch call of this thread (ldsr_last_device_ms)
 static thread_local double g_last_device_ms = 0.0;
 
 // ---- single-step batched entry points (one device: ctx device 0) ----------------------------
@@ -1932,6 +1932,90 @@ static Err posterior_rep_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, c
 }
 
 // ---- drought statistics of the conditioned replicates, reduced in the sampler's walk -------------------------
+// The checks and device set-up that the statistics and the yearly calls share.
+// A list of n window or run lengths: at most LDSR_STATS_MAX_WINDOWS, each 1 .. LDSR_STATS_MAX_WINDOW.
+static Err posterior_lengths(const char *name, int n, const int *v) {
+    if (n < 0 || n > LDSR_STATS_MAX_WINDOWS)
+        return fail(LDSR_ERR_ARG, "n_%s=%d, need 0 .. %d", name, n, LDSR_STATS_MAX_WINDOWS);
+    if (n > 0 && !v) return fail(LDSR_ERR_ARG, "%s is NULL", name);
+    for (int k = 0; k < n; k++)
+        if (v[k] < 1 || v[k] > LDSR_STATS_MAX_WINDOW)
+            return fail(LDSR_ERR_ARG, "%s[%d]=%d, need 1 .. %d", name, k, v[k], LDSR_STATS_MAX_WINDOW);
+    return Err();
+}
+
+// Per fit, the step range [lo, hi) (spec_range NULL: the whole series) and, when there is one, a finite threshold.
+static Err posterior_ranges(const ldsr_batch *b, const int *spec_range, const double *threshold,
+                            std::vector<int> &range) {
+    const int nf = b->n_fits;
+    range.assign((size_t)2 * nf, 0);
+    for (int f = 0; f < nf; f++) {
+        const int T = b->T[b->group_series[b->fit_group[f]]];
+        const int lo = spec_range ? spec_range[2 * f] : 0, hi = spec_range ? spec_range[2 * f + 1] : T;
+        if (!(0 <= lo && lo < hi && hi <= T))
+            return fail(LDSR_ERR_ARG, "fit %d: range [%d, %d), need 0 <= lo < hi <= T = %d", f, lo, hi, T);
+        if (threshold && !std::isfinite(threshold[f]))
+            return fail(LDSR_ERR_ARG, "fit %d: threshold %g is not finite", f, threshold[f]);
+        range[2 * f] = lo;
+        range[2 * f + 1] = hi;
+    }
+    return Err();
+}
+
+// One launch over every (fit, 32 replicates) block: caller noise uploaded whole (the test and parity path), the
+// ranges, thresholds and windows, and a Q ring of the smallest power of two >= the longest window.
+static cudaError_t posterior_reduce_params(Resources &cuda, const double *z, long long n_steps,
+                                           const std::vector<int> &range, const double *threshold, int nw,
+                                           const int *windows, PostRepParams &pp) {
+    const int nf = (int)(range.size() / 2);
+    pp.blk0 = 0;
+    pp.n_blk = (long long)nf * pp.wpf;
+    pp.out0 = 0;
+    cudaError_t ce = cudaSuccess;
+    if (z) {
+        double *dz;
+        const size_t nz = 2 * (size_t)pp.n_reps * (size_t)n_steps;
+        if ((ce = cuda.alloc(&dz, nz)) != cudaSuccess) return ce;
+        if ((ce = cudaMemcpyAsync(dz, z, nz * sizeof(double), cudaMemcpyHostToDevice, cuda.stream)) != cudaSuccess)
+            return ce;
+        pp.z = dz;
+    }
+    pp.n_win = nw;
+    int wmax = 0;
+    for (int k = 0; k < nw; k++) wmax = std::max(wmax, pp.win[k] = windows[k]);
+    pp.ring = 1;
+    while (pp.ring < wmax) pp.ring *= 2;
+    if (nw == 0) pp.ring = 0;
+    int *d_range;
+    if ((ce = cuda.upload(&d_range, range)) != cudaSuccess) return ce;
+    pp.range = d_range;
+    if (threshold) {
+        double *d_thr;
+        if ((ce = cuda.upload(&d_thr, std::vector<double>(threshold, threshold + nf))) != cudaSuccess) return ce;
+        pp.thr = d_thr;
+    }
+    return cudaSuccess;
+}
+
+// The one launch of a reducing mode, the copies of its outputs into the caller's arrays, and the device time.
+template <int MODE>
+static Err posterior_reduce_run(Resources &cuda, const PostRepParams &pp, bool with_z,
+                                const std::vector<std::function<cudaError_t()>> &copies) {
+    const size_t smem = posterior_stats_smem_bytes<REP_TT>(with_z, pp.ring);
+    CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)posterior_stats_smem_bytes<REP_TT>(true, POST_MAX_RING)));
+    CU(cuda.start());
+    posterior_rep_kernel<REP_TT, MODE>
+        <<<(unsigned)((pp.n_blk + REP_WARPS - 1) / REP_WARPS), REP_WARPS * 32, smem, cuda.stream>>>(pp);
+    CU(cudaGetLastError());
+    CU(cuda.stop());
+    for (auto &c : copies) CU(c());
+    CU(cudaStreamSynchronize(cuda.stream));
+    g_last_device_ms = 0.0;
+    CU(cuda.total_ms(&g_last_device_ms));
+    return Err();
+}
+
 static Err posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
                                  unsigned long long seed, const double *mu, int transform, const double *lambda,
                                  const ldsr_stats_spec *spec, const ldsr_stats_out *out) {
@@ -1940,59 +2024,19 @@ static Err posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps,
     if (!e.ok()) return e;
     if (!spec || !out) return fail(LDSR_ERR_ARG, "spec and out are required");
     const int nw = spec->n_windows, nf = b->n_fits;
-    if (nw < 0 || nw > LDSR_STATS_MAX_WINDOWS)
-        return fail(LDSR_ERR_ARG, "n_windows=%d, need 0 .. %d", nw, LDSR_STATS_MAX_WINDOWS);
-    if (nw > 0 && !spec->windows) return fail(LDSR_ERR_ARG, "windows is NULL");
-    int wmax = 0;
-    for (int k = 0; k < nw; k++) {
-        const int w = spec->windows[k];
-        if (w < 1 || w > LDSR_STATS_MAX_WINDOW)
-            return fail(LDSR_ERR_ARG, "windows[%d]=%d, need 1 .. %d", k, w, LDSR_STATS_MAX_WINDOW);
-        wmax = std::max(wmax, w);
-    }
+    if (!(e = posterior_lengths("windows", nw, spec->windows)).ok()) return e;
     if (nw == 0 && !spec->threshold) return fail(LDSR_ERR_ARG, "no statistics asked for: no window and no threshold");
     if (!spec->threshold && (out->run_len || out->run_at || out->deficit || out->deficit_at || out->n_runs))
         return fail(LDSR_ERR_ARG, "run outputs need a threshold");
-    std::vector<int> range((size_t)2 * nf);
-    for (int f = 0; f < nf; f++) {
-        const int T = b->T[b->group_series[b->fit_group[f]]];
-        const int lo = spec->range ? spec->range[2 * f] : 0, hi = spec->range ? spec->range[2 * f + 1] : T;
-        if (!(0 <= lo && lo < hi && hi <= T))
-            return fail(LDSR_ERR_ARG, "fit %d: range [%d, %d), need 0 <= lo < hi <= T = %d", f, lo, hi, T);
-        if (spec->threshold && !std::isfinite(spec->threshold[f]))
-            return fail(LDSR_ERR_ARG, "fit %d: threshold %g is not finite", f, spec->threshold[f]);
-        range[2 * f] = lo;
-        range[2 * f + 1] = hi;
-    }
+    std::vector<int> range;
+    if (!(e = posterior_ranges(b, spec->range, spec->threshold, range)).ok()) return e;
     PosteriorSetup S;
     if (!(e = posterior_setup(ctx, b, n_reps, seed, transform, par, S)).ok()) return e;
     Resources &cuda = S.plan->cuda;
     const long long rows = (long long)nf * n_reps, wrows = rows * nw;
     PostRepParams pp = S.pp;
-    pp.blk0 = 0;
-    pp.n_blk = (long long)nf * pp.wpf;
-    pp.out0 = 0;
-    if (z) { // the test and parity path: the whole noise array at once
-        double *dz;
-        const size_t nz = 2 * (size_t)n_reps * (size_t)S.fit_ptr[nf];
-        CU(cuda.alloc(&dz, nz));
-        CU(cudaMemcpyAsync(dz, z, nz * sizeof(double), cudaMemcpyHostToDevice, cuda.stream));
-        pp.z = dz;
-    }
-    pp.n_win = nw;
-    for (int k = 0; k < nw; k++) pp.win[k] = spec->windows[k];
-    pp.ring = 1;
-    while (pp.ring < wmax) pp.ring *= 2;
-    if (nw == 0) pp.ring = 0;
+    CU(posterior_reduce_params(cuda, z, S.fit_ptr[nf], range, spec->threshold, nw, spec->windows, pp));
     pp.n_rows = rows;
-    int *d_range;
-    CU(cuda.upload(&d_range, range));
-    pp.range = d_range;
-    if (spec->threshold) {
-        double *d_thr;
-        CU(cuda.upload(&d_thr, std::vector<double>(spec->threshold, spec->threshold + nf)));
-        pp.thr = d_thr;
-    }
     // device outputs of the requested statistics, copied into the caller's arrays once the kernel is done
     std::vector<std::function<cudaError_t()>> copies;
     auto out_block = [&](auto **dev, auto *host, long long n) -> cudaError_t {
@@ -2016,19 +2060,57 @@ static Err posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps,
     CU(out_block(&pp.deficit, out->deficit, rows));
     CU(out_block(&pp.deficit_at, out->deficit_at, rows));
     CU(out_block(&pp.n_runs, out->n_runs, rows));
-    const size_t smem = posterior_stats_smem_bytes<REP_TT>(z != nullptr, pp.ring);
-    CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)posterior_stats_smem_bytes<REP_TT>(true, POST_MAX_RING)));
-    CU(cuda.start());
-    posterior_rep_kernel<REP_TT, true>
-        <<<(unsigned)((pp.n_blk + REP_WARPS - 1) / REP_WARPS), REP_WARPS * 32, smem, cuda.stream>>>(pp);
-    CU(cudaGetLastError());
-    CU(cuda.stop());
-    for (auto &c : copies) CU(c());
-    CU(cudaStreamSynchronize(cuda.stream));
-    g_last_device_ms = 0.0;
-    CU(cuda.total_ms(&g_last_device_ms));
-    return Err();
+    return posterior_reduce_run<POST_STATS>(cuda, pp, z != nullptr, copies);
+}
+
+// ---- year-by-year drought counts of the conditioned replicates, reduced across replicates --------------------
+static Err posterior_yearly_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
+                                  unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                  const ldsr_yearly_spec *spec, const ldsr_yearly_out *out) {
+    std::vector<double> par;
+    Err e = posterior_args(b, n_reps, mu, transform, lambda, par);
+    if (!e.ok()) return e;
+    if (!spec || !out) return fail(LDSR_ERR_ARG, "spec and out are required");
+    const int nw = spec->n_windows, nl = spec->n_lengths, nf = b->n_fits;
+    if (!(e = posterior_lengths("windows", nw, spec->windows)).ok()) return e;
+    if (!(e = posterior_lengths("lengths", nl, spec->lengths)).ok()) return e;
+    if (!spec->threshold) return fail(LDSR_ERR_ARG, "threshold is required");
+    std::vector<int> range;
+    if (!(e = posterior_ranges(b, spec->range, spec->threshold, range)).ok()) return e;
+    PosteriorSetup S;
+    if (!(e = posterior_setup(ctx, b, n_reps, seed, transform, par, S)).ok()) return e;
+    Resources &cuda = S.plan->cuda;
+    const long long ns = S.fit_ptr[nf];
+    PostRepParams pp = S.pp;
+    CU(posterior_reduce_params(cuda, z, ns, range, spec->threshold, nw, spec->windows, pp));
+    pp.n_len = nl;
+    for (int k = 0; k < nl; k++) pp.delay = std::max(pp.delay, pp.len[k] = spec->lengths[k]);
+    pp.n_steps = ns;
+    // the counts start at 0 on the steps that have them (window k: starts lo .. hi - w) and -1 elsewhere; the
+    // kernel adds to them, and they are copied into the caller's arrays once it is done
+    std::vector<std::function<cudaError_t()>> copies;
+    auto out_block = [&](int **dev, int *host, int n, const int *w) -> cudaError_t {
+        *dev = nullptr;
+        if (!host) return cudaSuccess;
+        std::vector<int> init((size_t)n * ns, -1);
+        for (int k = 0; k < n; k++)
+            for (int f = 0; f < nf; f++) {
+                const long long hi = range[2 * f + 1] - (w ? w[k] - 1 : 0);
+                for (long long t = range[2 * f]; t < hi; t++) init[(size_t)(k * ns + S.fit_ptr[f] + t)] = 0;
+            }
+        cudaError_t ce = cuda.upload(dev, init);
+        if (ce == cudaSuccess) {
+            int *d = *dev;
+            const size_t bytes = init.size() * sizeof(int);
+            copies.push_back([=, &cuda] { return cudaMemcpyAsync(host, d, bytes, cudaMemcpyDeviceToHost, cuda.stream); });
+        }
+        return ce;
+    };
+    CU(out_block(&pp.y_below, out->below, 1, nullptr));
+    CU(out_block(&pp.y_in_run, out->in_run, nl, nullptr));
+    CU(out_block(&pp.y_wbelow, out->wbelow, nw, spec->windows));
+    CU(out_block(&pp.y_nonfinite, out->nonfinite, 1, nullptr));
+    return posterior_reduce_run<POST_YEARLY>(cuda, pp, z != nullptr, copies);
 }
 
 } // namespace ldsr
@@ -2157,6 +2239,13 @@ int ldsr_posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_rep
                                unsigned long long seed, const double *mu, int transform, const double *lambda,
                                const ldsr_stats_spec *spec, const ldsr_stats_out *out, char *errbuf, int errlen) {
     return report(posterior_stats_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, spec, out), errbuf,
+                  errlen);
+}
+
+int ldsr_posterior_yearly_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                                unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                const ldsr_yearly_spec *spec, const ldsr_yearly_out *out, char *errbuf, int errlen) {
+    return report(posterior_yearly_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, spec, out), errbuf,
                   errlen);
 }
 

@@ -345,6 +345,48 @@ LDS_rep_posterior_stats <- function(theta, Qa, u, v, start.year, transform = 'lo
   if (P$single) out[[1]] else out
 }
 
+# Year-by-year drought probabilities over LDS_rep_posterior's replicates (the same arguments and exact.rng / seed
+# give the same draws), counted on the device: no trajectory and no per-replicate value is returned, so 10^6
+# replicates and more fit.  A year is below when its flow is below threshold (NULL: mean of the observed Qa; a
+# non-finite flow is not); a run is a maximal stretch of years below it inside period (runs clipped to it).  Per year
+# of period = c(first.year, last.year) (NULL: the whole horizon): p.below, the share of replicates below; p.run.L, the
+# share inside a run of at least L years (lengths: up to 4 of 1..64); p.window.w, the share whose w-year mean flow
+# starting that year (all flows finite) is below threshold (windows: up to 4 of 1..64; NA past the period's end);
+# n.nonfinite, the replicates with a non-finite flow that year.  Returns a data.table by year (a list of them for an
+# ensemble), with the threshold as an attribute.
+LDS_rep_posterior_yearly <- function(theta, Qa, u, v, start.year, transform = 'log', num.reps = 100, exact.rng = TRUE,
+                                     seed = 0, windows = 10L, lengths = 5L, threshold = NULL, period = NULL) {
+  P <- .station_setup(list(Qa = Qa, u = u, v = v, start.year = start.year), transform)
+  thetas <- if (P$single) list(theta) else theta
+  if (length(thetas) != length(P$u)) stop('theta must be one model per ensemble member')
+  series <- lapply(seq_along(P$u), function(k) list(y = P$y, u = P$u[[k]], v = P$v[[k]]))
+  cols <- lapply(thetas, function(th) c(th$A, th$B, th$C, th$D, th$Q, th$R, th$mu1, th$V1))
+  stride <- max(lengths(cols))
+  th <- sapply(cols, function(x) c(x, rep(0, stride - length(x))))
+  n <- length(P$years); nm <- length(series); y0 <- P$years[1]
+  if (is.null(period)) period <- range(P$years)
+  rg <- c(period[1] - y0, period[2] - y0 + 1)
+  if (rg[1] < 0 || rg[2] > n || rg[1] >= rg[2]) stop('period must lie inside the reconstruction horizon')
+  if (is.null(threshold)) threshold <- mean(Qa$Qa)
+  z <- if (exact.rng) stats::rnorm(2 * num.reps * n * nm) else NULL
+  code <- switch(transform, none = 0L, log = 1L, boxcox = 2L)
+  m <- .Call('_ldsr_posterior_yearly_batch', series, matrix(th, nrow = stride), as.integer(num.reps), z,
+             as.numeric(seed), rep(P$mu, nm), code, if (transform == 'boxcox') rep(P$lambda, nm) else NULL,
+             as.integer(windows), as.integer(lengths), rep(as.numeric(threshold), nm), as.integer(rep(rg, nm)),
+             PACKAGE = 'ldsr')
+  share <- function(c) ifelse(c < 0, NA_real_, c / num.reps)
+  out <- lapply(seq_len(nm), function(k) {
+    r <- (k - 1) * n + seq(rg[1] + 1, rg[2])
+    dt <- data.table::data.table(year = P$years[seq(rg[1] + 1, rg[2])], p.below = share(m[[1]][r]),
+                                 n.nonfinite = m[[4]][r])
+    for (j in seq_along(lengths)) dt[[paste0('p.run.', lengths[j])]] <- share(m[[2]][r, j])
+    for (j in seq_along(windows)) dt[[paste0('p.window.', windows[j])]] <- share(m[[3]][r, j])
+    data.table::setattr(dt, 'threshold', threshold)
+    dt
+  })
+  if (P$single) out[[1]] else out
+}
+
 #' Kalman / RTS smoother for a state of dimension d > 1 (beyond ldsr, whose state is scalar).
 #' theta: list(A d x d, B d x p, C 1 x d, D 1 x q, Q d x d, R, mu1 d x 1, V1 d x d); y 1 x T with NA.
 #' method: 1 = associative scan over time (long series), 0 = sequential recursion.
