@@ -293,9 +293,49 @@ int ldsr_posterior_yearly_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_re
                                 unsigned long long seed, const double *mu, int transform, const double *lambda,
                                 const ldsr_yearly_spec *spec, const ldsr_yearly_out *out, char *errbuf, int errlen);
 
+/* Per-step quantiles of w-step mean flows over conditioned replicates (beyond the reference), selected exactly on
+ * the device: the replicates of ldsr_posterior_rep_batch with the same arguments (the same draws bit for bit, from
+ * seed or from z), of which no trajectory and no per-replicate value leaves the device.  For fit f let Q_t be a
+ * replicate's simQ, qf_t = Q_t with a non-finite flow replaced by 0, and [lo, hi) the fit's range of steps
+ * (range[2f], range[2f+1] with 0 <= lo < hi <= T_f; range NULL: the whole series).
+ *   Window value, per window w = windows[k] and start t with lo <= t <= hi - w: M = S / w, where S is a running sum
+ *   that starts at 0 at step hi - 1 and walks downwards: at step t, S = (S + qf_t) - qf_{t+w}, the subtraction
+ *   only once more than w steps of the range have been walked.  A window that holds a non-finite flow has no value;
+ *   such replicates are counted in nonfinite[k].
+ *   Quantile, per level p = levels[l]: with n the replicates that have a value at (k, t), the r-th smallest value
+ *   (1-based) for r = max(1, ceil(p * n)) evaluated in IEEE double (R's quantile type 1, numpy's
+ *   method="inverted_cdf").  Every output is a value some replicate took; p = 0 gives the minimum, p = 1 the
+ *   maximum; n = 0 gives NaN.
+ * Rows are ldsr_smoother_batch's: fit f's step t at fit_ptr[f] + t (fit_ptr the exclusive prefix sum of T over the
+ * fits, caller order).  q is [n_windows][n_levels][fit_ptr[n_fits]] and nonfinite [n_windows][fit_ptr[n_fits]];
+ * rows outside [lo, hi), and starts t > hi - w, are NaN in q and -1 in nonfinite.  Any output may be NULL, not
+ * all.  The selection is exact, so the result is the same bit for bit from run to run and does not depend on the
+ * other fits or on the outputs asked for.  The device runs the sampler several times (passes: the number of runs),
+ * with memory that does not grow with n_reps; if two runs disagree the call fails with LDSR_ERR_CUDA and names the
+ * fit, window and step.  Arguments are checked before a device is touched (as ldsr_posterior_rep_batch's, plus the
+ * spec); one device (ctx device 0), no CPU fallback.  ldsr_last_device_ms covers the coefficient pass, every
+ * sampler pass and the selection kernels. */
+#define LDSR_QUANT_MAX_LEVELS 8
+typedef struct {
+    int n_windows;        /* 1 .. LDSR_STATS_MAX_WINDOWS, each 1 .. LDSR_STATS_MAX_WINDOW */
+    const int *windows;   /* [n_windows] */
+    int n_levels;         /* 1 .. LDSR_QUANT_MAX_LEVELS */
+    const double *levels; /* [n_levels], each in [0, 1], strictly increasing */
+    const int *range;     /* [2*n_fits] or NULL */
+} ldsr_quant_spec;
+typedef struct {
+    double *q;      /* [n_windows][n_levels][fit_ptr[n_fits]] */
+    int *nonfinite; /* [n_windows][fit_ptr[n_fits]] */
+    int *passes;    /* [1] or NULL: the sampler runs of the call */
+} ldsr_quant_out;
+int ldsr_posterior_quantile_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                                  unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                  const ldsr_quant_spec *spec, const ldsr_quant_out *out, char *errbuf, int errlen);
+
 /* Device time in ms (CUDA events around the kernels, summed) of the last ldsr_rep_batch / ldsr_rep_batch_r /
- * ldsr_posterior_rep_batch / ldsr_posterior_stats_batch / ldsr_posterior_yearly_batch call made by the calling
- * thread: the measurement hook of bench.py's config-4 record. */
+ * ldsr_posterior_rep_batch / ldsr_posterior_stats_batch / ldsr_posterior_yearly_batch /
+ * ldsr_posterior_quantile_batch call made by the calling thread: the measurement hook of bench.py's config-4
+ * record. */
 double ldsr_last_device_ms(void);
 
 /* ---- the reference's random numbers (R's default generators after set.seed) ---------------

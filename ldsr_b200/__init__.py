@@ -12,6 +12,6 @@ from . import _lib  # noqa: F401
 from .api import (Kalman_smoother, Mstep, LDS_EM, LDS_EM_restart, LDS_reconstruction, cvLDS,  # noqa: F401
                   LDS_reconstruction_stations, cvLDS_stations,
                   one_lds_cv, propagate, LDS_rep, one_LDS_rep, LDS_rep_posterior, make_init, make_Z, calculate_metrics,
-                  LDS_rep_posterior_stats, LDS_rep_posterior_yearly,
+                  LDS_rep_posterior_stats, LDS_rep_posterior_yearly, LDS_rep_posterior_quantiles,
                   theta_to_vec, vec_to_theta, Kalman_smoother_d, tbrm)
 from ._lib import RRandom  # noqa: F401  (R's generators after set.seed: reproducible restarts / replicates)

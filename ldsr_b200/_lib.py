@@ -23,7 +23,7 @@ EXPORTS = ("ldsr_abi_version", "ldsr_device_count", "ldsr_ctx_create", "ldsr_ctx
            "ldsr_objective_batch", "ldsr_rep_batch_r", "ldsr_r_rng_create", "ldsr_r_rng_unif", "ldsr_r_rng_norm",
            "ldsr_r_rng_sample", "ldsr_r_rng_destroy", "ldsr_r_rnorm_device", "ldsr_last_device_ms",
            "ldsr_cv_metrics_stations", "ldsr_construct_rec_stations", "ldsr_posterior_rep_batch",
-           "ldsr_posterior_stats_batch", "ldsr_posterior_yearly_batch")
+           "ldsr_posterior_stats_batch", "ldsr_posterior_yearly_batch", "ldsr_posterior_quantile_batch")
 
 
 class LdsrError(RuntimeError):
@@ -60,6 +60,14 @@ class YearlySpec(C.Structure):
 
 class YearlyOut(C.Structure):
     _fields_ = [("below", _ip), ("in_run", _ip), ("wbelow", _ip), ("nonfinite", _ip)]
+
+
+class QuantSpec(C.Structure):
+    _fields_ = [("n_windows", C.c_int), ("windows", _ip), ("n_levels", C.c_int), ("levels", _dp), ("range", _ip)]
+
+
+class QuantOut(C.Structure):
+    _fields_ = [("q", _dp), ("nonfinite", _ip), ("passes", _ip)]
 
 
 POLL_FN = C.CFUNCTYPE(C.c_int, C.c_void_p)
@@ -518,6 +526,55 @@ def posterior_yearly_batch(series, group_series, held, fit_group, theta, n_reps,
     ptr = pb.fit_ptr
     res = {k: [o[:, ptr[f]:ptr[f + 1]] if k in ("in_run", "wbelow") else o[0, ptr[f]:ptr[f + 1]] for f in range(nf)]
            for k, o in outs.items()}
+    res["device_ms"] = float(lib().ldsr_last_device_ms())
+    return res
+
+
+QUANT_OUTPUTS = ("q", "nonfinite")
+
+
+def posterior_quantile_batch(series, group_series, held, fit_group, theta, n_reps, z=None, seed=0, mu=None,
+                             transform="log", lams=None, windows=(1, 10), levels=(0.05, 0.5, 0.95), ranges=None,
+                             want=QUANT_OUTPUTS, ctx=None):
+    """ldsr_posterior_quantile_batch: per step t and window w, the exact quantiles over posterior_rep_batch's
+    replicates (same arguments, the same draws) of the mean of Q_t .. Q_{t+w-1}, selected on the device.  windows:
+    1 to 4, in 1..64; levels: 1 to 8, in [0, 1], strictly increasing; the quantile at level p is the
+    max(1, ceil(p n))-th smallest of the n replicates whose window is finite (numpy's method="inverted_cdf"); ranges:
+    [n_fits, 2] step ranges [lo, hi) (None: whole series).  want: the outputs to return.  Returns, per requested
+    output, a list over fits: q [n_windows, n_levels, T_f] (NaN outside the range, at window starts past hi - w and
+    where no replicate has a value) and nonfinite [n_windows, T_f] int32 (-1 where q is undefined); the number of
+    sampler passes and the device time."""
+    pb = PackedBatch(series, group_series, held, fit_group, theta)
+    nf, n_reps = pb.n_fits, int(n_reps)
+    zz = None
+    if z is not None:
+        zz = np.ascontiguousarray(z, dtype=np.float64).ravel()
+        if zz.size != 2 * int(pb.fit_ptr[-1]) * n_reps:
+            raise ValueError("z must hold 2 * n_reps * sum(T) = %d values" % (2 * int(pb.fit_ptr[-1]) * n_reps))
+    code = TRANSFORMS[transform] if isinstance(transform, str) else int(transform)
+    mu_a = None if mu is None else np.ascontiguousarray(np.broadcast_to(np.asarray(mu, dtype=np.float64), (nf,)))
+    lam_a = None if lams is None else np.ascontiguousarray(np.broadcast_to(np.asarray(lams, dtype=np.float64), (nf,)))
+    win = np.ascontiguousarray(np.atleast_1d(np.asarray(windows if windows is not None else (), dtype=np.int32)))
+    lev = np.ascontiguousarray(np.atleast_1d(np.asarray(levels if levels is not None else (), dtype=np.float64)))
+    rng = None if ranges is None else np.ascontiguousarray(np.broadcast_to(np.asarray(ranges, dtype=np.int32),
+                                                                           (nf, 2)))
+    ns = int(pb.fit_ptr[-1])
+    outs = {}
+    if "q" in want:
+        outs["q"] = np.empty((win.size, lev.size, ns), dtype=np.float64)
+    if "nonfinite" in want:
+        outs["nonfinite"] = np.empty((win.size, ns), dtype=np.int32)
+    passes = np.zeros(1, dtype=np.int32)
+    spec = QuantSpec(win.size, _i(win) if win.size else None, lev.size, _d(lev) if lev.size else None, _i(rng))
+    out = QuantOut(_d(outs.get("q")), _i(outs.get("nonfinite")), _i(passes))
+    err = C.create_string_buffer(512)
+    rc = lib().ldsr_posterior_quantile_batch(ctx.h if isinstance(ctx, Ctx) else ctx, C.byref(pb.c), n_reps, _d(zz),
+                                             C.c_ulonglong(int(seed)), _d(mu_a), code, _d(lam_a), C.byref(spec),
+                                             C.byref(out), err, 512)
+    _check(rc, err)
+    ptr = pb.fit_ptr
+    res = {k: [o[..., ptr[f]:ptr[f + 1]] for f in range(nf)] for k, o in outs.items()}
+    res["passes"] = int(passes[0])
     res["device_ms"] = float(lib().ldsr_last_device_ms())
     return res
 

@@ -636,6 +636,32 @@ def LDS_rep_posterior_yearly(theta, Qa, u, v, start_year, transform="log", num_r
     return out[0] if S["single"] else out
 
 
+def LDS_rep_posterior_quantiles(theta, Qa, u, v, start_year, transform="log", num_reps=100, seed=0, z=None,
+                                windows=(1, 10), levels=(0.05, 0.5, 0.95), period=None):
+    """Per-year quantile bands of the w-year mean flow over LDS_rep_posterior's replicates (the same arguments give
+    the same draws), selected exactly on the device: no trajectory and no per-replicate value is written, so 10^6
+    replicates and more are practical.  windows: up to 4 lengths of 1..64 years (1: the annual flow); levels: up to
+    8, in [0, 1], strictly increasing.  For each year t of period = (first_year, last_year) (None: the whole horizon)
+    and window w, the w-year mean flow starting at t, over the replicates whose flows in that window are all finite;
+    its quantile at level p is the max(1, ceil(p n))-th smallest of those n values (R's quantile type 1, numpy's
+    method="inverted_cdf"), so every band edge is a value some replicate took.
+    Returns a dict with windows, levels, period, year (the period's years, each labelling the window that starts
+    there), q [n_windows, n_levels, n_years] (NaN where the window passes the period's end or no replicate has a
+    value) and n_nonfinite [n_windows, n_years] (replicates without a value; -1 where the window passes the end);
+    one dict per member for an ensemble.  One device call."""
+    S, thetas, y0, lo, hi, _ = _posterior_reduce_setup(theta, Qa, u, v, start_year, transform, None, period)
+    n = thetas.shape[0]
+    r = _lib.posterior_quantile_batch(S["series"], np.arange(n), None, np.arange(n), thetas, num_reps, z=z,
+                                      seed=seed, mu=np.full(n, S["mu"]), transform=transform,
+                                      lams=None if transform != "boxcox" else np.full(n, S["lam"]), windows=windows,
+                                      levels=levels, ranges=np.tile([lo, hi], (n, 1)))
+    out = [dict(windows=tuple(int(w) for w in np.atleast_1d(windows)),
+                levels=tuple(float(p) for p in np.atleast_1d(levels)), period=(y0 + lo, y0 + hi - 1),
+                year=np.arange(y0 + lo, y0 + hi), q=r["q"][k][..., lo:hi], n_nonfinite=r["nonfinite"][k][..., lo:hi])
+           for k in range(n)]
+    return out[0] if S["single"] else out
+
+
 def one_LDS_rep(rep_num, theta, u=None, v=None, years=None, mu=0.0, exp_trans=True, seed=0, z=None):
     """R/stochastics.R:18-47."""
     out = LDS_rep(theta, u, v, years, 1, mu, exp_trans, seed=seed + rep_num, z=None if z is None else z[None, :])

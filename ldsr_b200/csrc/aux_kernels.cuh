@@ -433,6 +433,38 @@ template <int PQ> __global__ void __launch_bounds__(REP_WARPS * 32) rep_kernel(c
 // ------------------------------------------------------------------------------------------
 constexpr int POST_MAX_WIN = 4;   // windows per statistics call (LDSR_STATS_MAX_WINDOWS)
 constexpr int POST_MAX_RING = 64; // longest window (LDSR_STATS_MAX_WINDOW): the Q ring covers the last 64 steps
+
+// Quantile mode (ldsr_posterior_quantile_batch): exact order statistics over replicates by radix selection on
+// order-preserving 64-bit keys, one sampler pass per round.  A slot is (window k, row fit_ptr[f] + t), at
+// k n_steps + fit_ptr[f] + t.  Each level of a slot keeps a bracket [lo, hi] of keys that holds its rank; the
+// distinct brackets of a pass are histogrammed (more than `cap` values) or collected (at most `cap`).
+constexpr int QUANT_MAX_LEV = 8;      // LDSR_QUANT_MAX_LEVELS
+constexpr int QUANT_MAX_CAP = 2048;   // values a collected bracket may hold (shared-memory sort)
+constexpr int QUANT_THREADS = 256;    // threads of the bracket kernel
+constexpr int QUANT_RANGE = 0, QUANT_SELECT = 1; // PostRepParams::qpass
+constexpr int QL_ACTIVE = 0, QL_DONE = 1, QL_NONE = 2; // QuantLevel::state (QL_NONE: no value, the output is NaN)
+struct QuantBracket {
+    unsigned long long lo, hi; // the keys it covers, both included
+    long long base;            // its first bin (histogram) or first segment entry (collected)
+    long long slot;
+    int count;                 // values in [lo, hi], from the previous pass
+    int shift;                 // histogram: bin = (key - lo) >> shift; -1: collected
+    int cursor;                // collected: values appended so far (the self-check compares it with count)
+};
+struct QuantLevel {
+    unsigned long long lo, hi, key; // the bracket that holds the rank; key: the answer once QL_DONE
+    int rank, below, count, state;  // rank among the slot's values (1-based), values below lo, values in [lo, hi]
+};
+// order-preserving map of a double onto an unsigned key (-0 below +0, NaN never occurs: windows with a non-finite
+// flow have no value) and back
+__device__ __forceinline__ unsigned long long quant_key(double v) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+    return b ^ (b >> 63 ? ~0ull : 1ull << 63);
+}
+__device__ __forceinline__ double quant_value(unsigned long long k) {
+    return __longlong_as_double((long long)(k ^ (k >> 63 ? 1ull << 63 : ~0ull)));
+}
+
 struct PostRepParams {
     const double *m, *o, *s, *J;  // coefficient rows, fit f's T_f steps at fit_ptr[f]
     const long long *fit_ptr;     // [n_fits + 1]
@@ -462,6 +494,17 @@ struct PostRepParams {
     int delay;                    // D = max L_k: step s is decided when the walk reaches s - D + 1 (0 without lengths)
     long long n_steps;            // fit_ptr[n_fits]
     int *y_below, *y_in_run, *y_wbelow, *y_nonfinite;
+    // quantile mode (posterior_rep_kernel<TT, POST_QUANT>, one launch per pass, blk0 = out0 = 0; win, n_win, ring,
+    // range and n_steps as above, n_win >= 1).  QUANT_RANGE adds, per slot, the values (q_n, which starts at 0 where
+    // the slot has values and at -1 elsewhere) and their smallest and largest key.  QUANT_SELECT adds each value to
+    // the histogram or the segment of the bracket of its slot that covers it, if any.
+    int qpass, n_lev;
+    int *q_n;
+    unsigned long long *q_min, *q_max;
+    const int *q_slot_nbr, *q_slot_br; // the slot's brackets: q_slot_br[slot n_lev + m], m < q_slot_nbr[slot]
+    QuantBracket *q_br;
+    unsigned *q_hist;
+    unsigned long long *q_seg;
 };
 
 __device__ __forceinline__ unsigned long long posterior_key(unsigned long long seed, int fit, long long rep) {
@@ -478,18 +521,41 @@ template <int TT> __host__ __device__ inline size_t posterior_stats_smem_bytes(b
 }
 
 // The modes of posterior_rep_kernel.  POST_STATS is 1, so the statistics mode may also be named <TT, true>.
-constexpr int POST_TRAJ = 0, POST_STATS = 1, POST_YEARLY = 2;
+constexpr int POST_TRAJ = 0, POST_STATS = 1, POST_YEARLY = 2, POST_QUANT = 3;
+
+// The quantile mode's selection pass: the value's key into the one bracket of its slot that covers it (brackets of
+// a slot are disjoint), as a bin count or a segment entry.  A collected bracket never takes more than its count;
+// the cursor still counts, so that the self-check sees any difference between passes.
+__device__ __forceinline__ void quant_select(const PostRepParams &P, long long slot, unsigned long long key) {
+    const int nb = P.q_slot_nbr[slot];
+    for (int m = 0; m < nb; m++) {
+        QuantBracket &B = P.q_br[P.q_slot_br[slot * P.n_lev + m]];
+        if (key < B.lo || key > B.hi) continue;
+        if (B.shift >= 0) {
+            atomicAdd(P.q_hist + B.base + (long long)((key - B.lo) >> B.shift), 1u);
+        } else {
+            const int pos = atomicAdd(&B.cursor, 1);
+            if (pos < B.count) P.q_seg[B.base + pos] = key;
+        }
+        return;
+    }
+}
 
 // POST_TRAJ: the trajectories (simX, simY, simQ).  POST_STATS: the same draws, reduced in the walk to each
 // replicate's drought statistics over its fit's range [lo, hi) (ldsr_posterior_stats_batch).  POST_YEARLY: the
-// same draws, reduced across replicates to per-step counts (ldsr_posterior_yearly_batch).  In the two reducing modes
-// no trajectory leaves the SM.  All modes run the one step body below, so a replicate's Q_t is the same value in each.
+// same draws, reduced across replicates to per-step counts (ldsr_posterior_yearly_batch).  POST_QUANT: the same
+// draws, one pass of the quantile selection (ldsr_posterior_quantile_batch; the pass is P.qpass, so that every pass
+// runs the same code and computes the same values).  In the reducing modes no trajectory leaves the SM.  All modes
+// run the one step body below, so a replicate's Q_t is the same value in each.
 // The statistics mode's accumulators take it to 168 registers: three CTAs an SM, stated so that ptxas does not cap
-// it at 128 and spill (0 leaves the other modes to ptxas's default: 96 registers for the trajectories).
+// it at 128 and spill (0 leaves the other modes to ptxas's default: 96 registers for the trajectories).  The
+// quantile mode would spill at 128 too and is bounded the same way.
 template <int TT, int MODE = POST_TRAJ>
-__global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS ? 3 : 0) posterior_rep_kernel(const PostRepParams P) {
+__global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS || MODE == POST_QUANT ? 3 : 0)
+    posterior_rep_kernel(const PostRepParams P) {
     static_assert(32 % TT == 0 && TT <= 16, "a tile's mask bits sit in one word; a half-warp loads a tile row");
-    constexpr bool STATS = MODE == POST_STATS, YEARLY = MODE == POST_YEARLY, REDUCE = STATS || YEARLY;
+    constexpr bool STATS = MODE == POST_STATS, YEARLY = MODE == POST_YEARLY, QUANT = MODE == POST_QUANT,
+                   REDUCE = STATS || YEARLY || QUANT;
     LDSR_DYN_SMEM(smem_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long blk = (long long)blockIdx.x * REP_WARPS + warp;
@@ -552,6 +618,7 @@ __global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS ? 3 : 0) po
     const int D = YEARLY ? P.delay : 1; // (1: the other modes never decide a step)
     unsigned long long below = 0ull, bad = 0ull;
     int up = 0, c_below = 0, c_bad = 0, c_win[POST_MAX_WIN] = {}, c_run[POST_MAX_WIN] = {};
+    unsigned long long k_min[POST_MAX_WIN], k_max[POST_MAX_WIN]; // quantile range pass: step j's keys, by lane j
     auto count = [&](int &c, bool pred, int j) { // c of lane j <- the live replicates with pred
         const int n = __popc(__ballot_sync(0xffffffffu, live && pred));
         if (lane == j) c = n;
@@ -639,6 +706,36 @@ __global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS ? 3 : 0) po
                 }
                 if (P.n_win > 0) ring[(t & rmask) * 32] = qf;
                 if (D > 0) decide(t + D - 1, j);
+            } else if constexpr (QUANT) {
+                // the yearly mode's window sums; the value of a window is its sum over w, as a key
+                const bool fin = fabs(q) < INFINITY;
+                bad = bad << 1 | (unsigned long long)!fin;
+                const double qf = fin ? q : 0.0;
+#pragma unroll
+                for (int k = 0; k < POST_MAX_WIN; k++) {
+                    if (k >= P.n_win) break;
+                    const int w = P.win[k];
+                    double sum = wsum[k] + qf;
+                    if (seen > w) sum -= ring[((t + w) & rmask) * 32];
+                    wsum[k] = sum;
+                    const bool has = live && seen >= w && !(bad & (~0ull >> (64 - w)));
+                    const unsigned long long key = quant_key(sum / (double)w);
+                    if (P.qpass == QUANT_RANGE) { // lane j <- step j's count and smallest and largest key
+                        count(c_win[k], has, j);
+                        unsigned long long mn = has ? key : ~0ull, mx = has ? key : 0ull;
+#pragma unroll
+                        for (int o = 16; o > 0; o >>= 1) {
+                            const unsigned long long a = __shfl_xor_sync(0xffffffffu, mn, o),
+                                                     b = __shfl_xor_sync(0xffffffffu, mx, o);
+                            mn = a < mn ? a : mn;
+                            mx = b > mx ? b : mx;
+                        }
+                        if (lane == j) k_min[k] = mn, k_max[k] = mx;
+                    } else if (has) {
+                        quant_select(P, k * P.n_steps + fp + t, key);
+                    }
+                }
+                ring[(t & rmask) * 32] = qf;
             } else {
 #pragma unroll
                 for (int k = 0; k < POST_MAX_WIN; k++) {
@@ -671,6 +768,21 @@ __global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS ? 3 : 0) po
             for (int k = 0; k < POST_MAX_WIN; k++) {
                 if (k < P.n_win) add(P.y_wbelow, k * P.n_steps + row, c_win[k]);
                 if (k < P.n_len) add(P.y_in_run, k * P.n_steps + row + D - 1, c_run[k]);
+            }
+        }
+        if constexpr (QUANT) { // lane j < TT holds step lo + j's count and keys
+            if (P.qpass == QUANT_RANGE) {
+#pragma unroll
+                for (int k = 0; k < POST_MAX_WIN; k++) {
+                    if (k >= P.n_win) break;
+                    if (c_win[k]) {
+                        const long long i = k * P.n_steps + fp + lo + lane;
+                        atomicAdd(P.q_n + i, c_win[k]);
+                        atomicMin(P.q_min + i, k_min[k]);
+                        atomicMax(P.q_max + i, k_max[k]);
+                        c_win[k] = 0;
+                    }
+                }
             }
         }
         if (!REDUCE) {
@@ -720,6 +832,197 @@ __global__ void __launch_bounds__(REP_WARPS * 32, MODE == POST_STATS ? 3 : 0) po
     if (P.deficit) P.deficit[row] = finite ? best_def : NAN;
     if (P.deficit_at) P.deficit_at[row] = finite ? best_def_at : -1;
     if (P.n_runs) P.n_runs[row] = finite ? n_runs : -1;
+}
+
+// ---- the quantile selection between the sampler's passes (ldsr_posterior_quantile_batch) ---------------------
+// quant_init_kernel (after the range pass) gives every level its rank and first bracket, [min, max] of its slot.
+// Then, until no level is active: quant_plan_kernel makes one bracket of each distinct active bracket, the sampler
+// runs its selection pass, and quant_bracket_kernel moves each level into the bin that holds its rank (histogram)
+// or picks it from the sorted segment (collected).  quant_out_kernel writes the outputs.  Each is a template of no
+// parameter, so that it is compiled where it is launched and not in every per-width unit.
+struct QuantParams {
+    long long n_slots, n_steps; // slots: n_windows n_steps
+    int n_lev, nb_log2, cap, n_reps; // levels; log2 of the bins of a histogram; most values of a collected bracket
+    double lev[QUANT_MAX_LEV];
+    const int *n;               // [n_slots] the values of the slot (-1: a slot without values)
+    const unsigned long long *kmin, *kmax;
+    QuantLevel *lv;             // [n_slots][n_lev]
+    QuantBracket *br;           // up to n_slots n_lev
+    int *slot_nbr, *slot_br;    // the slot's brackets (PostRepParams::q_slot_nbr, q_slot_br)
+    // [0] brackets, [1] histograms, [2] segment entries of the pass; [3] the lowest slot whose passes disagreed
+    // (~0: none)
+    unsigned long long *ctr;
+    const unsigned *hist;
+    const unsigned long long *seg;
+    long long n_br;             // brackets of the pass
+    double *q;                  // [n_windows][n_lev][n_steps]
+    int *nonfinite;             // [n_windows][n_steps]
+};
+
+// one thread per slot: rank max(1, ceil(p n)) in IEEE double; the minimum, the maximum and a slot of one key are
+// answered at once
+template <int = 0> __global__ void quant_init_kernel(const QuantParams Q) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= Q.n_slots) return;
+    const int n = Q.n[i];
+    const unsigned long long lo = Q.kmin[i], hi = Q.kmax[i];
+    for (int l = 0; l < Q.n_lev; l++) {
+        QuantLevel L;
+        L.lo = lo;
+        L.hi = hi;
+        L.key = 0ull;
+        L.below = 0;
+        L.count = n;
+        L.rank = 0;
+        L.state = QL_NONE;
+        if (n > 0) {
+            const long long r = (long long)ceil(Q.lev[l] * (double)n);
+            L.rank = r < 1 ? 1 : (int)r;
+            L.state = QL_ACTIVE;
+            if (lo == hi || L.rank == 1) L.state = QL_DONE, L.key = lo;
+            else if (L.rank == n) L.state = QL_DONE, L.key = hi;
+        }
+        Q.lv[i * Q.n_lev + l] = L;
+    }
+}
+
+// one thread per slot: a bracket for each distinct bracket of its active levels (the levels of one bracket are
+// adjacent, their ranks being ordered); histogram bins of 2^shift keys, the least shift that fits the span
+template <int = 0> __global__ void quant_plan_kernel(const QuantParams Q) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= Q.n_slots) return;
+    int nbr = 0;
+    unsigned long long plo = 0ull, phi = 0ull;
+    for (int l = 0; l < Q.n_lev; l++) {
+        const QuantLevel &L = Q.lv[i * Q.n_lev + l];
+        if (L.state != QL_ACTIVE || (nbr > 0 && L.lo == plo && L.hi == phi)) continue;
+        plo = L.lo;
+        phi = L.hi;
+        const long long id = (long long)atomicAdd(Q.ctr, 1ull);
+        QuantBracket B;
+        B.lo = L.lo;
+        B.hi = L.hi;
+        B.slot = i;
+        B.count = L.count;
+        B.cursor = 0;
+        if (L.count <= Q.cap) {
+            B.shift = -1;
+            B.base = (long long)atomicAdd(Q.ctr + 2, (unsigned long long)L.count);
+        } else {
+            int s = 0;
+            while (((L.hi - L.lo) >> s) >> Q.nb_log2) s++;
+            B.shift = s;
+            B.base = (long long)atomicAdd(Q.ctr + 1, 1ull) << Q.nb_log2;
+        }
+        Q.br[id] = B;
+        Q.slot_br[i * Q.n_lev + nbr++] = (int)id;
+    }
+    Q.slot_nbr[i] = nbr;
+}
+
+// Bracket bi of the pass, by a CTA of QUANT_THREADS.  Its levels are the slot's active levels with its bounds.
+// Histogram: an exclusive scan of the bins; the thread whose bins hold a level's rank moves the level into that bin
+// (a bin of one key answers it).  Collected: the segment, sorted (bitonic, in shared memory), gives each level's
+// rank.  Either way the values the pass found must be the bracket's count, else the slot is reported.
+__device__ __forceinline__ void quant_bracket(const QuantParams &Q, long long bi) {
+    LDSR_STATIC_SMEM(unsigned long long, keys[QUANT_MAX_CAP]);
+    LDSR_STATIC_SMEM(int, want[QUANT_MAX_LEV]);
+    LDSR_STATIC_SMEM(int, part[QUANT_THREADS / 32]);
+    const QuantBracket B = Q.br[bi];
+    const int tid = threadIdx.x;
+    QuantLevel *const lv = Q.lv + B.slot * Q.n_lev;
+    if (tid < QUANT_MAX_LEV) { // the rank inside the bracket of each of its levels, 0 for the others
+        want[tid] = 0;
+        if (tid < Q.n_lev) {
+            const QuantLevel L = lv[tid];
+            if (L.state == QL_ACTIVE && L.lo == B.lo && L.hi == B.hi) want[tid] = L.rank - L.below;
+        }
+    }
+    if (B.shift < 0) {
+        const int n = B.cursor;
+        if (n != B.count) {
+            if (tid == 0) atomicMin(Q.ctr + 3, (unsigned long long)B.slot);
+            return;
+        }
+        int m = 1;
+        while (m < n) m *= 2;
+        for (int j = tid; j < m; j += QUANT_THREADS) keys[j] = j < n ? Q.seg[B.base + j] : ~0ull;
+        __syncthreads();
+        for (int k = 2; k <= m; k *= 2)
+            for (int h = k / 2; h > 0; h /= 2) {
+                for (int j = tid; j < m; j += QUANT_THREADS) {
+                    const int o = j ^ h;
+                    if (o > j) {
+                        const unsigned long long a = keys[j], b = keys[o];
+                        if ((a > b) == ((j & k) == 0)) keys[j] = b, keys[o] = a;
+                    }
+                }
+                __syncthreads();
+            }
+        if (tid < Q.n_lev && want[tid] > 0) {
+            lv[tid].key = keys[want[tid] - 1];
+            lv[tid].state = QL_DONE;
+        }
+        return;
+    }
+    // bins [b0, b1) of this thread
+    const int nb = 1 << Q.nb_log2, per = (nb + QUANT_THREADS - 1) / QUANT_THREADS;
+    const int b0 = min(nb, tid * per), b1 = min(nb, b0 + per);
+    const unsigned *const h = Q.hist + B.base;
+    int mine = 0;
+    for (int b = b0; b < b1; b++) mine += (int)h[b];
+    // exclusive scan of `mine` across the CTA
+    const int lane = tid & 31, warp = tid >> 5;
+    int inc = mine;
+    for (int o = 1; o < 32; o *= 2) {
+        const int v = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += v;
+    }
+    if (lane == 31) part[warp] = inc;
+    __syncthreads();
+    int before = inc - mine, total = 0;
+    for (int w = 0; w < QUANT_THREADS / 32; w++) {
+        if (w < warp) before += part[w];
+        total += part[w];
+    }
+    if (total != B.count) {
+        if (tid == 0) atomicMin(Q.ctr + 3, (unsigned long long)B.slot);
+        return;
+    }
+    for (int l = 0; l < Q.n_lev; l++) {
+        const int r = want[l];
+        if (r <= before || r > before + mine) continue;
+        int c = before, b = b0;
+        while (c + (int)h[b] < r) c += (int)h[b++];
+        QuantLevel &L = lv[l];
+        L.below += c;
+        L.count = (int)h[b];
+        L.lo = B.lo + ((unsigned long long)b << B.shift);
+        const unsigned long long width = B.shift == 0 ? 0ull : (~0ull >> (64 - B.shift));
+        L.hi = L.lo + (B.hi - L.lo < width ? B.hi - L.lo : width);
+        if (L.lo == L.hi) L.state = QL_DONE, L.key = L.lo;
+    }
+}
+// the brackets of the pass, a CTA each (launched with one CTA per bracket; the CPU emulation runs a few CTAs)
+template <int = 0> __global__ void __launch_bounds__(QUANT_THREADS) quant_bracket_kernel(const QuantParams Q) {
+    for (long long bi = blockIdx.x; bi < Q.n_br; bi += gridDim.x) {
+        quant_bracket(Q, bi);
+        __syncthreads(); // the shared arrays are free again
+    }
+}
+
+// one thread per slot: the quantiles (NaN where a level has no value) and the replicates without a value
+// (-1 on a slot without values)
+template <int = 0> __global__ void quant_out_kernel(const QuantParams Q) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= Q.n_slots) return;
+    const int n = Q.n[i];
+    const long long k = i / Q.n_steps, row = i % Q.n_steps;
+    Q.nonfinite[i] = n < 0 ? -1 : Q.n_reps - n;
+    for (int l = 0; l < Q.n_lev; l++) {
+        const QuantLevel &L = Q.lv[i * Q.n_lev + l];
+        Q.q[(k * Q.n_lev + l) * Q.n_steps + row] = L.state == QL_DONE ? quant_value(L.key) : NAN;
+    }
 }
 
 } // namespace ldsr

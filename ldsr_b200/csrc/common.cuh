@@ -12,6 +12,27 @@
 // coroutine-per-thread emulator.  Never part of the product library.
 #define LDSR_DYN_SMEM(name) unsigned char *const name = ::hostsim::dyn_smem()
 #define LDSR_STATIC_SMEM(type, name) static type name
+// the atomics of the quantile selection (aux_kernels.cuh): one emulated thread runs at a time
+static inline unsigned atomicAdd(unsigned *p, unsigned v) {
+    const unsigned old = *p;
+    *p += v;
+    return old;
+}
+static inline unsigned long long atomicAdd(unsigned long long *p, unsigned long long v) {
+    const unsigned long long old = *p;
+    *p += v;
+    return old;
+}
+static inline unsigned long long atomicMin(unsigned long long *p, unsigned long long v) {
+    const unsigned long long old = *p;
+    *p = v < old ? v : old;
+    return old;
+}
+static inline unsigned long long atomicMax(unsigned long long *p, unsigned long long v) {
+    const unsigned long long old = *p;
+    *p = v > old ? v : old;
+    return old;
+}
 #endif
 
 // Plan-consistency checks inside the kernels (compute-sanitizer is not available on the GPU pool): always on in

@@ -1997,11 +1997,9 @@ static cudaError_t posterior_reduce_params(Resources &cuda, const double *z, lon
     return cudaSuccess;
 }
 
-// The one launch of a reducing mode, the copies of its outputs into the caller's arrays, and the device time.
-template <int MODE>
-static Err posterior_reduce_run(Resources &cuda, const PostRepParams &pp, bool with_z,
-                                const std::vector<std::function<cudaError_t()>> &copies) {
-    const size_t smem = posterior_stats_smem_bytes<REP_TT>(with_z, pp.ring);
+// One timed launch of a reducing mode over every (fit, 32 replicates) block.
+template <int MODE> static Err posterior_reduce_launch(Resources &cuda, const PostRepParams &pp) {
+    const size_t smem = posterior_stats_smem_bytes<REP_TT>(pp.z != nullptr, pp.ring);
     CU(cudaFuncSetAttribute(posterior_rep_kernel<REP_TT, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                             (int)posterior_stats_smem_bytes<REP_TT>(true, POST_MAX_RING)));
     CU(cuda.start());
@@ -2009,6 +2007,15 @@ static Err posterior_reduce_run(Resources &cuda, const PostRepParams &pp, bool w
         <<<(unsigned)((pp.n_blk + REP_WARPS - 1) / REP_WARPS), REP_WARPS * 32, smem, cuda.stream>>>(pp);
     CU(cudaGetLastError());
     CU(cuda.stop());
+    return Err();
+}
+
+// The one launch of a reducing mode, the copies of its outputs into the caller's arrays, and the device time.
+template <int MODE>
+static Err posterior_reduce_run(Resources &cuda, const PostRepParams &pp,
+                                const std::vector<std::function<cudaError_t()>> &copies) {
+    Err e = posterior_reduce_launch<MODE>(cuda, pp);
+    if (!e.ok()) return e;
     for (auto &c : copies) CU(c());
     CU(cudaStreamSynchronize(cuda.stream));
     g_last_device_ms = 0.0;
@@ -2060,7 +2067,7 @@ static Err posterior_stats_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps,
     CU(out_block(&pp.deficit, out->deficit, rows));
     CU(out_block(&pp.deficit_at, out->deficit_at, rows));
     CU(out_block(&pp.n_runs, out->n_runs, rows));
-    return posterior_reduce_run<POST_STATS>(cuda, pp, z != nullptr, copies);
+    return posterior_reduce_run<POST_STATS>(cuda, pp, copies);
 }
 
 // ---- year-by-year drought counts of the conditioned replicates, reduced across replicates --------------------
@@ -2110,7 +2117,142 @@ static Err posterior_yearly_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps
     CU(out_block(&pp.y_in_run, out->in_run, nl, nullptr));
     CU(out_block(&pp.y_wbelow, out->wbelow, nw, spec->windows));
     CU(out_block(&pp.y_nonfinite, out->nonfinite, 1, nullptr));
-    return posterior_reduce_run<POST_YEARLY>(cuda, pp, z != nullptr, copies);
+    return posterior_reduce_run<POST_YEARLY>(cuda, pp, copies);
+}
+
+// ---- per-step quantiles of w-step means over the conditioned replicates, selected exactly -----------------------
+// The sampler draws the same values on every run, so the selection takes passes instead of storing the values: a
+// range pass (count, smallest and largest key per slot), then selection passes until no level is active, each
+// followed by quant_bracket_kernel<>.  Each histogram pass removes log2(bins) bits of a bracket's span, so a level is
+// settled after at most ceil(64 / log2(bins)) of them and one collecting pass.
+static Err posterior_quantile_batch(ldsr_ctx *ctx, const ldsr_batch *b, int n_reps, const double *z,
+                                    unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                    const ldsr_quant_spec *spec, const ldsr_quant_out *out) {
+    std::vector<double> par;
+    Err e = posterior_args(b, n_reps, mu, transform, lambda, par);
+    if (!e.ok()) return e;
+    if (!spec || !out) return fail(LDSR_ERR_ARG, "spec and out are required");
+    const int nw = spec->n_windows, nl = spec->n_levels, nf = b->n_fits;
+    if (!(e = posterior_lengths("windows", nw, spec->windows)).ok()) return e;
+    if (nw == 0) return fail(LDSR_ERR_ARG, "n_windows=0, need at least one window");
+    if (nl < 1 || nl > LDSR_QUANT_MAX_LEVELS)
+        return fail(LDSR_ERR_ARG, "n_levels=%d, need 1 .. %d", nl, LDSR_QUANT_MAX_LEVELS);
+    if (!spec->levels) return fail(LDSR_ERR_ARG, "levels is NULL");
+    for (int l = 0; l < nl; l++) {
+        const double p = spec->levels[l];
+        if (!(p >= 0.0 && p <= 1.0)) return fail(LDSR_ERR_ARG, "levels[%d]=%g, need 0 <= p <= 1", l, p);
+        if (l > 0 && !(p > spec->levels[l - 1]))
+            return fail(LDSR_ERR_ARG, "levels[%d]=%g, need strictly increasing levels", l, p);
+    }
+    if (!out->q && !out->nonfinite && !out->passes) return fail(LDSR_ERR_ARG, "no output asked for");
+    std::vector<int> range;
+    if (!(e = posterior_ranges(b, spec->range, nullptr, range)).ok()) return e;
+    PosteriorSetup S;
+    if (!(e = posterior_setup(ctx, b, n_reps, seed, transform, par, S)).ok()) return e;
+    Resources &cuda = S.plan->cuda;
+    const long long ns = S.fit_ptr[nf], n_slots = nw * ns;
+    PostRepParams pp = S.pp;
+    CU(posterior_reduce_params(cuda, z, ns, range, nullptr, nw, spec->windows, pp));
+    pp.n_steps = ns;
+    pp.n_lev = nl;
+    // bins of a histogram and most values of a collected bracket (LDSR_QUANT_TINY=1, tests: 4 and 3, which takes
+    // every path of the selection at a few replicates)
+    static const bool tiny = std::getenv("LDSR_QUANT_TINY") != nullptr;
+    QuantParams Q{};
+    Q.n_slots = n_slots;
+    Q.n_steps = ns;
+    Q.n_lev = nl;
+    Q.nb_log2 = tiny ? 2 : 11;
+    Q.cap = tiny ? 3 : QUANT_MAX_CAP;
+    Q.n_reps = n_reps;
+    for (int l = 0; l < nl; l++) Q.lev[l] = spec->levels[l];
+    // values per slot: 0 where the slot has values (starts lo .. hi - w), -1 elsewhere
+    std::vector<int> n0((size_t)n_slots, -1);
+    for (int k = 0; k < nw; k++)
+        for (int f = 0; f < nf; f++)
+            for (long long t = range[2 * f]; t <= range[2 * f + 1] - spec->windows[k]; t++)
+                n0[(size_t)(k * ns + S.fit_ptr[f] + t)] = 0;
+    unsigned long long *d_min, *d_max, *d_ctr;
+    double *d_q;
+    int *d_nonfinite;
+    CU(cuda.upload(&pp.q_n, n0));
+    CU(cuda.alloc(&d_min, n_slots));
+    CU(cuda.alloc(&d_max, n_slots));
+    CU(cuda.alloc(&Q.lv, (size_t)n_slots * nl));
+    CU(cuda.alloc(&Q.br, (size_t)n_slots * nl));
+    CU(cuda.alloc(&Q.slot_nbr, n_slots));
+    CU(cuda.alloc(&Q.slot_br, (size_t)n_slots * nl));
+    CU(cuda.alloc(&d_ctr, 4));
+    CU(cuda.alloc(&d_q, (size_t)n_slots * nl));
+    CU(cuda.alloc(&d_nonfinite, n_slots));
+    CU(cudaMemsetAsync(d_min, 0xFF, n_slots * sizeof(unsigned long long), cuda.stream));
+    CU(cudaMemsetAsync(d_max, 0, n_slots * sizeof(unsigned long long), cuda.stream));
+    CU(cudaMemsetAsync(d_ctr, 0xFF, 4 * sizeof(unsigned long long), cuda.stream));
+    pp.q_min = d_min;
+    pp.q_max = d_max;
+    pp.q_slot_nbr = Q.slot_nbr;
+    pp.q_slot_br = Q.slot_br;
+    pp.q_br = Q.br;
+    Q.n = pp.q_n;
+    Q.kmin = d_min;
+    Q.kmax = d_max;
+    Q.ctr = d_ctr;
+    Q.q = d_q;
+    Q.nonfinite = d_nonfinite;
+    const unsigned slot_grid = (unsigned)((n_slots + 255) / 256);
+    auto small = [&](void (*kernel)(QuantParams), unsigned grid, unsigned block) -> Err {
+        CU(cuda.start());
+        kernel<<<grid, block, 0, cuda.stream>>>(Q);
+        CU(cudaGetLastError());
+        CU(cuda.stop());
+        return Err();
+    };
+    pp.qpass = QUANT_RANGE;
+    if (!(e = posterior_reduce_launch<POST_QUANT>(cuda, pp)).ok()) return e;
+    int passes = 1;
+    if (!(e = small(quant_init_kernel<>, slot_grid, 256)).ok()) return e;
+    // the histograms and the segments, grown when a pass needs more
+    unsigned *d_hist = nullptr;
+    unsigned long long *d_seg = nullptr;
+    size_t hist_cap = 0, seg_cap = 0;
+    const int max_passes = 2 + (64 + Q.nb_log2 - 1) / Q.nb_log2;
+    for (;;) {
+        CU(cudaMemsetAsync(d_ctr, 0, 3 * sizeof(unsigned long long), cuda.stream));
+        if (!(e = small(quant_plan_kernel<>, slot_grid, 256)).ok()) return e;
+        unsigned long long h[4];
+        CU(cudaMemcpyAsync(h, d_ctr, sizeof h, cudaMemcpyDeviceToHost, cuda.stream));
+        CU(cudaStreamSynchronize(cuda.stream));
+        if (h[3] != ~0ull) { // a bracket's values in the last pass were not those the pass before had counted
+            const long long k = (long long)(h[3] / ns), row = (long long)(h[3] % ns);
+            const int f = (int)(std::upper_bound(S.fit_ptr.begin(), S.fit_ptr.end(), row) - S.fit_ptr.begin()) - 1;
+            return fail(LDSR_ERR_CUDA, "fit %d, window %d, step %lld: two sampler passes disagreed", f,
+                        spec->windows[k], row - S.fit_ptr[f]);
+        }
+        if (h[0] == 0) break;
+        if (passes >= max_passes) return fail(LDSR_ERR_CUDA, "quantile selection did not settle in %d passes", passes);
+        const size_t bins = (size_t)h[1] << Q.nb_log2;
+        if (bins > hist_cap) CU(cuda.realloc(&d_hist, hist_cap = bins));
+        if (h[2] > seg_cap) CU(cuda.realloc(&d_seg, seg_cap = h[2]));
+        if (bins) CU(cudaMemsetAsync(d_hist, 0, bins * sizeof(unsigned), cuda.stream));
+        pp.qpass = QUANT_SELECT;
+        pp.q_hist = d_hist;
+        pp.q_seg = d_seg;
+        Q.hist = d_hist;
+        Q.seg = d_seg;
+        if (!(e = posterior_reduce_launch<POST_QUANT>(cuda, pp)).ok()) return e;
+        passes++;
+        Q.n_br = (long long)h[0];
+        if (!(e = small(quant_bracket_kernel<>, (unsigned)h[0], QUANT_THREADS)).ok()) return e;
+    }
+    if (!(e = small(quant_out_kernel<>, slot_grid, 256)).ok()) return e;
+    if (out->q) CU(cudaMemcpyAsync(out->q, d_q, (size_t)n_slots * nl * sizeof(double), cudaMemcpyDeviceToHost, cuda.stream));
+    if (out->nonfinite)
+        CU(cudaMemcpyAsync(out->nonfinite, d_nonfinite, (size_t)n_slots * sizeof(int), cudaMemcpyDeviceToHost, cuda.stream));
+    CU(cudaStreamSynchronize(cuda.stream));
+    if (out->passes) *out->passes = passes;
+    g_last_device_ms = 0.0;
+    CU(cuda.total_ms(&g_last_device_ms));
+    return Err();
 }
 
 } // namespace ldsr
@@ -2246,6 +2388,13 @@ int ldsr_posterior_yearly_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_re
                                 unsigned long long seed, const double *mu, int transform, const double *lambda,
                                 const ldsr_yearly_spec *spec, const ldsr_yearly_out *out, char *errbuf, int errlen) {
     return report(posterior_yearly_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, spec, out), errbuf,
+                  errlen);
+}
+
+int ldsr_posterior_quantile_batch(ldsr_ctx *ctx, const ldsr_batch *batch, int n_reps, const double *z,
+                                  unsigned long long seed, const double *mu, int transform, const double *lambda,
+                                  const ldsr_quant_spec *spec, const ldsr_quant_out *out, char *errbuf, int errlen) {
+    return report(posterior_quantile_batch(ctx, batch, n_reps, z, seed, mu, transform, lambda, spec, out), errbuf,
                   errlen);
 }
 

@@ -387,6 +387,45 @@ LDS_rep_posterior_yearly <- function(theta, Qa, u, v, start.year, transform = 'l
   if (P$single) out[[1]] else out
 }
 
+# Per-year quantile bands of the w-year mean flow over LDS_rep_posterior's replicates (the same arguments and
+# exact.rng / seed give the same draws), selected exactly on the device: no trajectory and no per-replicate value is
+# returned, so 10^6 replicates and more fit.  windows: up to 4 of 1..64 years (1: the annual flow); levels: up to 8
+# in [0, 1], strictly increasing.  For each year of period = c(first.year, last.year) (NULL: the whole horizon) and
+# window w, the quantile at level p of the w-year mean flow starting that year, over the replicates whose flows in it
+# are all finite, is the max(1, ceiling(p n))-th smallest of those n values (quantile(type = 1)).  Returns a
+# data.table with columns year, window, one column per level (q.0.05, ...; NA where the window passes the period's
+# end) and n.nonfinite, by window then year (a list of them for an ensemble).
+LDS_rep_posterior_quantiles <- function(theta, Qa, u, v, start.year, transform = 'log', num.reps = 100,
+                                        exact.rng = TRUE, seed = 0, windows = c(1L, 10L),
+                                        levels = c(0.05, 0.5, 0.95), period = NULL) {
+  P <- .station_setup(list(Qa = Qa, u = u, v = v, start.year = start.year), transform)
+  thetas <- if (P$single) list(theta) else theta
+  if (length(thetas) != length(P$u)) stop('theta must be one model per ensemble member')
+  series <- lapply(seq_along(P$u), function(k) list(y = P$y, u = P$u[[k]], v = P$v[[k]]))
+  cols <- lapply(thetas, function(th) c(th$A, th$B, th$C, th$D, th$Q, th$R, th$mu1, th$V1))
+  stride <- max(lengths(cols))
+  th <- sapply(cols, function(x) c(x, rep(0, stride - length(x))))
+  n <- length(P$years); nm <- length(series); y0 <- P$years[1]
+  if (is.null(period)) period <- range(P$years)
+  rg <- c(period[1] - y0, period[2] - y0 + 1)
+  if (rg[1] < 0 || rg[2] > n || rg[1] >= rg[2]) stop('period must lie inside the reconstruction horizon')
+  z <- if (exact.rng) stats::rnorm(2 * num.reps * n * nm) else NULL
+  code <- switch(transform, none = 0L, log = 1L, boxcox = 2L)
+  m <- .Call('_ldsr_posterior_quantile_batch', series, matrix(th, nrow = stride), as.integer(num.reps), z,
+             as.numeric(seed), rep(P$mu, nm), code, if (transform == 'boxcox') rep(P$lambda, nm) else NULL,
+             as.integer(windows), as.numeric(levels), as.integer(rep(rg, nm)), PACKAGE = 'ldsr')
+  out <- lapply(seq_len(nm), function(k) {
+    r <- (k - 1) * n + seq(rg[1] + 1, rg[2])
+    data.table::rbindlist(lapply(seq_along(windows), function(j) {
+      dt <- data.table::data.table(year = P$years[seq(rg[1] + 1, rg[2])], window = windows[j])
+      for (l in seq_along(levels)) dt[[paste0('q.', levels[l])]] <- m[[1]][r, (j - 1) * length(levels) + l]
+      dt[['n.nonfinite']] <- ifelse(m[[2]][r, j] < 0, NA_integer_, m[[2]][r, j])
+      dt
+    }))
+  })
+  if (P$single) out[[1]] else out
+}
+
 #' Kalman / RTS smoother for a state of dimension d > 1 (beyond ldsr, whose state is scalar).
 #' theta: list(A d x d, B d x p, C 1 x d, D 1 x q, Q d x d, R, mu1 d x 1, V1 d x d); y 1 x T with NA.
 #' method: 1 = associative scan over time (long series), 0 = sequential recursion.

@@ -17,6 +17,7 @@
  *     _ldsr_posterior_rep_batch(series,thetas,num_reps,z,seed,mu,transform,lambda)   8
  *     _ldsr_posterior_stats_batch(series,thetas,num_reps,z,seed,mu,transform,lambda,windows,threshold,range)   11
  *     _ldsr_posterior_yearly_batch(series,thetas,num_reps,z,seed,mu,transform,lambda,windows,lengths,threshold,range)   12
+ *     _ldsr_posterior_quantile_batch(series,thetas,num_reps,z,seed,mu,transform,lambda,windows,levels,range)   11
  *     _ldsr_cv_metrics(Ycv,target,Z,exp_trans)                                        4
  *     _ldsr_construct_rec(X,V,Y,C,R,mu,transform,lambda)                              8
  *     _ldsr_cv_metrics_stations(Ycv,target,Z,exp_trans)   lists, one element per station    4
@@ -468,6 +469,58 @@ SEXP _ldsr_posterior_yearly_batch(SEXP series, SEXP thetas, SEXP repsS, SEXP zS,
     return out;
 }
 
+/* Per-year quantiles of w-year mean flows over the same replicates, selected on the device
+ * (LDS_rep_posterior_quantiles in ldsr_b200.R): arguments as _ldsr_posterior_rep_batch, then windows (integer, 1 to
+ * 4 of 1..64), levels (double, 1 to 8 in [0, 1], strictly increasing) and range (a 2 x n integer matrix of 0-based
+ * [lo, hi) per series, or NULL).  Returns list(q, nonfinite, passes): q as a sum(T) x (n_levels n_windows) matrix
+ * (series by series, step by step; window k's level l in column k n_levels + l; NaN where undefined), nonfinite as a sum(T) x n_windows integer matrix (-1 where
+ * undefined), passes the sampler runs. */
+SEXP _ldsr_posterior_quantile_batch(SEXP series, SEXP thetas, SEXP repsS, SEXP zS, SEXP seedS, SEXP muS,
+                                    SEXP transformS, SEXP lambdaS, SEXP windowsS, SEXP levelsS, SEXP rangeS) {
+    const int ns = (int)XLENGTH(series), reps = Rf_asInteger(repsS);
+    const int nw = (int)XLENGTH(windowsS), nl = (int)XLENGTH(levelsS);
+    int *T = (int *)R_alloc(ns, sizeof(int)), *p = (int *)R_alloc(ns, sizeof(int)), *q = (int *)R_alloc(ns, sizeof(int));
+    int *idx = (int *)R_alloc(ns, sizeof(int));
+    const double **y = (const double **)R_alloc(ns, sizeof(double *));
+    const double **u = (const double **)R_alloc(ns, sizeof(double *));
+    const double **v = (const double **)R_alloc(ns, sizeof(double *));
+    R_xlen_t tot = 0, steps = 0;
+    for (int s = 0; s < ns; s++) {
+        SEXP e = VECTOR_ELT(series, s);
+        T[s] = Rf_ncols(list_get(e, "y"));
+        y[s] = REAL(list_get(e, "y"));
+        u[s] = input_ptr(list_get(e, "u"), T[s], &p[s]);
+        v[s] = input_ptr(list_get(e, "v"), T[s], &q[s]);
+        idx[s] = s;
+        tot += (R_xlen_t)reps * T[s];
+        steps += T[s];
+    }
+    if (Rf_ncols(thetas) != ns) Rf_error("ldsr: thetas must have one column per series");
+    if (XLENGTH(muS) != ns) Rf_error("ldsr: mu must have one value per series");
+    const double *z = Rf_isNull(zS) ? NULL : REAL(zS);
+    if (z && XLENGTH(zS) != 2 * tot) Rf_error("ldsr: z must hold 2 * num.reps * sum(T) draws");
+    const double *lam = Rf_isNull(lambdaS) ? NULL : REAL(lambdaS);
+    if (lam && XLENGTH(lambdaS) != ns) Rf_error("ldsr: lambda must have one value per series");
+    const int *range = Rf_isNull(rangeS) ? NULL : INTEGER(rangeS);
+    if (range && XLENGTH(rangeS) != 2 * (R_xlen_t)ns) Rf_error("ldsr: range must hold 2 values per series");
+    ldsr_batch b; memset(&b, 0, sizeof b);
+    b.n_series = ns; b.T = T; b.p = p; b.q = q; b.y = y; b.u = u; b.v = v;
+    b.n_groups = ns; b.group_series = idx;
+    b.n_fits = ns; b.fit_group = idx; b.theta0 = REAL(thetas); b.theta_stride = Rf_nrows(thetas);
+    ldsr_quant_spec spec = {nw, INTEGER(windowsS), nl, REAL(levelsS), range};
+    SEXP out = PROTECT(Rf_allocVector(VECSXP, 3));
+    SET_VECTOR_ELT(out, 0, Rf_allocMatrix(REALSXP, steps, nl * nw));
+    SET_VECTOR_ELT(out, 1, Rf_allocMatrix(INTSXP, steps, nw));
+    SET_VECTOR_ELT(out, 2, Rf_allocVector(INTSXP, 1));
+    ldsr_quant_out qo = {REAL(VECTOR_ELT(out, 0)), INTEGER(VECTOR_ELT(out, 1)), INTEGER(VECTOR_ELT(out, 2))};
+    char err[512] = "";
+    check(ldsr_posterior_quantile_batch(ctx(), &b, reps, z, (unsigned long long)Rf_asReal(seedS), REAL(muS),
+                                        Rf_asInteger(transformS), lam, &spec, &qo, err, sizeof err),
+          err);
+    UNPROTECT(1);
+    return out;
+}
+
 /* same shape as src/RcppExports.cpp:132-148 */
 /* mapply(calculate_metrics, sim = Ycv, z = Z, MoreArgs = list(obs = target)) in one call
  * (R/LDS_reconstruction.R:395): Ycv is an n x n_folds matrix, Z a list of integer vectors. */
@@ -701,6 +754,7 @@ static const R_CallMethodDef CallEntries[] = {
     {"_ldsr_posterior_rep_batch", (DL_FUNC)&_ldsr_posterior_rep_batch, 8},
     {"_ldsr_posterior_stats_batch", (DL_FUNC)&_ldsr_posterior_stats_batch, 11},
     {"_ldsr_posterior_yearly_batch", (DL_FUNC)&_ldsr_posterior_yearly_batch, 12},
+    {"_ldsr_posterior_quantile_batch", (DL_FUNC)&_ldsr_posterior_quantile_batch, 11},
     {"_ldsr_smoother_d", (DL_FUNC)&_ldsr_smoother_d, 6},
     {"_ldsr_cv_metrics", (DL_FUNC)&_ldsr_cv_metrics, 4},
     {"_ldsr_construct_rec", (DL_FUNC)&_ldsr_construct_rec, 8},
